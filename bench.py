@@ -7,7 +7,7 @@ all-reduce error statistics), one "step" = prediction + measurement() for every 
 Also measured at N=1 and reported in the same JSON line: the single large map (cfg4, n = 8,192, Sigma = 2.1 GB)
 whose streamed rank-2 sweep is the clean HBM-roofline kernel.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0.
@@ -17,11 +17,13 @@ import ctypes
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ for the modules imported from it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "tests")):
     if _p not in sys.path:
@@ -290,6 +292,24 @@ def parity_sharded(pkg, dist, local, n_lm, tr, min_corrections=10, sample_rows=N
 
 
 # ----------------------------------------------------------------------------- our arm
+DUMP_STATES = 65536  # filters whose state is written by --dump-outputs (22.5 MB of float64 at n = 20)
+DUMP_SIGMAS = 1024   # filters whose covariance is written (15.1 MB; all 65,536 would be 969 MB)
+
+
+def dump_batch_outputs(bt, out_dir, seed=0):
+    """What a caller of the timed path receives after its last step: the filters' states (bt.states()) and
+    covariances (bt.sigma(b)), for all filters or a fixed, seeded sample of them, as float64 .npy files.  The
+    *_filters.npy files hold the filter indices of each sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    st_ids = np.arange(bt.B) if bt.B <= DUMP_STATES else np.sort(rng.choice(bt.B, DUMP_STATES, replace=False))
+    sg_ids = np.sort(rng.choice(bt.B, min(DUMP_SIGMAS, bt.B), replace=False))
+    np.save(os.path.join(out_dir, "state.npy"), bt.states()[st_ids])
+    np.save(os.path.join(out_dir, "state_filters.npy"), st_ids.astype(np.float64))
+    np.save(os.path.join(out_dir, "sigma.npy"), np.stack([bt.sigma(int(b)) for b in sg_ids]))
+    np.save(os.path.join(out_dir, "sigma_filters.npy"), sg_ids.astype(np.float64))
+
+
 def cpu_reference_dense_scaling(pkg):
     """SURVEY.md section 8(d): the reference's own dense filter (oracle/_ref, one core) at growing map sizes, to show the
     cubic law that makes it intractable at cfg4 (2 N^3 flop per correction).  Whole-step time per correction."""
@@ -553,15 +573,16 @@ def single_filter_leg(pkg, device, steps=400):
             out[key + "_reference_cpu_1core"] = run(_oracle.RefEKF(N_SLOTS), known, True)
         except Exception as e:  # no reference build on this box
             out[key + "_reference_cpu_1core"] = {"unavailable": repr(e)}
-    exe = os.path.join(ROOT, "tests", "cpp", "facade_latency")
-    cmd = ["g++", "-std=c++17", "-O2", "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "cpp", "facade_latency.cpp"),
-           "-o", exe, "-L" + os.path.join(ROOT, "ekf-slam-ml_b200"), "-lekfslam_b200", "-Wl,-rpath," + os.path.join(ROOT, "ekf-slam-ml_b200")]
-    try:
-        subprocess.run(cmd, check=True, capture_output=True, timeout=300)
-        r = subprocess.run([exe, str(steps)], check=True, capture_output=True, text=True, timeout=300)
-        out["cpp_facade"] = json.loads(r.stdout.strip().splitlines()[-1])
-    except Exception as e:
-        out["cpp_facade"] = {"unavailable": repr(e)[:300]}
+    with tempfile.TemporaryDirectory() as tmp:  # built outside the tree, which may be read-only
+        exe = os.path.join(tmp, "facade_latency")
+        cmd = ["g++", "-std=c++17", "-O2", "-I" + os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "cpp", "facade_latency.cpp"),
+               "-o", exe, "-L" + os.path.join(ROOT, "ekf-slam-ml_b200"), "-lekfslam_b200", "-Wl,-rpath," + os.path.join(ROOT, "ekf-slam-ml_b200")]
+        try:
+            subprocess.run(cmd, check=True, capture_output=True, timeout=300)
+            r = subprocess.run([exe, str(steps)], check=True, capture_output=True, text=True, timeout=300)
+            out["cpp_facade"] = json.loads(r.stdout.strip().splitlines()[-1])
+        except Exception as e:
+            out["cpp_facade"] = {"unavailable": repr(e)[:300]}
     return out
 
 
@@ -824,6 +845,8 @@ def run_ours(args):
     barrier()
     clocks = sampler.stop()
     launches = bt.launch_count - l0
+    if args.dump_outputs and rank == 0:
+        dump_batch_outputs(bt, args.dump_outputs)  # untimed; legs B and C below continue the same filters
     # The timed region holds exactly K launches of one kernel on one stream, so the average launch duration of
     # the dominant kernel is total_ms / K (CUDA events on the launching stream).
     updates_A = int(upd_A[W:T].sum())
@@ -1020,7 +1043,14 @@ def main():
     ap.add_argument("--only-small", action="store_true", help="development aid: single_filter, large_map_unknown, scan_to_map")
     ap.add_argument("--sharded-n", type=int, default=40000, help="cfg5 landmarks (square number), N>1 only")
     ap.add_argument("--sharded-updates", type=int, default=96)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the headline leg, write its filters' states and a seeded sample of "
+                         "their covariances to DIR/*.npy (float64, under 64 MB; rank 0's batch)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.only_large or args.only_laser or args.only_sharded
+                              or args.only_small):
+        ap.error("--dump-outputs writes the headline leg's outputs: it cannot be combined with --impl reference "
+                 "or --only-*")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.only_large:

@@ -2,8 +2,8 @@
 """Generates tests/golden/*.npz by running the REFERENCE ITSELF (oracle/_ref/libekf_ref.so = the reference's
 rigid2d sources compiled unmodified, see oracle/Makefile) on seeded nurtlesim-shaped inputs.
 
-Run in the build container, where /root/reference is mounted:   python scripts/make_golden.py
-The fixtures travel with the repo; /root/reference does not exist on the GPU box.
+Run with a checkout of the reference:   EKF_SLAM_REFERENCE=<checkout> python scripts/make_golden.py
+The fixtures travel with the repo, so the tests need neither the reference nor oracle/_ref.
 """
 import ctypes
 import os
@@ -28,7 +28,7 @@ def main():
     os.makedirs(GOLD, exist_ok=True)
     _oracle.build_oracle()
     L = _oracle.ref_lib()
-    assert L is not None, "needs oracle/_ref (reference sources under /root/reference)"
+    assert L is not None, "needs oracle/_ref: set EKF_SLAM_REFERENCE to a checkout of the reference"
     tg = pkg.tracegen
     n = 20
     CK = [0, 1, 2, 5, 20, 59]
@@ -153,6 +153,15 @@ def main():
                          ctypes.c_double(wheels[k, 1]), o.ctypes.data_as(dp))
         tw[k] = o
     np.savez_compressed(os.path.join(GOLD, "helpers.npz"), angles=ang, normalized=norm, wheels=wheels, twists=tw)
+
+    # ---- DiffDrive::updatePose on the seeded cases of tests/test_oracle_cpu.py::test_odometry_restatement_is_pinned
+    pose_out = []
+    for pose, l, r in _oracle.odometry_inputs():
+        b = pose.copy()
+        L.ref_update_pose(ctypes.c_double(0.16), ctypes.c_double(0.033), b.ctypes.data_as(dp), ctypes.c_double(l),
+                          ctypes.c_double(r))
+        pose_out.append(b)
+    np.savez_compressed(os.path.join(GOLD, "odometry.npz"), pose_out=np.array(pose_out))
     for f in sorted(os.listdir(GOLD)):
         print(f, os.path.getsize(os.path.join(GOLD, f)))
 

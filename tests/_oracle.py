@@ -1,7 +1,7 @@
 """ctypes bindings for the CPU checkers under oracle/ (test infrastructure only).
 
 * ``RefEKF``     – the reference's own rigid2d::EKF_SLAM (oracle/_ref/libekf_ref.so, built from
-                   /root/reference by oracle/Makefile; present only where it was built).
+                   the checkout EKF_SLAM_REFERENCE names by oracle/Makefile; present only where it was built).
 * ``OracleEKF``  – the plain-C O(N^2) restatement (oracle/libekf_oracle.so, oracle/ekf_oracle.c).
 
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs import this module.
@@ -28,7 +28,7 @@ def _u8(a):
 
 
 def build_oracle():
-    """(Re)build oracle/libekf_oracle.so, and oracle/_ref when /root/reference is mounted."""
+    """(Re)build oracle/libekf_oracle.so (and oracle/_ref when EKF_SLAM_REFERENCE names a reference checkout)."""
     subprocess.run(["make", "-s", "-C", ORACLE_DIR, "all"], check=True, stdout=subprocess.DEVNULL)
 
 
@@ -150,7 +150,7 @@ class RefEKF:
     def __init__(self, n):
         self.L = ref_lib()
         if self.L is None:
-            raise RuntimeError("oracle/_ref/libekf_ref.so not built (needs /root/reference)")
+            raise RuntimeError("oracle/_ref/libekf_ref.so not built (set EKF_SLAM_REFERENCE to a reference checkout and build)")
         self.n = int(n)
         self.N = 3 + 2 * self.n
         self.h = ctypes.c_void_p(self.L.ref_ekf_create(self.n))
@@ -204,6 +204,17 @@ class RefEKF:
     @init_flag.setter
     def init_flag(self, v):
         self.L.ref_ekf_set_init_flag(self.h, ctypes.c_int(int(v)))
+
+
+def odometry_inputs():
+    """The 4,000 seeded (pose, left, right) cases on which DiffDrive::updatePose is pinned (tests/golden/odometry.npz)."""
+    rng = np.random.default_rng(5)
+    for k in range(4000):
+        pose = np.array([rng.normal(), rng.normal(), rng.uniform(-7, 7)])
+        l, r = (rng.uniform(-0.2, 0.2), rng.uniform(-0.2, 0.2)) if k % 3 else (rng.uniform(-40, 40), rng.uniform(-40, 40))
+        if k % 7 == 0:
+            r = l + rng.uniform(-1e-6, 1e-6)  # below the 1e-4 rad "straight line" threshold
+        yield pose, l, r
 
 
 def sigma_err(a, b):

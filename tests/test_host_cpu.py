@@ -34,15 +34,28 @@ def test_library_exports_every_declared_symbol(pkg):
     assert bound == decl, bound ^ decl
 
 
-def test_no_gpu_means_loud_failure_not_fallback(pkg):
-    if pkg.device_count() > 0:
-        pytest.skip("a GPU is visible here")
-    with pytest.raises(pkg.EkfError):
-        pkg.EKF_SLAM(20)
-    with pytest.raises(pkg.EkfError):
-        pkg.EKFBatch(8, 20)
-    with pytest.raises(pkg.EkfError):
-        pkg.CircleFitting().run_batch(np.ones((1, 360), np.float32))
+NO_GPU = r'''
+import sys
+import numpy as np
+import pytest
+sys.path.insert(0, sys.argv[1])
+import ekf_slam_ml_b200 as pkg
+assert pkg.device_count() == 0
+with pytest.raises(pkg.EkfError):
+    pkg.EKF_SLAM(20)
+with pytest.raises(pkg.EkfError):
+    pkg.EKFBatch(8, 20)
+with pytest.raises(pkg.EkfError):
+    pkg.CircleFitting().run_batch(np.ones((1, 360), np.float32))
+sys.stdout.write("no-gpu ok\n")
+'''
+
+
+def test_no_gpu_means_loud_failure_not_fallback():
+    """In a process that sees no device (CUDA_VISIBLE_DEVICES empty, so this runs on a GPU machine too)."""
+    r = subprocess.run([sys.executable, "-c", NO_GPU, ROOT], capture_output=True, text=True, timeout=240,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0 and "no-gpu ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_product_never_imports_the_oracle():

@@ -8,7 +8,7 @@ message sequences:
   the same paths, landmark maps and transforms as the same sources built against the reference's own rigid2d classes
   (section 8 f-2; GPU).
 
-The binaries are built where /root/reference is mounted and travel with the snapshot; tests skip without them."""
+The binaries are built by oracle/Makefile where EKF_SLAM_REFERENCE names a reference checkout; tests skip without them."""
 import numpy as np
 import pytest
 
@@ -37,7 +37,7 @@ def _tube_world_params(w):
 def test_tube_world_pins_the_trace_generator(pkg, case):
     binary = rl.node_path("node_tube_world")
     if binary is None:
-        pytest.skip("oracle/_ref/node_tube_world not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/node_tube_world not built (set EKF_SLAM_REFERENCE to a reference checkout and build)")
     tg = pkg.tracegen
     if case == "circle":
         w = _noise_free_world(tg)
@@ -104,7 +104,7 @@ def _known_scenario(tg, steps, seed):
 def test_slam_node_source_runs_on_the_facade(gpu_pkg):
     ref, ours = rl.node_path("node_slam_ref"), rl.node_path("node_slam_b200")
     if ref is None or ours is None:
-        pytest.skip("oracle/_ref/node_slam_* not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/node_slam_* not built (set EKF_SLAM_REFERENCE to a reference checkout and build)")
     sc, t_end = _known_scenario(gpu_pkg.tracegen, steps=110, seed=3)
     topics = ["slam_path", "slam_tube", "/tf"]
     a, _ = rl.run_node(ours, sc, t_end, topics)
@@ -131,7 +131,7 @@ def _scan_scenario(tg, n_scans, seed):
 def test_landmarks_node_source_runs_on_the_facade(gpu_pkg):
     ref, ours = rl.node_path("node_landmarks_ref"), rl.node_path("node_landmarks_b200")
     if ref is None or ours is None:
-        pytest.skip("oracle/_ref/node_landmarks_* not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/node_landmarks_* not built (set EKF_SLAM_REFERENCE to a reference checkout and build)")
     sc, t_end = _scan_scenario(gpu_pkg.tracegen, n_scans=12, seed=5)
     a, _ = rl.run_node(ours, sc, t_end, ["scan_sensor"])
     b, _ = rl.run_node(ref, sc, t_end, ["scan_sensor"])
@@ -144,7 +144,7 @@ def test_unknown_data_assoc_node_source_runs_on_the_facade(gpu_pkg):
     ref, ours = rl.node_path("node_unknown_data_assoc_ref"), rl.node_path("node_unknown_data_assoc_b200")
     lm = rl.node_path("node_landmarks_ref")
     if ref is None or ours is None or lm is None:
-        pytest.skip("oracle/_ref/node_unknown_data_assoc_* not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/node_unknown_data_assoc_* not built (set EKF_SLAM_REFERENCE to a reference checkout and build)")
     tg = gpu_pkg.tracegen
     w = tg.default_world()
     sim = tg.TubeWorldSim(w, 1, seed=9)
