@@ -19,13 +19,6 @@
 
 using namespace ekf;
 
-// multi-factor sweep: DMMA consumers (ekf_large_mma.cuh) unless the vector TMA path is asked for (comparison builds)
-#ifndef EKF_SWEEP_VECTOR
-#define EKF_SWEEP_LAUNCH launch_sweep_mma
-#else
-#define EKF_SWEEP_LAUNCH launch_sweep
-#endif
-
 namespace {
 
 thread_local char g_err[512] = "";
@@ -433,8 +426,8 @@ FusedParams fused_params(ekf_filter* h, int mode, int m_max) {
 // Apply the pending factors to Sigma in one sweep (ekf_large_delayed.cuh).
 int stream_flush(ekf_filter* h, int n_counted, const UpdateCmd* cmd) {
     if (h->pending == 0) return EKF_OK;
-    CU(EKF_SWEEP_LAUNCH(h->pending, h->d_sigma, h->ld, h->N, h->d_K2, h->d_W2, 0, h->d_nupd, n_counted, cmd, h->sm_count,
-                      h->stream));
+    CU(launch_sweep(h->pending, h->d_sigma, h->ld, h->N, h->d_K2, h->d_W2, 0, h->d_nupd, n_counted, cmd, h->sm_count,
+                    h->stream));
     h->launches += 1;
     h->sweeps += 1;
     h->pending = 0;
@@ -1012,9 +1005,6 @@ int ekf_device_pointers(ekf_filter* h, void** sigma, int64_t* ld, void** state) 
 // is bit-identical for every setting; 1 reproduces the reference's schedule of one full pass per correction.
 int ekf_set_max_pending(ekf_filter* h, int max_pending) {
     if (!h || max_pending < 1 || max_pending > kMaxPending) return fail(EKF_ERR_INVALID, "max_pending must be 1..%d", kMaxPending);
-#ifdef EKF_SWEEP_VECTOR  // the vector sweeps (ekf_large_tma.cuh) are instantiated up to 16 factors
-    if (max_pending > 16) return fail(EKF_ERR_UNSUPPORTED, "this build's vector sweep takes at most 16 corrections per pass");
-#endif
     h->max_pending = max_pending;
     if (h->pending >= max_pending) {
         DeviceGuard g(h->device);

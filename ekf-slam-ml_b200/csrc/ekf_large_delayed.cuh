@@ -13,7 +13,7 @@ namespace ekf {
 
 // Capacity (factor slots) and default depth of the delayed application.  Up to 14 pending corrections the sweep is
 // still a copy (0.90 of the measured HBM peak at N = 16,387: the DMMA time hides behind it) - that is the default.
-// Deeper groups (15..20, ekf_set_max_pending) go through the narrow-tile sweep of ekf_large_mma.cuh: fewer passes over
+// Deeper groups (15..20, ekf_set_max_pending) go through the 256-column tiles of k_large_sweep_mma: fewer passes over
 // Sigma per correction and more corrections/s (cfg4: 18.6k against 16.5k at 20), but the sweep is then bound by the
 // FP64 pipe, not by HBM (0.66 of the copy peak per sweep period).
 #ifndef EKF_MAX_PENDING
@@ -255,9 +255,10 @@ __global__ void __launch_bounds__(THREADS, 1)
     }
 }
 
-// Launch the sweep instantiation for `pending` factors.  One CTA per tile (ROWS x THREADS*4 columns): on B200 the
-// plain full grid beats a persistent grid-stride launch here (scripts/sweep_tune.cu: P=1 0.65 ms = 6.6 TB/s at
-// N = 16,387; P=4..6 0.79-0.82 ms; P=8 0.98 ms — the FMAs of a tile do not overlap its own loads).
+// One CTA per tile (ROWS x THREADS*4 columns): on B200 the plain full grid beats a persistent grid-stride launch here
+// (experiments/sweep_tune.cu: P=1 0.65 ms = 6.6 TB/s at N = 16,387; P=4..6 0.79-0.82 ms; P=8 0.98 ms — the FMAs of a
+// tile do not overlap its own loads).  So the register path only serves 1-2 factors; deeper groups go to
+// k_large_sweep_mma (ekf_large_mma.cuh).
 template <int P, int U, int ROWS, int THREADS>
 inline void launch_sweep_cfg(double* sig, long long ld, int n_rows, const double2* Kp, const double2* Wp, long long row0,
                              unsigned long long* n_updates, int n_counted, const UpdateCmd* cmd, cudaStream_t stream) {
@@ -269,16 +270,10 @@ inline void launch_sweep_cfg(double* sig, long long ld, int n_rows, const double
 
 inline cudaError_t launch_sweep_p(int pending, double* sig, long long ld, int n_rows, const double2* Kp, const double2* Wp,
                                   long long row0, unsigned long long* n_updates, int n_counted, const UpdateCmd* cmd,
-                                  int /*sm_count*/, cudaStream_t stream) {
+                                  cudaStream_t stream) {
     switch (pending) {
         case 1: launch_sweep_cfg<1, 4, 32, 256>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
         case 2: launch_sweep_cfg<2, 4, 32, 256>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 3: launch_sweep_cfg<3, 4, 64, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 4: launch_sweep_cfg<4, 4, 64, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 5: launch_sweep_cfg<5, 4, 64, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 6: launch_sweep_cfg<6, 4, 64, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 7: launch_sweep_cfg<7, 4, 128, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
-        case 8: launch_sweep_cfg<8, 4, 64, 128>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

@@ -5,195 +5,60 @@
 // which mma.sync.m8n8k4.f64 (SASS DMMA.8x8x4) does in ceil(2P / 4) instructions.  DMMA accumulates its k = 0..3 terms
 // as a chain of FMAs in order (experiments/dmma_rate.cu), and the k axis is laid out factor by factor, x before y, so
 // every element still sees exactly the FMA sequence of sequential sweeps: the result is bit-identical to
-// k_large_sweep_p / k_large_sweep_tma (tests/test_gpu_ekf.py::test_delayed_application_is_bit_identical).
+// k_large_sweep_p (tests/test_gpu_ekf.py::test_delayed_application_is_bit_identical).
 //
-// What changes is the instruction mix.  The vector consumers of k_large_sweep_tma issue 2P DFMA per element plus one
-// shared-memory K fetch per four of them, which at P = 14 pushed the sweep from the copy time (0.66 ms at N = 16,387)
-// to 0.85 ms.  Here a warp issues ceil(P/2) DMMA per 64 elements; its B fragments (the W pairs of its 64 columns) sit
-// in registers for the whole work unit and the A fragments (the stage's K rows) cost ceil(P/2) 8-byte loads per stage.
-// The FP64 pipe time is the same as for the vector form (both run at 64 FMA / clk / SM), but it is the ONLY cost left
-// next to the copy, and it stays below the copy time up to P ~ 22.
+// What DMMA changes is the instruction mix.  Vector consumers issue 2P DFMA per element plus one shared-memory K fetch
+// per four of them, which at P = 14 pushed the sweep from the copy time (0.66 ms at N = 16,387) to 0.85 ms.  Here a
+// warp issues ceil(P/2) DMMA per 64 elements; its B fragments (the W pairs of its columns) sit in registers for the
+// whole work unit and the A fragments (the stage's K rows) cost ceil(P/2) 8-byte loads per 8 rows.  The FP64 pipe time
+// is the same as for the vector form (both run at 64 FMA / clk / SM), but it is the ONLY cost left next to the copy,
+// and it stays below the copy time up to P ~ 22.
 //
-// Pipeline as in ekf_large_tma.cuh: CTA = 1 producer warp + 8 consumer warps + 1 store warp, one CTA per SM,
-// persistent over work units of 512 columns x 128 rows, stages of 8 rows moved by the bulk copy engine
-// (cp.async.bulk, SASS UBLKCP) with mbarriers.  Stage rows are padded to 520 doubles so that the fragment accesses
-// (lane (g, t) touches row g, columns 2t, 2t+1 of a block) are bank-conflict free.
+// CTA = 1 producer warp + 8 consumer warps + 1 store warp, one CTA per SM, persistent over work units of SweepTile<P>
+// columns x kUnitRows rows, moved by the bulk copy engine (cp.async.bulk, SASS UBLKCP) through a ring of mbarrier
+// stages:
+//   producer : waits empty[s], bulk-loads the stage's row segments and its K rows (P x SROWS pairs); full[s] counts bytes;
+//   consumers: wait full[s], run the DMMA blocks of their columns in place in shared memory, arrive on done[s];
+//   storer   : waits done[s], bulk-stores the row segments, and hands stage s-1 back (empty[s-1]) once the store of
+//              s-1 has finished reading shared memory.
+// Stage rows are padded by 8 doubles so that the fragment accesses (lane (g, t) touches row g, columns 2t, 2t+1 of a
+// block) are bank-conflict free.
 #pragma once
-#include "ekf_large_tma.cuh"
+#include "bulk_copy.cuh"
+#include "ekf_large_delayed.cuh"
 
 namespace ekf {
 
-#ifndef EKF_MMA_STAGES
-#define EKF_MMA_STAGES 4
-#endif
-constexpr int kMmaStages = EKF_MMA_STAGES;   // 4 x (33 KB tile + K rows); 6 stages measured slower (748 vs 727 us at P = 14)
-constexpr int kMmaRowStride = kTmaCols + 8;  // doubles: 4,160 B = 64 B past a multiple of 128 B
-constexpr int kMmaTileBytes = kStageRows * kMmaRowStride * 8;
-constexpr int kMmaSmemBytes = kMmaStages * (kMmaTileBytes + kKBytes) + 3 * kMmaStages * 8 + 64;
+constexpr int kUnitRows = 128;  // rows of a work unit
+constexpr int kTmaConsumerWarps = 8;
+constexpr int kTmaThreads = 32 * (kTmaConsumerWarps + 2);
 
+// The sweep's geometry, from P alone.  A consumer warp keeps NBW x ceil(P/2) W fragment doubles in registers: at 64
+// columns per warp that fits up to P = 14, so deeper groups get 256-column tiles (32 columns per warp) with 16-row
+// stages, which keeps a stage at ~33 KB.  Measured on B200 (experiments/README.md): 6 stages slower, 256 columns 8 %
+// slower at P = 14, unguarded DMMA blocks slower.
 template <int P>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-    k_large_sweep_mma(double* __restrict__ sig, long long ld, int n_rows, const double2* __restrict__ Kp,
-                      const double2* __restrict__ Wp, long long row0, unsigned long long* __restrict__ n_updates,
-                      int n_counted, const UpdateCmd* __restrict__ cmd) {
-    constexpr int KS = (2 * P + 3) / 4;  // DMMA k-steps
-    constexpr int NBW = 8;               // 8 x 8 blocks per consumer warp and stage (64 columns)
-    pdl_prologue();
-    if (cmd && !cmd->do_update) return;
-    if (blockIdx.x == 0 && threadIdx.x == 0 && n_updates) *n_updates += (unsigned long long)n_counted;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    double* tiles = reinterpret_cast<double*>(smem_raw);                                     // [kMmaStages][8][520]
-    double2* ksm = reinterpret_cast<double2*>(smem_raw + (size_t)kMmaStages * kMmaTileBytes);   // [kMmaStages][kMaxPending][8]
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)kMmaStages * (kMmaTileBytes + kKBytes));
-    uint64_t* done = full + kMmaStages;
-    uint64_t* empty = done + kMmaStages;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) {
-        for (int s = 0; s < kMmaStages; ++s) {
-            mbar_init(full + s, 1);
-            mbar_init(done + s, kTmaConsumerWarps);
-            mbar_init(empty + s, 1);
-        }
-        fence_mbar_init();
-    }
-    __syncthreads();
-
-    const int chunks = (int)((ld + kTmaCols - 1) / kTmaCols);
-    const int row_units = (n_rows + kUnitRows - 1) / kUnitRows;
-    const long long units = (long long)chunks * row_units;
-    int stage = 0;
-    uint32_t phase = 0;
-    bool first = true;
-
-    for (long long u = blockIdx.x; u < units; u += gridDim.x) {
-        const int cu = (int)(u % chunks), ru = (int)(u / chunks);
-        const long long c0 = (long long)cu * kTmaCols;
-        const int width = (int)(ld - c0 < kTmaCols ? ld - c0 : kTmaCols);  // multiple of 16 doubles
-        const int r_begin = ru * kUnitRows;
-        const int r_end = r_begin + kUnitRows < n_rows ? r_begin + kUnitRows : n_rows;
-        const int groups = (r_end - r_begin + kStageRows - 1) / kStageRows;
-        if (warp == 0) {
-            // ---------------------------------------------------------------- producer
-            if (lane == 0) {
-                for (int g = 0; g < groups; ++g) {
-                    mbar_wait(empty + stage, phase ^ 1u);
-                    const int r = r_begin + g * kStageRows;
-                    const int nr = r_end - r < kStageRows ? r_end - r : kStageRows;
-                    mbar_arrive_expect_tx(full + stage, (uint32_t)(nr * width * 8 + P * kStageRows * 16));
-                    double* tile = tiles + (size_t)stage * kStageRows * kMmaRowStride;
-                    for (int k = 0; k < nr; ++k)
-                        bulk_g2s(tile + k * kMmaRowStride, sig + (long long)(r + k) * ld + c0, (uint32_t)(width * 8), full + stage);
-                    for (int j = 0; j < P; ++j)
-                        bulk_g2s(ksm + ((size_t)stage * kMaxPending + j) * kStageRows, Kp + (long long)j * ld + row0 + r,
-                                 kStageRows * 16, full + stage);
-                    if (++stage == kMmaStages) {
-                        stage = 0;
-                        phase ^= 1u;
-                    }
-                }
-            }
-        } else if (warp <= kTmaConsumerWarps) {
-            // ---------------------------------------------------------------- consumers
-            const int w = warp - 1;
-            const int g = lane >> 2, t = lane & 3;
-            const int wc0 = 64 * w;  // this warp's first column inside the tile
-            // B fragments: B[k][n] of k-step s and block b = W_j[c0 + wc0 + 8 b + g].{x | y}, j = (4 s + t) / 2,
-            // component (4 s + t) % 2; zero beyond the last factor or the tile's width
-            double bf[NBW][KS];
-#pragma unroll
-            for (int b = 0; b < NBW; ++b) {
-                const int c = wc0 + 8 * b + g;
-#pragma unroll
-                for (int s = 0; s < KS; ++s) {
-                    const int kk = 4 * s + t, j = kk >> 1;
-                    bf[b][s] = (j < P && c < width)
-                                   ? reinterpret_cast<const double*>(Wp + (long long)j * ld + c0 + c)[kk & 1]
-                                   : 0.0;
-                }
-            }
-            const int nblk = width - wc0 >= 64 ? NBW : (width - wc0 > 0 ? (width - wc0) / 8 : 0);  // warp-uniform
-            for (int gi = 0; gi < groups; ++gi) {
-                mbar_wait(full + stage, phase);
-                double* tile = tiles + (size_t)stage * kStageRows * kMmaRowStride;
-                const double* kst = reinterpret_cast<const double*>(ksm + (size_t)stage * kMaxPending * kStageRows);
-                // A fragments: A[g][k] = -K_j[row g of the stage].{x | y}
-                double af[KS];
-#pragma unroll
-                for (int s = 0; s < KS; ++s) {
-                    const int kk = 4 * s + t, j = kk >> 1;
-                    af[s] = j < P ? -kst[2 * (j * kStageRows + g) + (kk & 1)] : 0.0;
-                }
-                double* cp = tile + g * kMmaRowStride + wc0 + 2 * t;
-                double2 cf[NBW];
-#pragma unroll
-                for (int b = 0; b < NBW; ++b)
-                    if (b < nblk) cf[b] = *reinterpret_cast<const double2*>(cp + 8 * b);
-#pragma unroll
-                for (int s = 0; s < KS; ++s)
-#pragma unroll
-                    for (int b = 0; b < NBW; ++b)
-                        if (b < nblk)
-                            asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                                         : "+d"(cf[b].x), "+d"(cf[b].y)
-                                         : "d"(af[s]), "d"(bf[b][s]));
-#pragma unroll
-                for (int b = 0; b < NBW; ++b)
-                    if (b < nblk) *reinterpret_cast<double2*>(cp + 8 * b) = cf[b];
-                fence_proxy_async_smem();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(done + stage);
-                if (++stage == kMmaStages) {
-                    stage = 0;
-                    phase ^= 1u;
-                }
-            }
-        } else {
-            // ---------------------------------------------------------------- store warp
-            if (lane == 0) {
-                for (int g = 0; g < groups; ++g) {
-                    const int r = r_begin + g * kStageRows;
-                    const int nr = r_end - r < kStageRows ? r_end - r : kStageRows;
-                    mbar_wait(done + stage, phase);
-                    double* tile = tiles + (size_t)stage * kStageRows * kMmaRowStride;
-                    for (int k = 0; k < nr; ++k)
-                        bulk_s2g(sig + (long long)(r + k) * ld + c0, tile + k * kMmaRowStride, (uint32_t)(width * 8));
-                    bulk_commit();
-                    bulk_wait_read_1();  // every store but the newest has finished reading shared memory
-                    if (!first) mbar_arrive(empty + (stage == 0 ? kMmaStages - 1 : stage - 1));
-                    first = false;
-                    if (++stage == kMmaStages) {
-                        stage = 0;
-                        phase ^= 1u;
-                    }
-                }
-            }
-        }
-    }
-    if (warp == kTmaConsumerWarps + 1 && lane == 0) bulk_wait_all();  // drain before the CTA's shared memory goes away
-}
-
-// ---- more than 14 corrections per pass ------------------------------------------------------------------------
-// Above P = 14 the W fragments of a 64-column consumer warp (8 blocks x ceil(P/2) doubles) no longer fit the register
-// file.  This variant cuts the tile to 256 columns (32 per consumer warp: 4 x ceil(P/2) fragment doubles) and makes
-// a stage 16 rows instead of 8, so a stage is still 33 KB and one mbarrier round trip buys the same amount of work.
-template <int P, int COLS, int SROWS, int STAGES>
-struct MmaT {
-    static constexpr int KS = (2 * P + 3) / 4;
-    static constexpr int NBW = COLS / (8 * kTmaConsumerWarps);
-    static constexpr int RG = SROWS / 8;
+struct SweepTile {
+    static constexpr int COLS = P <= 14 ? 512 : 256;  // tile width
+    static constexpr int SROWS = P <= 14 ? 8 : 16;    // rows per stage
+    static constexpr int STAGES = 4;
+    static constexpr int KS = (2 * P + 3) / 4;                  // DMMA k-steps
+    static constexpr int NBW = COLS / (8 * kTmaConsumerWarps);  // 8 x 8 blocks per consumer warp and 8 rows
+    static constexpr int RG = SROWS / 8;                        // 8-row groups per stage
     static constexpr int RS = COLS + 8;  // row stride in doubles: 64 B past a multiple of 128 B
     static constexpr int kTileBytes = SROWS * RS * 8;
     static constexpr int kKBytes = P * SROWS * 16;
     static constexpr int kSmemBytes = STAGES * (kTileBytes + kKBytes) + 3 * STAGES * 8 + 64;
 };
 
-template <int P, int COLS, int SROWS, int STAGES>
+template <int P>
 __global__ void __launch_bounds__(kTmaThreads, 1)
-    k_large_sweep_mma_t(double* __restrict__ sig, long long ld, int n_rows, const double2* __restrict__ Kp,
-                        const double2* __restrict__ Wp, long long row0, unsigned long long* __restrict__ n_updates,
-                        int n_counted, const UpdateCmd* __restrict__ cmd) {
-    using T = MmaT<P, COLS, SROWS, STAGES>;
-    constexpr int KS = T::KS, NBW = T::NBW, RG = T::RG, RS = T::RS;
+    k_large_sweep_mma(double* __restrict__ sig, long long ld, int n_rows, const double2* __restrict__ Kp,
+                      const double2* __restrict__ Wp, long long row0, unsigned long long* __restrict__ n_updates,
+                      int n_counted, const UpdateCmd* __restrict__ cmd) {
+    using T = SweepTile<P>;
+    constexpr int COLS = T::COLS, SROWS = T::SROWS, STAGES = T::STAGES, KS = T::KS, NBW = T::NBW, RG = T::RG,
+                  RS = T::RS;
     pdl_prologue();
     if (cmd && !cmd->do_update) return;
     if (blockIdx.x == 0 && threadIdx.x == 0 && n_updates) *n_updates += (unsigned long long)n_counted;
@@ -252,7 +117,9 @@ __global__ void __launch_bounds__(kTmaThreads, 1)
             const int w = warp - 1;
             const int g = lane >> 2, t = lane & 3;
             const int wc0 = 8 * NBW * w;  // this warp's first column inside the tile
-            double bf[NBW][KS];           // B[k][n] of k-step s and block b, as in k_large_sweep_mma
+            // B fragments: B[k][n] of k-step s and block b = W_j[c0 + wc0 + 8 b + g].{x | y}, j = (4 s + t) / 2,
+            // component (4 s + t) % 2; zero beyond the last factor or the tile's width
+            double bf[NBW][KS];
 #pragma unroll
             for (int b = 0; b < NBW; ++b) {
                 const int c = wc0 + 8 * b + g;
@@ -327,83 +194,62 @@ __global__ void __launch_bounds__(kTmaThreads, 1)
     if (warp == kTmaConsumerWarps + 1 && lane == 0) bulk_wait_all();  // drain before the CTA's shared memory goes away
 }
 
-#ifndef EKF_MMA_T_COLS
-#define EKF_MMA_T_COLS 256
-#endif
-#ifndef EKF_MMA_T_SROWS
-#define EKF_MMA_T_SROWS 16
-#endif
-#ifndef EKF_MMA_T_STAGES
-#define EKF_MMA_T_STAGES 4
-#endif
+// One persistent CTA per SM (at most one per work unit).  P is at most kMaxPending: the factor buffers have no more
+// slots, and -DEKF_MAX_PENDING=14 builds no deeper kernel.
+template <int P>
+cudaError_t launch_sweep_mma(double* sig, long long ld, int n_rows, const double2* Kp, const double2* Wp, long long row0,
+                             unsigned long long* n_updates, int n_counted, const UpdateCmd* cmd, int sm_count,
+                             cudaStream_t stream) {
+    if constexpr (P > kMaxPending) {
+        return cudaErrorInvalidValue;
+    } else {
+        using T = SweepTile<P>;
+        // the shared-memory opt-in is per device: one flag per device, indexed by the device the launch goes to
+        static bool attr_set[64] = {false};
+        int dev = -1;
+        if (cudaGetDevice(&dev) != cudaSuccess) dev = -1;
+        if (dev < 0 || dev >= 64 || !attr_set[dev]) {
+            cudaError_t e = cudaFuncSetAttribute(k_large_sweep_mma<P>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 T::kSmemBytes);
+            if (e != cudaSuccess) return e;
+            if (dev >= 0 && dev < 64) attr_set[dev] = true;
+        }
+        const long long units = ((ld + T::COLS - 1) / T::COLS) * ((n_rows + kUnitRows - 1) / kUnitRows);
+        const unsigned grid = (unsigned)(units < sm_count ? (units < 1 ? 1 : units) : sm_count);
+        k_large_sweep_mma<P><<<grid, kTmaThreads, T::kSmemBytes, stream>>>(sig, ld, n_rows, Kp, Wp, row0, n_updates,
+                                                                          n_counted, cmd);
+        return cudaGetLastError();
+    }
+}
 
-// Dispatch: register path for 1-2 factors, DMMA pipeline from 3 on.  Kp must have at least kStageRows pairs of slack
-// after its last used row (the stage's K rows are fetched 8 at a time).
-inline cudaError_t launch_sweep_mma(int pending, double* sig, long long ld, int n_rows, const double2* Kp,
-                                    const double2* Wp, long long row0, unsigned long long* n_updates, int n_counted,
-                                    const UpdateCmd* cmd, int sm_count, cudaStream_t stream) {
-    if (pending <= 2) return launch_sweep_p(pending, sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
-    const long long units = ((ld + kTmaCols - 1) / kTmaCols) * ((n_rows + kUnitRows - 1) / kUnitRows);
-    const unsigned grid = (unsigned)(units < sm_count ? (units < 1 ? 1 : units) : sm_count);
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) dev = -1;
-#define EKF_MMA_CASE(PP)                                                                                              \
-    case PP: {                                                                                                        \
-        static bool attr_set[64] = {false};                                                                           \
-        if (dev < 0 || dev >= 64 || !attr_set[dev]) {                                                                 \
-            cudaError_t e = cudaFuncSetAttribute(k_large_sweep_mma<PP>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                                 kMmaSmemBytes);                                                      \
-            if (e != cudaSuccess) return e;                                                                           \
-            if (dev >= 0 && dev < 64) attr_set[dev] = true;                                                           \
-        }                                                                                                             \
-        k_large_sweep_mma<PP><<<grid, kTmaThreads, kMmaSmemBytes, stream>>>(sig, ld, n_rows, Kp, Wp, row0, n_updates, \
-                                                                             n_counted, cmd);                        \
-        break;                                                                                                        \
-    }
-#define EKF_MMA_T_CASE(PP)                                                                                            \
-    case PP: {                                                                                                        \
-        using TT = MmaT<PP, EKF_MMA_T_COLS, EKF_MMA_T_SROWS, EKF_MMA_T_STAGES>;                                       \
-        auto kern = k_large_sweep_mma_t<PP, EKF_MMA_T_COLS, EKF_MMA_T_SROWS, EKF_MMA_T_STAGES>;                       \
-        static bool attr_set[64] = {false};                                                                           \
-        if (dev < 0 || dev >= 64 || !attr_set[dev]) {                                                                 \
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TT::kSmemBytes);  \
-            if (e != cudaSuccess) return e;                                                                           \
-            if (dev >= 0 && dev < 64) attr_set[dev] = true;                                                           \
-        }                                                                                                             \
-        const long long units_t = ((ld + EKF_MMA_T_COLS - 1) / EKF_MMA_T_COLS) * ((n_rows + kUnitRows - 1) / kUnitRows); \
-        const unsigned grid_t = (unsigned)(units_t < sm_count ? (units_t < 1 ? 1 : units_t) : sm_count);             \
-        kern<<<grid_t, kTmaThreads, TT::kSmemBytes, stream>>>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd); \
-        break;                                                                                                        \
-    }
+// Apply `pending` factor pairs: the register path for 1-2 factors, the DMMA pipeline from 3 on.  Kp must have at least
+// 16 pairs of slack after its last used row (a stage's K rows are fetched SweepTile<P>::SROWS at a time).
+inline cudaError_t launch_sweep(int pending, double* sig, long long ld, int n_rows, const double2* Kp, const double2* Wp,
+                                long long row0, unsigned long long* n_updates, int n_counted, const UpdateCmd* cmd,
+                                int sm_count, cudaStream_t stream) {
     switch (pending) {
-        EKF_MMA_CASE(3)
-        EKF_MMA_CASE(4)
-        EKF_MMA_CASE(5)
-        EKF_MMA_CASE(6)
-        EKF_MMA_CASE(7)
-        EKF_MMA_CASE(8)
-        EKF_MMA_CASE(9)
-        EKF_MMA_CASE(10)
-        EKF_MMA_CASE(11)
-        EKF_MMA_CASE(12)
-        EKF_MMA_CASE(13)
-        EKF_MMA_CASE(14)
-#if EKF_MAX_PENDING > 14
-        EKF_MMA_T_CASE(15)
-        EKF_MMA_T_CASE(16)
-#endif
-#if EKF_MAX_PENDING > 16
-        EKF_MMA_T_CASE(17)
-        EKF_MMA_T_CASE(18)
-        EKF_MMA_T_CASE(19)
-        EKF_MMA_T_CASE(20)
-#endif
-        default:
-            return cudaErrorInvalidValue;
+        case 1:
+        case 2: return launch_sweep_p(pending, sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, stream);
+        case 3: return launch_sweep_mma<3>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 4: return launch_sweep_mma<4>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 5: return launch_sweep_mma<5>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 6: return launch_sweep_mma<6>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 7: return launch_sweep_mma<7>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 8: return launch_sweep_mma<8>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 9: return launch_sweep_mma<9>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 10: return launch_sweep_mma<10>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 11: return launch_sweep_mma<11>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 12: return launch_sweep_mma<12>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 13: return launch_sweep_mma<13>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 14: return launch_sweep_mma<14>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 15: return launch_sweep_mma<15>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 16: return launch_sweep_mma<16>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 17: return launch_sweep_mma<17>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 18: return launch_sweep_mma<18>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 19: return launch_sweep_mma<19>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        case 20: return launch_sweep_mma<20>(sig, ld, n_rows, Kp, Wp, row0, n_updates, n_counted, cmd, sm_count, stream);
+        default: return cudaErrorInvalidValue;
     }
-#undef EKF_MMA_CASE
-#undef EKF_MMA_T_CASE
-    return cudaGetLastError();
 }
 
 }  // namespace ekf

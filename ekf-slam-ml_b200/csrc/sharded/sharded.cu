@@ -20,13 +20,6 @@
 
 using namespace ekf;
 
-// multi-factor sweep: DMMA consumers (ekf_large_mma.cuh) unless the vector TMA path is asked for (comparison builds)
-#ifndef EKF_SWEEP_VECTOR
-#define EKF_SWEEP_LAUNCH launch_sweep_mma
-#else
-#define EKF_SWEEP_LAUNCH launch_sweep
-#endif
-
 namespace {
 
 thread_local char g_err[512] = "";
@@ -951,8 +944,8 @@ int flush(ekf_sharded* h, int n_counted, bool use_cmd) {
     }
     for (auto& s : h->sh) {
         if (s.rows > 0) {
-            CU(EKF_SWEEP_LAUNCH(h->pending, s.sig, h->ld, s.rows, s.K2, s.W2, s.r0, s.nupd, n_counted, use_cmd ? s.cmd : nullptr,
-                              h->sm_count, h->stream));
+            CU(launch_sweep(h->pending, s.sig, h->ld, s.rows, s.K2, s.W2, s.r0, s.nupd, n_counted, use_cmd ? s.cmd : nullptr,
+                            h->sm_count, h->stream));
             h->launches++;
         }
     }

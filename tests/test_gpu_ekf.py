@@ -647,14 +647,15 @@ def test_scan_to_map_pipeline(gpu_pkg):
 
 
 def test_delayed_application_is_bit_identical(gpu_pkg):
-    """Accumulating up to 8 corrections per pass over Sigma (ekf_large_delayed.cuh) must give exactly the bits of
+    """Accumulating up to 20 corrections per pass over Sigma (ekf_large_delayed.cuh) must give exactly the bits of
     the reference's schedule (one pass per correction): every element sees the same FMA sequence."""
     n = 300
     tg = gpu_pkg.tracegen
     w = tg.grid_world(20, 15, pitch=0.4, n_slots=n, max_visible=1.2)
     tr = tg.simulate_known(w, 1, 8, seed=21)
     outs = []
-    for k in (1, 3, 8, 14, 20):  # 3..14: DMMA sweep on 512-column tiles, 15..20: the narrow-tile variant
+    ks = (1, 2, 3, 8, 14, 15, 20)  # 1..2: register sweep; 3..20: DMMA sweep, 512-column tiles to 14, 256 from 15
+    for k in ks:
         f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
         f.set_max_pending(k)
         f.set_carry_pending(False)  # groups end with the measurement() call
@@ -666,7 +667,7 @@ def test_delayed_application_is_bit_identical(gpu_pkg):
     for st, sg, _ in outs[1:]:
         assert np.array_equal(st.view(np.uint64), outs[0][0].view(np.uint64))
         assert np.array_equal(sg.view(np.uint64), outs[0][1].view(np.uint64))
-    assert outs[4][2] < outs[2][2] < outs[0][2]  # fewer launches: fewer sweeps
+    assert outs[ks.index(20)][2] < outs[ks.index(8)][2] < outs[0][2]  # fewer launches: fewer sweeps
 
 
 def test_pending_factors_carried_across_prediction(gpu_pkg):
