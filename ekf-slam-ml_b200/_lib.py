@@ -63,6 +63,8 @@ SIGNATURES = {
     "ekf_batch_create": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_void_pp]),
     "ekf_batch_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "ekf_batch_size": (ctypes.c_int64, [ctypes.c_void_p]),
+    "ekf_batch_engine": (ctypes.c_int, [ctypes.c_void_p]),
+    "ekf_batch_sweep_count": (ctypes.c_int, [ctypes.c_void_p, c_u64_p]),
     "ekf_batch_step_known": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_batch_step_unknown": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                               ctypes.c_int, ctypes.c_void_p]),

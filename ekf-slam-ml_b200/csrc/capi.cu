@@ -14,6 +14,7 @@
 #include "ekf_fused.cuh"
 #include "ekf_fused_sym.cuh"
 #include "ekf_fused_tile.cuh"
+#include "ekf_batch_wide.cuh"
 #include "ekf_large.cuh"
 #include "ekf_large_mma.cuh"
 
@@ -1071,16 +1072,22 @@ struct ekf_batch {
     int n = 0, N = 0, device = 0;
     int sig_stride = 0, st_stride = 0;
     bool tiled = false;  // n == 20: register-resident tile layout (ekf_fused_tile.cuh); else symmetric staircase
+    bool wide = false;   // n > kFusedMaxN: dense N x ld Sigma per filter in HBM (ekf_batch_wide.cuh)
+    long long ld = 0;    // wide: row stride of a filter's Sigma
+    int grid = 0;        // wide: CTAs of the step kernel (each owns a set of factor slots)
     cudaStream_t stream = nullptr;       // compute
     cudaStream_t copy_stream = nullptr;  // H2D of the next step's inputs
     cudaStream_t out_stream = nullptr;   // D2H of results
     uint64_t launches = 0;
-    double* d_sigma = nullptr;  // [B][sig_stride], symmetric staircase layout (ekf_fused_sym.cuh)
+    double* d_sigma = nullptr;  // [B][sig_stride]: staircase (ekf_fused_sym.cuh), tile, or dense N x ld (wide)
     double* d_dense = nullptr;  // N x N scratch of ekf_batch_get_sigma
     double* d_state = nullptr;
     int32_t* d_init_flag = nullptr;
     uint8_t* d_known = nullptr;
     unsigned long long* d_nupd = nullptr;
+    unsigned long long* d_sweeps = nullptr;  // wide: passes over a filter's Sigma, summed over the batch
+    double2* d_wK = nullptr;                 // wide: [grid][kWidePending * ld + 16] factor slots
+    double2* d_wW = nullptr;
     // double-buffered device inputs
     int m_cap = 0;
     double* d_twists[2] = {nullptr, nullptr};
@@ -1111,6 +1118,9 @@ int free_batch(ekf_batch* b) {
     cudaFree(b->d_init_flag);
     cudaFree(b->d_known);
     cudaFree(b->d_nupd);
+    cudaFree(b->d_sweeps);
+    cudaFree(b->d_wK);
+    cudaFree(b->d_wW);
     for (int s = 0; s < 2; ++s) {
         cudaFree(b->d_twists[s]);
         cudaFree(b->d_xy[s]);
@@ -1175,6 +1185,36 @@ FusedParams batch_params(ekf_batch* b, int mode, int m_max, const double* tw, co
     return p;
 }
 
+// One step of a wide batch: dense readings (offsets == nullptr) or the marker list.
+int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint8_t* vis, const int32_t* offsets,
+                long long total) {
+    WideParams p;
+    memset(&p, 0, sizeof(p));
+    p.sigma = b->d_sigma;
+    p.state = b->d_state;
+    p.init_flag = b->d_init_flag;
+    p.n_updates = b->d_nupd;
+    p.n_sweeps = b->d_sweeps;
+    p.Kp = b->d_wK;
+    p.Wp = b->d_wW;
+    p.twists = twists;
+    p.xy = xy;
+    p.vis = vis;
+    p.offsets = offsets;
+    p.sparse_total = total;
+    p.B = b->B;
+    p.ld = b->ld;
+    p.slot_stride = (long long)kWidePending * b->ld + 16;
+    p.n = b->n;
+    p.N = b->N;
+    p.st_stride = b->st_stride;
+    CU(launch_wide_step(p, b->grid, b->stream));
+    return EKF_OK;
+}
+
+// The marker list carries uint8_t landmark ids.
+constexpr int kMarkerMaxN = 256;
+
 }  // namespace
 
 extern "C" {
@@ -1183,7 +1223,11 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
     if (!out) return fail(EKF_ERR_INVALID, "null out pointer");
     *out = nullptr;
     if (B <= 0 || n <= 0) return fail(EKF_ERR_INVALID, "invalid batch shape");
-    if (n > kFusedMaxN) return fail(EKF_ERR_UNSUPPORTED, "batched filters use the fused engine: n <= %d", kFusedMaxN);
+    if (n > kWideMaxN)
+        return fail(EKF_ERR_UNSUPPORTED,
+                    "batched filters support n <= %d landmarks; for a larger map use one streamed filter per map, "
+                    "ekf_create_ex(n, device, EKF_ENGINE_STREAM, &h)",
+                    kWideMaxN);
     int count = 0;
     int rc = ekf_device_count(&count);
     if (rc) return rc;
@@ -1196,9 +1240,16 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
     b->N = 3 + 2 * n;
     b->device = device;
     b->tiled = (n == tile::kNL);
-    // tiled: one block per filter holds Sigma (fragment layout) and the state, so that one bulk copy stages it
-    b->sig_stride = b->tiled ? tile::kStride : sym_sig_stride(b->N);
-    b->st_stride = b->tiled ? tile::kStride : sym_st_stride(b->N);
+    b->wide = n > kFusedMaxN;
+    if (b->wide) {  // the streamed engine's layout: row-major N x ld, ld = N rounded up to 16 doubles
+        b->ld = fused_round16(b->N);
+        b->sig_stride = b->N * (int)b->ld;
+        b->st_stride = fused_round16(b->N);
+    } else {
+        // tiled: one block per filter holds Sigma (fragment layout) and the state, so that one bulk copy stages it
+        b->sig_stride = b->tiled ? tile::kStride : sym_sig_stride(b->N);
+        b->st_stride = b->tiled ? tile::kStride : sym_st_stride(b->N);
+    }
 #define CUB(expr)                          \
     do {                                   \
         cudaError_t e_ = (expr);           \
@@ -1238,7 +1289,23 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
         free_batch(b);
         return fail(EKF_ERR_INVALID, "batch too large");
     }
-    if (b->tiled)
+    if (b->wide) {
+        int sms = 0;
+        CUB(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+        b->grid = (int)std::min<long long>(B, std::max(sms, 1));
+        const size_t slots = (size_t)b->grid * ((size_t)kWidePending * b->ld + 16);
+        CUB(cudaMalloc(&b->d_wK, sizeof(double2) * slots));
+        CUB(cudaMalloc(&b->d_wW, sizeof(double2) * slots));
+        CUB(cudaMalloc(&b->d_sweeps, sizeof(unsigned long long)));
+        CUB(cudaMemsetAsync(b->d_wK, 0, sizeof(double2) * slots, b->stream));
+        CUB(cudaMemsetAsync(b->d_wW, 0, sizeof(double2) * slots, b->stream));
+        CUB(cudaMemsetAsync(b->d_sweeps, 0, sizeof(unsigned long long), b->stream));
+        CUB(cudaMemsetAsync(b->d_sigma, 0, sizeof(double) * (size_t)b->sig_stride * B, b->stream));
+        CUB(cudaMemsetAsync(b->d_state, 0, sizeof(double) * (size_t)b->st_stride * B, b->stream));
+        CUB(cudaMemsetAsync(b->d_init_flag, 0, sizeof(int32_t) * (size_t)B, b->stream));
+        const long long diag = B * (b->N - 3);
+        k_wide_init_sigma<<<(unsigned)((diag + 255) / 256), 256, 0, b->stream>>>(b->d_sigma, B, b->N, b->ld);
+    } else if (b->tiled)
         tile::k_fused_tile_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_init_flag, B);
     else
         k_fused_sym_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_state, b->d_init_flag, B, b->N,
@@ -1258,11 +1325,28 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
 
 int ekf_batch_destroy(ekf_batch* b) { return free_batch(b); }
 int64_t ekf_batch_size(const ekf_batch* b) { return b ? b->B : EKF_ERR_INVALID; }
+int ekf_batch_engine(const ekf_batch* b) { return b ? (b->wide ? EKF_ENGINE_STREAM : EKF_ENGINE_FUSED) : EKF_ERR_INVALID; }
+int ekf_batch_sweep_count(ekf_batch* b, uint64_t* out) {
+    if (!b || !out) return fail(EKF_ERR_INVALID, "null argument");
+    *out = 0;
+    if (!b->wide) return EKF_OK;  // the on-chip engines never sweep a covariance in HBM
+    DeviceGuard g(b->device);
+    unsigned long long v = 0;
+    CU(cudaMemcpyAsync(&v, b->d_sweeps, sizeof(v), cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    *out = v;
+    return EKF_OK;
+}
 void* ekf_batch_stream(ekf_batch* b) { return b ? (void*)b->stream : nullptr; }
 
 int ekf_batch_step_known_dev(ekf_batch* b, const double* d_twists, const double* d_xy, const uint8_t* d_visible) {
     if (!b || !d_twists || !d_xy || !d_visible) return fail(EKF_ERR_INVALID, "null argument");
     DeviceGuard g(b->device);
+    if (b->wide) {
+        int rc = launch_wide(b, d_twists, d_xy, d_visible, nullptr, 0);
+        b->launches += 1;
+        return rc;
+    }
     FusedParams p = batch_params(b, kDoPredict | kDoMeasurement, 1, d_twists, d_xy, d_visible, nullptr, nullptr);
     int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_sym(p, b->stream, b->device);
     b->launches += 1;
@@ -1272,6 +1356,9 @@ int ekf_batch_step_known_dev(ekf_batch* b, const double* d_twists, const double*
 int ekf_batch_step_unknown_dev(ekf_batch* b, const double* d_twists, const double* d_meas, const int32_t* d_count,
                                int m_max, int32_t* d_assoc_out) {
     if (!b || !d_twists || !d_meas || m_max <= 0) return fail(EKF_ERR_INVALID, "invalid argument");
+    if (b->wide)
+        return fail(EKF_ERR_UNSUPPORTED, "unknown data association is not available for batches with n > %d landmarks",
+                    kFusedMaxN);
     DeviceGuard g(b->device);
     FusedParams p = batch_params(b, kDoPredict | kDoAssociation, m_max, d_twists, d_meas, nullptr, d_count, d_assoc_out);
     int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_sym(p, b->stream, b->device);
@@ -1301,7 +1388,15 @@ int ekf_batch_step_known(ekf_batch* b, const double* twists, const double* xy, c
 int ekf_batch_step_known_sparse_dev(ekf_batch* b, const double* d_twists, const int32_t* d_offsets, const uint8_t* d_ids,
                                     const double* d_xy, int64_t total) {
     if (!b || !d_twists || !d_offsets || !d_ids || !d_xy || total < 0) return fail(EKF_ERR_INVALID, "invalid argument");
+    if (b->n > kMarkerMaxN)
+        return fail(EKF_ERR_UNSUPPORTED, "the marker list carries uint8 ids: n <= %d landmarks (use the dense arrays)",
+                    kMarkerMaxN);
     DeviceGuard g(b->device);
+    if (b->wide) {
+        int rc = launch_wide(b, d_twists, d_xy, d_ids, d_offsets, total);
+        b->launches += 1;
+        return rc;
+    }
     FusedParams p = batch_params(b, kDoPredict | kDoMeasurement | kSparseReadings, 1, d_twists, d_xy, d_ids, d_offsets,
                                  nullptr);
     p.sparse_total = total;
@@ -1315,6 +1410,9 @@ int ekf_batch_step_known_sparse(ekf_batch* b, const double* twists, const int32_
     if (!b || !twists || !offsets || total < 0 || (total > 0 && (!ids || !xy)))
         return fail(EKF_ERR_INVALID, "null argument");
     if (total > (int64_t)b->n * b->B) return fail(EKF_ERR_INVALID, "marker list longer than n markers per filter");
+    if (b->n > kMarkerMaxN)
+        return fail(EKF_ERR_UNSUPPORTED, "the marker list carries uint8 ids: n <= %d landmarks (use the dense arrays)",
+                    kMarkerMaxN);
     DeviceGuard g(b->device);
     const int s = b->slot;
     b->slot ^= 1;
@@ -1337,6 +1435,9 @@ int ekf_batch_step_known_sparse(ekf_batch* b, const double* twists, const int32_
 int ekf_batch_step_unknown(ekf_batch* b, const double* twists, const double* meas, const int32_t* count, int m_max,
                            int32_t* assoc_out) {
     if (!b || !twists || !meas || !count || m_max <= 0) return fail(EKF_ERR_INVALID, "invalid argument");
+    if (b->wide)
+        return fail(EKF_ERR_UNSUPPORTED, "unknown data association is not available for batches with n > %d landmarks",
+                    kFusedMaxN);
     DeviceGuard g(b->device);
     int rc = batch_ensure_xy(b, m_max);
     if (rc) return rc;
@@ -1395,7 +1496,13 @@ int ekf_batch_get_states(ekf_batch* b, double* out) {
 int ekf_batch_get_sigma(ekf_batch* b, int64_t filter, double* out, int64_t ld) {
     if (!b || !out || filter < 0 || filter >= b->B || ld < b->N) return fail(EKF_ERR_INVALID, "invalid argument");
     DeviceGuard g(b->device);
-    // the batch keeps Sigma in the symmetric staircase layout; expand one filter's copy to dense N x N
+    if (b->wide) {  // already dense: one 2-D copy
+        CU(cudaMemcpy2DAsync(out, sizeof(double) * ld, b->d_sigma + (size_t)filter * b->sig_stride, sizeof(double) * b->ld,
+                             sizeof(double) * b->N, b->N, cudaMemcpyDeviceToHost, b->stream));
+        CU(cudaStreamSynchronize(b->stream));
+        return EKF_OK;
+    }
+    // the on-chip engines keep Sigma in the staircase or tile layout; expand one filter's copy to dense N x N
     if (!b->d_dense) CU(cudaMalloc(&b->d_dense, sizeof(double) * (size_t)b->N * b->N));
     if (b->tiled)
         tile::k_fused_tile_unpack<<<(b->N * b->N + 255) / 256, 256, 0, b->stream>>>(
@@ -1417,8 +1524,8 @@ int ekf_batch_get_known(ekf_batch* b, uint8_t* out) {
     CU(cudaStreamSynchronize(b->stream));
     return EKF_OK;
 }
-// Checkpoint / resume of the whole batch: the arrays exactly as the engine keeps them (Sigma in its packed symmetric
-// layout, per-filter strides as reported by ekf_batch_checkpoint_size).  No conversion, so a restored batch continues
+// Checkpoint / resume of the whole batch: the arrays exactly as the engine keeps them (Sigma in the engine's layout:
+// packed symmetric, tile or dense N x ld; per-filter strides as reported by ekf_batch_checkpoint_size).  No conversion, so a restored batch continues
 // bit-identically.
 int ekf_batch_checkpoint_size(ekf_batch* b, int64_t* sigma_doubles, int64_t* state_doubles) {
     if (!b) return fail(EKF_ERR_INVALID, "null handle");

@@ -51,42 +51,56 @@ struct SweepTile {
     static constexpr int kSmemBytes = STAGES * (kTileBytes + kKBytes) + 3 * STAGES * 8 + 64;
 };
 
+// Where one thread stands in the CTA's stage ring: each role (producer lane, consumer warps, store lane) advances its own
+// copy.  A kernel that sweeps several times keeps it across calls, so the ring runs on as one stream of stages.
+struct SweepRing {
+    int stage = 0;
+    uint32_t phase = 0;
+    bool first = true;  // store lane: no earlier stage to hand back yet
+};
+
+// The barriers of the stage ring in the dynamic shared memory `smem_raw` (laid out as SweepTile<P>); every thread of the
+// CTA must pass a __syncthreads() before the first sweep.
 template <int P>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-    k_large_sweep_mma(double* __restrict__ sig, long long ld, int n_rows, const double2* __restrict__ Kp,
-                      const double2* __restrict__ Wp, long long row0, unsigned long long* __restrict__ n_updates,
-                      int n_counted, const UpdateCmd* __restrict__ cmd) {
+__device__ __forceinline__ uint64_t* sweep_mma_barriers(unsigned char* smem_raw) {
+    using T = SweepTile<P>;
+    return reinterpret_cast<uint64_t*>(smem_raw + (size_t)T::STAGES * (T::kTileBytes + T::kKBytes));
+}
+template <int P>
+__device__ __forceinline__ void sweep_mma_init(unsigned char* smem_raw) {
+    uint64_t* full = sweep_mma_barriers<P>(smem_raw);
+    for (int s = 0; s < SweepTile<P>::STAGES; ++s) {
+        mbar_init(full + s, 1);
+        mbar_init(full + SweepTile<P>::STAGES + s, kTmaConsumerWarps);
+        mbar_init(full + 2 * SweepTile<P>::STAGES + s, 1);
+    }
+    fence_mbar_init();
+}
+
+// The work units of one sweep, run by all kTmaThreads threads of the CTA: blockIdx.x, blockIdx.x + gridDim.x, ... when
+// the grid shares the sweep (GRID), all of them otherwise.  The bulk stores of the last stages may still be in flight
+// on return: the store lane drains them (bulk_wait_all) before anything reads the swept rows or the CTA exits.
+template <int P, bool GRID>
+__device__ __forceinline__ void sweep_mma_units(double* sig, long long ld, int n_rows, const double2* Kp, const double2* Wp,
+                                                long long row0, unsigned char* smem_raw, SweepRing& ring) {
     using T = SweepTile<P>;
     constexpr int COLS = T::COLS, SROWS = T::SROWS, STAGES = T::STAGES, KS = T::KS, NBW = T::NBW, RG = T::RG,
                   RS = T::RS;
-    pdl_prologue();
-    if (cmd && !cmd->do_update) return;
-    if (blockIdx.x == 0 && threadIdx.x == 0 && n_updates) *n_updates += (unsigned long long)n_counted;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
     double* tiles = reinterpret_cast<double*>(smem_raw);                                   // [STAGES][SROWS][RS]
     double2* ksm = reinterpret_cast<double2*>(smem_raw + (size_t)STAGES * T::kTileBytes);  // [STAGES][P][SROWS]
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)STAGES * (T::kTileBytes + T::kKBytes));
+    uint64_t* full = sweep_mma_barriers<P>(smem_raw);
     uint64_t* done = full + STAGES;
     uint64_t* empty = done + STAGES;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) {
-        for (int s = 0; s < STAGES; ++s) {
-            mbar_init(full + s, 1);
-            mbar_init(done + s, kTmaConsumerWarps);
-            mbar_init(empty + s, 1);
-        }
-        fence_mbar_init();
-    }
-    __syncthreads();
 
     const int chunks = (int)((ld + COLS - 1) / COLS);
     const int row_units = (n_rows + kUnitRows - 1) / kUnitRows;
     const long long units = (long long)chunks * row_units;
-    int stage = 0;
-    uint32_t phase = 0;
-    bool first = true;
+    int stage = ring.stage;
+    uint32_t phase = ring.phase;
+    bool first = ring.first;
 
-    for (long long u = blockIdx.x; u < units; u += gridDim.x) {
+    for (long long u = GRID ? blockIdx.x : 0; u < units; u += GRID ? gridDim.x : 1) {
         const int cu = (int)(u % chunks), ru = (int)(u / chunks);
         const long long c0 = (long long)cu * COLS;
         const int width = (int)(ld - c0 < COLS ? ld - c0 : COLS);  // multiple of 16 doubles
@@ -191,7 +205,25 @@ __global__ void __launch_bounds__(kTmaThreads, 1)
             }
         }
     }
-    if (warp == kTmaConsumerWarps + 1 && lane == 0) bulk_wait_all();  // drain before the CTA's shared memory goes away
+    ring.stage = stage;
+    ring.phase = phase;
+    ring.first = first;
+}
+
+template <int P>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+    k_large_sweep_mma(double* __restrict__ sig, long long ld, int n_rows, const double2* __restrict__ Kp,
+                      const double2* __restrict__ Wp, long long row0, unsigned long long* __restrict__ n_updates,
+                      int n_counted, const UpdateCmd* __restrict__ cmd) {
+    pdl_prologue();
+    if (cmd && !cmd->do_update) return;
+    if (blockIdx.x == 0 && threadIdx.x == 0 && n_updates) *n_updates += (unsigned long long)n_counted;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    if (threadIdx.x == 0) sweep_mma_init<P>(smem_raw);
+    __syncthreads();
+    SweepRing ring;
+    sweep_mma_units<P, true>(sig, ld, n_rows, Kp, Wp, row0, smem_raw, ring);
+    if (threadIdx.x == 32 * (kTmaConsumerWarps + 1)) bulk_wait_all();  // drain before the CTA's shared memory goes away
 }
 
 // One persistent CTA per SM (at most one per work unit).  P is at most kMaxPending: the factor buffers have no more

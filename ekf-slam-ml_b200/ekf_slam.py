@@ -338,8 +338,8 @@ def marker_list(xy, visible):
     (offsets [B+1] int32, ids [total] uint8, xy [total,2]); only visible markers are listed, in id order."""
     vis = np.asarray(visible) != 0
     B, n = vis.shape
-    if n > 255:
-        raise ValueError("marker ids are uint8")
+    if n > 256:
+        raise ValueError("marker ids are uint8: n <= 256")
     offsets = np.zeros(B + 1, dtype=np.int32)
     np.cumsum(vis.sum(axis=1), out=offsets[1:])
     rows, ids = np.nonzero(vis)
@@ -348,7 +348,10 @@ def marker_list(xy, visible):
 
 
 class EKFBatch:
-    """B independent reference-sized filters on one GPU (Monte-Carlo noise-seed sweep, SURVEY.md §8d cfg3)."""
+    """B independent filters on one GPU (Monte-Carlo noise-seed sweep, SURVEY.md §8d cfg3).  Up to 64 landmarks the
+    covariance stays on chip during a step (`engine` == ENGINE_FUSED); from 65 to 1,024 it lives in HBM and each filter
+    is bit-identical to an EKF_SLAM(n, engine=ENGINE_STREAM) with set_carry_pending(False) (`engine` ==
+    ENGINE_STREAM; unknown association is not available there)."""
 
     def __init__(self, n_filters, n_measurements=20, device=0):
         self._L = _lib.load()
@@ -365,6 +368,18 @@ class EKFBatch:
             self._h = None
 
     __del__ = close
+
+    @property
+    def engine(self):
+        """ENGINE_FUSED (covariance on chip, n <= 64) or ENGINE_STREAM (covariance in HBM, 64 < n <= 1024)."""
+        return self._L.ekf_batch_engine(self._h)
+
+    @property
+    def sweep_count(self):
+        """Passes over a filter's covariance in HBM so far, summed over the filters (0 for the on-chip engines)."""
+        v = ctypes.c_uint64()
+        check(self._L.ekf_batch_sweep_count(self._h, ctypes.byref(v)))
+        return v.value
 
     def step_known(self, twists, xy, visible):
         """prediction + measurement for every filter; host arrays [B,2], [B,2n], [B,n] (uint8)."""
@@ -467,8 +482,8 @@ class EKFBatch:
         return ms.value
 
     def checkpoint(self):
-        """Everything needed to resume the batch bit-identically (dict of numpy arrays; Sigma in the engine's packed
-        symmetric layout).  save_checkpoint / load_checkpoint put it in an .npz file."""
+        """Everything needed to resume the batch bit-identically (dict of numpy arrays; Sigma in the engine's own layout,
+        see device_pointers).  save_checkpoint / load_checkpoint put it in an .npz file."""
         ns, nst = ctypes.c_int64(), ctypes.c_int64()
         check(self._L.ekf_batch_checkpoint_size(self._h, ctypes.byref(ns), ctypes.byref(nst)))
         ck = {"sigma_packed": np.empty(ns.value), "state": np.empty(nst.value),
@@ -502,6 +517,9 @@ class EKFBatch:
             self.restore({k: z[k] for k in z.files})
 
     def device_pointers(self):
+        """(sigma, sigma_stride, state, state_stride): device addresses and per-filter strides in doubles.  Sigma is in
+        the engine's layout: tile (n = 20), packed symmetric staircase (n <= 64), or dense N x ld rows with
+        ld = N rounded up to 16 (n > 64, sigma_stride = N * ld)."""
         s, st = ctypes.c_void_p(), ctypes.c_void_p()
         ss, sts = ctypes.c_int64(), ctypes.c_int64()
         check(self._L.ekf_batch_device_pointers(self._h, ctypes.byref(s), ctypes.byref(ss), ctypes.byref(st),

@@ -121,9 +121,19 @@ void* ekf_stream(ekf_filter* h); /* cudaStream_t */
 /* ------------------------------------------------------------------ batch of independent filters */
 typedef struct ekf_batch ekf_batch;
 
+/* n_landmarks <= 64: Sigma stays on chip during a step (EKF_ENGINE_FUSED engines).  64 < n_landmarks <= 1024: the
+ * "wide" engine (EKF_ENGINE_STREAM): every filter's Sigma lives in HBM and each filter is bit-identical to an
+ * ekf_create_ex(n, device, EKF_ENGINE_STREAM, ...) filter with ekf_set_carry_pending(h, 0) fed the same inputs; it
+ * serves the known-association verbs (dense, marker list for n <= 256, device-resident), and ekf_batch_step_unknown
+ * returns EKF_ERR_UNSUPPORTED.  n_landmarks > 1024 returns EKF_ERR_UNSUPPORTED: one streamed filter per map. */
 int ekf_batch_create(int64_t n_filters, int n_landmarks, int device, ekf_batch** out);
 int ekf_batch_destroy(ekf_batch* b);
 int64_t ekf_batch_size(const ekf_batch* b);
+/* EKF_ENGINE_FUSED (Sigma on chip, n <= 64) or EKF_ENGINE_STREAM (Sigma in HBM, the wide engine); mirrors ekf_engine */
+int ekf_batch_engine(const ekf_batch* b);
+/* passes over a filter's Sigma in HBM so far, summed over the filters (0 for the on-chip engines); mirrors
+ * ekf_sweep_count.  A wide filter sweeps ceil(c / 14) times in a step with c corrections. */
+int ekf_batch_sweep_count(ekf_batch* b, uint64_t* out);
 
 /* One SLAM-node step for every filter: prediction(twist) then measurement(xy, visible)
  * (nuslam/src/slam.cpp:433-434).  HOST buffers: twists [B][2] = {dtheta, dx}, xy [B][2n], visible [B][n].
@@ -154,13 +164,14 @@ int ekf_batch_get_poses(ekf_batch* b, double* out /* [B][3] theta,x,y */);
 /* asynchronous read-back into pinned memory; complete after ekf_batch_sync() */
 int ekf_batch_get_poses_async(ekf_batch* b, double* pinned_out);
 int ekf_batch_get_states(ekf_batch* b, double* out /* [B][N] */);
-/* one filter's covariance as a dense row-major N x N matrix (expanded from the engine's symmetric storage) */
+/* one filter's covariance as a dense row-major N x N matrix (expanded from the on-chip engines' storage) */
 int ekf_batch_get_sigma(ekf_batch* b, int64_t filter, double* out, int64_t ld);
 int ekf_batch_get_known(ekf_batch* b, uint8_t* out /* [B][n] */);
 int ekf_batch_set_known(ekf_batch* b, const uint8_t* in);
 int ekf_batch_update_count(ekf_batch* b, uint64_t* out);
 /* Checkpoint / resume (the reference keeps the filter only in the node's memory, slam.cpp:427-430): the batch's arrays
- * exactly as the engine holds them — Sigma packed symmetric, sizes from ekf_batch_checkpoint_size — plus
+ * exactly as the engine holds them — Sigma in the layout of ekf_batch_device_pointers, sizes from
+ * ekf_batch_checkpoint_size — plus
  * landmark_init_flag [B], known_list [B][n] and the update counter.  A batch of the same shape restored with
  * ekf_batch_import continues bit-identically. */
 int ekf_batch_checkpoint_size(ekf_batch* b, int64_t* sigma_doubles, int64_t* state_doubles);
@@ -172,9 +183,13 @@ int ekf_batch_import(ekf_batch* b, const double* sigma, const double* state, con
 int ekf_batch_pose_error(ekf_batch* b, const double* truth, double* out4);
 int ekf_batch_sync(ekf_batch* b);
 /* Raw device arrays of the batch.  state: [B][state_stride] doubles (theta, x, y, m1x, m1y, ...).  sigma:
- * [B][sigma_stride] doubles in the engine's SYMMETRIC block-staircase layout: row r stores the columns
- * [16*floor(r/16), N) only, rows back to back (element (r, c) with c < 16*floor(r/16) is the stored (c, r)); use
- * ekf_batch_get_sigma() for a dense copy. */
+ * [B][sigma_stride] doubles in the engine's layout:
+ *   n == 20      the tile engine's register-fragment layout, with the state inside each filter's block;
+ *   n <= 64      the SYMMETRIC block-staircase layout: row r stores the columns [16*floor(r/16), N) only, rows back to
+ *                back (element (r, c) with c < 16*floor(r/16) is the stored (c, r));
+ *   64 < n       (wide engine) a dense row-major N x ld matrix, ld = N rounded up to a multiple of 16 doubles (the
+ *                streamed engine's layout; columns N..ld-1 are padding), sigma_stride = N * ld.
+ * ekf_batch_get_sigma() returns a dense copy of any of them. */
 int ekf_batch_device_pointers(ekf_batch* b, void** sigma, int64_t* sigma_stride, void** state,
                               int64_t* state_stride);
 void* ekf_batch_stream(ekf_batch* b);
