@@ -38,7 +38,8 @@ __device__ __forceinline__ void pdl_prologue() {
 
 // ---------------------------------------------------------------- prediction (ekf_slam.cpp:55-106)
 // One warp: lane 0 does the motion model, state[0..2], the 3x3 robot block of At*Sigma*At^T + Q, and (a1, a2) for the
-// strips; lane j < pending carries pending factor j across the prediction (see k_large_predict_factors below).
+// strips; lane j < pending carries pending factor j across the prediction (ekf_large_delayed.cuh).  The row-sharded
+// engine runs it on every rank: `sig` is then the rank's 3 x ld copy of rows 0..2, or its own rows on rank 0.
 __global__ void k_large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
                                double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
                                double2* __restrict__ Wp, int pending) {
@@ -126,23 +127,24 @@ __device__ __forceinline__ void assoc_merge(double& best, double& second, int& b
     }
 }
 
-__global__ void __launch_bounds__(256)
-    k_large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
-                  const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
-                  AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
-                  UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
-                  double* __restrict__ second_out, uint8_t* __restrict__ created_out) {
+// Distances to the landmarks [i_begin, i_end), grid-strided, then the minimum and runner-up over the grid: warp
+// shuffles, the CTA's warps, and the last CTA to finish merges the per-CTA partials in CTA order.  Returns true on
+// thread 0 of that last CTA only, with the grid's result in best / second / best_i.  Rows 0..2 of Sigma are read from
+// `robot`, rows 3+2i and 4+2i from `lm_rows`, which holds the global rows from r0 on.
+__device__ __forceinline__ bool assoc_scan(const double* __restrict__ robot, const double* __restrict__ lm_rows,
+                                           long long ld, long long r0, int i_begin, int i_end,
+                                           const double* __restrict__ state, double zr, double zphi, double theta,
+                                           double x, double y, AssocPartial* __restrict__ partials,
+                                           unsigned int* __restrict__ done_counter, double& best, double& second,
+                                           int& best_i) {
     __shared__ AssocPartial sh[8];
     __shared__ bool is_last;
-    const int known_count = *known_count_p;
-    const double sx = meas[2 * j], sy = meas[2 * j + 1];
-    double zr, zphi;
-    range_bearing(sx, sy, zr, zphi);
-    const double theta = state[0], x = state[1], y = state[2];
-    double best = INFINITY, second = INFINITY;
-    int best_i = 0x7fffffff;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < known_count; i += gridDim.x * blockDim.x) {
-        double d = maha_distance(sig, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, theta, x, y);
+    best = INFINITY;
+    second = INFINITY;
+    best_i = 0x7fffffff;
+    for (int i = i_begin + blockIdx.x * blockDim.x + threadIdx.x; i < i_end; i += gridDim.x * blockDim.x) {
+        const double* lm = lm_rows + ((3 + 2 * (long long)i) - r0) * ld;
+        double d = maha_distance_rows(robot, lm, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, theta, x, y);
         if (!(d == d)) d = INFINITY;
         if (d < best) {
             second = best;
@@ -170,7 +172,7 @@ __global__ void __launch_bounds__(256)
         is_last = (t == gridDim.x - 1);
     }
     __syncthreads();
-    if (!is_last || threadIdx.x != 0) return;
+    if (!is_last || threadIdx.x != 0) return false;
     __threadfence();
     best = INFINITY;
     second = INFINITY;
@@ -180,6 +182,18 @@ __global__ void __launch_bounds__(256)
         assoc_merge(best, second, best_i, pp->best, pp->second, pp->best_i);
     }
     *done_counter = 0;  // re-arm for the next measurement (stream-ordered)
+    return true;
+}
+
+// The decision for measurement j = (sx, sy) from the merged minimum (ekf_slam.cpp:293-330): a new landmark when no
+// known one is within kGateNew, an update when the distance is below kGateUpdate.  Writes the command block, the
+// new landmark's state and known count, and those of the four outputs that are not null.
+__device__ __forceinline__ void assoc_decide(double best, double second, int best_i, int known_count, int n, int j,
+                                             double sx, double sy, double theta, double x, double y,
+                                             double* __restrict__ state, int* __restrict__ known_count_p,
+                                             UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out,
+                                             double* __restrict__ dmin_out, double* __restrict__ second_out,
+                                             uint8_t* __restrict__ created_out) {
     double min_d = kGateNew;
     int min_idx = known_count;
     if (best < kGateNew) {
@@ -211,6 +225,26 @@ __global__ void __launch_bounds__(256)
     if (created_out) created_out[j] = (uint8_t)created;
 }
 
+__global__ void __launch_bounds__(256)
+    k_large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
+                  const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
+                  AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
+                  UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
+                  double* __restrict__ second_out, uint8_t* __restrict__ created_out) {
+    const int known_count = *known_count_p;
+    const double sx = meas[2 * j], sy = meas[2 * j + 1];
+    double zr, zphi;
+    range_bearing(sx, sy, zr, zphi);
+    const double theta = state[0], x = state[1], y = state[2];
+    double best, second;
+    int best_i;
+    if (!assoc_scan(sig, sig, ld, 0, 0, known_count, state, zr, zphi, theta, x, y, partials, done_counter, best,
+                    second, best_i))
+        return;
+    assoc_decide(best, second, best_i, known_count, n, j, sx, sy, theta, x, y, state, known_count_p, cmd, assoc_out,
+                 dmin_out, second_out, created_out);
+}
+
 // ---------------------------------------------------------------- 256-bit global accesses (LDG/STG.E.256 on sm_100a)
 __device__ __forceinline__ void ld256(const double* p, double& a, double& b, double& c, double& d) {
     asm volatile("ld.global.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a), "=d"(b), "=d"(c), "=d"(d) : "l"(p));
@@ -218,9 +252,6 @@ __device__ __forceinline__ void ld256(const double* p, double& a, double& b, dou
 __device__ __forceinline__ void st256(double* p, double a, double b, double c, double d) {
     asm volatile("st.global.v4.f64 [%0], {%1,%2,%3,%4};" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d) : "memory");
 }
-
-constexpr int kSweepThreads = 256;
-constexpr int kSweepRows = 32;
 
 // Sigma0 = blockdiag(0_3, 100 I) (ekf_slam.cpp:29-36) on an already-zeroed buffer.
 __global__ void k_large_init_sigma(double* __restrict__ sig, long long ld, int N) {

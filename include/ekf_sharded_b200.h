@@ -39,7 +39,9 @@ int ekf_sharded_destroy(ekf_sharded* h);
  * for partial W, stores, flags, gain and state update - waits on per-block flags instead of on an ncclAllReduce.  The caller allocates one symmetric, zero-filled buffer of
  * ekf_sharded_exchange_bytes() bytes per rank (e.g. torch.distributed._symmetric_memory, or cudaIpc) and passes every
  * rank's mapping of it (peer_bases[0..world-1]) and the multicast address (0 = none).  Collective; the buffers must
- * outlive the handle.  Results are identical to the all-reduce path. */
+ * outlive the handle.  Results are identical to the all-reduce path.  The correction kernel's CTAs wait for one another,
+ * so its whole grid (ld / 256 CTAs) has to be resident on the device at once: for larger maps (on a B200, from about
+ * n = 94,700 landmarks) the call returns an error, attaches nothing, and the handle keeps the all-reduce. */
 int ekf_sharded_exchange_bytes(ekf_sharded* h, uint64_t* bytes);
 int ekf_sharded_attach_exchange(ekf_sharded* h, int world, const uint64_t* peer_bases, uint64_t multicast_base);
 
