@@ -141,7 +141,9 @@ int ekf_batch_sweep_count(ekf_batch* b, uint64_t* out);
  * blocks, and the caller must leave them untouched until ekf_batch_sync() (cudaMemcpyAsync rules). */
 int ekf_batch_step_known(ekf_batch* b, const double* twists, const double* xy, const uint8_t* visible);
 /* prediction(twist) then data_association(measures) (nuslam/src/unknown_data_assoc.cpp:414-415).
- * meas [B][m_max][2], count [B] valid measurements per filter; assoc_out [B][m_max] host, optional. */
+ * meas [B][m_max][2], count [B] valid measurements per filter; assoc_out [B][m_max] host, optional.
+ * A count below 0 is an empty list (prediction only, that filter's outputs all -1), a count above m_max is m_max;
+ * assoc_out[b][j] = -1 for every j at or beyond filter b's count. */
 int ekf_batch_step_unknown(ekf_batch* b, const double* twists, const double* meas, const int32_t* count,
                            int m_max, int32_t* assoc_out);
 /* The same step fed with the fake_sensor message as it is on the wire: only the visible markers, each with its
@@ -153,7 +155,8 @@ int ekf_batch_step_unknown(ekf_batch* b, const double* twists, const double* mea
  * those dense arrays, with about a third of the host-to-device bytes. */
 int ekf_batch_step_known_sparse(ekf_batch* b, const double* twists, const int32_t* offsets, const uint8_t* ids,
                                 const double* xy, int64_t total);
-/* Same verbs with inputs already resident in HBM (device pointers, same layouts). */
+/* Same verbs with inputs already resident in HBM (device pointers, same layouts).  ekf_batch_step_unknown_dev clamps
+ * the counts as above; a null d_count means m_max measurements for every filter. */
 int ekf_batch_step_known_sparse_dev(ekf_batch* b, const double* d_twists, const int32_t* d_offsets, const uint8_t* d_ids,
                                     const double* d_xy, int64_t total);
 int ekf_batch_step_known_dev(ekf_batch* b, const double* d_twists, const double* d_xy, const uint8_t* d_visible);
