@@ -78,64 +78,35 @@ int max_smem_optin(int device) {
     return v;
 }
 
-// Launch the fused one-warp-per-filter kernel (n = 20 gets the fully unrolled instantiation).
-#ifndef EKF_DEBUG_EXTRA_SMEM
-#define EKF_DEBUG_EXTRA_SMEM 0  // occupancy experiments only
-#endif
-
-int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
-    FusedSmem L(p.n, p.m_max);
-    L.total += EKF_DEBUG_EXTRA_SMEM;
-    if (L.total > max_smem_optin(device))
-        return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for n=%d", L.total, p.n);
+// Launch one of the shared-memory kernels (ekf_fused_kernel, ekf_fused_sym_kernel): one single-warp CTA per filter
+// with `smem` bytes of shared memory.
+template <void (*Kernel)(FusedParams)>
+int launch_smem_kernel(int smem, const FusedParams& p, cudaStream_t stream, int device) {
+    if (smem > max_smem_optin(device))
+        return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for n=%d", smem, p.n);
     if (p.B <= 0) return EKF_OK;
     if (p.B > 0x7fffffffLL) return fail(EKF_ERR_INVALID, "batch too large for one launch");
-    static int set20[64] = {0}, set0[64] = {0};
-    if (p.n == 20) {
-        if (set20[device] < L.total) {
-            CU(cudaFuncSetAttribute(ekf_fused_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-            set20[device] = L.total;
-        }
-        ekf_fused_kernel<20><<<(unsigned)p.B, 32, L.total, stream>>>(p);
-    } else {
-        if (set0[device] < L.total) {
-            CU(cudaFuncSetAttribute(ekf_fused_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-            set0[device] = L.total;
-        }
-        ekf_fused_kernel<0><<<(unsigned)p.B, 32, L.total, stream>>>(p);
+    static int smem_set[64] = {0};  // per device: the largest shared-memory size this kernel is enabled for
+    if (smem_set[device] < smem) {
+        CU(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        CU(cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        smem_set[device] = smem;
     }
+    Kernel<<<(unsigned)p.B, 32, smem, stream>>>(p);
     CU(cudaGetLastError());
     return EKF_OK;
 }
 
-// Batched engine: symmetric staircase Sigma (ekf_fused_sym.cuh).
-int launch_fused_sym(const FusedParams& p, cudaStream_t stream, int device) {
-    SymSmem L(p.n, p.m_max);
-    if (L.total > max_smem_optin(device))
-        return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for n=%d", L.total, p.n);
-    if (p.B <= 0) return EKF_OK;
-    if (p.B > 0x7fffffffLL) return fail(EKF_ERR_INVALID, "batch too large for one launch");
-    L.total += EKF_DEBUG_EXTRA_SMEM;
-    static int set20[64] = {0}, set0[64] = {0};
-    if (p.n == 20) {
-        if (set20[device] < L.total) {
-            CU(cudaFuncSetAttribute(ekf_fused_sym_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-            CU(cudaFuncSetAttribute(ekf_fused_sym_kernel<20>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                    cudaSharedmemCarveoutMaxShared));
-            set20[device] = L.total;
-        }
-        ekf_fused_sym_kernel<20><<<(unsigned)p.B, 32, L.total, stream>>>(p);
-    } else {
-        if (set0[device] < L.total) {
-            CU(cudaFuncSetAttribute(ekf_fused_sym_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-            CU(cudaFuncSetAttribute(ekf_fused_sym_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                    cudaSharedmemCarveoutMaxShared));
-            set0[device] = L.total;
-        }
-        ekf_fused_sym_kernel<0><<<(unsigned)p.B, 32, L.total, stream>>>(p);
-    }
-    CU(cudaGetLastError());
-    return EKF_OK;
+// Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.
+int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
+    const int smem = FusedSmem(p.n, p.m_max).total;
+    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20>>(smem, p, stream, device)
+                     : launch_smem_kernel<ekf_fused_kernel<0>>(smem, p, stream, device);
+}
+
+// Batch with n <= 64, n != 20: symmetric staircase Sigma (ekf_fused_sym.cuh).
+int launch_fused_staircase(const FusedParams& p, cudaStream_t stream, int device) {
+    return launch_smem_kernel<ekf_fused_sym_kernel>(SymSmem(p.n, p.m_max).total, p, stream, device);
 }
 
 // Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh).
@@ -1348,7 +1319,7 @@ int ekf_batch_step_known_dev(ekf_batch* b, const double* d_twists, const double*
         return rc;
     }
     FusedParams p = batch_params(b, kDoPredict | kDoMeasurement, 1, d_twists, d_xy, d_visible, nullptr, nullptr);
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_sym(p, b->stream, b->device);
+    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
     b->launches += 1;
     return rc;
 }
@@ -1361,7 +1332,7 @@ int ekf_batch_step_unknown_dev(ekf_batch* b, const double* d_twists, const doubl
                     kFusedMaxN);
     DeviceGuard g(b->device);
     FusedParams p = batch_params(b, kDoPredict | kDoAssociation, m_max, d_twists, d_meas, nullptr, d_count, d_assoc_out);
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_sym(p, b->stream, b->device);
+    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
     b->launches += 1;
     return rc;
 }
@@ -1400,7 +1371,7 @@ int ekf_batch_step_known_sparse_dev(ekf_batch* b, const double* d_twists, const 
     FusedParams p = batch_params(b, kDoPredict | kDoMeasurement | kSparseReadings, 1, d_twists, d_xy, d_ids, d_offsets,
                                  nullptr);
     p.sparse_total = total;
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_sym(p, b->stream, b->device);
+    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
     b->launches += 1;
     return rc;
 }

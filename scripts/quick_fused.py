@@ -1,6 +1,9 @@
 """Development aid: time the batched fused step (cfg3 shape) and check a few filters against the oracle.
 
-    python scripts/quick_fused.py [--filters 65536] [--steps 10] [--warmup 3] [--unknown] [--check 8]
+    python scripts/quick_fused.py [--filters 65536] [--landmarks 20] [--steps 10] [--warmup 3] [--unknown] [--check 8]
+
+n = 20 runs the tile kernel on the cfg3 world (the shape bench.py times); any other n <= 64 runs the staircase kernel on
+a grid of n landmarks that are all in sight.
 
 Not part of the product or of bench.py; it exists so that a kernel change can be judged in one short GPU run.
 """
@@ -15,9 +18,20 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
 
 
+def world(tg, n):
+    if n == 20:
+        return tg.dense_world(n)
+    # dense_world's rejection sampling cannot place much more than 40 tubes
+    nx = int(np.ceil(np.sqrt(n)))
+    w = tg.grid_world(nx, -(-n // nx), pitch=0.3, n_slots=n, max_visible=3.0)
+    w.tubes_x, w.tubes_y = w.tubes_x[:n], w.tubes_y[:n]
+    return w
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--filters", type=int, default=65536)
+    ap.add_argument("--landmarks", type=int, default=20)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--check", type=int, default=8)
@@ -30,16 +44,16 @@ def main():
     from _oracle import OracleEKF, sigma_err, state_err
 
     tg = pkg.tracegen
-    B, n, T = a.filters, 20, a.steps + a.warmup
+    B, n, T = a.filters, a.landmarks, a.steps + a.warmup
     t0 = time.time()
     if a.unknown:
         M = 12
-        tr = tg.simulate_unknown(tg.dense_world(n), B, T, seed=4242, m_max=M)
+        tr = tg.simulate_unknown(world(tg, n), B, T, seed=4242, m_max=M)
         d_tw = torch.from_numpy(np.ascontiguousarray(tr["twists"])).cuda()
         d_me = torch.from_numpy(np.ascontiguousarray(tr["meas"])).cuda()
         d_ct = torch.from_numpy(np.ascontiguousarray(tr["count"])).cuda()
     else:
-        tr = tg.simulate_known(tg.dense_world(n), B, T + 1, seed=2026, workers=os.cpu_count())
+        tr = tg.simulate_known(world(tg, n), B, T + 1, seed=2026, workers=os.cpu_count())
         d_tw = torch.from_numpy(np.ascontiguousarray(tr["twists"])).cuda()
         d_xy = torch.from_numpy(np.ascontiguousarray(tr["xy"])).cuda()
         d_vis = torch.from_numpy(np.ascontiguousarray(tr["vis"])).cuda()

@@ -1,4 +1,4 @@
-"""The batch engine for maps of up to 64 landmarks other than n = 20: ekf_fused_sym_kernel<0>, which keeps each filter's
+"""The batch engine for maps of up to 64 landmarks other than n = 20: ekf_fused_sym_kernel, which keeps each filter's
 covariance in the packed symmetric staircase layout of csrc/ekf_fused_sym.cuh, against the CPU oracle.
 
 Its code depends on the size in ways the n = 20 tile kernel never sees: the staircase offsets where N = 3 + 2n crosses a
