@@ -88,6 +88,11 @@ SIGNATURES = {
     "ekf_batch_set_known": (ctypes.c_int, [ctypes.c_void_p, c_u8_p]),
     "ekf_batch_update_count": (ctypes.c_int, [ctypes.c_void_p, c_u64_p]),
     "ekf_batch_pose_error": (ctypes.c_int, [ctypes.c_void_p, c_double_p, c_double_p]),
+    "ekf_batch_get_marginals": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "ekf_batch_nees": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p,
+                                      ctypes.c_void_p]),
+    "ekf_batch_nees_dev": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
+                                          ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_batch_sync": (ctypes.c_int, [ctypes.c_void_p]),
     "ekf_batch_device_pointers": (ctypes.c_int, [ctypes.c_void_p, c_void_pp, c_i64_p, c_void_pp, c_i64_p]),
     "ekf_batch_stream": (ctypes.c_void_p, [ctypes.c_void_p]),

@@ -15,6 +15,7 @@
 #include "ekf_fused_sym.cuh"
 #include "ekf_fused_tile.cuh"
 #include "ekf_batch_wide.cuh"
+#include "ekf_batch_consistency.cuh"
 #include "ekf_large.cuh"
 #include "ekf_large_mma.cuh"
 
@@ -1074,6 +1075,16 @@ struct ekf_batch {
     double* d_poses = nullptr;
     double* d_acc4 = nullptr;
     double* d_truth = nullptr;
+    // consistency read-out (ekf_batch_consistency.cuh), allocated on first use
+    int cons_grid = 0;
+    double* d_cons_part = nullptr;      // [cons_grid][8] per-CTA partials
+    unsigned int* d_cons_done = nullptr;
+    double* d_marg_pose = nullptr;      // [B][6]
+    double* d_marg_lm = nullptr;        // [B][n][3]
+    double* d_nees_lm = nullptr;        // landmark truth of ekf_batch_nees, lm_cap doubles
+    long long lm_cap = 0;
+    double* d_nees_pf = nullptr;        // [B][3]
+    double* d_nees_out = nullptr;       // [8]
     cudaEvent_t t0 = nullptr, t1[3] = {nullptr, nullptr, nullptr};
 };
 
@@ -1104,6 +1115,13 @@ int free_batch(ekf_batch* b) {
     cudaFree(b->d_poses);
     cudaFree(b->d_acc4);
     cudaFree(b->d_truth);
+    cudaFree(b->d_cons_part);
+    cudaFree(b->d_cons_done);
+    cudaFree(b->d_marg_pose);
+    cudaFree(b->d_marg_lm);
+    cudaFree(b->d_nees_lm);
+    cudaFree(b->d_nees_pf);
+    cudaFree(b->d_nees_out);
     if (b->ev_step) cudaEventDestroy(b->ev_step);
     if (b->ev_out) cudaEventDestroy(b->ev_out);
     if (b->t0) cudaEventDestroy(b->t0);
@@ -1185,6 +1203,59 @@ int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint
 
 // The marker list carries uint8_t landmark ids.
 constexpr int kMarkerMaxN = 256;
+
+// One launch of k_batch_consistency on the compute stream, in the batch's Sigma layout.  The grid is what fits the
+// device at once (each warp walks filters w, w + warps, ...), fixed for the handle so that the reduction order is too.
+template <class At>
+int launch_consistency_at(ekf_batch* b, const ConsistencyParams& p, At at) {
+    if (!b->cons_grid) {
+        int sms = 0, per_sm = 0;
+        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_batch_consistency<At>, kConsWarps * 32, 0));
+        const long long resident = (long long)std::max(sms, 1) * std::max(per_sm, 1);
+        const int grid = (int)std::min<long long>((b->B + kConsWarps - 1) / kConsWarps, resident);
+        CU(cudaMalloc(&b->d_cons_part, sizeof(double) * 8 * (size_t)grid));
+        CU(cudaMalloc(&b->d_cons_done, sizeof(unsigned int)));
+        CU(cudaMemsetAsync(b->d_cons_done, 0, sizeof(unsigned int), b->stream));
+        b->cons_grid = grid;
+    }
+    ConsistencyParams q = p;
+    q.partials = b->d_cons_part;
+    q.done = b->d_cons_done;
+    k_batch_consistency<At><<<b->cons_grid, kConsWarps * 32, 0, b->stream>>>(q, at);
+    b->launches += 1;
+    CU(cudaGetLastError());
+    return EKF_OK;
+}
+
+int launch_consistency(ekf_batch* b, const double* truth, const double* lm_truth, long long lm_stride,
+                       double* per_filter, double* pose_cov, double* lm_cov, double* out8) {
+    ConsistencyParams p;
+    memset(&p, 0, sizeof(p));
+    p.state = b->d_state;
+    p.init_flag = b->d_init_flag;
+    p.known = b->d_known;
+    p.truth = truth;
+    p.lm_truth = lm_truth;
+    p.per_filter = per_filter;
+    p.pose_cov = pose_cov;
+    p.lm_cov = lm_cov;
+    p.out8 = out8;
+    p.B = b->B;
+    p.st_stride = b->st_stride;
+    p.lm_stride = lm_stride;
+    p.n = b->n;
+    if (b->wide) return launch_consistency_at(b, p, WideAt{b->d_sigma, b->sig_stride, b->ld});
+    if (b->tiled) return launch_consistency_at(b, p, TileAt{b->d_sigma});
+    return launch_consistency_at(b, p, StairAt{b->d_sigma, b->sig_stride, b->N});
+}
+
+int check_nees_args(ekf_batch* b, const double* truth, int64_t lm_truth_stride, const double* out8) {
+    if (!b || !truth || !out8) return fail(EKF_ERR_INVALID, "null argument");
+    if (lm_truth_stride != 0 && lm_truth_stride != 2LL * b->n)
+        return fail(EKF_ERR_INVALID, "lm_truth_stride must be 0 (shared landmark truth) or 2n = %d", 2 * b->n);
+    return EKF_OK;
+}
 
 }  // namespace
 
@@ -1572,6 +1643,57 @@ int ekf_batch_pose_error(ekf_batch* b, const double* truth, double* out4) {
     CU(cudaStreamSynchronize(b->stream));
     out4[3] = (double)b->B;
     return EKF_OK;
+}
+int ekf_batch_get_marginals(ekf_batch* b, double* pose_cov, double* lm_cov) {
+    if (!b) return fail(EKF_ERR_INVALID, "null handle");
+    if (!pose_cov && !lm_cov) return EKF_OK;
+    DeviceGuard g(b->device);
+    const size_t B = (size_t)b->B;
+    if (pose_cov && !b->d_marg_pose) CU(cudaMalloc(&b->d_marg_pose, sizeof(double) * 6 * B));
+    if (lm_cov && !b->d_marg_lm) CU(cudaMalloc(&b->d_marg_lm, sizeof(double) * 3 * (size_t)b->n * B));
+    int rc = launch_consistency(b, nullptr, nullptr, 0, nullptr, pose_cov ? b->d_marg_pose : nullptr,
+                                lm_cov ? b->d_marg_lm : nullptr, nullptr);
+    if (rc) return rc;
+    if (pose_cov) CU(cudaMemcpyAsync(pose_cov, b->d_marg_pose, sizeof(double) * 6 * B, cudaMemcpyDeviceToHost, b->stream));
+    if (lm_cov)
+        CU(cudaMemcpyAsync(lm_cov, b->d_marg_lm, sizeof(double) * 3 * (size_t)b->n * B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    return EKF_OK;
+}
+int ekf_batch_nees(ekf_batch* b, const double* truth, const double* lm_truth, int64_t lm_truth_stride, double* per_filter,
+                   double* out8) {
+    int rc = check_nees_args(b, truth, lm_truth_stride, out8);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    const size_t B = (size_t)b->B;
+    const long long lm_len = lm_truth ? 2LL * b->n * (lm_truth_stride ? b->B : 1) : 0;
+    if (lm_len > b->lm_cap) {
+        CU(cudaStreamSynchronize(b->stream));
+        cudaFree(b->d_nees_lm);
+        b->d_nees_lm = nullptr;
+        b->lm_cap = 0;
+        CU(cudaMalloc(&b->d_nees_lm, sizeof(double) * (size_t)lm_len));
+        b->lm_cap = lm_len;
+    }
+    if (per_filter && !b->d_nees_pf) CU(cudaMalloc(&b->d_nees_pf, sizeof(double) * 3 * B));
+    if (!b->d_nees_out) CU(cudaMalloc(&b->d_nees_out, sizeof(double) * 8));
+    CU(cudaMemcpyAsync(b->d_truth, truth, sizeof(double) * 3 * B, cudaMemcpyHostToDevice, b->stream));
+    if (lm_truth)
+        CU(cudaMemcpyAsync(b->d_nees_lm, lm_truth, sizeof(double) * (size_t)lm_len, cudaMemcpyHostToDevice, b->stream));
+    rc = launch_consistency(b, b->d_truth, lm_truth ? b->d_nees_lm : nullptr, lm_truth_stride,
+                            per_filter ? b->d_nees_pf : nullptr, nullptr, nullptr, b->d_nees_out);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out8, b->d_nees_out, sizeof(double) * 8, cudaMemcpyDeviceToHost, b->stream));
+    if (per_filter) CU(cudaMemcpyAsync(per_filter, b->d_nees_pf, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    return EKF_OK;
+}
+int ekf_batch_nees_dev(ekf_batch* b, const double* d_truth, const double* d_lm_truth, int64_t lm_truth_stride,
+                       double* d_per_filter, double* d_out8) {
+    int rc = check_nees_args(b, d_truth, lm_truth_stride, d_out8);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    return launch_consistency(b, d_truth, d_lm_truth, lm_truth_stride, d_per_filter, nullptr, nullptr, d_out8);
 }
 int ekf_batch_sync(ekf_batch* b) {
     if (!b) return fail(EKF_ERR_INVALID, "null handle");

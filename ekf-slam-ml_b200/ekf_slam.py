@@ -470,6 +470,57 @@ class EKFBatch:
         check(self._L.ekf_batch_pose_error(self._h, t.ctypes.data_as(c_double_p), out.ctypes.data_as(c_double_p)))
         return out
 
+    # --- consistency (no reference counterpart; read on the device, in the engine's layout)
+    def marginals(self):
+        """(pose [B,3,3] in state order theta, x, y; landmarks [B,n,2,2]), both symmetric: the stored entries of
+        sigma(b), bit for bit, without pulling whole covariances to the host."""
+        pc = np.empty((self.B, 6))
+        lc = np.empty((self.B, self.n, 3))
+        check(self._L.ekf_batch_get_marginals(self._h, pc.ctypes.data, lc.ctypes.data))
+        pose = pc[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(self.B, 3, 3)
+        lm = lc[:, :, [0, 1, 1, 2]].reshape(self.B, self.n, 2, 2)
+        return pose, lm
+
+    def _lm_stride(self, shape):
+        if shape == (self.n, 2):
+            return 0
+        if shape == (self.B, self.n, 2):
+            return 2 * self.n
+        raise ValueError(f"lm_truth must be [n,2] or [B,n,2], got {shape}")
+
+    def nees(self, truth_xyt, lm_truth=None, per_filter=False):
+        """Normalised estimation error squared of every filter against truth [B,3] = (x, y, theta) and, optionally,
+        landmark truth [n,2] (shared by every filter) or [B,n,2]; NaN entries are not scored.  A landmark slot is scored
+        once the filter has initialised it (first measurement(), or known[b, i] on the association path).  Returns
+        consistency.anees_from_stats() of the batch partial, the partial itself as "stats" (additive: multi-GPU runs
+        sum it with sharding.allreduce_sum), and with per_filter the arrays "pose_nees" [B] (NaN where not scored),
+        "landmark_nees_sum" [B] and "landmark_nees_count" [B]."""
+        from .consistency import anees_from_stats
+        t = np.ascontiguousarray(truth_xyt, dtype=np.float64)
+        if t.shape != (self.B, 3):
+            raise ValueError(f"truth must be [B,3], got {t.shape}")
+        lm = stride = None
+        if lm_truth is not None:
+            lm = np.ascontiguousarray(lm_truth, dtype=np.float64)
+            stride = self._lm_stride(lm.shape)
+        pf = np.empty((self.B, 3)) if per_filter else None
+        out = np.zeros(8)
+        check(self._L.ekf_batch_nees(self._h, t.ctypes.data, lm.ctypes.data if lm is not None else None, stride or 0,
+                                     pf.ctypes.data if per_filter else None, out.ctypes.data))
+        res = anees_from_stats(out)
+        res["stats"] = out
+        if per_filter:
+            res["pose_nees"], res["landmark_nees_sum"], res["landmark_nees_count"] = pf[:, 0], pf[:, 1], pf[:, 2]
+        return res
+
+    def nees_dev(self, d_truth, d_out8, d_lm_truth=None, lm_truth_stride=0, d_per_filter=None):
+        """ekf_batch_nees_dev: the same read-out from device pointers (truth [B][3], landmark truth [n][2] with stride 0
+        or [B][n][2] with stride 2n, per-filter [B][3], out8 [8]), enqueued on the batch's stream without a
+        synchronisation; the results are valid after sync()."""
+        check(self._L.ekf_batch_nees_dev(self._h, int(d_truth) if d_truth else None, int(d_lm_truth) if d_lm_truth else None,
+                                         int(lm_truth_stride), int(d_per_filter) if d_per_filter else None,
+                                         int(d_out8) if d_out8 else None))
+
     def sync(self):
         check(self._L.ekf_batch_sync(self._h))
 

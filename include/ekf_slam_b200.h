@@ -184,6 +184,30 @@ int ekf_batch_import(ekf_batch* b, const double* sigma, const double* state, con
 /* error statistics against ground-truth poses truth[B][3] = {x, y, theta}:
  * out4 = {sum dx^2, sum dy^2, sum wrap(dtheta)^2, B} — the per-GPU partial that ranks all-reduce. */
 int ekf_batch_pose_error(ekf_batch* b, const double* truth, double* out4);
+/* Consistency of the batch (no reference counterpart: the reference never scores its covariance).  One kernel reads
+ * each filter's stored Sigma entries in place, in any of the three layouts below, plus the state, landmark_init_flag and
+ * known_list; it writes nothing the filters own.  It is enqueued on ekf_batch_stream(), after any step already there.
+ *
+ * Marginals: pose_cov [B][6] = (00, 01, 02, 11, 12, 22) of Sigma[0:3, 0:3] (state order theta, x, y), lm_cov [B][n][3]
+ * = (xx, xy, yy) of each landmark slot's 2 x 2 block; either may be NULL.  Bit-identical to the same entries
+ * (row <= column) of ekf_batch_get_sigma(). */
+int ekf_batch_get_marginals(ekf_batch* b, double* pose_cov, double* lm_cov);
+/* Normalised estimation error squared against truth [B][3] = {x, y, theta} (the convention of ekf_batch_pose_error):
+ *   NEES_pose = e^T P^-1 e, e = (wrap(theta_hat - theta), x_hat - x, y_hat - y), P = Sigma[0:3, 0:3];
+ *   NEES_i    = the same with landmark slot i's 2 x 2 block and lm_truth.
+ * lm_truth is [n][2] shared by every filter (lm_truth_stride = 0) or [B][n][2] (lm_truth_stride = 2n); NULL scores no
+ * landmark.  Slot i of filter b is scored iff its truth is finite and (landmark_init_flag[b] != 0 or known_list[b][i]
+ * != 0).  A block whose Cholesky pivot is not positive and finite is singular: its NEES is NaN and it is counted apart.
+ * per_filter [B][3] = {NEES_pose, sum of NEES_i, number of NEES_i}, optional.
+ * out8 = {sum NEES_pose, sum NEES_pose^2, #pose, sum NEES_i, sum NEES_i^2, #landmarks, #singular pose, #singular
+ * landmark}: additive, so ranks all-reduce it like out4.  The reduction runs in a fixed order without floating-point
+ * atomics: two calls on the same state and device return bit-identical results.  HOST buffers; synchronises. */
+int ekf_batch_nees(ekf_batch* b, const double* truth, const double* lm_truth, int64_t lm_truth_stride,
+                   double* per_filter, double* out8);
+/* The same with DEVICE pointers (e.g. the truth of tubeworld_outputs()), enqueued on ekf_batch_stream() and not
+ * synchronised: the results are valid after ekf_batch_sync(), so a per-step series costs no host round trip. */
+int ekf_batch_nees_dev(ekf_batch* b, const double* d_truth, const double* d_lm_truth, int64_t lm_truth_stride,
+                       double* d_per_filter, double* d_out8);
 int ekf_batch_sync(ekf_batch* b);
 /* Raw device arrays of the batch.  state: [B][state_stride] doubles (theta, x, y, m1x, m1y, ...).  sigma:
  * [B][sigma_stride] doubles in the engine's layout:
