@@ -4,9 +4,9 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <vector>
 
@@ -18,60 +18,14 @@
 #include "ekf_batch_consistency.cuh"
 #include "ekf_large.cuh"
 #include "ekf_large_mma.cuh"
+#include "host_util.cuh"
 
 using namespace ekf;
 
 namespace {
 
-thread_local char g_err[512] = "";
-
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
-
-#define CU(expr)                                                                                         \
-    do {                                                                                                 \
-        cudaError_t e_ = (expr);                                                                         \
-        if (e_ != cudaSuccess) {                                                                         \
-            cudaGetLastError();                                                                          \
-            return fail((int)e_, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-        }                                                                                                \
-    } while (0)
-
-// Launch with the programmatic-stream-serialization attribute (see pdl_prologue in ekf_large.cuh): only for kernels
-// that start with pdl_prologue().
-template <class... KArgs, class... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 constexpr int kFusedMaxN = 64;  // landmarks; Sigma (131^2 fp64 = 137 KB) must fit shared memory
 constexpr int kRing = 8;
-
-struct DeviceGuard {
-    int prev = -1;
-    explicit DeviceGuard(int dev) {
-        cudaGetDevice(&prev);
-        if (prev != dev) cudaSetDevice(dev);
-    }
-    ~DeviceGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
 
 int max_smem_optin(int device) {
     int v = 0;
@@ -86,13 +40,7 @@ int launch_smem_kernel(int smem, const FusedParams& p, cudaStream_t stream, int 
     if (smem > max_smem_optin(device))
         return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for n=%d", smem, p.n);
     if (p.B <= 0) return EKF_OK;
-    if (p.B > 0x7fffffffLL) return fail(EKF_ERR_INVALID, "batch too large for one launch");
-    static int smem_set[64] = {0};  // per device: the largest shared-memory size this kernel is enabled for
-    if (smem_set[device] < smem) {
-        CU(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        CU(cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        smem_set[device] = smem;
-    }
+    CU(kernel_setup<Kernel>(device, 32, smem, true));
     Kernel<<<(unsigned)p.B, 32, smem, stream>>>(p);
     CU(cudaGetLastError());
     return EKF_OK;
@@ -111,53 +59,31 @@ int launch_fused_staircase(const FusedParams& p, cudaStream_t stream, int device
 }
 
 // Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh).
-int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device) {
-    const bool assoc = (p.mode & kDoAssociation) != 0;
-    const tile::TileSmem L(p.m_max, assoc);
+template <bool Assoc>
+int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
+    const tile::TileSmem L(p.m_max, Assoc);
     if (L.total > max_smem_optin(device))
         return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for m_max=%d", L.total, p.m_max);
     if (p.sig_stride != tile::kStride || p.st_stride != tile::kStride || p.n != tile::kNL ||
         p.state != p.sigma + tile::kStOff)
         return fail(EKF_ERR_STATE, "tile engine: unexpected batch layout");
     if (p.B <= 0) return EKF_OK;
-    if (p.B > 0x7fffffffLL) return fail(EKF_ERR_INVALID, "batch too large for one launch");
     // persistent warps: as many single-warp CTAs as fit the device at once, each walking filters b, b + grid, ...
-    static int sms[64] = {0}, per_sm[64][2] = {{0}}, smem_set[64][2] = {{0}};
-    const int v = assoc ? 1 : 0;
-    const void* fn = assoc ? (const void*)tile::ekf_fused_tile_kernel<true> : (const void*)tile::ekf_fused_tile_kernel<false>;
-    if (smem_set[device][v] < L.total) {
-        CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-        CU(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        if (!sms[device]) CU(cudaDeviceGetAttribute(&sms[device], cudaDevAttrMultiProcessorCount, device));
-        int nb = 0;
-        if (assoc)
-            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, tile::ekf_fused_tile_kernel<true>, 32, L.total));
-        else
-            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, tile::ekf_fused_tile_kernel<false>, 32, L.total));
-        per_sm[device][v] = nb > 0 ? nb : 1;
-        smem_set[device][v] = L.total;
-    }
-    const long long resident = (long long)sms[device] * per_sm[device][v];
-    const unsigned grid = (unsigned)std::min<long long>(p.B, resident);
-    if (assoc)
-        tile::ekf_fused_tile_kernel<true><<<grid, 32, L.total, stream>>>(p);
-    else
-        tile::ekf_fused_tile_kernel<false><<<grid, 32, L.total, stream>>>(p);
+    int per_sm = 0;
+    CU(kernel_setup<tile::ekf_fused_tile_kernel<Assoc>>(device, 32, L.total, true, &per_sm));
+    const long long resident = (long long)sm_count * std::max(per_sm, 1);
+    tile::ekf_fused_tile_kernel<Assoc><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
     CU(cudaGetLastError());
     return EKF_OK;
 }
 
-__global__ void k_fused_init(double* sigma, double* state, int32_t* init_flag, long long B, int N, int sig_stride,
-                             int st_stride) {
-    const long long b = blockIdx.x;
-    if (b >= B) return;
-    double* s = sigma + b * (long long)sig_stride;
-    for (int e = threadIdx.x; e < sig_stride; e += blockDim.x) {
-        const int r = e / N, c = e - r * N;
-        s[e] = (e < N * N && r == c && r >= 3) ? kSigma0 : 0.0;
-    }
-    for (int e = threadIdx.x; e < st_stride; e += blockDim.x) state[b * (long long)st_stride + e] = 0.0;
-    if (threadIdx.x == 0) init_flag[b] = 0;
+// Sigma0 = blockdiag(0_3, 100 I) (ekf_slam.cpp:29-36) for B filters of an already-zeroed buffer: dense rows of stride
+// ld, one filter every `stride` doubles.
+__global__ void k_init_sigma(double* __restrict__ sigma, long long B, int N, long long ld, long long stride) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= B * (N - 3)) return;
+    const long long b = e / (N - 3), k = 3 + e - b * (N - 3);
+    sigma[b * stride + k * ld + k] = kSigma0;
 }
 
 __global__ void k_maha_one(const double* sig, long long ld, const double* state, int i, double sx, double sy,
@@ -233,8 +159,6 @@ struct ekf_filter {
     int m_cap = 0;
     double* d_in = nullptr;       // xy (2n) or meas (2 m_cap)
     uint8_t* d_flags = nullptr;   // visible (n) / known (n)
-    int32_t* d_mcount = nullptr;
-    double* d_twist = nullptr;
     int32_t* d_assoc = nullptr;
     double* d_dmin = nullptr;
     double* d_second = nullptr;
@@ -290,8 +214,6 @@ int free_filter(ekf_filter* h) {
     cudaFree(h->d_nupd);
     cudaFree(h->d_in);
     cudaFree(h->d_flags);
-    cudaFree(h->d_mcount);
-    cudaFree(h->d_twist);
     cudaFree(h->d_assoc);
     cudaFree(h->d_dmin);
     cudaFree(h->d_second);
@@ -370,21 +292,13 @@ int ring_acquire(ekf_filter* h, unsigned char** slot, cudaEvent_t* ev) {
     return EKF_OK;
 }
 
+// The filter's own buffers; each verb points the inputs and outputs of its mode at its pinned slot.
 FusedParams fused_params(ekf_filter* h, int mode, int m_max) {
     FusedParams p;
     memset(&p, 0, sizeof(p));
     p.sigma = h->d_sigma;
     p.state = h->d_state;
     p.init_flag = h->d_init_flag;
-    p.known = h->d_flags;
-    p.twists = h->d_twist;
-    p.xy = h->d_in;
-    p.vis = h->d_flags;
-    p.mcount = h->d_mcount;
-    p.assoc_out = h->d_assoc;
-    p.dmin_out = h->d_dmin;
-    p.second_out = h->d_second;
-    p.created_out = h->d_created;
     p.n_updates = h->d_nupd;
     p.pose_out = h->h_pose;
     p.B = 1;
@@ -452,6 +366,57 @@ int stream_settle(ekf_filter* h) {
     return stream_flush(h, h->pending, nullptr);
 }
 
+// Buffers and initial state (Sigma0, zero state) of a new filter; on failure the caller frees the half-made handle.
+int alloc_filter(ekf_filter* h) {
+    const int n = h->n;
+    CU(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
+    for (int i = 0; i < kRing; ++i) CU(cudaEventCreateWithFlags(&h->ring_ev[i], cudaEventDisableTiming));
+    h->st_stride = fused_round16(h->N);
+    if (h->engine == EKF_ENGINE_FUSED) {
+        h->ld = h->N;
+        h->sig_elems = fused_round16(h->N * h->N);
+    } else {
+        h->ld = fused_round16(h->N);
+        h->sig_elems = (long long)h->N * h->ld;
+    }
+    CU(cudaMalloc(&h->d_sigma, sizeof(double) * (size_t)h->sig_elems));
+    CU(cudaMalloc(&h->d_state, sizeof(double) * h->st_stride));
+    CU(cudaMalloc(&h->d_init_flag, sizeof(int32_t)));
+    CU(cudaMalloc(&h->d_nupd, sizeof(unsigned long long)));
+    CU(cudaMalloc(&h->d_flags, (size_t)n + 16));
+    CU(cudaMalloc(&h->d_scalar, sizeof(double)));
+    CU(cudaMemsetAsync(h->d_nupd, 0, sizeof(unsigned long long), h->stream));
+    CU(cudaMemsetAsync(h->d_sigma, 0, sizeof(double) * (size_t)h->sig_elems, h->stream));
+    CU(cudaMemsetAsync(h->d_state, 0, sizeof(double) * h->st_stride, h->stream));
+    CU(cudaMemsetAsync(h->d_init_flag, 0, sizeof(int32_t), h->stream));
+    k_init_sigma<<<(h->N - 3 + 255) / 256, 256, 0, h->stream>>>(h->d_sigma, 1, h->N, h->ld, h->sig_elems);
+    h->launches += 1;
+    CU(cudaGetLastError());
+    if (h->engine == EKF_ENGINE_FUSED) {
+        CU(cudaMallocHost((void**)&h->h_pose, 64));
+    } else {
+        CU(cudaMalloc(&h->d_K2, sizeof(double2) * ((size_t)h->ld * kMaxPending + 16)));
+        CU(cudaMalloc(&h->d_W2, sizeof(double2) * ((size_t)h->ld * kMaxPending + 16)));
+        CU(cudaMalloc(&h->d_state_alt, sizeof(double) * h->st_stride));
+        CU(cudaMemsetAsync(h->d_state_alt, 0, sizeof(double) * h->st_stride, h->stream));
+        CU(cudaMalloc(&h->d_motion, 2 * sizeof(double)));
+        CU(cudaMalloc(&h->d_pose0, 3 * sizeof(double)));
+        CU(cudaMalloc(&h->d_cmd, sizeof(UpdateCmd)));
+        h->assoc_blocks = std::max(1, std::min((n + 255) / 256, 1024));
+        CU(cudaMalloc(&h->d_partials, sizeof(AssocPartial) * h->assoc_blocks));
+        CU(cudaMalloc(&h->d_done, sizeof(unsigned int)));
+        CU(cudaMalloc(&h->d_known_count, sizeof(int)));
+        CU(cudaMemsetAsync(h->d_done, 0, sizeof(unsigned int), h->stream));
+        CU(cudaMemsetAsync(h->d_cmd, 0, sizeof(UpdateCmd), h->stream));
+        CU(cudaMemsetAsync(h->d_K2, 0, sizeof(double2) * (size_t)h->ld * kMaxPending, h->stream));
+        CU(cudaMemsetAsync(h->d_W2, 0, sizeof(double2) * (size_t)h->ld * kMaxPending, h->stream));
+    }
+    int rc = ensure_m_cap(h, std::max(n, 32));
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(h->stream));
+    return EKF_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -486,10 +451,8 @@ int ekf_create_ex(int n, int device, int engine, ekf_filter** out) {
     if (!out) return fail(EKF_ERR_INVALID, "null out pointer");
     *out = nullptr;
     if (n <= 0 || n > 500000) return fail(EKF_ERR_INVALID, "n_landmarks=%d out of range", n);
-    int count = 0;
-    int rc = ekf_device_count(&count);
+    int rc = check_device(device);
     if (rc) return rc;
-    if (device < 0 || device >= count) return fail(EKF_ERR_INVALID, "device %d not available (%d visible)", device, count);
     if (engine == EKF_ENGINE_AUTO) engine = (n <= kFusedMaxN) ? EKF_ENGINE_FUSED : EKF_ENGINE_STREAM;
     if (engine != EKF_ENGINE_FUSED && engine != EKF_ENGINE_STREAM) return fail(EKF_ERR_INVALID, "unknown engine %d", engine);
     if (engine == EKF_ENGINE_FUSED && n > kFusedMaxN)
@@ -502,69 +465,11 @@ int ekf_create_ex(int n, int device, int engine, ekf_filter** out) {
     h->device = device;
     h->engine = engine;
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
-#define CUH(expr)                          \
-    do {                                   \
-        cudaError_t e_ = (expr);           \
-        if (e_ != cudaSuccess) {           \
-            cudaGetLastError();            \
-            int code_ = fail((int)e_, "%s failed: %s", #expr, cudaGetErrorString(e_)); \
-            free_filter(h);                \
-            return code_;                  \
-        }                                  \
-    } while (0)
-    CUH(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-    for (int i = 0; i < kRing; ++i) CUH(cudaEventCreateWithFlags(&h->ring_ev[i], cudaEventDisableTiming));
-    h->st_stride = fused_round16(h->N);
-    if (engine == EKF_ENGINE_FUSED) {
-        h->ld = h->N;
-        h->sig_elems = fused_round16(h->N * h->N);
-    } else {
-        h->ld = fused_round16(h->N);
-        h->sig_elems = (long long)h->N * h->ld;
-    }
-    CUH(cudaMalloc(&h->d_sigma, sizeof(double) * (size_t)h->sig_elems));
-    CUH(cudaMalloc(&h->d_state, sizeof(double) * h->st_stride));
-    CUH(cudaMalloc(&h->d_init_flag, sizeof(int32_t)));
-    CUH(cudaMalloc(&h->d_nupd, sizeof(unsigned long long)));
-    CUH(cudaMalloc(&h->d_flags, (size_t)n + 16));
-    CUH(cudaMalloc(&h->d_mcount, sizeof(int32_t)));
-    CUH(cudaMalloc(&h->d_twist, 2 * sizeof(double)));
-    CUH(cudaMalloc(&h->d_scalar, sizeof(double)));
-    CUH(cudaMemsetAsync(h->d_nupd, 0, sizeof(unsigned long long), h->stream));
-    if (engine == EKF_ENGINE_FUSED) {
-        CUH(cudaMallocHost((void**)&h->h_pose, 64));
-        k_fused_init<<<1, 256, 0, h->stream>>>(h->d_sigma, h->d_state, h->d_init_flag, 1, h->N, (int)h->sig_elems,
-                                                h->st_stride);
-    } else {
-        CUH(cudaMemsetAsync(h->d_sigma, 0, sizeof(double) * (size_t)h->sig_elems, h->stream));
-        CUH(cudaMemsetAsync(h->d_state, 0, sizeof(double) * h->st_stride, h->stream));
-        CUH(cudaMemsetAsync(h->d_init_flag, 0, sizeof(int32_t), h->stream));
-        k_large_init_sigma<<<(h->N + 255) / 256, 256, 0, h->stream>>>(h->d_sigma, h->ld, h->N);
-        CUH(cudaMalloc(&h->d_K2, sizeof(double2) * ((size_t)h->ld * kMaxPending + 16)));
-        CUH(cudaMalloc(&h->d_W2, sizeof(double2) * ((size_t)h->ld * kMaxPending + 16)));
-        CUH(cudaMalloc(&h->d_state_alt, sizeof(double) * h->st_stride));
-        CUH(cudaMemsetAsync(h->d_state_alt, 0, sizeof(double) * h->st_stride, h->stream));
-        CUH(cudaMalloc(&h->d_motion, 2 * sizeof(double)));
-        CUH(cudaMalloc(&h->d_pose0, 3 * sizeof(double)));
-        CUH(cudaMalloc(&h->d_cmd, sizeof(UpdateCmd)));
-        h->assoc_blocks = std::max(1, std::min((n + 255) / 256, 1024));
-        CUH(cudaMalloc(&h->d_partials, sizeof(AssocPartial) * h->assoc_blocks));
-        CUH(cudaMalloc(&h->d_done, sizeof(unsigned int)));
-        CUH(cudaMalloc(&h->d_known_count, sizeof(int)));
-        CUH(cudaMemsetAsync(h->d_done, 0, sizeof(unsigned int), h->stream));
-        CUH(cudaMemsetAsync(h->d_cmd, 0, sizeof(UpdateCmd), h->stream));
-        CUH(cudaMemsetAsync(h->d_K2, 0, sizeof(double2) * (size_t)h->ld * kMaxPending, h->stream));
-        CUH(cudaMemsetAsync(h->d_W2, 0, sizeof(double2) * (size_t)h->ld * kMaxPending, h->stream));
-    }
-    h->launches += 1;
-    CUH(cudaGetLastError());
-    rc = ensure_m_cap(h, std::max(n, 32));
+    rc = alloc_filter(h);
     if (rc) {
         free_filter(h);
         return rc;
     }
-    CUH(cudaStreamSynchronize(h->stream));
-#undef CUH
     *out = h;
     return EKF_OK;
 }
@@ -1039,12 +944,16 @@ int ekf_timer_stop(ekf_filter* h, float* ms_out) {
 }  // extern "C"
 
 // ======================================================================================= batch
+// Sigma layout of a batch: register tile (n = 20, ekf_fused_tile.cuh), symmetric staircase (other n <= 64,
+// ekf_fused_sym.cuh), or dense N x ld rows per filter in HBM (64 < n <= 1,024, ekf_batch_wide.cuh).
+enum class Layout { Tile, Stair, Wide };
+
 struct ekf_batch {
     long long B = 0;
-    int n = 0, N = 0, device = 0;
-    int sig_stride = 0, st_stride = 0;
-    bool tiled = false;  // n == 20: register-resident tile layout (ekf_fused_tile.cuh); else symmetric staircase
-    bool wide = false;   // n > kFusedMaxN: dense N x ld Sigma per filter in HBM (ekf_batch_wide.cuh)
+    int n = 0, N = 0, device = 0, sm_count = 0;
+    Layout layout = Layout::Stair;
+    int sig_stride = 0, st_stride = 0;  // doubles per filter in d_sigma and d_state
+    int st_len = 0;      // doubles per filter in the state array of a checkpoint
     long long ld = 0;    // wide: row stride of a filter's Sigma
     int grid = 0;        // wide: CTAs of the step kernel (each owns a set of factor slots)
     cudaStream_t stream = nullptr;       // compute
@@ -1096,7 +1005,7 @@ int free_batch(ekf_batch* b) {
     cudaDeviceSynchronize();
     cudaFree(b->d_sigma);
     cudaFree(b->d_dense);
-    if (!b->tiled) cudaFree(b->d_state);  // tiled: the state lives inside the filter's block of d_sigma
+    if (b->layout != Layout::Tile) cudaFree(b->d_state);  // tile: the state lives inside the filter's block of d_sigma
     cudaFree(b->d_init_flag);
     cudaFree(b->d_known);
     cudaFree(b->d_nupd);
@@ -1151,27 +1060,87 @@ int batch_ensure_xy(ekf_batch* b, int m_max) {
     return EKF_OK;
 }
 
-FusedParams batch_params(ekf_batch* b, int mode, int m_max, const double* tw, const double* xy, const uint8_t* vis,
-                         const int32_t* cnt, int32_t* assoc) {
-    FusedParams p;
-    memset(&p, 0, sizeof(p));
-    p.sigma = b->d_sigma;
-    p.state = b->d_state;
-    p.init_flag = b->d_init_flag;
-    p.known = b->d_known;
-    p.twists = tw;
-    p.xy = xy;
-    p.vis = vis;
-    p.mcount = cnt;
-    p.assoc_out = assoc;
-    p.n_updates = b->d_nupd;
-    p.B = b->B;
-    p.n = b->n;
-    p.m_max = m_max;
-    p.mode = mode;
-    p.sig_stride = b->sig_stride;
-    p.st_stride = b->st_stride;
-    return p;
+// Layout and strides of a batch of n-landmark filters.
+void batch_geometry(ekf_batch* b) {
+    if (b->n == tile::kNL) {
+        // one block per filter holds Sigma (fragment layout) and the state, so that one bulk copy stages it; a
+        // checkpoint keeps the state as its own compact array as well
+        b->layout = Layout::Tile;
+        b->sig_stride = b->st_stride = tile::kStride;
+        b->st_len = tile::kStLen;
+    } else if (b->n <= kFusedMaxN) {
+        b->layout = Layout::Stair;
+        b->sig_stride = sym_sig_stride(b->N);
+        b->st_stride = b->st_len = sym_st_stride(b->N);
+    } else {  // the streamed engine's layout: row-major N x ld, ld = N rounded up to 16 doubles
+        b->layout = Layout::Wide;
+        b->ld = fused_round16(b->N);
+        b->sig_stride = b->N * (int)b->ld;
+        b->st_stride = b->st_len = (int)b->ld;
+    }
+}
+
+// Buffers and initial state of a new batch; on failure the caller frees the half-made handle.
+int alloc_batch(ekf_batch* b) {
+    const long long B = b->B;
+    const int n = b->n;
+    CU(cudaDeviceGetAttribute(&b->sm_count, cudaDevAttrMultiProcessorCount, b->device));
+    CU(cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&b->out_stream, cudaStreamNonBlocking));
+    CU(cudaMalloc(&b->d_sigma, sizeof(double) * (size_t)b->sig_stride * B));
+    if (b->layout == Layout::Tile)
+        b->d_state = b->d_sigma + tile::kStOff;
+    else
+        CU(cudaMalloc(&b->d_state, sizeof(double) * (size_t)b->st_stride * B));
+    CU(cudaMalloc(&b->d_init_flag, sizeof(int32_t) * (size_t)B));
+    CU(cudaMalloc(&b->d_known, (size_t)n * B));
+    CU(cudaMalloc(&b->d_nupd, sizeof(unsigned long long)));
+    CU(cudaMalloc(&b->d_poses, sizeof(double) * 3 * (size_t)B));
+    CU(cudaMalloc(&b->d_acc4, sizeof(double) * 4));
+    CU(cudaMalloc(&b->d_truth, sizeof(double) * 3 * (size_t)B));
+    for (int s = 0; s < 2; ++s) {
+        CU(cudaMalloc(&b->d_twists[s], sizeof(double) * 2 * (size_t)B));
+        CU(cudaMalloc(&b->d_vis[s], (size_t)n * B));
+        CU(cudaMalloc(&b->d_count[s], sizeof(int32_t) * ((size_t)B + 1)));
+        CU(cudaEventCreateWithFlags(&b->ev_copied[s], cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&b->ev_consumed[s], cudaEventDisableTiming));
+    }
+    CU(cudaEventCreateWithFlags(&b->ev_step, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&b->ev_out, cudaEventDisableTiming));
+    CU(cudaMemsetAsync(b->d_known, 0, (size_t)n * B, b->stream));
+    CU(cudaMemsetAsync(b->d_nupd, 0, sizeof(unsigned long long), b->stream));
+    switch (b->layout) {
+        case Layout::Tile:
+            tile::k_fused_tile_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_init_flag, B);
+            break;
+        case Layout::Stair:
+            k_fused_sym_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_state, b->d_init_flag, B, b->N,
+                                                                 b->sig_stride, b->st_stride);
+            break;
+        case Layout::Wide: {
+            b->grid = (int)std::min<long long>(B, std::max(b->sm_count, 1));
+            const size_t slots = (size_t)b->grid * ((size_t)kWidePending * b->ld + 16);
+            CU(cudaMalloc(&b->d_wK, sizeof(double2) * slots));
+            CU(cudaMalloc(&b->d_wW, sizeof(double2) * slots));
+            CU(cudaMalloc(&b->d_sweeps, sizeof(unsigned long long)));
+            CU(cudaMemsetAsync(b->d_wK, 0, sizeof(double2) * slots, b->stream));
+            CU(cudaMemsetAsync(b->d_wW, 0, sizeof(double2) * slots, b->stream));
+            CU(cudaMemsetAsync(b->d_sweeps, 0, sizeof(unsigned long long), b->stream));
+            CU(cudaMemsetAsync(b->d_sigma, 0, sizeof(double) * (size_t)b->sig_stride * B, b->stream));
+            CU(cudaMemsetAsync(b->d_state, 0, sizeof(double) * (size_t)b->st_stride * B, b->stream));
+            CU(cudaMemsetAsync(b->d_init_flag, 0, sizeof(int32_t) * (size_t)B, b->stream));
+            const long long diag = B * (b->N - 3);
+            k_init_sigma<<<(unsigned)((diag + 255) / 256), 256, 0, b->stream>>>(b->d_sigma, B, b->N, b->ld, b->sig_stride);
+            break;
+        }
+    }
+    b->launches += 1;
+    CU(cudaGetLastError());
+    int rc = batch_ensure_xy(b, n);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(b->stream));
+    return EKF_OK;
 }
 
 // One step of a wide batch: dense readings (offsets == nullptr) or the marker list.
@@ -1197,7 +1166,74 @@ int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint
     p.n = b->n;
     p.N = b->N;
     p.st_stride = b->st_stride;
-    CU(launch_wide_step(p, b->grid, b->stream));
+    CU(launch_wide_step(p, b->grid, b->stream, b->device));
+    return EKF_OK;
+}
+
+// One step of the whole batch in the kernel of its layout, counted as one launch.  `mode` as in FusedParams; `vis`
+// holds the visible flags, or the marker ids with kSparseReadings; `cnt` the marker list's CSR offsets, or the
+// per-filter measurement counts of unknown association.
+int batch_launch(ekf_batch* b, int mode, int m_max, const double* tw, const double* xy, const uint8_t* vis,
+                 const int32_t* cnt, int32_t* assoc, long long total) {
+    const bool association = (mode & kDoAssociation) != 0;
+    int rc;
+    if (b->layout == Layout::Wide) {
+        if (association)
+            return fail(EKF_ERR_UNSUPPORTED,
+                        "unknown data association is not available for batches with n > %d landmarks", kFusedMaxN);
+        rc = launch_wide(b, tw, xy, vis, cnt, total);
+    } else {
+        FusedParams p;
+        memset(&p, 0, sizeof(p));
+        p.sigma = b->d_sigma;
+        p.state = b->d_state;
+        p.init_flag = b->d_init_flag;
+        p.known = b->d_known;
+        p.twists = tw;
+        p.xy = xy;
+        p.vis = vis;
+        p.mcount = cnt;
+        p.assoc_out = assoc;
+        p.n_updates = b->d_nupd;
+        p.B = b->B;
+        p.n = b->n;
+        p.m_max = m_max;
+        p.mode = mode;
+        p.sig_stride = b->sig_stride;
+        p.st_stride = b->st_stride;
+        p.sparse_total = total;
+        if (b->layout == Layout::Stair)
+            rc = launch_fused_staircase(p, b->stream, b->device);
+        else if (association)
+            rc = launch_fused_tile<true>(p, b->stream, b->device, b->sm_count);
+        else
+            rc = launch_fused_tile<false>(p, b->stream, b->device, b->sm_count);
+    }
+    b->launches += 1;
+    return rc;
+}
+
+struct HostCopy {
+    void* dst;
+    const void* src;
+    size_t bytes;  // 0: skipped
+};
+
+// A step fed from host memory through the double-buffered device inputs: `copies` fill input slot b->slot on the copy
+// stream once the step that last read that slot has finished, and step() is enqueued on the compute stream behind
+// them.  The next host-fed step uses the other slot.
+template <class Step>
+int batch_host_step(ekf_batch* b, std::initializer_list<HostCopy> copies, Step step) {
+    const int s = b->slot;
+    b->slot ^= 1;
+    CU(cudaStreamWaitEvent(b->copy_stream, b->ev_consumed[s], 0));
+    for (const HostCopy& c : copies)
+        if (c.bytes) CU(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyHostToDevice, b->copy_stream));
+    CU(cudaEventRecord(b->ev_copied[s], b->copy_stream));
+    CU(cudaStreamWaitEvent(b->stream, b->ev_copied[s], 0));
+    const int rc = step();
+    if (rc) return rc;
+    CU(cudaEventRecord(b->ev_consumed[s], b->stream));
     return EKF_OK;
 }
 
@@ -1209,10 +1245,9 @@ constexpr int kMarkerMaxN = 256;
 template <class At>
 int launch_consistency_at(ekf_batch* b, const ConsistencyParams& p, At at) {
     if (!b->cons_grid) {
-        int sms = 0, per_sm = 0;
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, b->device));
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_batch_consistency<At>, kConsWarps * 32, 0));
-        const long long resident = (long long)std::max(sms, 1) * std::max(per_sm, 1);
+        int per_sm = 0;
+        CU(kernel_setup<k_batch_consistency<At>>(b->device, kConsWarps * 32, 0, false, &per_sm));
+        const long long resident = (long long)std::max(b->sm_count, 1) * std::max(per_sm, 1);
         const int grid = (int)std::min<long long>((b->B + kConsWarps - 1) / kConsWarps, resident);
         CU(cudaMalloc(&b->d_cons_part, sizeof(double) * 8 * (size_t)grid));
         CU(cudaMalloc(&b->d_cons_done, sizeof(unsigned int)));
@@ -1245,8 +1280,8 @@ int launch_consistency(ekf_batch* b, const double* truth, const double* lm_truth
     p.st_stride = b->st_stride;
     p.lm_stride = lm_stride;
     p.n = b->n;
-    if (b->wide) return launch_consistency_at(b, p, WideAt{b->d_sigma, b->sig_stride, b->ld});
-    if (b->tiled) return launch_consistency_at(b, p, TileAt{b->d_sigma});
+    if (b->layout == Layout::Wide) return launch_consistency_at(b, p, WideAt{b->d_sigma, b->sig_stride, b->ld});
+    if (b->layout == Layout::Tile) return launch_consistency_at(b, p, TileAt{b->d_sigma});
     return launch_consistency_at(b, p, StairAt{b->d_sigma, b->sig_stride, b->N});
 }
 
@@ -1265,15 +1300,14 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
     if (!out) return fail(EKF_ERR_INVALID, "null out pointer");
     *out = nullptr;
     if (B <= 0 || n <= 0) return fail(EKF_ERR_INVALID, "invalid batch shape");
+    if (B > 0x7fffffffLL) return fail(EKF_ERR_INVALID, "batch too large");
     if (n > kWideMaxN)
         return fail(EKF_ERR_UNSUPPORTED,
                     "batched filters support n <= %d landmarks; for a larger map use one streamed filter per map, "
                     "ekf_create_ex(n, device, EKF_ENGINE_STREAM, &h)",
                     kWideMaxN);
-    int count = 0;
-    int rc = ekf_device_count(&count);
+    int rc = check_device(device);
     if (rc) return rc;
-    if (device < 0 || device >= count) return fail(EKF_ERR_INVALID, "device %d not available (%d visible)", device, count);
     DeviceGuard g(device);
     ekf_batch* b = new (std::nothrow) ekf_batch();
     if (!b) return fail(EKF_ERR_STATE, "out of host memory");
@@ -1281,97 +1315,25 @@ int ekf_batch_create(int64_t B, int n, int device, ekf_batch** out) {
     b->n = n;
     b->N = 3 + 2 * n;
     b->device = device;
-    b->tiled = (n == tile::kNL);
-    b->wide = n > kFusedMaxN;
-    if (b->wide) {  // the streamed engine's layout: row-major N x ld, ld = N rounded up to 16 doubles
-        b->ld = fused_round16(b->N);
-        b->sig_stride = b->N * (int)b->ld;
-        b->st_stride = fused_round16(b->N);
-    } else {
-        // tiled: one block per filter holds Sigma (fragment layout) and the state, so that one bulk copy stages it
-        b->sig_stride = b->tiled ? tile::kStride : sym_sig_stride(b->N);
-        b->st_stride = b->tiled ? tile::kStride : sym_st_stride(b->N);
-    }
-#define CUB(expr)                          \
-    do {                                   \
-        cudaError_t e_ = (expr);           \
-        if (e_ != cudaSuccess) {           \
-            cudaGetLastError();            \
-            int code_ = fail((int)e_, "%s failed: %s", #expr, cudaGetErrorString(e_)); \
-            free_batch(b);                 \
-            return code_;                  \
-        }                                  \
-    } while (0)
-    CUB(cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking));
-    CUB(cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking));
-    CUB(cudaStreamCreateWithFlags(&b->out_stream, cudaStreamNonBlocking));
-    CUB(cudaMalloc(&b->d_sigma, sizeof(double) * (size_t)b->sig_stride * B));
-    if (b->tiled)
-        b->d_state = b->d_sigma + tile::kStOff;
-    else
-        CUB(cudaMalloc(&b->d_state, sizeof(double) * (size_t)b->st_stride * B));
-    CUB(cudaMalloc(&b->d_init_flag, sizeof(int32_t) * (size_t)B));
-    CUB(cudaMalloc(&b->d_known, (size_t)n * B));
-    CUB(cudaMalloc(&b->d_nupd, sizeof(unsigned long long)));
-    CUB(cudaMalloc(&b->d_poses, sizeof(double) * 3 * (size_t)B));
-    CUB(cudaMalloc(&b->d_acc4, sizeof(double) * 4));
-    CUB(cudaMalloc(&b->d_truth, sizeof(double) * 3 * (size_t)B));
-    for (int s = 0; s < 2; ++s) {
-        CUB(cudaMalloc(&b->d_twists[s], sizeof(double) * 2 * (size_t)B));
-        CUB(cudaMalloc(&b->d_vis[s], (size_t)n * B));
-        CUB(cudaMalloc(&b->d_count[s], sizeof(int32_t) * ((size_t)B + 1)));
-        CUB(cudaEventCreateWithFlags(&b->ev_copied[s], cudaEventDisableTiming));
-        CUB(cudaEventCreateWithFlags(&b->ev_consumed[s], cudaEventDisableTiming));
-    }
-    CUB(cudaEventCreateWithFlags(&b->ev_step, cudaEventDisableTiming));
-    CUB(cudaEventCreateWithFlags(&b->ev_out, cudaEventDisableTiming));
-    CUB(cudaMemsetAsync(b->d_known, 0, (size_t)n * B, b->stream));
-    CUB(cudaMemsetAsync(b->d_nupd, 0, sizeof(unsigned long long), b->stream));
-    if (B > 0x7fffffffLL) {
-        free_batch(b);
-        return fail(EKF_ERR_INVALID, "batch too large");
-    }
-    if (b->wide) {
-        int sms = 0;
-        CUB(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-        b->grid = (int)std::min<long long>(B, std::max(sms, 1));
-        const size_t slots = (size_t)b->grid * ((size_t)kWidePending * b->ld + 16);
-        CUB(cudaMalloc(&b->d_wK, sizeof(double2) * slots));
-        CUB(cudaMalloc(&b->d_wW, sizeof(double2) * slots));
-        CUB(cudaMalloc(&b->d_sweeps, sizeof(unsigned long long)));
-        CUB(cudaMemsetAsync(b->d_wK, 0, sizeof(double2) * slots, b->stream));
-        CUB(cudaMemsetAsync(b->d_wW, 0, sizeof(double2) * slots, b->stream));
-        CUB(cudaMemsetAsync(b->d_sweeps, 0, sizeof(unsigned long long), b->stream));
-        CUB(cudaMemsetAsync(b->d_sigma, 0, sizeof(double) * (size_t)b->sig_stride * B, b->stream));
-        CUB(cudaMemsetAsync(b->d_state, 0, sizeof(double) * (size_t)b->st_stride * B, b->stream));
-        CUB(cudaMemsetAsync(b->d_init_flag, 0, sizeof(int32_t) * (size_t)B, b->stream));
-        const long long diag = B * (b->N - 3);
-        k_wide_init_sigma<<<(unsigned)((diag + 255) / 256), 256, 0, b->stream>>>(b->d_sigma, B, b->N, b->ld);
-    } else if (b->tiled)
-        tile::k_fused_tile_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_init_flag, B);
-    else
-        k_fused_sym_init<<<(unsigned)B, 128, 0, b->stream>>>(b->d_sigma, b->d_state, b->d_init_flag, B, b->N,
-                                                             b->sig_stride, b->st_stride);
-    b->launches += 1;
-    CUB(cudaGetLastError());
-    rc = batch_ensure_xy(b, n);
+    batch_geometry(b);
+    rc = alloc_batch(b);
     if (rc) {
         free_batch(b);
         return rc;
     }
-    CUB(cudaStreamSynchronize(b->stream));
-#undef CUB
     *out = b;
     return EKF_OK;
 }
 
 int ekf_batch_destroy(ekf_batch* b) { return free_batch(b); }
 int64_t ekf_batch_size(const ekf_batch* b) { return b ? b->B : EKF_ERR_INVALID; }
-int ekf_batch_engine(const ekf_batch* b) { return b ? (b->wide ? EKF_ENGINE_STREAM : EKF_ENGINE_FUSED) : EKF_ERR_INVALID; }
+int ekf_batch_engine(const ekf_batch* b) {
+    return b ? (b->layout == Layout::Wide ? EKF_ENGINE_STREAM : EKF_ENGINE_FUSED) : EKF_ERR_INVALID;
+}
 int ekf_batch_sweep_count(ekf_batch* b, uint64_t* out) {
     if (!b || !out) return fail(EKF_ERR_INVALID, "null argument");
     *out = 0;
-    if (!b->wide) return EKF_OK;  // the on-chip engines never sweep a covariance in HBM
+    if (b->layout != Layout::Wide) return EKF_OK;  // the on-chip engines never sweep a covariance in HBM
     DeviceGuard g(b->device);
     unsigned long long v = 0;
     CU(cudaMemcpyAsync(&v, b->d_sweeps, sizeof(v), cudaMemcpyDeviceToHost, b->stream));
@@ -1384,47 +1346,29 @@ void* ekf_batch_stream(ekf_batch* b) { return b ? (void*)b->stream : nullptr; }
 int ekf_batch_step_known_dev(ekf_batch* b, const double* d_twists, const double* d_xy, const uint8_t* d_visible) {
     if (!b || !d_twists || !d_xy || !d_visible) return fail(EKF_ERR_INVALID, "null argument");
     DeviceGuard g(b->device);
-    if (b->wide) {
-        int rc = launch_wide(b, d_twists, d_xy, d_visible, nullptr, 0);
-        b->launches += 1;
-        return rc;
-    }
-    FusedParams p = batch_params(b, kDoPredict | kDoMeasurement, 1, d_twists, d_xy, d_visible, nullptr, nullptr);
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
-    b->launches += 1;
-    return rc;
+    return batch_launch(b, kDoPredict | kDoMeasurement, 1, d_twists, d_xy, d_visible, nullptr, nullptr, 0);
 }
 
 int ekf_batch_step_unknown_dev(ekf_batch* b, const double* d_twists, const double* d_meas, const int32_t* d_count,
                                int m_max, int32_t* d_assoc_out) {
     if (!b || !d_twists || !d_meas || m_max <= 0) return fail(EKF_ERR_INVALID, "invalid argument");
-    if (b->wide)
-        return fail(EKF_ERR_UNSUPPORTED, "unknown data association is not available for batches with n > %d landmarks",
-                    kFusedMaxN);
     DeviceGuard g(b->device);
-    FusedParams p = batch_params(b, kDoPredict | kDoAssociation, m_max, d_twists, d_meas, nullptr, d_count, d_assoc_out);
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
-    b->launches += 1;
-    return rc;
+    return batch_launch(b, kDoPredict | kDoAssociation, m_max, d_twists, d_meas, nullptr, d_count, d_assoc_out, 0);
 }
 
 int ekf_batch_step_known(ekf_batch* b, const double* twists, const double* xy, const uint8_t* visible) {
     if (!b || !twists || !xy || !visible) return fail(EKF_ERR_INVALID, "null argument");
     DeviceGuard g(b->device);
+    const size_t B = (size_t)b->B, n = (size_t)b->n;
     const int s = b->slot;
-    b->slot ^= 1;
-    const size_t B = (size_t)b->B;
-    // the copy stream may overwrite slot s only after the step that last read it has finished
-    CU(cudaStreamWaitEvent(b->copy_stream, b->ev_consumed[s], 0));
-    CU(cudaMemcpyAsync(b->d_twists[s], twists, sizeof(double) * 2 * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaMemcpyAsync(b->d_xy[s], xy, sizeof(double) * 2 * b->n * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaMemcpyAsync(b->d_vis[s], visible, (size_t)b->n * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaEventRecord(b->ev_copied[s], b->copy_stream));
-    CU(cudaStreamWaitEvent(b->stream, b->ev_copied[s], 0));
-    int rc = ekf_batch_step_known_dev(b, b->d_twists[s], b->d_xy[s], b->d_vis[s]);
-    if (rc) return rc;
-    CU(cudaEventRecord(b->ev_consumed[s], b->stream));
-    return EKF_OK;
+    return batch_host_step(b,
+                           {{b->d_twists[s], twists, sizeof(double) * 2 * B},
+                            {b->d_xy[s], xy, sizeof(double) * 2 * n * B},
+                            {b->d_vis[s], visible, n * B}},
+                           [&] {
+                               return batch_launch(b, kDoPredict | kDoMeasurement, 1, b->d_twists[s], b->d_xy[s],
+                                                   b->d_vis[s], nullptr, nullptr, 0);
+                           });
 }
 
 int ekf_batch_step_known_sparse_dev(ekf_batch* b, const double* d_twists, const int32_t* d_offsets, const uint8_t* d_ids,
@@ -1434,17 +1378,8 @@ int ekf_batch_step_known_sparse_dev(ekf_batch* b, const double* d_twists, const 
         return fail(EKF_ERR_UNSUPPORTED, "the marker list carries uint8 ids: n <= %d landmarks (use the dense arrays)",
                     kMarkerMaxN);
     DeviceGuard g(b->device);
-    if (b->wide) {
-        int rc = launch_wide(b, d_twists, d_xy, d_ids, d_offsets, total);
-        b->launches += 1;
-        return rc;
-    }
-    FusedParams p = batch_params(b, kDoPredict | kDoMeasurement | kSparseReadings, 1, d_twists, d_xy, d_ids, d_offsets,
-                                 nullptr);
-    p.sparse_total = total;
-    int rc = b->tiled ? launch_fused_tile(p, b->stream, b->device) : launch_fused_staircase(p, b->stream, b->device);
-    b->launches += 1;
-    return rc;
+    return batch_launch(b, kDoPredict | kDoMeasurement | kSparseReadings, 1, d_twists, d_xy, d_ids, d_offsets, nullptr,
+                        total);
 }
 
 int ekf_batch_step_known_sparse(ekf_batch* b, const double* twists, const int32_t* offsets, const uint8_t* ids,
@@ -1456,49 +1391,38 @@ int ekf_batch_step_known_sparse(ekf_batch* b, const double* twists, const int32_
         return fail(EKF_ERR_UNSUPPORTED, "the marker list carries uint8 ids: n <= %d landmarks (use the dense arrays)",
                     kMarkerMaxN);
     DeviceGuard g(b->device);
-    const int s = b->slot;
-    b->slot ^= 1;
     const size_t B = (size_t)b->B;
-    CU(cudaStreamWaitEvent(b->copy_stream, b->ev_consumed[s], 0));
-    CU(cudaMemcpyAsync(b->d_twists[s], twists, sizeof(double) * 2 * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaMemcpyAsync(b->d_count[s], offsets, sizeof(int32_t) * (B + 1), cudaMemcpyHostToDevice, b->copy_stream));
-    if (total > 0) {
-        CU(cudaMemcpyAsync(b->d_vis[s], ids, (size_t)total, cudaMemcpyHostToDevice, b->copy_stream));
-        CU(cudaMemcpyAsync(b->d_xy[s], xy, sizeof(double) * 2 * (size_t)total, cudaMemcpyHostToDevice, b->copy_stream));
-    }
-    CU(cudaEventRecord(b->ev_copied[s], b->copy_stream));
-    CU(cudaStreamWaitEvent(b->stream, b->ev_copied[s], 0));
-    int rc = ekf_batch_step_known_sparse_dev(b, b->d_twists[s], b->d_count[s], b->d_vis[s], b->d_xy[s], total);
-    if (rc) return rc;
-    CU(cudaEventRecord(b->ev_consumed[s], b->stream));
-    return EKF_OK;
+    const int s = b->slot;
+    return batch_host_step(b,
+                           {{b->d_twists[s], twists, sizeof(double) * 2 * B},
+                            {b->d_count[s], offsets, sizeof(int32_t) * (B + 1)},
+                            {b->d_vis[s], ids, (size_t)total},
+                            {b->d_xy[s], xy, sizeof(double) * 2 * (size_t)total}},
+                           [&] {
+                               return batch_launch(b, kDoPredict | kDoMeasurement | kSparseReadings, 1, b->d_twists[s],
+                                                   b->d_xy[s], b->d_vis[s], b->d_count[s], nullptr, total);
+                           });
 }
 
 int ekf_batch_step_unknown(ekf_batch* b, const double* twists, const double* meas, const int32_t* count, int m_max,
                            int32_t* assoc_out) {
     if (!b || !twists || !meas || !count || m_max <= 0) return fail(EKF_ERR_INVALID, "invalid argument");
-    if (b->wide)
-        return fail(EKF_ERR_UNSUPPORTED, "unknown data association is not available for batches with n > %d landmarks",
-                    kFusedMaxN);
     DeviceGuard g(b->device);
     int rc = batch_ensure_xy(b, m_max);
     if (rc) return rc;
-    const int s = b->slot;
-    b->slot ^= 1;
     const size_t B = (size_t)b->B;
-    CU(cudaStreamWaitEvent(b->copy_stream, b->ev_consumed[s], 0));
-    CU(cudaMemcpyAsync(b->d_twists[s], twists, sizeof(double) * 2 * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaMemcpyAsync(b->d_xy[s], meas, sizeof(double) * 2 * m_max * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaMemcpyAsync(b->d_count[s], count, sizeof(int32_t) * B, cudaMemcpyHostToDevice, b->copy_stream));
-    CU(cudaEventRecord(b->ev_copied[s], b->copy_stream));
-    CU(cudaStreamWaitEvent(b->stream, b->ev_copied[s], 0));
-    rc = ekf_batch_step_unknown_dev(b, b->d_twists[s], b->d_xy[s], b->d_count[s], m_max, assoc_out ? b->d_assoc : nullptr);
-    if (rc) return rc;
-    CU(cudaEventRecord(b->ev_consumed[s], b->stream));
-    if (assoc_out) {
-        CU(cudaMemcpyAsync(assoc_out, b->d_assoc, sizeof(int32_t) * m_max * B, cudaMemcpyDeviceToHost, b->stream));
-        CU(cudaStreamSynchronize(b->stream));
-    }
+    const int s = b->slot;
+    rc = batch_host_step(b,
+                         {{b->d_twists[s], twists, sizeof(double) * 2 * B},
+                          {b->d_xy[s], meas, sizeof(double) * 2 * m_max * B},
+                          {b->d_count[s], count, sizeof(int32_t) * B}},
+                         [&] {
+                             return batch_launch(b, kDoPredict | kDoAssociation, m_max, b->d_twists[s], b->d_xy[s],
+                                                 nullptr, b->d_count[s], assoc_out ? b->d_assoc : nullptr, 0);
+                         });
+    if (rc || !assoc_out) return rc;
+    CU(cudaMemcpyAsync(assoc_out, b->d_assoc, sizeof(int32_t) * m_max * B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
     return EKF_OK;
 }
 
@@ -1538,22 +1462,20 @@ int ekf_batch_get_states(ekf_batch* b, double* out) {
 int ekf_batch_get_sigma(ekf_batch* b, int64_t filter, double* out, int64_t ld) {
     if (!b || !out || filter < 0 || filter >= b->B || ld < b->N) return fail(EKF_ERR_INVALID, "invalid argument");
     DeviceGuard g(b->device);
-    if (b->wide) {  // already dense: one 2-D copy
-        CU(cudaMemcpy2DAsync(out, sizeof(double) * ld, b->d_sigma + (size_t)filter * b->sig_stride, sizeof(double) * b->ld,
-                             sizeof(double) * b->N, b->N, cudaMemcpyDeviceToHost, b->stream));
-        CU(cudaStreamSynchronize(b->stream));
-        return EKF_OK;
+    const double* src = b->d_sigma + (size_t)filter * b->sig_stride;
+    long long src_ld = b->ld;
+    if (b->layout != Layout::Wide) {  // the on-chip layouts: expand the filter's copy to dense N x N first
+        if (!b->d_dense) CU(cudaMalloc(&b->d_dense, sizeof(double) * (size_t)b->N * b->N));
+        const int blocks = (b->N * b->N + 255) / 256;
+        if (b->layout == Layout::Tile)
+            tile::k_fused_tile_unpack<<<blocks, 256, 0, b->stream>>>(src, b->d_dense);
+        else
+            k_fused_sym_unpack<<<blocks, 256, 0, b->stream>>>(src, b->d_dense, b->N);
+        CU(cudaGetLastError());
+        src = b->d_dense;
+        src_ld = b->N;
     }
-    // the on-chip engines keep Sigma in the staircase or tile layout; expand one filter's copy to dense N x N
-    if (!b->d_dense) CU(cudaMalloc(&b->d_dense, sizeof(double) * (size_t)b->N * b->N));
-    if (b->tiled)
-        tile::k_fused_tile_unpack<<<(b->N * b->N + 255) / 256, 256, 0, b->stream>>>(
-            b->d_sigma + (size_t)filter * b->sig_stride, b->d_dense);
-    else
-        k_fused_sym_unpack<<<(b->N * b->N + 255) / 256, 256, 0, b->stream>>>(b->d_sigma + (size_t)filter * b->sig_stride,
-                                                                            b->d_dense, b->N);
-    CU(cudaGetLastError());
-    CU(cudaMemcpy2DAsync(out, sizeof(double) * ld, b->d_dense, sizeof(double) * b->N, sizeof(double) * b->N, b->N,
+    CU(cudaMemcpy2DAsync(out, sizeof(double) * ld, src, sizeof(double) * src_ld, sizeof(double) * b->N, b->N,
                          cudaMemcpyDeviceToHost, b->stream));
     CU(cudaStreamSynchronize(b->stream));
     return EKF_OK;
@@ -1572,7 +1494,7 @@ int ekf_batch_get_known(ekf_batch* b, uint8_t* out) {
 int ekf_batch_checkpoint_size(ekf_batch* b, int64_t* sigma_doubles, int64_t* state_doubles) {
     if (!b) return fail(EKF_ERR_INVALID, "null handle");
     if (sigma_doubles) *sigma_doubles = (int64_t)b->sig_stride * b->B;
-    if (state_doubles) *state_doubles = (int64_t)(b->tiled ? tile::kStLen : b->st_stride) * b->B;
+    if (state_doubles) *state_doubles = (int64_t)b->st_len * b->B;
     return EKF_OK;
 }
 int ekf_batch_export(ekf_batch* b, double* sigma, double* state, int32_t* init_flag, uint8_t* known, uint64_t* updates) {
@@ -1581,11 +1503,8 @@ int ekf_batch_export(ekf_batch* b, double* sigma, double* state, int32_t* init_f
     const size_t B = (size_t)b->B;
     CU(cudaStreamSynchronize(b->copy_stream));
     CU(cudaMemcpyAsync(sigma, b->d_sigma, sizeof(double) * b->sig_stride * B, cudaMemcpyDeviceToHost, b->stream));
-    if (b->tiled)  // the state sits inside the Sigma blocks; it is exported as its own compact [B][44] array as well
-        CU(cudaMemcpy2DAsync(state, sizeof(double) * tile::kStLen, b->d_state, sizeof(double) * b->st_stride,
-                             sizeof(double) * tile::kStLen, B, cudaMemcpyDeviceToHost, b->stream));
-    else
-        CU(cudaMemcpyAsync(state, b->d_state, sizeof(double) * b->st_stride * B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaMemcpy2DAsync(state, sizeof(double) * b->st_len, b->d_state, sizeof(double) * b->st_stride,
+                         sizeof(double) * b->st_len, B, cudaMemcpyDeviceToHost, b->stream));
     CU(cudaMemcpyAsync(init_flag, b->d_init_flag, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, b->stream));
     CU(cudaMemcpyAsync(known, b->d_known, (size_t)b->n * B, cudaMemcpyDeviceToHost, b->stream));
     unsigned long long u = 0;
@@ -1602,11 +1521,8 @@ int ekf_batch_import(ekf_batch* b, const double* sigma, const double* state, con
     CU(cudaStreamSynchronize(b->copy_stream));
     CU(cudaStreamSynchronize(b->out_stream));
     CU(cudaMemcpyAsync(b->d_sigma, sigma, sizeof(double) * b->sig_stride * B, cudaMemcpyHostToDevice, b->stream));
-    if (b->tiled)
-        CU(cudaMemcpy2DAsync(b->d_state, sizeof(double) * b->st_stride, state, sizeof(double) * tile::kStLen,
-                             sizeof(double) * tile::kStLen, B, cudaMemcpyHostToDevice, b->stream));
-    else
-        CU(cudaMemcpyAsync(b->d_state, state, sizeof(double) * b->st_stride * B, cudaMemcpyHostToDevice, b->stream));
+    CU(cudaMemcpy2DAsync(b->d_state, sizeof(double) * b->st_stride, state, sizeof(double) * b->st_len,
+                         sizeof(double) * b->st_len, B, cudaMemcpyHostToDevice, b->stream));
     CU(cudaMemcpyAsync(b->d_init_flag, init_flag, sizeof(int32_t) * B, cudaMemcpyHostToDevice, b->stream));
     CU(cudaMemcpyAsync(b->d_known, known, (size_t)b->n * B, cudaMemcpyHostToDevice, b->stream));
     const unsigned long long u = (unsigned long long)updates;
@@ -1759,10 +1675,8 @@ int ekf_batch_launch_count(ekf_batch* b, uint64_t* out) {
 int ekf_normalize_angles(const double* in, double* out, int64_t count, int device) {
     if (!in || !out || count < 0) return fail(EKF_ERR_INVALID, "invalid argument");
     if (count == 0) return EKF_OK;
-    int ndev = 0;
-    int rc = ekf_device_count(&ndev);
+    int rc = check_device(device);
     if (rc) return rc;
-    if (device < 0 || device >= ndev) return fail(EKF_ERR_INVALID, "device %d not available", device);
     DeviceGuard g(device);
     double *d_in = nullptr, *d_out = nullptr;
     CU(cudaMalloc(&d_in, sizeof(double) * count));

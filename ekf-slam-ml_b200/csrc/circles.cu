@@ -7,13 +7,13 @@
 // One kernel launch per batch of scans; nothing is computed on the host.
 #include <cuda_runtime.h>
 
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <new>
 
 #include "../../include/circle_fit_b200.h"
 #include "ekf_math.cuh"
+#include "host_util.cuh"
 
 namespace circ {
 
@@ -495,23 +495,6 @@ __global__ void __launch_bounds__(128)
     }
 }
 
-thread_local char g_err[512] = "";
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
-#define CCU(expr)                                                                            \
-    do {                                                                                     \
-        cudaError_t e_ = (expr);                                                             \
-        if (e_ != cudaSuccess) {                                                             \
-            cudaGetLastError();                                                              \
-            return circ::fail((int)e_, "%s failed: %s", #expr, cudaGetErrorString(e_));      \
-        }                                                                                    \
-    } while (0)
-
 }  // namespace circ
 
 struct circles_ctx {
@@ -526,46 +509,30 @@ struct circles_ctx {
 };
 
 namespace {
-struct Dev {
-    int prev = -1;
-    explicit Dev(int d) {
-        cudaGetDevice(&prev);
-        if (prev != d) cudaSetDevice(d);
-    }
-    ~Dev() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 template <typename T>
 int run_scans(circles_ctx* c, const T* d_ranges, long long B) {
     circ::k_circles_scan<T><<<(unsigned)B, circ::kCtaThreads, 0, c->stream>>>(d_ranges, B, c->n_beams, c->max_c, c->o);
     c->launches += 1;
     c->last_B = B;
-    CCU(cudaGetLastError());
+    CU(cudaGetLastError());
     return 0;
 }
 }  // namespace
 
 extern "C" {
 
-const char* circles_last_error(void) { return circ::g_err; }
+const char* circles_last_error(void) { return g_err; }
 
 int circles_create(int64_t max_scans, int n_beams, int max_circles, int device, circles_ctx** out) {
-    if (!out) return circ::fail(-1, "null out pointer");
+    if (!out) return fail(-1, "null out pointer");
     *out = nullptr;
-    if (max_scans <= 0 || n_beams < 2 || max_circles <= 0) return circ::fail(-1, "invalid shape");
-    if (n_beams > circ::kMaxBeams) return circ::fail(-2, "n_beams=%d exceeds %d", n_beams, circ::kMaxBeams);
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return circ::fail((int)e, "cudaGetDeviceCount: %s", cudaGetErrorString(e));
-    }
-    if (device < 0 || device >= count) return circ::fail(-1, "device %d not available (%d visible)", device, count);
-    Dev g(device);
+    if (max_scans <= 0 || n_beams < 2 || max_circles <= 0) return fail(-1, "invalid shape");
+    if (n_beams > circ::kMaxBeams) return fail(-2, "n_beams=%d exceeds %d", n_beams, circ::kMaxBeams);
+    int rc = check_device(device);
+    if (rc) return rc;
+    DeviceGuard g(device);
     circles_ctx* c = new (std::nothrow) circles_ctx();
-    if (!c) return circ::fail(-3, "out of host memory");
+    if (!c) return fail(-3, "out of host memory");
     c->cap = max_scans;
     c->n_beams = n_beams;
     c->device = device;
@@ -586,7 +553,7 @@ int circles_create(int64_t max_scans, int n_beams, int max_circles, int device, 
     A((void**)&c->o.counts, B * sizeof(int32_t));
     if (err != cudaSuccess) {
         cudaGetLastError();
-        int code = circ::fail((int)err, "allocation failed: %s", cudaGetErrorString(err));
+        int code = fail((int)err, "allocation failed: %s", cudaGetErrorString(err));
         circles_destroy(c);
         return code;
     }
@@ -596,7 +563,7 @@ int circles_create(int64_t max_scans, int n_beams, int max_circles, int device, 
 
 int circles_destroy(circles_ctx* c) {
     if (!c) return 0;
-    Dev g(c->device);
+    DeviceGuard g(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
     cudaFree(c->d_ranges);
     cudaFree(c->o.n_clusters);
@@ -616,38 +583,38 @@ int circles_destroy(circles_ctx* c) {
 
 static int fetch_results(circles_ctx* c, long long B, double* centers, int32_t* counts) {
     if (centers)
-        CCU(cudaMemcpyAsync(centers, c->o.centers, sizeof(double) * 2 * c->max_c * B, cudaMemcpyDeviceToHost, c->stream));
-    if (counts) CCU(cudaMemcpyAsync(counts, c->o.counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, c->stream));
-    CCU(cudaStreamSynchronize(c->stream));
+        CU(cudaMemcpyAsync(centers, c->o.centers, sizeof(double) * 2 * c->max_c * B, cudaMemcpyDeviceToHost, c->stream));
+    if (counts) CU(cudaMemcpyAsync(counts, c->o.counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
     return 0;
 }
 
 int circles_run_f32(circles_ctx* c, const float* ranges, int64_t B, double* centers, int32_t* counts) {
-    if (!c || !ranges || B <= 0 || B > c->cap) return circ::fail(-1, "invalid argument");
-    Dev g(c->device);
-    CCU(cudaMemcpyAsync(c->d_ranges, ranges, sizeof(float) * c->n_beams * B, cudaMemcpyHostToDevice, c->stream));
+    if (!c || !ranges || B <= 0 || B > c->cap) return fail(-1, "invalid argument");
+    DeviceGuard g(c->device);
+    CU(cudaMemcpyAsync(c->d_ranges, ranges, sizeof(float) * c->n_beams * B, cudaMemcpyHostToDevice, c->stream));
     int rc = run_scans<float>(c, static_cast<const float*>(c->d_ranges), B);
     if (rc) return rc;
     return fetch_results(c, B, centers, counts);
 }
 
 int circles_run_f64(circles_ctx* c, const double* ranges, int64_t B, double* centers, int32_t* counts) {
-    if (!c || !ranges || B <= 0 || B > c->cap) return circ::fail(-1, "invalid argument");
-    Dev g(c->device);
-    CCU(cudaMemcpyAsync(c->d_ranges, ranges, sizeof(double) * c->n_beams * B, cudaMemcpyHostToDevice, c->stream));
+    if (!c || !ranges || B <= 0 || B > c->cap) return fail(-1, "invalid argument");
+    DeviceGuard g(c->device);
+    CU(cudaMemcpyAsync(c->d_ranges, ranges, sizeof(double) * c->n_beams * B, cudaMemcpyHostToDevice, c->stream));
     int rc = run_scans<double>(c, static_cast<const double*>(c->d_ranges), B);
     if (rc) return rc;
     return fetch_results(c, B, centers, counts);
 }
 
 int circles_run_dev_f32(circles_ctx* c, const float* d_ranges, int64_t B) {
-    if (!c || !d_ranges || B <= 0 || B > c->cap) return circ::fail(-1, "invalid argument");
-    Dev g(c->device);
+    if (!c || !d_ranges || B <= 0 || B > c->cap) return fail(-1, "invalid argument");
+    DeviceGuard g(c->device);
     return run_scans<float>(c, d_ranges, B);
 }
 
 int circles_device_outputs(circles_ctx* c, void** d_centers, void** d_counts) {
-    if (!c) return circ::fail(-1, "null handle");
+    if (!c) return fail(-1, "null handle");
     if (d_centers) *d_centers = c->o.centers;
     if (d_counts) *d_counts = c->o.counts;
     return 0;
@@ -655,15 +622,15 @@ int circles_device_outputs(circles_ctx* c, void** d_centers, void** d_counts) {
 
 int circles_last_clusters(circles_ctx* c, int64_t scan, int32_t* n_clusters, int32_t* segs, double* cxr,
                           uint8_t* flags, double* xy) {
-    if (!c || scan < 0 || scan >= c->last_B) return circ::fail(-1, "invalid argument");
-    Dev g(c->device);
+    if (!c || scan < 0 || scan >= c->last_B) return fail(-1, "invalid argument");
+    DeviceGuard g(c->device);
     const int M = circ::kMaxClusters;
-    if (n_clusters) CCU(cudaMemcpyAsync(n_clusters, c->o.n_clusters + scan, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    if (segs) CCU(cudaMemcpyAsync(segs, c->o.segs + scan * M * 4, sizeof(int32_t) * M * 4, cudaMemcpyDeviceToHost, c->stream));
-    if (cxr) CCU(cudaMemcpyAsync(cxr, c->o.cxr + scan * M * 4, sizeof(double) * M * 4, cudaMemcpyDeviceToHost, c->stream));
-    if (flags) CCU(cudaMemcpyAsync(flags, c->o.flags + scan * M, M, cudaMemcpyDeviceToHost, c->stream));
-    if (xy) CCU(cudaMemcpyAsync(xy, c->o.xy + scan * c->n_beams * 2, sizeof(double) * 2 * c->n_beams, cudaMemcpyDeviceToHost, c->stream));
-    CCU(cudaStreamSynchronize(c->stream));
+    if (n_clusters) CU(cudaMemcpyAsync(n_clusters, c->o.n_clusters + scan, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (segs) CU(cudaMemcpyAsync(segs, c->o.segs + scan * M * 4, sizeof(int32_t) * M * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (cxr) CU(cudaMemcpyAsync(cxr, c->o.cxr + scan * M * 4, sizeof(double) * M * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (flags) CU(cudaMemcpyAsync(flags, c->o.flags + scan * M, M, cudaMemcpyDeviceToHost, c->stream));
+    if (xy) CU(cudaMemcpyAsync(xy, c->o.xy + scan * c->n_beams * 2, sizeof(double) * 2 * c->n_beams, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
     return 0;
 }
 
@@ -672,15 +639,15 @@ int circles_max_beams(void) { return circ::kMaxBeams; }
 
 int circles_fit_clusters(circles_ctx* c, const double* flat_xy, const int32_t* sizes, int n_clusters, double* cxr,
                          uint8_t* flags) {
-    if (!c || !flat_xy || !sizes || n_clusters <= 0 || !cxr || !flags) return circ::fail(-1, "invalid argument");
-    Dev g(c->device);
+    if (!c || !flat_xy || !sizes || n_clusters <= 0 || !cxr || !flags) return fail(-1, "invalid argument");
+    DeviceGuard g(c->device);
     int total = 0;
     int* offs = new (std::nothrow) int[n_clusters + 1];
-    if (!offs) return circ::fail(-3, "out of host memory");
+    if (!offs) return fail(-3, "out of host memory");
     for (int i = 0; i < n_clusters; ++i) {
         if (sizes[i] < 1 || sizes[i] > circ::kMaxBeams) {
             delete[] offs;
-            return circ::fail(-2, "cluster %d has %d points (supported: 1..%d)", i, sizes[i], circ::kMaxBeams);
+            return fail(-2, "cluster %d has %d points (supported: 1..%d)", i, sizes[i], circ::kMaxBeams);
         }
         offs[i] = total;
         total += sizes[i];
@@ -710,46 +677,46 @@ int circles_fit_clusters(circles_ctx* c, const double* flat_xy, const int32_t* s
     delete[] offs;
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return circ::fail((int)e, "circles_fit_clusters: %s", cudaGetErrorString(e));
+        return fail((int)e, "circles_fit_clusters: %s", cudaGetErrorString(e));
     }
     return 0;
 }
 
 int circles_sync(circles_ctx* c) {
-    if (!c) return circ::fail(-1, "null handle");
-    Dev g(c->device);
-    CCU(cudaStreamSynchronize(c->stream));
+    if (!c) return fail(-1, "null handle");
+    DeviceGuard g(c->device);
+    CU(cudaStreamSynchronize(c->stream));
     return 0;
 }
 int circles_timer_start(circles_ctx* c) {
-    if (!c) return circ::fail(-1, "null handle");
-    Dev g(c->device);
+    if (!c) return fail(-1, "null handle");
+    DeviceGuard g(c->device);
     if (!c->t0) {
-        CCU(cudaEventCreate(&c->t0));
-        CCU(cudaEventCreate(&c->t1));
+        CU(cudaEventCreate(&c->t0));
+        CU(cudaEventCreate(&c->t1));
     }
-    CCU(cudaEventRecord(c->t0, c->stream));
+    CU(cudaEventRecord(c->t0, c->stream));
     return 0;
 }
 int circles_timer_stop(circles_ctx* c, float* ms_out) {
-    if (!c || !ms_out || !c->t0) return circ::fail(-1, "timer not started");
-    Dev g(c->device);
-    CCU(cudaEventRecord(c->t1, c->stream));
-    CCU(cudaEventSynchronize(c->t1));
-    CCU(cudaEventElapsedTime(ms_out, c->t0, c->t1));
+    if (!c || !ms_out || !c->t0) return fail(-1, "timer not started");
+    DeviceGuard g(c->device);
+    CU(cudaEventRecord(c->t1, c->stream));
+    CU(cudaEventSynchronize(c->t1));
+    CU(cudaEventElapsedTime(ms_out, c->t0, c->t1));
     return 0;
 }
 // 1: runs return only what approxCirclePositions() returns (accepted centres + counts); clusters that fail the
 // inscribed-angle test are not fitted and circles_last_clusters() reports NaN for them.  0 (default): every cluster is
 // fitted, as circleRegression() does.  The accepted centres are identical in both modes.
 int circles_set_centres_only(circles_ctx* c, int on) {
-    if (!c) return circ::fail(-1, "null handle");
+    if (!c) return fail(-1, "null handle");
     c->o.centres_only = on ? 1 : 0;
     return 0;
 }
 
 int circles_launch_count(circles_ctx* c, uint64_t* out) {
-    if (!c || !out) return circ::fail(-1, "null argument");
+    if (!c || !out) return fail(-1, "null argument");
     *out = c->launches;
     return 0;
 }

@@ -258,25 +258,10 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
     if (threadIdx.x == 32 * (kTmaConsumerWarps + 1)) bulk_wait_all();
 }
 
-// Sigma_0 = blockdiag(0_3, 100 I) for every filter of an already-zeroed batch.
-__global__ void k_wide_init_sigma(double* __restrict__ sigma, long long B, int N, long long ld) {
-    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= B * (N - 3)) return;
-    const long long b = e / (N - 3), k = 3 + e - b * (N - 3);
-    sigma[b * N * ld + k * ld + k] = kSigma0;
-}
-
-// One step of the whole batch.  grid = the number of CTAs the factor slots were allocated for.
-inline cudaError_t launch_wide_step(const WideParams& p, int grid, cudaStream_t stream) {
-    static bool attr_set[64] = {false};
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) dev = -1;
-    const int smem = wide_smem_bytes(kWideMaxN);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(k_wide_step, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
+// One step of the whole batch on `device`.  grid = the number of CTAs the factor slots were allocated for.
+inline cudaError_t launch_wide_step(const WideParams& p, int grid, cudaStream_t stream, int device) {
+    const cudaError_t e = kernel_setup<k_wide_step>(device, kTmaThreads, wide_smem_bytes(kWideMaxN), false);
+    if (e != cudaSuccess) return e;
     k_wide_step<<<(unsigned)grid, kTmaThreads, wide_smem_bytes(p.n), stream>>>(p);
     return cudaGetLastError();
 }

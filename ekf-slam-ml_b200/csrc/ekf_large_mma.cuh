@@ -26,6 +26,7 @@
 #pragma once
 #include "bulk_copy.cuh"
 #include "ekf_large_delayed.cuh"
+#include "host_util.cuh"
 
 namespace ekf {
 
@@ -236,16 +237,10 @@ cudaError_t launch_sweep_mma(double* sig, long long ld, int n_rows, const double
         return cudaErrorInvalidValue;
     } else {
         using T = SweepTile<P>;
-        // the shared-memory opt-in is per device: one flag per device, indexed by the device the launch goes to
-        static bool attr_set[64] = {false};
         int dev = -1;
         if (cudaGetDevice(&dev) != cudaSuccess) dev = -1;
-        if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-            cudaError_t e = cudaFuncSetAttribute(k_large_sweep_mma<P>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 T::kSmemBytes);
-            if (e != cudaSuccess) return e;
-            if (dev >= 0 && dev < 64) attr_set[dev] = true;
-        }
+        const cudaError_t e = kernel_setup<k_large_sweep_mma<P>>(dev, kTmaThreads, T::kSmemBytes, false);
+        if (e != cudaSuccess) return e;
         const long long units = ((ld + T::COLS - 1) / T::COLS) * ((n_rows + kUnitRows - 1) / kUnitRows);
         const unsigned grid = (unsigned)(units < sm_count ? (units < 1 ? 1 : units) : sm_count);
         k_large_sweep_mma<P><<<grid, kTmaThreads, T::kSmemBytes, stream>>>(sig, ld, n_rows, Kp, Wp, row0, n_updates,

@@ -9,7 +9,6 @@
 #include <nccl.h>
 
 #include <algorithm>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <new>
@@ -17,27 +16,12 @@
 
 #include "../../../include/ekf_sharded_b200.h"
 #include "../ekf_large_mma.cuh"
+#include "../host_util.cuh"
 
 using namespace ekf;
 
 namespace {
 
-thread_local char g_err[512] = "";
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
-#define CU(expr)                                                                               \
-    do {                                                                                       \
-        cudaError_t e_ = (expr);                                                               \
-        if (e_ != cudaSuccess) {                                                               \
-            cudaGetLastError();                                                                \
-            return fail((int)e_, "%s failed: %s (line %d)", #expr, cudaGetErrorString(e_), __LINE__); \
-        }                                                                                      \
-    } while (0)
 #define NC(expr)                                                                               \
     do {                                                                                       \
         ncclResult_t r_ = (expr);                                                              \
@@ -479,32 +463,6 @@ struct ekf_sharded {
 
 namespace {
 
-template <class... KArgs, class... Args>
-cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
-struct Dev {
-    int prev = -1;
-    explicit Dev(int d) {
-        cudaGetDevice(&prev);
-        if (prev != d) cudaSetDevice(d);
-    }
-    ~Dev() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 void partition(ekf_sharded* h) {
     const int per = (h->n + h->world - 1) / h->world;
     h->r0_of.resize(h->world);
@@ -721,13 +679,8 @@ int create_common(int n, int world, int device, ekf_sharded** out, ekf_sharded**
     if (!out) return fail(-1, "null out pointer");
     *out = nullptr;
     if (n <= 0 || world <= 0 || n < world) return fail(-1, "invalid shape: n=%d world=%d", n, world);
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return fail((int)e, "cudaGetDeviceCount: %s", cudaGetErrorString(e));
-    }
-    if (device < 0 || device >= count) return fail(-1, "device %d not available (%d visible)", device, count);
+    const int rc = check_device(device);
+    if (rc) return rc;
     ekf_sharded* h = new (std::nothrow) ekf_sharded();
     if (!h) return fail(-3, "out of host memory");
     h->n = n;
@@ -758,7 +711,7 @@ int ekf_sharded_unique_id(void* id128) {
 
 int ekf_sharded_destroy(ekf_sharded* h) {
     if (!h) return 0;
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
     for (auto& s : h->sh) {
         cudaFree(s.sig);
@@ -803,7 +756,7 @@ int ekf_sharded_create(int n, int rank, int world, const void* id128, int device
     ekf_sharded* h = nullptr;
     int rc = create_common(n, world, device, out, &h);
     if (rc) return rc;
-    Dev g(device);
+    DeviceGuard g(device);
     cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         ekf_sharded_destroy(h);
@@ -849,10 +802,10 @@ int ekf_sharded_attach_exchange(ekf_sharded* h, int world, const uint64_t* peer_
     if (!h || !peer_bases) return fail(-1, "null argument");
     if (h->local) return fail(-1, "the push exchange needs real ranks (not the single-GPU emulation)");
     if (world != h->world || world > 8) return fail(-1, "push exchange: world size %d not supported", world);
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {   // k_sh_correct_push's CTAs wait for one another: the whole grid has to be resident at once
         int per_sm = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sh_correct_push, 256, 0));
+        CU(kernel_setup<k_sh_correct_push>(h->device, 256, 0, false, &per_sm));
         const long long blocks = (h->ld + 255) / 256;
         if (blocks > (long long)per_sm * h->sm_count)
             return fail(-1, "push exchange: the correction needs %lld resident CTAs, the device holds %d (%d SMs x %d)",
@@ -884,7 +837,7 @@ int ekf_sharded_create_local(int n, int world, int device, ekf_sharded** out) {
     ekf_sharded* h = nullptr;
     int rc = create_common(n, world, device, out, &h);
     if (rc) return rc;
-    Dev g(device);
+    DeviceGuard g(device);
     h->local = true;
     cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
@@ -904,7 +857,7 @@ int ekf_sharded_create_local(int n, int world, int device, ekf_sharded** out) {
 
 int ekf_sharded_predict(ekf_sharded* h, double dtheta, double dx) {
     if (!h) return fail(-1, "null handle");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     if (!h->carry_pending) {
         int rc = settle(h);
         if (rc) return rc;
@@ -930,7 +883,7 @@ int ekf_sharded_predict(ekf_sharded* h, double dtheta, double dx) {
 
 int ekf_sharded_measurement(ekf_sharded* h, const double* xy, const uint8_t* visible) {
     if (!h || !xy || !visible) return fail(-1, "null argument");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     const int n = h->n;
     if (!h->init_flag_host) {
         CU(cudaStreamSynchronize(h->stream));
@@ -957,7 +910,7 @@ int ekf_sharded_data_association(ekf_sharded* h, const double* xy, int m, uint8_
                                  double* dmin_out, double* second_out, uint8_t* created_out) {
     if (!h || !known || m < 0 || (m > 0 && !xy)) return fail(-1, "invalid argument");
     if (m == 0) return 0;
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;
@@ -1021,7 +974,7 @@ int ekf_sharded_data_association(ekf_sharded* h, const double* xy, int m, uint8_
 
 int ekf_sharded_get_state(ekf_sharded* h, double* out) {
     if (!h || !out) return fail(-1, "null argument");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     CU(cudaMemcpyAsync(out, h->sh[0].state, sizeof(double) * h->N, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     return 0;
@@ -1034,7 +987,7 @@ int ekf_sharded_rows(ekf_sharded* h, int shard, int64_t* row_begin, int64_t* row
 }
 int ekf_sharded_get_sigma_rows(ekf_sharded* h, int shard, double* out, int64_t ld) {
     if (!h || !out || shard < 0 || shard >= (int)h->sh.size() || ld < h->N) return fail(-1, "invalid argument");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;
@@ -1053,7 +1006,7 @@ int ekf_sharded_get_sigma_row_list(ekf_sharded* h, int shard, const int64_t* row
     Shard& s = h->sh[shard];
     for (int k = 0; k < count; ++k)
         if (rows[k] < s.r0 || rows[k] >= s.r1) return fail(-1, "row %lld is not owned by this shard", (long long)rows[k]);
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;
@@ -1066,7 +1019,7 @@ int ekf_sharded_get_sigma_row_list(ekf_sharded* h, int shard, const int64_t* row
 }
 int ekf_sharded_update_count(ekf_sharded* h, uint64_t* out) {
     if (!h || !out) return fail(-1, "null argument");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;
@@ -1079,7 +1032,7 @@ int ekf_sharded_update_count(ekf_sharded* h, uint64_t* out) {
 }
 int ekf_sharded_set_max_pending(ekf_sharded* h, int max_pending) {
     if (!h || max_pending < 1 || max_pending > kMaxPending) return fail(-1, "max_pending must be 1..%d", kMaxPending);
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     h->max_pending = max_pending;
     return h->pending >= max_pending ? settle(h) : 0;
 }
@@ -1092,7 +1045,7 @@ int ekf_sharded_set_carry_pending(ekf_sharded* h, int carry) {
     if (!h) return fail(-1, "null handle");
     h->carry_pending = carry ? 1 : 0;
     if (!h->carry_pending) {
-        Dev g(h->device);
+        DeviceGuard g(h->device);
         return settle(h);
     }
     return 0;
@@ -1104,7 +1057,7 @@ int ekf_sharded_launch_count(ekf_sharded* h, uint64_t* out) {
 }
 int ekf_sharded_sync(ekf_sharded* h) {
     if (!h) return fail(-1, "null handle");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;
@@ -1114,7 +1067,7 @@ int ekf_sharded_sync(ekf_sharded* h) {
 }
 int ekf_sharded_timer_start(ekf_sharded* h) {
     if (!h) return fail(-1, "null handle");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     if (!h->t0) {
         CU(cudaEventCreate(&h->t0));
         CU(cudaEventCreate(&h->t1));
@@ -1124,7 +1077,7 @@ int ekf_sharded_timer_start(ekf_sharded* h) {
 }
 int ekf_sharded_timer_stop(ekf_sharded* h, float* ms_out) {
     if (!h || !ms_out || !h->t0) return fail(-1, "timer not started");
-    Dev g(h->device);
+    DeviceGuard g(h->device);
     {
         int rc_ = settle(h);
         if (rc_) return rc_;

@@ -4,13 +4,13 @@
 // transcendental functions differ from numpy's in the last bits only.
 #include <cuda_runtime.h>
 
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <new>
 
 #include "../../include/tube_world_b200.h"
 #include "ekf_math.cuh"
+#include "host_util.cuh"
 
 namespace tw {
 
@@ -215,34 +215,6 @@ __global__ void __launch_bounds__(128)
     ranges[g] = (float)(min_r + p.range_std * noise);
 }
 
-thread_local char g_err[512] = "";
-int fail(int code, const char* fmt, ...) {
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(g_err, sizeof(g_err), fmt, ap);
-    va_end(ap);
-    return code;
-}
-#define TCU(expr)                                                                       \
-    do {                                                                                \
-        cudaError_t e_ = (expr);                                                        \
-        if (e_ != cudaSuccess) {                                                        \
-            cudaGetLastError();                                                         \
-            return tw::fail((int)e_, "%s failed: %s", #expr, cudaGetErrorString(e_));   \
-        }                                                                               \
-    } while (0)
-
-struct Dev {
-    int prev = -1;
-    explicit Dev(int d) {
-        cudaGetDevice(&prev);
-        if (prev != d) cudaSetDevice(d);
-    }
-    ~Dev() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 }  // namespace tw
 
 struct tubeworld {
@@ -262,11 +234,11 @@ struct tubeworld {
 
 extern "C" {
 
-const char* tubeworld_last_error(void) { return tw::g_err; }
+const char* tubeworld_last_error(void) { return g_err; }
 
 int tubeworld_destroy(tubeworld* w) {
     if (!w) return 0;
-    tw::Dev g(w->device);
+    DeviceGuard g(w->device);
     /* a borrowed stream may already be gone when the consumer was closed first: never touch it here */
     if (w->stream && w->own_stream) cudaStreamSynchronize(w->stream);
     else cudaDeviceSynchronize();
@@ -287,21 +259,16 @@ int tubeworld_destroy(tubeworld* w) {
 
 int tubeworld_create(int64_t B, const tubeworld_params* p, const double* tubes_x, const double* tubes_y, int n_tubes,
                      uint64_t seed, int64_t first_filter, int device, tubeworld** out) {
-    if (!out) return tw::fail(-1, "null out pointer");
+    if (!out) return fail(-1, "null out pointer");
     *out = nullptr;
     if (B <= 0 || !p || n_tubes < 0 || (n_tubes > 0 && (!tubes_x || !tubes_y)) || p->n_slots <= 0)
-        return tw::fail(-1, "invalid argument");
-    if (n_tubes > 255) return tw::fail(-2, "at most 255 tubes (RNG counter layout)");
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return tw::fail((int)e, "cudaGetDeviceCount: %s", cudaGetErrorString(e));
-    }
-    if (device < 0 || device >= count) return tw::fail(-1, "device %d not available (%d visible)", device, count);
-    tw::Dev g(device);
+        return fail(-1, "invalid argument");
+    if (n_tubes > 255) return fail(-2, "at most 255 tubes (RNG counter layout)");
+    const int rc = check_device(device);
+    if (rc) return rc;
+    DeviceGuard g(device);
     tubeworld* w = new (std::nothrow) tubeworld();
-    if (!w) return tw::fail(-3, "out of host memory");
+    if (!w) return fail(-3, "out of host memory");
     w->B = B;
     w->first_filter = first_filter;
     w->seed = seed;
@@ -326,7 +293,7 @@ int tubeworld_create(int64_t B, const tubeworld_params* p, const double* tubes_x
     if (err == cudaSuccess) err = cudaStreamSynchronize(w->stream);
     if (err != cudaSuccess) {
         cudaGetLastError();
-        int code = tw::fail((int)err, "tubeworld_create: %s", cudaGetErrorString(err));
+        int code = fail((int)err, "tubeworld_create: %s", cudaGetErrorString(err));
         tubeworld_destroy(w);
         return code;
     }
@@ -337,26 +304,26 @@ int tubeworld_create(int64_t B, const tubeworld_params* p, const double* tubes_x
 }
 
 int tubeworld_step_known(tubeworld* w) {
-    if (!w) return tw::fail(-1, "null handle");
-    tw::Dev g(w->device);
+    if (!w) return fail(-1, "null handle");
+    DeviceGuard g(w->device);
     const unsigned blocks = (unsigned)((w->B + 127) / 128);
     tw::k_step_known<<<blocks, 128, 0, w->stream>>>(w->p, w->d_tx, w->d_ty, w->n_tubes, w->seed, w->first_filter, w->B, w->tick,
                                                    11, w->R, w->calls > 0 ? 1 : 0, w->d_twists, w->d_xy, w->d_vis, w->d_truth,
                                                    w->d_odom);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     w->tick += 11;
     w->calls += 1;
     return 0;
 }
 
 int tubeworld_step_scan(tubeworld* w, int ticks, int n_beams) {
-    if (!w || ticks < 0 || n_beams < 2 || n_beams > 511) return tw::fail(-1, "invalid argument");
-    tw::Dev g(w->device);
+    if (!w || ticks < 0 || n_beams < 2 || n_beams > 511) return fail(-1, "invalid argument");
+    DeviceGuard g(w->device);
     if (n_beams > w->n_beams_cap) {
-        TCU(cudaStreamSynchronize(w->stream));
+        CU(cudaStreamSynchronize(w->stream));
         cudaFree(w->d_ranges);
         w->d_ranges = nullptr;
-        TCU(cudaMalloc((void**)&w->d_ranges, sizeof(float) * (size_t)n_beams * (size_t)w->B));
+        CU(cudaMalloc((void**)&w->d_ranges, sizeof(float) * (size_t)n_beams * (size_t)w->B));
         w->n_beams_cap = n_beams;
     }
     if (ticks > 0) {
@@ -368,13 +335,13 @@ int tubeworld_step_scan(tubeworld* w, int ticks, int n_beams) {
     const long long total = w->B * n_beams;
     tw::k_scan<<<(unsigned)((total + 127) / 128), 128, 0, w->stream>>>(w->p, w->d_tx, w->d_ty, w->n_tubes, w->seed,
                                                                      w->first_filter, w->B, w->tick, n_beams, w->R, w->d_ranges);
-    TCU(cudaGetLastError());
+    CU(cudaGetLastError());
     w->n_beams_last = n_beams;
     return 0;
 }
 
 int tubeworld_outputs(tubeworld* w, void** d_twists, void** d_xy, void** d_vis, void** d_truth, void** d_ranges) {
-    if (!w) return tw::fail(-1, "null handle");
+    if (!w) return fail(-1, "null handle");
     if (d_twists) *d_twists = w->d_twists;
     if (d_xy) *d_xy = w->d_xy;
     if (d_vis) *d_vis = w->d_vis;
@@ -384,45 +351,45 @@ int tubeworld_outputs(tubeworld* w, void** d_twists, void** d_xy, void** d_vis, 
 }
 
 int tubeworld_download(tubeworld* w, double* twists, double* xy, uint8_t* vis, double* truth, float* ranges) {
-    if (!w) return tw::fail(-1, "null handle");
-    tw::Dev g(w->device);
+    if (!w) return fail(-1, "null handle");
+    DeviceGuard g(w->device);
     const size_t B = (size_t)w->B, n = (size_t)w->p.n_slots;
-    if (twists) TCU(cudaMemcpyAsync(twists, w->d_twists, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, w->stream));
-    if (xy) TCU(cudaMemcpyAsync(xy, w->d_xy, sizeof(double) * 2 * n * B, cudaMemcpyDeviceToHost, w->stream));
-    if (vis) TCU(cudaMemcpyAsync(vis, w->d_vis, n * B, cudaMemcpyDeviceToHost, w->stream));
-    if (truth) TCU(cudaMemcpyAsync(truth, w->d_truth, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, w->stream));
+    if (twists) CU(cudaMemcpyAsync(twists, w->d_twists, sizeof(double) * 2 * B, cudaMemcpyDeviceToHost, w->stream));
+    if (xy) CU(cudaMemcpyAsync(xy, w->d_xy, sizeof(double) * 2 * n * B, cudaMemcpyDeviceToHost, w->stream));
+    if (vis) CU(cudaMemcpyAsync(vis, w->d_vis, n * B, cudaMemcpyDeviceToHost, w->stream));
+    if (truth) CU(cudaMemcpyAsync(truth, w->d_truth, sizeof(double) * 3 * B, cudaMemcpyDeviceToHost, w->stream));
     if (ranges) {
-        if (!w->d_ranges) return tw::fail(-3, "no scan has been generated yet");
-        TCU(cudaMemcpyAsync(ranges, w->d_ranges, sizeof(float) * (size_t)w->n_beams_last * B, cudaMemcpyDeviceToHost, w->stream));
+        if (!w->d_ranges) return fail(-3, "no scan has been generated yet");
+        CU(cudaMemcpyAsync(ranges, w->d_ranges, sizeof(float) * (size_t)w->n_beams_last * B, cudaMemcpyDeviceToHost, w->stream));
     }
-    TCU(cudaStreamSynchronize(w->stream));
+    CU(cudaStreamSynchronize(w->stream));
     return 0;
 }
 
 int tubeworld_odometry(tubeworld* w, void** d_odom, double* odom) {
-    if (!w) return tw::fail(-1, "null handle");
+    if (!w) return fail(-1, "null handle");
     if (d_odom) *d_odom = w->d_odom;
     if (odom) {
-        tw::Dev g(w->device);
-        TCU(cudaMemcpyAsync(odom, w->d_odom, sizeof(double) * 3 * (size_t)w->B, cudaMemcpyDeviceToHost, w->stream));
-        TCU(cudaStreamSynchronize(w->stream));
+        DeviceGuard g(w->device);
+        CU(cudaMemcpyAsync(odom, w->d_odom, sizeof(double) * 3 * (size_t)w->B, cudaMemcpyDeviceToHost, w->stream));
+        CU(cudaStreamSynchronize(w->stream));
     }
     return 0;
 }
 
 int tubeworld_sync(tubeworld* w) {
-    if (!w) return tw::fail(-1, "null handle");
-    tw::Dev g(w->device);
-    TCU(cudaStreamSynchronize(w->stream));
+    if (!w) return fail(-1, "null handle");
+    DeviceGuard g(w->device);
+    CU(cudaStreamSynchronize(w->stream));
     return 0;
 }
 void* tubeworld_stream(tubeworld* w) { return w ? (void*)w->stream : nullptr; }
 // Run the generator on the consumer's stream (e.g. ekf_batch_stream()): generation and filtering are then
 // stream-ordered and need no host synchronisation in between.
 int tubeworld_set_stream(tubeworld* w, void* stream) {
-    if (!w || !stream) return tw::fail(-1, "null argument");
-    tw::Dev g(w->device);
-    TCU(cudaStreamSynchronize(w->stream));
+    if (!w || !stream) return fail(-1, "null argument");
+    DeviceGuard g(w->device);
+    CU(cudaStreamSynchronize(w->stream));
     if (w->own_stream) cudaStreamDestroy(w->stream);
     w->stream = (cudaStream_t)stream;
     w->own_stream = false;
