@@ -93,6 +93,9 @@ SIGNATURES = {
                                       ctypes.c_void_p]),
     "ekf_batch_nees_dev": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64,
                                           ctypes.c_void_p, ctypes.c_void_p]),
+    "ekf_batch_set_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "ekf_batch_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]),
+    "ekf_batch_nis_dev": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]),
     "ekf_batch_sync": (ctypes.c_int, [ctypes.c_void_p]),
     "ekf_batch_device_pointers": (ctypes.c_int, [ctypes.c_void_p, c_void_pp, c_i64_p, c_void_pp, c_i64_p]),
     "ekf_batch_stream": (ctypes.c_void_p, [ctypes.c_void_p]),

@@ -1,4 +1,5 @@
-"""Filter consistency statistics on the host side of EKFBatch.nees() / nees_dev() (numpy and the standard library only).
+"""Filter consistency statistics on the host side of EKFBatch.nees() / nees_dev() and nis() / nis_dev() (numpy and the
+standard library only).
 
 A consistent filter's NEES (normalised estimation error squared, e^T P^-1 e) is chi-square distributed with as many
 degrees of freedom as the block it scores: 3 for the pose, 2 for a landmark.  Averaged over `runs` independent
@@ -7,7 +8,11 @@ lies inside chi2_bounds(dof, runs) with probability p; an ANEES above the interv
 
 The batch partial of ekf_batch_nees, out8 = {sum NEES_pose, sum NEES_pose^2, #pose, sum NEES_lm, sum NEES_lm^2, #lm,
 #singular pose, #singular lm}, is additive: a multi-GPU run sums the ranks' vectors with sharding.allreduce_sum and
-passes the sum to anees_from_stats."""
+passes the sum to anees_from_stats.
+
+NIS (normalised innovation squared, nu^T S^-1 nu of one range-bearing correction) needs no truth and is chi-square with
+2 degrees of freedom for a consistent filter.  The batch total of EKFBatch.nis() / ekf_batch_nis, out4 = {sum NIS,
+sum NIS^2, #scored, #non-finite}, is additive in the same way; anis_from_stats gives the ANIS and its interval."""
 from statistics import NormalDist
 
 import numpy as np
@@ -27,6 +32,22 @@ def anees_from_stats(out8):
     lm, lv = mean_var(s[3], s[4], s[5])
     return {"pose_anees": pm, "pose_nees_var": pv, "pose_count": int(s[2]), "pose_singular": int(s[6]),
             "landmark_anees": lm, "landmark_nees_var": lv, "landmark_count": int(s[5]), "landmark_singular": int(s[7])}
+
+
+def anis_from_stats(out4):
+    """NIS partial of EKFBatch.nis() / ekf_batch_nis, out4 = {sum NIS, sum NIS^2, #scored, #non-finite} (one batch, or
+    the sum over batches or ranks) -> ANIS, its sample variance, the counts, and the 95 % interval of a consistent
+    filter's ANIS over that many corrections (the NIS of one range-bearing correction is chi-square with 2 degrees of
+    freedom)."""
+    s = np.asarray(out4, dtype=np.float64).reshape(4)
+    count = int(s[2])
+    if count > 0:
+        m = s[0] / count
+        mean, var = float(m), float(s[1] / count - m * m)
+    else:
+        mean = var = float("nan")
+    return {"anis": mean, "nis_var": var, "count": count, "nonfinite": int(s[3]), "dof": 2,
+            "bounds_95": chi2_bounds(2, count)}
 
 
 def chi2_quantile(q, k):

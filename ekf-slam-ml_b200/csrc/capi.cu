@@ -55,13 +55,15 @@ int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
 
 // Batch with n <= 64, n != 20: symmetric staircase Sigma (ekf_fused_sym.cuh).
 int launch_fused_staircase(const FusedParams& p, cudaStream_t stream, int device) {
-    return launch_smem_kernel<ekf_fused_sym_kernel>(SymSmem(p.n, p.m_max).total, p, stream, device);
+    const int smem = SymSmem(p.n, p.m_max, p.nis != nullptr).total;
+    return p.nis ? launch_smem_kernel<ekf_fused_sym_kernel<true>>(smem, p, stream, device)
+                 : launch_smem_kernel<ekf_fused_sym_kernel<false>>(smem, p, stream, device);
 }
 
 // Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh).
-template <bool Assoc>
+template <bool Assoc, bool Nis>
 int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
-    const tile::TileSmem L(p.m_max, Assoc);
+    const tile::TileSmem L(p.m_max, Assoc, Nis);
     if (L.total > max_smem_optin(device))
         return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for m_max=%d", L.total, p.m_max);
     if (p.sig_stride != tile::kStride || p.st_stride != tile::kStride || p.n != tile::kNL ||
@@ -70,9 +72,9 @@ int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int
     if (p.B <= 0) return EKF_OK;
     // persistent warps: as many single-warp CTAs as fit the device at once, each walking filters b, b + grid, ...
     int per_sm = 0;
-    CU(kernel_setup<tile::ekf_fused_tile_kernel<Assoc>>(device, 32, L.total, true, &per_sm));
+    CU((kernel_setup<tile::ekf_fused_tile_kernel<Assoc, Nis>>(device, 32, L.total, true, &per_sm)));
     const long long resident = (long long)sm_count * std::max(per_sm, 1);
-    tile::ekf_fused_tile_kernel<Assoc><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
+    tile::ekf_fused_tile_kernel<Assoc, Nis><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
     CU(cudaGetLastError());
     return EKF_OK;
 }
@@ -994,6 +996,14 @@ struct ekf_batch {
     long long lm_cap = 0;
     double* d_nees_pf = nullptr;        // [B][3]
     double* d_nees_out = nullptr;       // [8]
+    // NIS (ekf_batch_set_nis): per-filter accumulators, allocated and zeroed on first use; read-out buffers
+    bool nis_on = false;
+    double* d_nis = nullptr;            // [B][4] = {sum NIS, sum NIS^2, #scored, #non-finite}
+    int nis_grid = 0;
+    double* d_nis_part = nullptr;       // [nis_grid][4] per-CTA partials of k_batch_nis
+    unsigned int* d_nis_done = nullptr;
+    double* d_nis_pf = nullptr;         // [B][4] host read-out staging
+    double* d_nis_out = nullptr;        // [4]
     cudaEvent_t t0 = nullptr, t1[3] = {nullptr, nullptr, nullptr};
 };
 
@@ -1031,6 +1041,11 @@ int free_batch(ekf_batch* b) {
     cudaFree(b->d_nees_lm);
     cudaFree(b->d_nees_pf);
     cudaFree(b->d_nees_out);
+    cudaFree(b->d_nis);
+    cudaFree(b->d_nis_part);
+    cudaFree(b->d_nis_done);
+    cudaFree(b->d_nis_pf);
+    cudaFree(b->d_nis_out);
     if (b->ev_step) cudaEventDestroy(b->ev_step);
     if (b->ev_out) cudaEventDestroy(b->ev_out);
     if (b->t0) cudaEventDestroy(b->t0);
@@ -1166,11 +1181,16 @@ int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint
     p.n = b->n;
     p.N = b->N;
     p.st_stride = b->st_stride;
-    CU(launch_wide_step(p, b->grid, b->stream, b->device));
+    p.nis = b->nis_on ? b->d_nis : nullptr;
+    if (p.nis)
+        CU(launch_wide_step<true>(p, b->grid, b->stream, b->device));
+    else
+        CU(launch_wide_step<false>(p, b->grid, b->stream, b->device));
     return EKF_OK;
 }
 
-// One step of the whole batch in the kernel of its layout, counted as one launch.  `mode` as in FusedParams; `vis`
+// One step of the whole batch in the kernel of its layout, counted as one launch; with NIS on, the NIS variant of that
+// kernel (ekf_batch_set_nis).  `mode` as in FusedParams; `vis`
 // holds the visible flags, or the marker ids with kSparseReadings; `cnt` the marker list's CSR offsets, or the
 // per-filter measurement counts of unknown association.
 int batch_launch(ekf_batch* b, int mode, int m_max, const double* tw, const double* xy, const uint8_t* vis,
@@ -1202,12 +1222,15 @@ int batch_launch(ekf_batch* b, int mode, int m_max, const double* tw, const doub
         p.sig_stride = b->sig_stride;
         p.st_stride = b->st_stride;
         p.sparse_total = total;
+        p.nis = b->nis_on ? b->d_nis : nullptr;
         if (b->layout == Layout::Stair)
             rc = launch_fused_staircase(p, b->stream, b->device);
         else if (association)
-            rc = launch_fused_tile<true>(p, b->stream, b->device, b->sm_count);
+            rc = p.nis ? launch_fused_tile<true, true>(p, b->stream, b->device, b->sm_count)
+                       : launch_fused_tile<true, false>(p, b->stream, b->device, b->sm_count);
         else
-            rc = launch_fused_tile<false>(p, b->stream, b->device, b->sm_count);
+            rc = p.nis ? launch_fused_tile<false, true>(p, b->stream, b->device, b->sm_count)
+                       : launch_fused_tile<false, false>(p, b->stream, b->device, b->sm_count);
     }
     b->launches += 1;
     return rc;
@@ -1283,6 +1306,31 @@ int launch_consistency(ekf_batch* b, const double* truth, const double* lm_truth
     if (b->layout == Layout::Wide) return launch_consistency_at(b, p, WideAt{b->d_sigma, b->sig_stride, b->ld});
     if (b->layout == Layout::Tile) return launch_consistency_at(b, p, TileAt{b->d_sigma});
     return launch_consistency_at(b, p, StairAt{b->d_sigma, b->sig_stride, b->N});
+}
+
+// One launch of k_batch_nis on the compute stream; the grid is fixed for the handle, so the reduction order is too.
+int launch_nis(ekf_batch* b, double* per_filter, double* out4, int reset) {
+    if (!b->nis_grid) {
+        int per_sm = 0;
+        CU(kernel_setup<k_batch_nis>(b->device, kConsWarps * 32, 0, false, &per_sm));
+        const long long resident = (long long)std::max(b->sm_count, 1) * std::max(per_sm, 1);
+        const int grid = (int)std::min<long long>((b->B + kConsWarps * 32 - 1) / (kConsWarps * 32), resident);
+        CU(cudaMalloc(&b->d_nis_part, sizeof(double) * 4 * (size_t)grid));
+        CU(cudaMalloc(&b->d_nis_done, sizeof(unsigned int)));
+        CU(cudaMemsetAsync(b->d_nis_done, 0, sizeof(unsigned int), b->stream));
+        b->nis_grid = grid;
+    }
+    k_batch_nis<<<b->nis_grid, kConsWarps * 32, 0, b->stream>>>(b->d_nis, b->B, per_filter, reset != 0, b->d_nis_part,
+                                                              b->d_nis_done, out4);
+    b->launches += 1;
+    CU(cudaGetLastError());
+    return EKF_OK;
+}
+
+int check_nis_args(ekf_batch* b, const double* out4) {
+    if (!b || !out4) return fail(EKF_ERR_INVALID, "null argument");
+    if (!b->d_nis) return fail(EKF_ERR_STATE, "NIS was never enabled on this batch (ekf_batch_set_nis)");
+    return EKF_OK;
 }
 
 int check_nees_args(ekf_batch* b, const double* truth, int64_t lm_truth_stride, const double* out8) {
@@ -1610,6 +1658,36 @@ int ekf_batch_nees_dev(ekf_batch* b, const double* d_truth, const double* d_lm_t
     if (rc) return rc;
     DeviceGuard g(b->device);
     return launch_consistency(b, d_truth, d_lm_truth, lm_truth_stride, d_per_filter, nullptr, nullptr, d_out8);
+}
+int ekf_batch_set_nis(ekf_batch* b, int on) {
+    if (!b) return fail(EKF_ERR_INVALID, "null handle");
+    DeviceGuard g(b->device);
+    if (on && !b->d_nis) {
+        CU(cudaMalloc(&b->d_nis, sizeof(double) * 4 * (size_t)b->B));
+        CU(cudaMemsetAsync(b->d_nis, 0, sizeof(double) * 4 * (size_t)b->B, b->stream));
+    }
+    b->nis_on = on != 0;
+    return EKF_OK;
+}
+int ekf_batch_nis(ekf_batch* b, double* per_filter, double* out4, int reset) {
+    int rc = check_nis_args(b, out4);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    const size_t B = (size_t)b->B;
+    if (per_filter && !b->d_nis_pf) CU(cudaMalloc(&b->d_nis_pf, sizeof(double) * 4 * B));
+    if (!b->d_nis_out) CU(cudaMalloc(&b->d_nis_out, sizeof(double) * 4));
+    rc = launch_nis(b, per_filter ? b->d_nis_pf : nullptr, b->d_nis_out, reset);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out4, b->d_nis_out, sizeof(double) * 4, cudaMemcpyDeviceToHost, b->stream));
+    if (per_filter) CU(cudaMemcpyAsync(per_filter, b->d_nis_pf, sizeof(double) * 4 * B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    return EKF_OK;
+}
+int ekf_batch_nis_dev(ekf_batch* b, double* d_per_filter, double* d_out4, int reset) {
+    int rc = check_nis_args(b, d_out4);
+    if (rc) return rc;
+    DeviceGuard g(b->device);
+    return launch_nis(b, d_per_filter, d_out4, reset);
 }
 int ekf_batch_sync(ekf_batch* b) {
     if (!b) return fail(EKF_ERR_INVALID, "null handle");

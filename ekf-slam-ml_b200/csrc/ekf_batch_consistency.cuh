@@ -10,6 +10,8 @@
 // Only stored entries (r <= c) are read, through the layouts' own index helpers, so every value is bit-identical to
 // entry (r, c) of ekf_batch_get_sigma().  The kernel reads Sigma, the state, the init flags and the known lists and
 // writes nothing the filters own.
+// k_batch_nis reads out the NIS accumulators the step kernels' NIS variants keep (ekf_batch_set_nis), with the same
+// fixed-order reduction (reduce_batch_partials).
 #pragma once
 #include "ekf_fused_sym.cuh"
 #include "ekf_fused_tile.cuh"
@@ -33,7 +35,42 @@ struct WideAt {  // 64 < n <= 1,024: dense N x ld rows, upper triangle (ekf_batc
     __device__ double operator()(long long b, int r, int c) const { return sigma[b * stride + r * ld + c]; }
 };
 
-constexpr int kConsWarps = 8;  // warps per CTA of k_batch_consistency
+constexpr int kConsWarps = 8;  // warps per CTA of k_batch_consistency and k_batch_nis
+
+// Batch total of K per-lane partials in a fixed order: warp (shuffle tree), then the kConsWarps warps of the CTA in index
+// order into partials[blockIdx.x][K], then CTAs in index order by the last CTA to finish, into out[K].  `done` counts
+// finished CTAs and is zero between launches (the last CTA resets it).  Every thread of the CTA calls this, with
+// lane = threadIdx.x % 32 and warp = threadIdx.x / 32.
+template <int K>
+__device__ __forceinline__ void reduce_batch_partials(const double (&acc)[K], const int lane, const int warp,
+                                                      double* partials, unsigned int* done, double* out) {
+    __shared__ double red[kConsWarps][K];
+    __shared__ bool last;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        double v = acc[k];
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+        if (lane == 0) red[warp][k] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < K) {
+        double s = 0.0;
+        for (int w = 0; w < kConsWarps; ++w) s += red[w][threadIdx.x];
+        partials[K * blockIdx.x + threadIdx.x] = s;
+        __threadfence();
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) last = atomicAdd(done, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    if (threadIdx.x < K) {
+        double s = 0.0;
+        for (unsigned g = 0; g < gridDim.x; ++g) s += __ldcg(partials + K * g + threadIdx.x);
+        out[threadIdx.x] = s;
+    }
+    if (threadIdx.x == 0) *done = 0;
+}
 
 struct ConsistencyParams {
     const double* state;       // [B][st_stride]: theta, x, y, m1x, m1y, ...
@@ -124,33 +161,32 @@ __global__ void __launch_bounds__(kConsWarps * 32) k_batch_consistency(Consisten
         }
     }
     if (!p.out8) return;
-    // warp (shuffle tree), then warps in index order, then CTAs in index order
-    __shared__ double red[kConsWarps][8];
-    __shared__ bool last;
+    reduce_batch_partials<8>(acc, lane, warp, p.partials, p.done, p.out8);
+}
+
+// NIS read-out of a batch (ekf_batch_nis): the [B][4] accumulators {sum NIS, sum NIS^2, #scored, #non-finite} that
+// the step kernels' NIS variants keep, copied to per_filter (optional) and summed over the batch in the fixed order of
+// reduce_batch_partials: each thread adds its filters b = thread, thread + threads, ... in filter order first.  reset
+// zeroes the accumulators after they were read (each filter is read and cleared by the same thread).
+__global__ void __launch_bounds__(kConsWarps * 32) k_batch_nis(double* acc4, long long B, double* per_filter,
+                                                               int reset, double* partials, unsigned int* done,
+                                                               double* out4) {
+    double acc[4] = {0, 0, 0, 0};
+    for (long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
+        double v[4];
 #pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        double v = acc[k];
-        for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-        if (lane == 0) red[warp][k] = v;
+        for (int k = 0; k < 4; ++k) {
+            v[k] = acc4[4 * b + k];
+            acc[k] += v[k];
+        }
+        if (per_filter)
+#pragma unroll
+            for (int k = 0; k < 4; ++k) per_filter[4 * b + k] = v[k];
+        if (reset)
+#pragma unroll
+            for (int k = 0; k < 4; ++k) acc4[4 * b + k] = 0.0;
     }
-    __syncthreads();
-    if (threadIdx.x < 8) {
-        double s = 0.0;
-        for (int w = 0; w < kConsWarps; ++w) s += red[w][threadIdx.x];
-        p.partials[8 * blockIdx.x + threadIdx.x] = s;
-        __threadfence();
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) last = atomicAdd(p.done, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!last) return;
-    __threadfence();
-    if (threadIdx.x < 8) {
-        double s = 0.0;
-        for (unsigned g = 0; g < gridDim.x; ++g) s += __ldcg(p.partials + 8 * g + threadIdx.x);
-        p.out8[threadIdx.x] = s;
-    }
-    if (threadIdx.x == 0) *p.done = 0;
+    reduce_batch_partials<4>(acc, threadIdx.x & 31, threadIdx.x >> 5, partials, done, out4);
 }
 
 }  // namespace ekf

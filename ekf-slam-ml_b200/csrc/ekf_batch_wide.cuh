@@ -37,6 +37,7 @@ struct WideParams {
     long long ld;
     long long slot_stride;  // double2 per CTA in Kp / Wp
     int n, N, st_stride;
+    double* nis;  // [B][4] NIS accumulators of k_wide_step<true> (nis() / nis_add())
 };
 
 // dynamic shared memory: the sweep's stage ring, then the readings [2n] and visible flags [n] of the current filter
@@ -58,6 +59,9 @@ __device__ __forceinline__ void wide_sweep(double* sig, long long ld, int N, con
     __syncthreads();
 }
 
+// NIS: also accumulate the NIS of the step's corrections (none on a filter's first call) into p.nis[b]; thread 0 keeps
+// the running sums in shared memory.
+template <bool NIS>
 __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* zxy = reinterpret_cast<double*>(smem_raw + WideTile::kSmemBytes);
@@ -65,6 +69,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
     __shared__ GainSharedP g;
     __shared__ double s_a[2], s_pose[3];
     __shared__ int s_init;
+    __shared__ double s_nis[4];
     // per-CTA loop state of the corrections, and the sweep ring's position per role (producer, consumers, storer)
     __shared__ struct {
         int i, pending, dirty;
@@ -180,6 +185,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
             L.pending = 0;
             L.corrections = 0;
             L.sweeps = 0;
+            if (NIS) s_nis[0] = s_nis[1] = s_nis[2] = s_nis[3] = 0.0;
         }
         __syncthreads();
         for (;;) {
@@ -202,6 +208,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
                                g);
                 }
                 __syncthreads();
+                if (NIS && tid == 0 && s_init) nis_add(s_nis, nis(g.si, g.nu0, g.nu1));
                 double2* Kout = Kp + (long long)pending * ld;
                 double2* Wout = Wp + (long long)pending * ld;
                 const long long i3l = (long long)i3 * ld;
@@ -252,6 +259,9 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
         if (tid == 0 && L.corrections) {
             atomicAdd(p.n_updates, L.corrections);
             atomicAdd(p.n_sweeps, L.sweeps);
+            if (NIS) {
+                for (int k = 0; k < 4; ++k) p.nis[4 * b + k] += s_nis[k];
+            }
         }
         __syncthreads();  // zxy / zvis are refilled for the next filter
     }
@@ -259,10 +269,11 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
 }
 
 // One step of the whole batch on `device`.  grid = the number of CTAs the factor slots were allocated for.
+template <bool NIS>
 inline cudaError_t launch_wide_step(const WideParams& p, int grid, cudaStream_t stream, int device) {
-    const cudaError_t e = kernel_setup<k_wide_step>(device, kTmaThreads, wide_smem_bytes(kWideMaxN), false);
+    const cudaError_t e = kernel_setup<k_wide_step<NIS>>(device, kTmaThreads, wide_smem_bytes(kWideMaxN), false);
     if (e != cudaSuccess) return e;
-    k_wide_step<<<(unsigned)grid, kTmaThreads, wide_smem_bytes(p.n), stream>>>(p);
+    k_wide_step<NIS><<<(unsigned)grid, kTmaThreads, wide_smem_bytes(p.n), stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -37,6 +37,7 @@ struct FusedParams {
     int sig_stride;  // doubles
     int st_stride;   // doubles
     long long sparse_total;  // marker-list mode: number of listed markers (offsets are checked against it)
+    double* nis;             // [B][4] NIS accumulators of the batch kernels' NIS variants (nis() / nis_add())
 };
 
 __host__ __device__ inline int fused_round16(int v) { return (v + 15) & ~15; }
@@ -264,7 +265,8 @@ __device__ __forceinline__ int fused_assoc_inputs(const FusedParams& p, const lo
 // data_association(): Mahalanobis nearest neighbour + landmark initialisation (ekf_slam.cpp:278-402) for the m
 // readings in zbuf.  The Sigma layout enters through two calls only:
 //   dist(i, zr, zphi, theta, x, y)  distance of known landmark i (each lane scans its own landmarks);
-//   correct(i, h, zr, zphi)         gain, state update and rank-2 update of landmark i (whole warp; h from the live pose).
+//   correct(i, h, zr, zphi, created) gain, state update and rank-2 update of landmark i (whole warp; h from the live
+//                                    pose); `created` is set when this very reading initialised the landmark.
 template <class Dist, class Correct>
 __device__ __forceinline__ void fused_association(const FusedParams& p, const long long b, const int n, const int m,
                                                   const int lane, double* st, const double* zbuf,
@@ -344,7 +346,7 @@ __device__ __forceinline__ void fused_association(const FusedParams& p, const lo
         if (min_d < kGateUpdate) {  // :330
             const double th_l = st[0], x_l = st[1], y_l = st[2];  // live pose (:331-333)
             const Hj h = make_hj(st[3 + 2 * min_idx], st[4 + 2 * min_idx], th_l, x_l, y_l);
-            correct(min_idx, h, zr, zphi);  // the next distances need the new Sigma
+            correct(min_idx, h, zr, zphi, created);  // the next distances need the new Sigma
             ++n_corr;
             assoc = min_idx;
         }
@@ -481,7 +483,7 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
             [&](int i, double zr, double zphi, double theta, double x, double y) {
                 return maha_distance(sig, N, i, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y);
             },
-            [&](int i, const Hj& h, double zr, double zphi) {
+            [&](int i, const Hj& h, double zr, double zphi, int) {
                 warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, i, h, zr, zphi);
                 warp_rank2<NL, 1>(sig, K2, W2, nullptr, nullptr, N, lane);
             });

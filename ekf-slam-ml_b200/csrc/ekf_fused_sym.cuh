@@ -37,8 +37,8 @@ __host__ __device__ constexpr int sym_sig_stride(int N) { return (stair_size(N) 
 __host__ __device__ constexpr int sym_st_stride(int N) { return (N + 1) & ~1; }
 
 struct SymSmem {
-    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, total;
-    __host__ __device__ SymSmem(int n, int m_max) {
+    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_nis, total;
+    __host__ __device__ SymSmem(int n, int m_max, bool nis = false) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;
@@ -59,6 +59,8 @@ struct SymSmem {
         o += zc * 8;  // n = 20: 13,536 B per CTA: 16 CTAs of 13,568 B (+1 KB reserve each) fit one SM's 228 KB
         off_bar = o;
         o += 16;
+        off_nis = o;  // NIS only: the step's sums {sum, sum^2, #scored, #non-finite}, kept by lane 0
+        o += nis ? 4 * 8 : 0;
         total = o;
     }
 };
@@ -68,9 +70,10 @@ constexpr int kSymSlots = 5;  // column slots per lane (n <= 64 -> N <= 131)
 // Gain of one correction from five ROWS of the symmetric Sigma: W = Hj Sigma -> Wout, K = W^T S^-1 -> Kout,
 // state += K nu.  With PEND the stored Sigma still misses the previous correction's factor (Kpend, Wpend); the
 // entries read here are rebuilt with the FMAs the rank-2 pass will apply to them (in their stored orientation).
-// cmv[s] = offset of the mirror row of the lane's column slot s (loop invariant, computed once per launch).
+// cmv[s] = offset of the mirror row of the lane's column slot s (loop invariant, computed once per launch).  Returns
+// S^-1 (warp-uniform) for the NIS of the correction.
 template <bool PEND, class H>
-__device__ __forceinline__ void sym_warp_gain(const double* __restrict__ sig, double* __restrict__ st,
+__device__ __forceinline__ Sym2 sym_warp_gain(const double* __restrict__ sig, double* __restrict__ st,
                                               const double2* __restrict__ Kpend, const double2* __restrict__ Wpend,
                                               double2* __restrict__ Kout, double2* __restrict__ Wout, const int N,
                                               const int lane, const int* __restrict__ cmv, const int i, const H h,
@@ -134,6 +137,7 @@ __device__ __forceinline__ void sym_warp_gain(const double* __restrict__ sig, do
         }
     }
     __syncwarp();
+    return si;
 }
 
 // Sigma <- Sigma - Ka Wa [- Kb Wb] over the stored entries, block row by block row (rows 16 rb .. 16 rb + 15,
@@ -208,11 +212,14 @@ static __device__ __noinline__ void landmark_from_reading_cold(double sx, double
     landmark_from_reading(sx, sy, theta, x, y, mx, my);
 }
 
+// NIS: also accumulate the NIS of the step's scored corrections into p.nis[b]; lane 0 keeps the running sums in shared
+// memory, not in registers.
+template <bool NIS>
 __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int n = p.n;
     const int N = 3 + 2 * n;
-    const SymSmem L(n, p.m_max);
+    const SymSmem L(n, p.m_max, NIS);
     double* sig = reinterpret_cast<double*>(smem_raw + L.off_sig);
     double* st = reinterpret_cast<double*>(smem_raw + L.off_st);
     double2* K2 = reinterpret_cast<double2*>(smem_raw + L.off_k2);
@@ -221,6 +228,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
     double2* W2b = reinterpret_cast<double2*>(smem_raw + L.off_w2b);
     double* zbuf = reinterpret_cast<double*>(smem_raw + L.off_z);
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + L.off_bar);
+    double* nacc = reinterpret_cast<double*>(smem_raw + L.off_nis);
 
     const int lane = threadIdx.x;
     const long long b = blockIdx.x;
@@ -228,6 +236,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
     double* g_sig = p.sigma + b * (long long)p.sig_stride;
     double* g_st = p.state + b * (long long)p.st_stride;
     const uint32_t sig_bytes = (uint32_t)p.sig_stride * 8u, st_bytes = (uint32_t)p.st_stride * 8u;
+    if (NIS && lane == 0) nacc[0] = nacc[1] = nacc[2] = nacc[3] = 0.0;
 
     int cmv[kSymSlots];  // mirror-row offsets of this lane's column slots (see sym_warp_gain)
 #pragma unroll
@@ -309,6 +318,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
     // ---- measurement(): known association (ekf_slam.cpp:108-197)
     if (p.mode & kDoMeasurement) {
         const double theta = st[0], x = st[1], y = st[2];  // read once; stale for later i (:109-111)
+        const bool score = init_flag != 0;  // the first call's readings initialised every landmark: nu ~ 0
         if (!init_flag) {
             if (p.mode & kSparseReadings) {
                 // unlisted slots read (0, 0): the landmark starts at the robot's position, as with dense zeros
@@ -355,10 +365,12 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
             while (rem) {
                 const int ic = base + __ffs(rem) - 1;
                 rem &= rem - 1;
+                Sym2 si;
                 if (!second)
-                    sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, ic, h, h.nu0, h.nu1);
+                    si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, ic, h, h.nu0, h.nu1);
                 else
-                    sym_warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, cmv, ic, h, h.nu0, h.nu1);
+                    si = sym_warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, cmv, ic, h, h.nu0, h.nu1);
+                if (NIS && score && lane == 0) nis_add(nacc, nis(si, h.nu0, h.nu1));
                 ++n_corr;
                 if (rem) {
                     const int in = base + __ffs(rem) - 1;
@@ -382,9 +394,10 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
                 const double rob[6] = {sig[0], sig[1], sig[2], sig[N + 1], sig[N + 2], sig[2 * N + 2]};
                 return sym_maha_distance(sig, N, i, rob, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y);
             },
-            [&](int i, const Hj& h, double zr, double zphi) {
-                sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, i, h, __dsub_rn(zr, h.zr),
-                                     normalize_angle(__dsub_rn(zphi, h.zphi)));  // :182-183
+            [&](int i, const Hj& h, double zr, double zphi, int created) {
+                const double nu0 = __dsub_rn(zr, h.zr), nu1 = normalize_angle(__dsub_rn(zphi, h.zphi));  // :182-183
+                const Sym2 si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, i, h, nu0, nu1);
+                if (NIS && !created && lane == 0) nis_add(nacc, nis(si, nu0, nu1));  // a new landmark starts at its reading
                 sym_warp_rank2<1>(sig, K2, W2, nullptr, nullptr, N, lane);
             });
     }
@@ -399,6 +412,10 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
         bulk_commit();
         p.init_flag[b] = init_flag;
         if (p.n_updates && n_corr) atomicAdd(p.n_updates, n_corr);
+        if (NIS) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) p.nis[4 * b + k] += nacc[k];
+        }
         bulk_wait_read();  // shared memory must outlive the copy engine's reads; the writes drain with the grid
     }
 }

@@ -237,6 +237,25 @@ __device__ __forceinline__ Sym2 inv2x2(double s00, double s01, double s10, doubl
     return r;
 }
 
+// Normalised innovation squared nu^T S^-1 nu of one correction, from exactly the S^-1 and nu its gain uses (the batch
+// engines' NIS variants).  Every product and sum is rounded on its own, so a host restatement without FMA contraction
+// gives the same value from the same inputs.
+__device__ __forceinline__ double nis(const Sym2& si, double nu0, double nu1) {
+    const double t0 = __dadd_rn(__dmul_rn(si.i00, nu0), __dmul_rn(si.i10, nu1));
+    const double t1 = __dadd_rn(__dmul_rn(si.i01, nu0), __dmul_rn(si.i11, nu1));
+    return __dadd_rn(__dmul_rn(nu0, t0), __dmul_rn(nu1, t1));
+}
+// acc = {sum NIS, sum NIS^2, #scored, #non-finite}: a value that is not finite is counted in acc[3] only
+__device__ __forceinline__ void nis_add(double* acc, double v) {
+    if (isfinite(v)) {
+        acc[0] = __dadd_rn(acc[0], v);
+        acc[1] = __dadd_rn(acc[1], __dmul_rn(v, v));
+        acc[2] += 1.0;
+    } else {
+        acc[3] += 1.0;
+    }
+}
+
 // Mahalanobis distance of measurement (zr, zphi) to landmark i, from the 5x5 block Sigma[idx, idx]
 // (ekf_slam.cpp:217-276).  The bearing innovation is NOT wrapped (:269).  `sig` may point to shared or
 // global memory; ld is the row stride in doubles.

@@ -521,6 +521,33 @@ class EKFBatch:
                                          int(lm_truth_stride), int(d_per_filter) if d_per_filter else None,
                                          int(d_out8) if d_out8 else None))
 
+    def set_nis(self, on=True):
+        """ekf_batch_set_nis: with on, the following steps also accumulate every filter's normalised innovation squared
+        (NIS = nu^T S^-1 nu of each scored correction; the accumulators are allocated and zeroed on first use); with
+        off, the plain step kernels run again and the accumulators are kept.  Checkpoints do not carry them."""
+        check(self._L.ekf_batch_set_nis(self._h, 1 if on else 0))
+
+    def nis(self, per_filter=False, reset=False):
+        """NIS read-out, the consistency test that needs no truth: consistency.anis_from_stats() of the batch total
+        {sum NIS, sum NIS^2, #scored, #non-finite} (also returned as "stats"; additive across ranks), and with
+        per_filter the arrays "nis_sum", "nis_sq_sum", "nis_count" and "nis_nonfinite" [B].  reset zeroes the
+        accumulators after the read.  Raises before set_nis() was ever called."""
+        from .consistency import anis_from_stats
+        pf = np.empty((self.B, 4)) if per_filter else None
+        out = np.zeros(4)
+        check(self._L.ekf_batch_nis(self._h, pf.ctypes.data if per_filter else None, out.ctypes.data, 1 if reset else 0))
+        res = anis_from_stats(out)
+        res["stats"] = out
+        if per_filter:
+            res["nis_sum"], res["nis_sq_sum"], res["nis_count"], res["nis_nonfinite"] = pf[:, 0], pf[:, 1], pf[:, 2], pf[:, 3]
+        return res
+
+    def nis_dev(self, d_out4, d_per_filter=None, reset=False):
+        """ekf_batch_nis_dev: the same read-out into device pointers (out4 [4], per-filter [B][4]), enqueued on the
+        batch's stream without a synchronisation; the results are valid after sync()."""
+        check(self._L.ekf_batch_nis_dev(self._h, int(d_per_filter) if d_per_filter else None,
+                                        int(d_out4) if d_out4 else None, 1 if reset else 0))
+
     def sync(self):
         check(self._L.ekf_batch_sync(self._h))
 

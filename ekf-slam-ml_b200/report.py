@@ -43,6 +43,7 @@ def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0)
     sim = pkg.TubeWorld(world, robots, seed=seed, device=device)
     slam = pkg.EKFBatch(robots, n, device=device)
     blind = pkg.EKFBatch(robots, n, device=device)
+    slam.set_nis(True)  # innovation consistency of every correction, on the device
     sim.use_stream(slam.stream)
     p = sim.device_pointers()
     no_vis = torch.zeros(robots * n, dtype=torch.uint8, device=f"cuda:{device}")
@@ -81,6 +82,9 @@ def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0)
     ns, nb = slam.nees(truth, lm_truth)["stats"], blind.nees(truth)["stats"]
     out["consistency"] = {"slam": {"pose": _anees(cs, ns, "pose", 3), "landmarks": _anees(cs, ns, "landmark", 2)},
                           "prediction_only": {"pose": _anees(cs, nb, "pose", 3)}}
+    ni = slam.nis()
+    out["consistency"]["slam"]["innovations"] = {"anis": ni["anis"], "dof": 2, "bounds_95": list(ni["bounds_95"]),
+                                                 "corrections": ni["count"], "nonfinite": ni["nonfinite"]}
     if series_at:
         out["consistency"]["pose_anees_series"] = {
             "steps": series_at, "anees": [cs.anees_from_stats(v)["pose_anees"] for v in series.cpu().numpy()]}
@@ -106,8 +110,15 @@ def markdown(r):
             e = c[key][block]
             rows.append(f"{name} | {block} | {e['dof']} | {e['anees']:.3f} | {e['bounds_95'][0]:.3f} .. "
                         f"{e['bounds_95'][1]:.3f} | {e['runs']} | {e['singular']}")
+        e = c["slam"].get("innovations")
+        if e:  # NIS needs no truth: ANIS over every scored correction (columns: ANIS, corrections, non-finite)
+            rows.append(f"Slam | innovations | {e['dof']} | {e['anis']:.3f} | {e['bounds_95'][0]:.3f} .. "
+                        f"{e['bounds_95'][1]:.3f} | {e['corrections']} | {e['nonfinite']}")
         text += ("\n\nANEES: mean NEES over the runs; a consistent filter lies inside the interval, an overconfident one "
                  "above it.\n\n" + "\n".join(rows))
+        if e:
+            text += ("\n\nInnovations: ANIS, the mean NIS over every scored correction (needs no truth); its runs column "
+                     "counts corrections, its singular column non-finite values.")
         sr = c.get("pose_anees_series")
         if sr:
             text += "\n\nSlam pose ANEES by step: " + ", ".join(f"{t}: {v:.3f}" for t, v in zip(sr["steps"], sr["anees"]))

@@ -208,6 +208,24 @@ int ekf_batch_nees(ekf_batch* b, const double* truth, const double* lm_truth, in
  * synchronised: the results are valid after ekf_batch_sync(), so a per-step series costs no host round trip. */
 int ekf_batch_nees_dev(ekf_batch* b, const double* d_truth, const double* d_lm_truth, int64_t lm_truth_stride,
                        double* d_per_filter, double* d_out8);
+/* Normalised innovation squared, the consistency test that needs no truth.  Per correction NIS = nu^T S^-1 nu with
+ * nu = (z_r - zhat_r, wrap(z_phi - zhat_phi)) and S = H_j Sigma H_j^T + R, from exactly the S^-1 and nu of the
+ * correction's gain (known association: entry-time pose; unknown: live pose); chi^2(2) for a consistent filter.  Every
+ * correction a step applies is scored, except those of a filter's first measurement (landmark_init_flag == 0 at step
+ * entry) and, with unknown association, that of a landmark created by the same reading (nu ~ 0 in both).  Per filter
+ * the kernel sums the step's values in correction order and adds them to {sum NIS, sum NIS^2, #scored, #non-finite};
+ * a value that is not finite counts in #non-finite only.  No floating-point atomics: replicas of one trajectory get
+ * bit-identical accumulators.
+ *
+ * 1: the following steps run the NIS variants of the step kernels and accumulate per filter (allocated and zeroed on
+ * first use); 0: the plain kernels again, accumulators kept.  Not part of checkpoints: export / import ignore them. */
+int ekf_batch_set_nis(ekf_batch* b, int on);
+/* per_filter [B][4] = {sum NIS, sum NIS^2, #scored, #non-finite} (optional), out4 = the same summed over the batch in a
+ * fixed order (additive across ranks).  reset != 0 zeroes the accumulators after the read.  EKF_ERR_STATE before NIS
+ * was ever enabled.  HOST buffers; synchronises. */
+int ekf_batch_nis(ekf_batch* b, double* per_filter, double* out4, int reset);
+/* the same with DEVICE pointers, enqueued on ekf_batch_stream(), no synchronisation (a per-step series with reset = 1) */
+int ekf_batch_nis_dev(ekf_batch* b, double* d_per_filter, double* d_out4, int reset);
 int ekf_batch_sync(ekf_batch* b);
 /* Raw device arrays of the batch.  state: [B][state_stride] doubles (theta, x, y, m1x, m1y, ...).  sigma:
  * [B][sigma_stride] doubles in the engine's layout:
