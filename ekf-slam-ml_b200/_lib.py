@@ -59,6 +59,8 @@ SIGNATURES = {
     "ekf_launch_count": (ctypes.c_int, [ctypes.c_void_p, c_u64_p]),
     "ekf_sweep_count": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint64)]),
     "ekf_set_carry_pending": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "ekf_set_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
+    "ekf_get_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_set_max_pending": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "ekf_batch_create": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_void_pp]),
     "ekf_batch_destroy": (ctypes.c_int, [ctypes.c_void_p]),
@@ -96,6 +98,8 @@ SIGNATURES = {
     "ekf_batch_set_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "ekf_batch_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]),
     "ekf_batch_nis_dev": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]),
+    "ekf_batch_set_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64]),
+    "ekf_batch_get_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_batch_sync": (ctypes.c_int, [ctypes.c_void_p]),
     "ekf_batch_device_pointers": (ctypes.c_int, [ctypes.c_void_p, c_void_pp, c_i64_p, c_void_pp, c_i64_p]),
     "ekf_batch_stream": (ctypes.c_void_p, [ctypes.c_void_p]),

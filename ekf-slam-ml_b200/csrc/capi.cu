@@ -22,6 +22,8 @@
 
 using namespace ekf;
 
+static_assert(kQ == EKF_DEFAULT_Q && kR == EKF_DEFAULT_R, "the kernels' default noise is the header's");
+
 namespace {
 
 constexpr int kFusedMaxN = 64;  // landmarks; Sigma (131^2 fp64 = 137 KB) must fit shared memory
@@ -46,24 +48,34 @@ int launch_smem_kernel(int smem, const FusedParams& p, cudaStream_t stream, int 
     return EKF_OK;
 }
 
-// Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.
+// Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.  With p.noise, the NOISE
+// variant.
+template <bool NoiseOn>
+int launch_fused_nz(const FusedParams& p, cudaStream_t stream, int device) {
+    const int smem = FusedSmem(p.n, p.m_max, NoiseOn).total;
+    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20, NoiseOn>>(smem, p, stream, device)
+                     : launch_smem_kernel<ekf_fused_kernel<0, NoiseOn>>(smem, p, stream, device);
+}
 int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
-    const int smem = FusedSmem(p.n, p.m_max).total;
-    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20>>(smem, p, stream, device)
-                     : launch_smem_kernel<ekf_fused_kernel<0>>(smem, p, stream, device);
+    return p.noise ? launch_fused_nz<true>(p, stream, device) : launch_fused_nz<false>(p, stream, device);
 }
 
 // Batch with n <= 64, n != 20: symmetric staircase Sigma (ekf_fused_sym.cuh).
+template <bool Nis>
+int launch_fused_staircase_nis(const FusedParams& p, cudaStream_t stream, int device) {
+    return p.noise ? launch_smem_kernel<ekf_fused_sym_kernel<Nis, true>>(SymSmem(p.n, p.m_max, Nis, true).total, p, stream,
+                                                                        device)
+                   : launch_smem_kernel<ekf_fused_sym_kernel<Nis, false>>(SymSmem(p.n, p.m_max, Nis).total, p, stream,
+                                                                         device);
+}
 int launch_fused_staircase(const FusedParams& p, cudaStream_t stream, int device) {
-    const int smem = SymSmem(p.n, p.m_max, p.nis != nullptr).total;
-    return p.nis ? launch_smem_kernel<ekf_fused_sym_kernel<true>>(smem, p, stream, device)
-                 : launch_smem_kernel<ekf_fused_sym_kernel<false>>(smem, p, stream, device);
+    return p.nis ? launch_fused_staircase_nis<true>(p, stream, device) : launch_fused_staircase_nis<false>(p, stream, device);
 }
 
 // Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh).
-template <bool Assoc, bool Nis>
+template <bool Assoc, bool Nis, bool NoiseOn>
 int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
-    const tile::TileSmem L(p.m_max, Assoc, Nis);
+    const tile::TileSmem L(p.m_max, Assoc, Nis, NoiseOn);
     if (L.total > max_smem_optin(device))
         return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for m_max=%d", L.total, p.m_max);
     if (p.sig_stride != tile::kStride || p.st_stride != tile::kStride || p.n != tile::kNL ||
@@ -72,11 +84,16 @@ int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int
     if (p.B <= 0) return EKF_OK;
     // persistent warps: as many single-warp CTAs as fit the device at once, each walking filters b, b + grid, ...
     int per_sm = 0;
-    CU((kernel_setup<tile::ekf_fused_tile_kernel<Assoc, Nis>>(device, 32, L.total, true, &per_sm)));
+    CU((kernel_setup<tile::ekf_fused_tile_kernel<Assoc, Nis, NoiseOn>>(device, 32, L.total, true, &per_sm)));
     const long long resident = (long long)sm_count * std::max(per_sm, 1);
-    tile::ekf_fused_tile_kernel<Assoc, Nis><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
+    tile::ekf_fused_tile_kernel<Assoc, Nis, NoiseOn><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
     CU(cudaGetLastError());
     return EKF_OK;
+}
+template <bool Assoc, bool Nis>
+int launch_fused_tile_nis(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
+    return p.noise ? launch_fused_tile<Assoc, Nis, true>(p, stream, device, sm_count)
+                   : launch_fused_tile<Assoc, Nis, false>(p, stream, device, sm_count);
 }
 
 // Sigma0 = blockdiag(0_3, 100 I) (ekf_slam.cpp:29-36) for B filters of an already-zeroed buffer: dense rows of stride
@@ -88,11 +105,52 @@ __global__ void k_init_sigma(double* __restrict__ sigma, long long B, int N, lon
     sigma[b * stride + k * ld + k] = kSigma0;
 }
 
-__global__ void k_maha_one(const double* sig, long long ld, const double* state, int i, double sx, double sy,
-                           double* out) {
+__device__ __forceinline__ void maha_one(const double* sig, long long ld, const double* state, int i, double sx,
+                                         double sy, double* out, const Noise& nz) {
     double zr, zphi;
     range_bearing(sx, sy, zr, zphi);
-    *out = maha_distance(sig, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, state[0], state[1], state[2]);
+    *out = maha_distance(sig, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, state[0], state[1], state[2], nz);
+}
+__global__ void k_maha_one(const double* sig, long long ld, const double* state, int i, double sx, double sy,
+                           double* out) {
+    maha_one(sig, ld, state, i, sx, sy, out, ref_noise());
+}
+
+// NOISE variants of the single filter's kernels that use Q or R (ekf_set_noise): the handle's row travels as a kernel
+// argument.  The fused engine reads it from the device copy instead (FusedParams::noise).
+__global__ void k_maha_one_noise(const double* sig, long long ld, const double* state, int i, double sx, double sy,
+                                 double* out, const Noise nz) {
+    maha_one(sig, ld, state, i, sx, sy, out, nz);
+}
+__global__ void k_large_motion_noise(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
+                                     double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
+                                     double2* __restrict__ Wp, int pending, const Noise nz) {
+    large_motion(state, sig, ld, dtheta, dx, motion_out, Kp, Wp, pending, nz);
+}
+__global__ void __launch_bounds__(kGainThreads)
+    k_large_gain_p_noise(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
+                         double* __restrict__ state_out, const double* __restrict__ pose_src,
+                         const UpdateCmd* __restrict__ cmd, int lm_arg, double sx_arg, double sy_arg,
+                         double2* __restrict__ Kp, double2* __restrict__ Wp, int p, const Noise nz) {
+    large_gain_p(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p, nz);
+}
+__global__ void __launch_bounds__(256)
+    k_large_assoc_noise(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
+                        const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
+                        AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
+                        UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
+                        double* __restrict__ second_out, uint8_t* __restrict__ created_out, const Noise nz) {
+    large_assoc(sig, ld, state, n, meas, j, known_count_p, partials, done_counter, cmd, assoc_out, dmin_out, second_out,
+                created_out, nz);
+}
+
+// Rows {q_theta, q_x, q_y, r_range, r_bearing}: every entry finite, q >= 0, r > 0.
+bool noise_rows_valid(const double* rows, long long count) {
+    for (long long k = 0; k < 5 * count; ++k) {
+        const double v = rows[k];
+        if (!std::isfinite(v) || v < 0.0 || (k % 5 >= 3 && v == 0.0)) return false;
+    }
+    return true;
 }
 
 __global__ void k_update_pose(double wheel_base, double wheel_radius, long long count, double* poses,
@@ -199,6 +257,11 @@ struct ekf_filter {
     int* d_known_count = nullptr;
     int assoc_blocks = 0;
     int sm_count = 148;
+    // ekf_set_noise: with noise_on the NOISE kernels run with `noise` (streamed engine: kernel arguments; fused
+    // engine: the device copy d_noise)
+    bool noise_on = false;
+    Noise noise = ref_noise();
+    double* d_noise = nullptr;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
 };
 
@@ -230,6 +293,7 @@ int free_filter(ekf_filter* h) {
     cudaFree(h->d_partials);
     cudaFree(h->d_done);
     cudaFree(h->d_known_count);
+    cudaFree(h->d_noise);
     for (int i = 0; i < kRing; ++i) {
         if (h->h_ring[i]) cudaFreeHost(h->h_ring[i]);
         if (h->ring_ev[i]) cudaEventDestroy(h->ring_ev[i]);
@@ -309,6 +373,7 @@ FusedParams fused_params(ekf_filter* h, int mode, int m_max) {
     p.mode = mode;
     p.sig_stride = (int)h->sig_elems;
     p.st_stride = h->st_stride;
+    p.noise = h->noise_on ? h->d_noise : nullptr;
     return p;
 }
 
@@ -327,8 +392,12 @@ int stream_flush(ekf_filter* h, int n_counted, const UpdateCmd* cmd) {
 // touched when kMaxPending factors have piled up or the verb ends.
 int stream_correct(ekf_filter* h, const double* pose_src, const UpdateCmd* cmd, int lm, double sx, double sy) {
     const int gb = (int)((h->ld + 255) / 256);
-    CU(launch_pdl(k_large_gain_p, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N, h->d_state, h->d_state_alt,
-                  pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending));
+    if (h->noise_on)
+        CU(launch_pdl(k_large_gain_p_noise, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
+                      h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise));
+    else
+        CU(launch_pdl(k_large_gain_p, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N, h->d_state,
+                      h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending));
     h->launches += 1;
     std::swap(h->d_state, h->d_state_alt);
     h->pending += 1;
@@ -508,6 +577,16 @@ int ekf_clone(ekf_filter* src, ekf_filter** out) {
     h->init_flag_host = src->init_flag_host;
     h->max_pending = src->max_pending;
     h->carry_pending = src->carry_pending;
+    if (src->noise_on) {
+        const Noise nz = src->noise;
+        const double row[5] = {nz.q0, nz.q1, nz.q2, nz.r0, nz.r1};
+        rc = ekf_set_noise(h, row);
+        if (rc) {
+            free_filter(h);
+            *out = nullptr;
+            return rc;
+        }
+    }
     return EKF_OK;
 }
 
@@ -533,8 +612,12 @@ int ekf_predict(ekf_filter* h, double dtheta, double dx) {
     }
     // motion model + robot block + the pending factors carried across the prediction (ekf_large_delayed.cuh), then
     // the robot-landmark strips
-    CU(launch_pdl(k_large_motion, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld, dtheta, dx, h->d_motion,
-                  h->d_K2, h->d_W2, h->pending));
+    if (h->noise_on)
+        CU(launch_pdl(k_large_motion_noise, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld, dtheta, dx,
+                      h->d_motion, h->d_K2, h->d_W2, h->pending, h->noise));
+    else
+        CU(launch_pdl(k_large_motion, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld, dtheta, dx,
+                      h->d_motion, h->d_K2, h->d_W2, h->pending));
     CU(launch_pdl(k_large_predict_strips, dim3((h->N - 3 + 255) / 256), dim3(256), 0, h->stream, h->d_sigma, h->ld, h->N,
                   (const double*)h->d_motion));
     h->launches += 2;
@@ -649,9 +732,15 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
         CU(cudaMemcpyAsync(h->d_known_count, slot_i + 1, sizeof(int), cudaMemcpyHostToDevice, h->stream));
         CU(cudaEventRecord(ev, h->stream));
         for (int j = 0; j < m; ++j) {
-            k_large_assoc<<<h->assoc_blocks, 256, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, n, h->d_in, j,
-                                                                   h->d_known_count, h->d_partials, h->d_done, h->d_cmd,
-                                                                   h->d_assoc, h->d_dmin, h->d_second, h->d_created);
+            if (h->noise_on)
+                k_large_assoc_noise<<<h->assoc_blocks, 256, 0, h->stream>>>(
+                    h->d_sigma, h->ld, h->d_state, n, h->d_in, j, h->d_known_count, h->d_partials, h->d_done, h->d_cmd,
+                    h->d_assoc, h->d_dmin, h->d_second, h->d_created, h->noise);
+            else
+                k_large_assoc<<<h->assoc_blocks, 256, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, n, h->d_in, j,
+                                                                       h->d_known_count, h->d_partials, h->d_done,
+                                                                       h->d_cmd, h->d_assoc, h->d_dmin, h->d_second,
+                                                                       h->d_created);
             h->launches += 1;
             // the next measurement's distances need the corrected Sigma: one factor, applied at once
             rc = stream_correct(h, h->d_state, h->d_cmd, 0, 0.0, 0.0);
@@ -706,11 +795,44 @@ int ekf_maha(ekf_filter* h, double mx, double my, int landmark, double* d_out) {
         int rc_ = stream_settle(h);
         if (rc_) return rc_;
     }
-    k_maha_one<<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar);
+    if (h->noise_on)
+        k_maha_one_noise<<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar, h->noise);
+    else
+        k_maha_one<<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar);
     h->launches += 1;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(d_out, h->d_scalar, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
+    return EKF_OK;
+}
+
+int ekf_set_noise(ekf_filter* h, const double* noise5) {
+    if (!h) return fail(EKF_ERR_INVALID, "null handle");
+    if (noise5 && !noise_rows_valid(noise5, 1))
+        return fail(EKF_ERR_INVALID, "noise: every entry must be finite, q >= 0 and r > 0");
+    DeviceGuard g(h->device);
+    int rc = settle_prediction(h);  // a deferred prediction of the fused engine goes first, with the old Q
+    if (rc) return rc;
+    if (!noise5) {
+        h->noise_on = false;
+        h->noise = ref_noise();
+        return EKF_OK;
+    }
+    h->noise = Noise{noise5[0], noise5[1], noise5[2], noise5[3], noise5[4]};
+    if (h->engine == EKF_ENGINE_FUSED) {
+        if (!h->d_noise) CU(cudaMalloc(&h->d_noise, sizeof(Noise)));
+        // from pageable memory: staged before the call returns, applied in stream order behind enqueued kernels
+        CU(cudaMemcpyAsync(h->d_noise, &h->noise, sizeof(Noise), cudaMemcpyHostToDevice, h->stream));
+    }
+    h->noise_on = true;
+    return EKF_OK;
+}
+
+int ekf_get_noise(ekf_filter* h, double* out5) {
+    if (!h || !out5) return fail(EKF_ERR_INVALID, "null argument");
+    const Noise nz = h->noise;
+    const double row[5] = {nz.q0, nz.q1, nz.q2, nz.r0, nz.r1};
+    memcpy(out5, row, sizeof(row));
     return EKF_OK;
 }
 
@@ -1004,6 +1126,9 @@ struct ekf_batch {
     unsigned int* d_nis_done = nullptr;
     double* d_nis_pf = nullptr;         // [B][4] host read-out staging
     double* d_nis_out = nullptr;        // [4]
+    // per-filter noise (ekf_batch_set_noise): with noise_on every step runs the NOISE variant of its kernel
+    bool noise_on = false;
+    double* d_noise = nullptr;          // [B][5] = {q_theta, q_x, q_y, r_range, r_bearing}, allocated on first use
     cudaEvent_t t0 = nullptr, t1[3] = {nullptr, nullptr, nullptr};
 };
 
@@ -1046,6 +1171,7 @@ int free_batch(ekf_batch* b) {
     cudaFree(b->d_nis_done);
     cudaFree(b->d_nis_pf);
     cudaFree(b->d_nis_out);
+    cudaFree(b->d_noise);
     if (b->ev_step) cudaEventDestroy(b->ev_step);
     if (b->ev_out) cudaEventDestroy(b->ev_out);
     if (b->t0) cudaEventDestroy(b->t0);
@@ -1182,10 +1308,13 @@ int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint
     p.N = b->N;
     p.st_stride = b->st_stride;
     p.nis = b->nis_on ? b->d_nis : nullptr;
+    p.noise = b->noise_on ? b->d_noise : nullptr;
     if (p.nis)
-        CU(launch_wide_step<true>(p, b->grid, b->stream, b->device));
+        CU((p.noise ? launch_wide_step<true, true>(p, b->grid, b->stream, b->device)
+                    : launch_wide_step<true, false>(p, b->grid, b->stream, b->device)));
     else
-        CU(launch_wide_step<false>(p, b->grid, b->stream, b->device));
+        CU((p.noise ? launch_wide_step<false, true>(p, b->grid, b->stream, b->device)
+                    : launch_wide_step<false, false>(p, b->grid, b->stream, b->device)));
     return EKF_OK;
 }
 
@@ -1223,14 +1352,15 @@ int batch_launch(ekf_batch* b, int mode, int m_max, const double* tw, const doub
         p.st_stride = b->st_stride;
         p.sparse_total = total;
         p.nis = b->nis_on ? b->d_nis : nullptr;
+        p.noise = b->noise_on ? b->d_noise : nullptr;
         if (b->layout == Layout::Stair)
             rc = launch_fused_staircase(p, b->stream, b->device);
         else if (association)
-            rc = p.nis ? launch_fused_tile<true, true>(p, b->stream, b->device, b->sm_count)
-                       : launch_fused_tile<true, false>(p, b->stream, b->device, b->sm_count);
+            rc = p.nis ? launch_fused_tile_nis<true, true>(p, b->stream, b->device, b->sm_count)
+                       : launch_fused_tile_nis<true, false>(p, b->stream, b->device, b->sm_count);
         else
-            rc = p.nis ? launch_fused_tile<false, true>(p, b->stream, b->device, b->sm_count)
-                       : launch_fused_tile<false, false>(p, b->stream, b->device, b->sm_count);
+            rc = p.nis ? launch_fused_tile_nis<false, true>(p, b->stream, b->device, b->sm_count)
+                       : launch_fused_tile_nis<false, false>(p, b->stream, b->device, b->sm_count);
     }
     b->launches += 1;
     return rc;
@@ -1688,6 +1818,38 @@ int ekf_batch_nis_dev(ekf_batch* b, double* d_per_filter, double* d_out4, int re
     if (rc) return rc;
     DeviceGuard g(b->device);
     return launch_nis(b, d_per_filter, d_out4, reset);
+}
+int ekf_batch_set_noise(ekf_batch* b, const double* noise, int64_t stride) {
+    if (!b) return fail(EKF_ERR_INVALID, "null handle");
+    if (!noise) {
+        b->noise_on = false;
+        return EKF_OK;
+    }
+    if (stride != 0 && stride != 5) return fail(EKF_ERR_INVALID, "noise stride must be 0 (one row for all) or 5");
+    const long long rows = stride ? b->B : 1;
+    if (!noise_rows_valid(noise, rows))
+        return fail(EKF_ERR_INVALID, "noise: every entry must be finite, q >= 0 and r > 0");
+    DeviceGuard g(b->device);
+    if (!b->d_noise) CU(cudaMalloc(&b->d_noise, sizeof(double) * 5 * (size_t)b->B));
+    // staged in pageable memory, which cudaMemcpyAsync copies out before it returns: the caller's buffer (pinned or
+    // not) may be reused at once, and the rows reach the device in stream order behind the steps already enqueued
+    std::vector<double> all((size_t)5 * b->B);
+    for (long long k = 0; k < b->B; ++k) memcpy(all.data() + 5 * k, noise + (stride ? 5 * k : 0), 5 * sizeof(double));
+    CU(cudaMemcpyAsync(b->d_noise, all.data(), sizeof(double) * all.size(), cudaMemcpyHostToDevice, b->stream));
+    b->noise_on = true;
+    return EKF_OK;
+}
+int ekf_batch_get_noise(ekf_batch* b, double* out) {
+    if (!b || !out) return fail(EKF_ERR_INVALID, "null argument");
+    if (!b->noise_on) {
+        const double row[5] = {ref_noise().q0, ref_noise().q1, ref_noise().q2, ref_noise().r0, ref_noise().r1};
+        for (long long k = 0; k < b->B; ++k) memcpy(out + 5 * k, row, sizeof(row));
+        return EKF_OK;
+    }
+    DeviceGuard g(b->device);
+    CU(cudaMemcpyAsync(out, b->d_noise, sizeof(double) * 5 * (size_t)b->B, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    return EKF_OK;
 }
 int ekf_batch_sync(ekf_batch* b) {
     if (!b) return fail(EKF_ERR_INVALID, "null handle");

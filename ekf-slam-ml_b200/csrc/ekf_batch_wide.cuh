@@ -37,7 +37,8 @@ struct WideParams {
     long long ld;
     long long slot_stride;  // double2 per CTA in Kp / Wp
     int n, N, st_stride;
-    double* nis;  // [B][4] NIS accumulators of k_wide_step<true> (nis() / nis_add())
+    double* nis;  // [B][4] NIS accumulators of k_wide_step<true, *> (nis() / nis_add())
+    const double* noise;  // [B][5] per-filter {q_theta, q_x, q_y, r_range, r_bearing} of k_wide_step<*, true>
 };
 
 // dynamic shared memory: the sweep's stage ring, then the readings [2n] and visible flags [n] of the current filter
@@ -60,8 +61,9 @@ __device__ __forceinline__ void wide_sweep(double* sig, long long ld, int N, con
 }
 
 // NIS: also accumulate the NIS of the step's corrections (none on a filter's first call) into p.nis[b]; thread 0 keeps
-// the running sums in shared memory.
-template <bool NIS>
+// the running sums in shared memory.  NOISE: Q and R from the filter's row of p.noise, loaded once per filter into
+// shared memory.
+template <bool NIS, bool NOISE>
 __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* zxy = reinterpret_cast<double*>(smem_raw + WideTile::kSmemBytes);
@@ -70,6 +72,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
     __shared__ double s_a[2], s_pose[3];
     __shared__ int s_init;
     __shared__ double s_nis[4];
+    __shared__ Noise s_noise;
     // per-CTA loop state of the corrections, and the sweep ring's position per role (producer, consumers, storer)
     __shared__ struct {
         int i, pending, dirty;
@@ -127,6 +130,8 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
         // ---- prediction: motion model and robot block (k_large_motion), then the strips (k_large_predict_strips).
         // Sigma is read with ld.global.cg: the sweep's bulk stores bypass L1, so no line of Sigma may live there.
         if (tid == 0) {
+            if (NOISE) s_noise = load_noise(p.noise + 5 * b);
+            const Noise nz = NOISE ? s_noise : ref_noise();
             const Motion m = motion_model(st[0], p.twists[2 * b], p.twists[2 * b + 1]);
             double s[3][3];
             for (int r = 0; r < 3; ++r)
@@ -139,9 +144,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
                 s[r][1] = fma(s[r][0], m.a1, s[r][1]);
                 s[r][2] = fma(s[r][0], m.a2, s[r][2]);
             }
-            s[0][0] += kQ;
-            s[1][1] += kQ;
-            s[2][2] += kQ;
+            add_process_noise(s, nz);
             for (int r = 0; r < 3; ++r)
                 for (int c = 0; c < 3; ++c) sig[r * ld + c] = s[r][c];
             st[0] = st[0] + m.u0;
@@ -205,7 +208,7 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
                     const GainBlockEntry e = gain_block_entry(lane, i3);
                     const Hj h = make_hj(st[i3], st[i3 + 1], s_pose[0], s_pose[1], s_pose[2]);
                     gain_block(lane, e, __ldcg(sig + e.ida * ld + e.idl), Wp, ld, pending, h, zxy[2 * i], zxy[2 * i + 1],
-                               g);
+                               NOISE ? s_noise : ref_noise(), g);
                 }
                 __syncthreads();
                 if (NIS && tid == 0 && s_init) nis_add(s_nis, nis(g.si, g.nu0, g.nu1));
@@ -269,11 +272,11 @@ __global__ void __launch_bounds__(kTmaThreads, 1) k_wide_step(WideParams p) {
 }
 
 // One step of the whole batch on `device`.  grid = the number of CTAs the factor slots were allocated for.
-template <bool NIS>
+template <bool NIS, bool NOISE>
 inline cudaError_t launch_wide_step(const WideParams& p, int grid, cudaStream_t stream, int device) {
-    const cudaError_t e = kernel_setup<k_wide_step<NIS>>(device, kTmaThreads, wide_smem_bytes(kWideMaxN), false);
+    const cudaError_t e = kernel_setup<k_wide_step<NIS, NOISE>>(device, kTmaThreads, wide_smem_bytes(kWideMaxN), false);
     if (e != cudaSuccess) return e;
-    k_wide_step<NIS><<<(unsigned)grid, kTmaThreads, wide_smem_bytes(p.n), stream>>>(p);
+    k_wide_step<NIS, NOISE><<<(unsigned)grid, kTmaThreads, wide_smem_bytes(p.n), stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -38,14 +38,15 @@ struct FusedParams {
     int st_stride;   // doubles
     long long sparse_total;  // marker-list mode: number of listed markers (offsets are checked against it)
     double* nis;             // [B][4] NIS accumulators of the batch kernels' NIS variants (nis() / nis_add())
+    const double* noise;     // [B][5] per-filter {q_theta, q_x, q_y, r_range, r_bearing} of the NOISE variants
 };
 
 __host__ __device__ inline int fused_round16(int v) { return (v + 15) & ~15; }
 
 // shared memory carve-up (bytes), identical on host and device
 struct FusedSmem {
-    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, total;
-    __host__ __device__ FusedSmem(int n, int m_max) {
+    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_noise, total;
+    __host__ __device__ FusedSmem(int n, int m_max, bool noise = false) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;
@@ -66,6 +67,8 @@ struct FusedSmem {
         o += zc * 8;  // n = 20: 18,320 B per CTA in total, so that 12 CTAs (+1 KB reserve each) fit one SM's 227 KB
         off_bar = o;
         o += 16;
+        off_noise = o;  // NOISE only: the filter's row, read where it is used instead of held in registers
+        o += noise ? (int)sizeof(Noise) : 0;
         total = o;
     }
 };
@@ -84,7 +87,8 @@ template <bool PEND>
 __device__ __forceinline__ void warp_gain(const double* __restrict__ sig, double* __restrict__ st,
                                           const double2* __restrict__ Kpend, const double2* __restrict__ Wpend,
                                           double2* __restrict__ Kout, double2* __restrict__ Wout, const int N,
-                                          const int lane, const int i, const Hj h, const double zr, const double zphi) {
+                                          const int lane, const int i, const Hj h, const double zr, const double zphi,
+                                          const Noise& nz) {
     const int i3 = 3 + 2 * i, i4 = i3 + 1;
     double2 ka[5], wa[5];
     if (PEND) {
@@ -116,10 +120,10 @@ __device__ __forceinline__ void warp_gain(const double* __restrict__ sig, double
     __syncwarp();
     // S = (Hj Sigma) Hj^T + R from W at the five columns; closed-form inverse
     const double2 w0 = Wout[0], w1 = Wout[1], w2 = Wout[2], w3 = Wout[i3], w4 = Wout[i4];
-    const double s00 = h_row0(h, w1.x, w2.x, w3.x, w4.x) + kR;
+    const double s00 = h_row0(h, w1.x, w2.x, w3.x, w4.x) + nz.r0;
     const double s01 = h_row1(h, w0.x, w1.x, w2.x, w3.x, w4.x);
     const double s10 = h_row0(h, w1.y, w2.y, w3.y, w4.y);
-    const double s11 = h_row1(h, w0.y, w1.y, w2.y, w3.y, w4.y) + kR;
+    const double s11 = h_row1(h, w0.y, w1.y, w2.y, w3.y, w4.y) + nz.r1;
     const Sym2 si = inv2x2(s00, s01, s10, s11);
     const double nu0 = __dsub_rn(zr, h.zr);
     const double nu1 = normalize_angle(__dsub_rn(zphi, h.zphi));  // :182-183
@@ -220,7 +224,7 @@ __device__ __forceinline__ void warp_rank2(double* __restrict__ sig, const doubl
 // Rows 1, 2 take a * row 0 over all N columns; columns 1, 2 take a * column 0 in the rows below col_rows: all N rows
 // of a dense Sigma, the first diagonal block of the staircase (beyond it, columns 1, 2 ARE rows 1, 2).
 __device__ __forceinline__ Motion fused_predict(double* sig, double* st, const int N, const int col_rows, const int lane,
-                                                const double dtheta, const double dxv) {
+                                                const double dtheta, const double dxv, const Noise nz) {
     const Motion mo = motion_model(st[0], dtheta, dxv);
     __syncwarp();
     for (int c = lane; c < N; c += 32) {
@@ -236,9 +240,9 @@ __device__ __forceinline__ Motion fused_predict(double* sig, double* st, const i
     }
     __syncwarp();
     if (lane == 0) {
-        sig[0] += kQ;
-        sig[N + 1] += kQ;
-        sig[2 * N + 2] += kQ;
+        sig[0] += nz.q0;
+        sig[N + 1] += nz.q1;
+        sig[2 * N + 2] += nz.q2;
         st[0] = st[0] + mo.u0;  // theta is not wrapped here (:99)
         st[1] = st[1] + mo.u1;
         st[2] = st[2] + mo.u2;
@@ -367,12 +371,13 @@ __device__ __forceinline__ void fused_association(const FusedParams& p, const lo
     }
 }
 
-template <int NL>
+// NOISE: Q and R from p.noise (one row: this kernel runs the single fused filter), kept in shared memory by lane 0.
+template <int NL, bool NOISE>
 __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int n = NL ? NL : p.n;
     const int N = 3 + 2 * n;
-    const FusedSmem L(n, p.m_max);
+    const FusedSmem L(n, p.m_max, NOISE);
     double* sig = reinterpret_cast<double*>(smem_raw + L.off_sig);
     double* st = reinterpret_cast<double*>(smem_raw + L.off_st);
     double2* K2 = reinterpret_cast<double2*>(smem_raw + L.off_k2);
@@ -381,6 +386,8 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     double2* W2b = reinterpret_cast<double2*>(smem_raw + L.off_w2b);
     double* zbuf = reinterpret_cast<double*>(smem_raw + L.off_z);
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + L.off_bar);
+    Noise* nzs = reinterpret_cast<Noise*>(smem_raw + L.off_noise);
+    const auto nz = [&]() { return NOISE ? *nzs : ref_noise(); };
 
     const int lane = threadIdx.x;
     const long long b = blockIdx.x;
@@ -404,6 +411,7 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
         dxv = p.twists[2 * b + 1];
     }
     int init_flag = p.init_flag[b];
+    if (NOISE && lane == 0) *nzs = load_noise(p.noise + 5 * b);
     int m = 0;
     if (p.mode & kDoMeasurement) {
         // z = (range, bearing) of every slot's reading, lane-parallel (ekf_slam.cpp:140-146)
@@ -421,7 +429,7 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     mbar_wait(bar, 0);
 
     // ---- prediction (ekf_slam.cpp:55-106)
-    if (p.mode & kDoPredict) fused_predict(sig, st, N, N, lane, dtheta, dxv);
+    if (p.mode & kDoPredict) fused_predict(sig, st, N, N, lane, dtheta, dxv, nz());
 
     unsigned long long n_corr = 0;
 
@@ -456,13 +464,13 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
             while (rem) {
                 const int ia = base + __ffs(rem) - 1;
                 rem &= rem - 1;
-                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, ia, h, zbuf[2 * ia], zbuf[2 * ia + 1]);
+                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, ia, h, zbuf[2 * ia], zbuf[2 * ia + 1], nz());
                 ++n_corr;
                 if (rem) {
                     const int ib = base + __ffs(rem) - 1;
                     rem &= rem - 1;
                     h = make_hj(st[3 + 2 * ib], st[4 + 2 * ib], theta, x, y);
-                    warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, ib, h, zbuf[2 * ib], zbuf[2 * ib + 1]);
+                    warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, ib, h, zbuf[2 * ib], zbuf[2 * ib + 1], nz());
                     ++n_corr;
                     if (rem) {
                         const int in = base + __ffs(rem) - 1;
@@ -481,10 +489,10 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
         fused_association(
             p, b, n, m, lane, st, zbuf, n_corr,
             [&](int i, double zr, double zphi, double theta, double x, double y) {
-                return maha_distance(sig, N, i, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y);
+                return maha_distance(sig, N, i, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y, nz());
             },
             [&](int i, const Hj& h, double zr, double zphi, int) {
-                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, i, h, zr, zphi);
+                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, i, h, zr, zphi, nz());
                 warp_rank2<NL, 1>(sig, K2, W2, nullptr, nullptr, N, lane);
             });
     }

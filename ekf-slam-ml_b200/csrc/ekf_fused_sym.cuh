@@ -37,8 +37,8 @@ __host__ __device__ constexpr int sym_sig_stride(int N) { return (stair_size(N) 
 __host__ __device__ constexpr int sym_st_stride(int N) { return (N + 1) & ~1; }
 
 struct SymSmem {
-    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_nis, total;
-    __host__ __device__ SymSmem(int n, int m_max, bool nis = false) {
+    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_nis, off_noise, total;
+    __host__ __device__ SymSmem(int n, int m_max, bool nis = false, bool noise = false) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;
@@ -61,6 +61,8 @@ struct SymSmem {
         o += 16;
         off_nis = o;  // NIS only: the step's sums {sum, sum^2, #scored, #non-finite}, kept by lane 0
         o += nis ? 4 * 8 : 0;
+        off_noise = o;  // NOISE only: the filter's row, read where it is used instead of held in registers
+        o += noise ? (int)sizeof(Noise) : 0;
         total = o;
     }
 };
@@ -77,7 +79,7 @@ __device__ __forceinline__ Sym2 sym_warp_gain(const double* __restrict__ sig, do
                                               const double2* __restrict__ Kpend, const double2* __restrict__ Wpend,
                                               double2* __restrict__ Kout, double2* __restrict__ Wout, const int N,
                                               const int lane, const int* __restrict__ cmv, const int i, const H h,
-                                              const double nu0, const double nu1) {
+                                              const double nu0, const double nu1, const double r0, const double r1) {
     const int i3 = 3 + 2 * i, i4 = i3 + 1;
     const int b3 = i3 & ~15, b4 = i4 & ~15;
     // row offsets of the landmark's two rows: lane r % 32 already holds stair_row_base(r) - (r & ~15) in cmv[r / 32]
@@ -121,7 +123,7 @@ __device__ __forceinline__ Sym2 sym_warp_gain(const double* __restrict__ sig, do
     double s00, s01, s10, s11;
     h_rows(h, w0.x, w1.x, w2.x, w3.x, w4.x, s00, s01);
     h_rows(h, w0.y, w1.y, w2.y, w3.y, w4.y, s10, s11);
-    const Sym2 si = inv2x2(s00 + kR, s01, s10, s11 + kR);
+    const Sym2 si = inv2x2(s00 + r0, s01, s10, s11 + r1);
     // K = W^T S^-1 folded with nu: state += K nu
 #pragma unroll
     for (int sl = 0; sl < kSymSlots; ++sl) {
@@ -181,7 +183,7 @@ __device__ __forceinline__ void sym_warp_rank2(double* __restrict__ sig, const d
 // (00 01 02 11 12 22) is the same for every landmark and is fetched once per measurement by the caller.
 __device__ __forceinline__ double sym_maha_distance(const double* __restrict__ sig, int N, int i, const double* rob,
                                                     double mx, double my, double zr, double zphi, double theta,
-                                                    double x, double y) {
+                                                    double x, double y, double r0, double r1) {
     const Hj h = make_hj(mx, my, theta, x, y);
     const int i3 = 3 + 2 * i, i4 = i3 + 1;
     const int rb3 = stair_row_base(i3, N) - (i3 & ~15), rb4 = stair_row_base(i4, N) - (i4 & ~15);
@@ -199,7 +201,7 @@ __device__ __forceinline__ double sym_maha_distance(const double* __restrict__ s
     double p00, p01, p10, p11;
     h_rows(h, wl0[0], wl0[1], wl0[2], wl0[3], wl0[4], p00, p01);
     h_rows(h, wl1[0], wl1[1], wl1[2], wl1[3], wl1[4], p10, p11);
-    const Sym2 pi = inv2x2(p00 + kR, p01, p10, p11 + kR);
+    const Sym2 pi = inv2x2(p00 + r0, p01, p10, p11 + r1);
     const double v0 = __dsub_rn(zr, h.zr), v1 = __dsub_rn(zphi, h.zphi);
     const double t0 = __dadd_rn(__dmul_rn(v0, pi.i00), __dmul_rn(v1, pi.i10));
     const double t1 = __dadd_rn(__dmul_rn(v0, pi.i01), __dmul_rn(v1, pi.i11));
@@ -213,13 +215,13 @@ static __device__ __noinline__ void landmark_from_reading_cold(double sx, double
 }
 
 // NIS: also accumulate the NIS of the step's scored corrections into p.nis[b]; lane 0 keeps the running sums in shared
-// memory, not in registers.
-template <bool NIS>
+// memory, not in registers.  NOISE: Q and R from the filter's row of p.noise, kept in shared memory by lane 0.
+template <bool NIS, bool NOISE>
 __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int n = p.n;
     const int N = 3 + 2 * n;
-    const SymSmem L(n, p.m_max, NIS);
+    const SymSmem L(n, p.m_max, NIS, NOISE);
     double* sig = reinterpret_cast<double*>(smem_raw + L.off_sig);
     double* st = reinterpret_cast<double*>(smem_raw + L.off_st);
     double2* K2 = reinterpret_cast<double2*>(smem_raw + L.off_k2);
@@ -229,6 +231,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
     double* zbuf = reinterpret_cast<double*>(smem_raw + L.off_z);
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + L.off_bar);
     double* nacc = reinterpret_cast<double*>(smem_raw + L.off_nis);
+    Noise* nzs = reinterpret_cast<Noise*>(smem_raw + L.off_noise);
 
     const int lane = threadIdx.x;
     const long long b = blockIdx.x;
@@ -260,6 +263,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
         dxv = p.twists[2 * b + 1];
     }
     int init_flag = p.init_flag[b];
+    if (NOISE && lane == 0) *nzs = load_noise(p.noise + 5 * b);
     int m = 0;
     // visible landmarks as warp-uniform bit masks (slots 0..31 and 32..63), readings as {zr, ux, uy} per slot
     unsigned vismask[2] = {0u, 0u};
@@ -309,7 +313,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
     double sth = 0.0, cth = 1.0;
     bool have_sincos = false;
     if (p.mode & kDoPredict) {
-        const Motion mo = fused_predict(sig, st, N, N < 16 ? N : 16, lane, dtheta, dxv);
+        const Motion mo = fused_predict(sig, st, N, N < 16 ? N : 16, lane, dtheta, dxv, NOISE ? *nzs : ref_noise());
         sth = mo.s_new, cth = mo.c_new, have_sincos = true;
     }
 
@@ -367,9 +371,11 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
                 rem &= rem - 1;
                 Sym2 si;
                 if (!second)
-                    si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, ic, h, h.nu0, h.nu1);
+                    si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, ic, h, h.nu0, h.nu1,
+                                              NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);
                 else
-                    si = sym_warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, cmv, ic, h, h.nu0, h.nu1);
+                    si = sym_warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, cmv, ic, h, h.nu0, h.nu1,
+                                             NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);
                 if (NIS && score && lane == 0) nis_add(nacc, nis(si, h.nu0, h.nu1));
                 ++n_corr;
                 if (rem) {
@@ -392,11 +398,13 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
             p, b, n, m, lane, st, zbuf, n_corr,
             [&](int i, double zr, double zphi, double theta, double x, double y) {
                 const double rob[6] = {sig[0], sig[1], sig[2], sig[N + 1], sig[N + 2], sig[2 * N + 2]};
-                return sym_maha_distance(sig, N, i, rob, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y);
+                return sym_maha_distance(sig, N, i, rob, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y,
+                                         NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);
             },
             [&](int i, const Hj& h, double zr, double zphi, int created) {
                 const double nu0 = __dsub_rn(zr, h.zr), nu1 = normalize_angle(__dsub_rn(zphi, h.zphi));  // :182-183
-                const Sym2 si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, i, h, nu0, nu1);
+                const Sym2 si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, i, h, nu0, nu1,
+                                                     NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);
                 if (NIS && !created && lane == 0) nis_add(nacc, nis(si, nu0, nu1));  // a new landmark starts at its reading
                 sym_warp_rank2<1>(sig, K2, W2, nullptr, nullptr, N, lane);
             });

@@ -40,9 +40,11 @@ __device__ __forceinline__ void pdl_prologue() {
 // One warp: lane 0 does the motion model, state[0..2], the 3x3 robot block of At*Sigma*At^T + Q, and (a1, a2) for the
 // strips; lane j < pending carries pending factor j across the prediction (ekf_large_delayed.cuh).  The row-sharded
 // engine runs it on every rank: `sig` is then the rank's 3 x ld copy of rows 0..2, or its own rows on rank 0.
-__global__ void k_large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
-                               double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
-                               double2* __restrict__ Wp, int pending) {
+// The body is shared by k_large_motion (the reference's Q) and the single filter's noise variant (capi.cu).
+__device__ __forceinline__ void large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld,
+                                             double dtheta, double dx, double* __restrict__ motion_out,
+                                             double2* __restrict__ Kp, double2* __restrict__ Wp, int pending,
+                                             const Noise& nz) {
     pdl_prologue();
     if (blockIdx.x != 0 || threadIdx.x >= 32) return;
     Motion m = {};
@@ -72,9 +74,7 @@ __global__ void k_large_motion(double* __restrict__ state, double* __restrict__ 
         s[r][1] = fma(s[r][0], m.a1, s[r][1]);
         s[r][2] = fma(s[r][0], m.a2, s[r][2]);
     }
-    s[0][0] += kQ;
-    s[1][1] += kQ;
-    s[2][2] += kQ;
+    add_process_noise(s, nz);
     for (int r = 0; r < 3; ++r)
         for (int c = 0; c < 3; ++c) sig[r * ld + c] = s[r][c];
     state[0] = state[0] + m.u0;
@@ -82,6 +82,11 @@ __global__ void k_large_motion(double* __restrict__ state, double* __restrict__ 
     state[2] = state[2] + m.u2;
     motion_out[0] = m.a1;
     motion_out[1] = m.a2;
+}
+__global__ void k_large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
+                               double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
+                               double2* __restrict__ Wp, int pending) {
+    large_motion(state, sig, ld, dtheta, dx, motion_out, Kp, Wp, pending, ref_noise());
 }
 
 // Robot-landmark strips: rows 1,2 += a*row0 and cols 1,2 += a*col0 for indices k >= 3.  6N doubles touched.
@@ -136,7 +141,7 @@ __device__ __forceinline__ bool assoc_scan(const double* __restrict__ robot, con
                                            const double* __restrict__ state, double zr, double zphi, double theta,
                                            double x, double y, AssocPartial* __restrict__ partials,
                                            unsigned int* __restrict__ done_counter, double& best, double& second,
-                                           int& best_i) {
+                                           int& best_i, const Noise& nz) {
     __shared__ AssocPartial sh[8];
     __shared__ bool is_last;
     best = INFINITY;
@@ -144,7 +149,7 @@ __device__ __forceinline__ bool assoc_scan(const double* __restrict__ robot, con
     best_i = 0x7fffffff;
     for (int i = i_begin + blockIdx.x * blockDim.x + threadIdx.x; i < i_end; i += gridDim.x * blockDim.x) {
         const double* lm = lm_rows + ((3 + 2 * (long long)i) - r0) * ld;
-        double d = maha_distance_rows(robot, lm, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, theta, x, y);
+        double d = maha_distance_rows(robot, lm, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, theta, x, y, nz);
         if (!(d == d)) d = INFINITY;
         if (d < best) {
             second = best;
@@ -225,12 +230,14 @@ __device__ __forceinline__ void assoc_decide(double best, double second, int bes
     if (created_out) created_out[j] = (uint8_t)created;
 }
 
-__global__ void __launch_bounds__(256)
-    k_large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
-                  const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
-                  AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
-                  UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
-                  double* __restrict__ second_out, uint8_t* __restrict__ created_out) {
+// The body is shared by k_large_assoc (the reference's R) and the single filter's noise variant (capi.cu).
+__device__ __forceinline__ void large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state,
+                                            int n, const double* __restrict__ meas, int j,
+                                            int* __restrict__ known_count_p, AssocPartial* __restrict__ partials,
+                                            unsigned int* __restrict__ done_counter, UpdateCmd* __restrict__ cmd,
+                                            int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
+                                            double* __restrict__ second_out, uint8_t* __restrict__ created_out,
+                                            const Noise nz) {
     const int known_count = *known_count_p;
     const double sx = meas[2 * j], sy = meas[2 * j + 1];
     double zr, zphi;
@@ -239,10 +246,19 @@ __global__ void __launch_bounds__(256)
     double best, second;
     int best_i;
     if (!assoc_scan(sig, sig, ld, 0, 0, known_count, state, zr, zphi, theta, x, y, partials, done_counter, best,
-                    second, best_i))
+                    second, best_i, nz))
         return;
     assoc_decide(best, second, best_i, known_count, n, j, sx, sy, theta, x, y, state, known_count_p, cmd, assoc_out,
                  dmin_out, second_out, created_out);
+}
+__global__ void __launch_bounds__(256)
+    k_large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
+                  const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
+                  AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
+                  UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
+                  double* __restrict__ second_out, uint8_t* __restrict__ created_out) {
+    large_assoc(sig, ld, state, n, meas, j, known_count_p, partials, done_counter, cmd, assoc_out, dmin_out, second_out,
+                created_out, ref_noise());
 }
 
 // ---------------------------------------------------------------- 256-bit global accesses (LDG/STG.E.256 on sm_100a)

@@ -53,12 +53,12 @@ __device__ __forceinline__ GainBlockEntry gain_block_entry(int lane, int i3) {
 
 // S^-1 and the innovation nu = z - h(x) from H_j, W = H_j Sigma at the five columns {0, 1, 2, i3, i4} and the measured
 // range and bearing.  Also used by the row-sharded engine (sharded/sharded.cu).
-__device__ __forceinline__ void gain_scalars(const Hj& h, const double2 (&w5)[5], double sx, double sy, Sym2& si,
-                                             double& nu0, double& nu1) {
-    const double s00 = h_row0(h, w5[1].x, w5[2].x, w5[3].x, w5[4].x) + kR;
+__device__ __forceinline__ void gain_scalars(const Hj& h, const double2 (&w5)[5], double sx, double sy, const Noise& nz,
+                                             Sym2& si, double& nu0, double& nu1) {
+    const double s00 = h_row0(h, w5[1].x, w5[2].x, w5[3].x, w5[4].x) + nz.r0;
     const double s01 = h_row1(h, w5[0].x, w5[1].x, w5[2].x, w5[3].x, w5[4].x);
     const double s10 = h_row0(h, w5[1].y, w5[2].y, w5[3].y, w5[4].y);
-    const double s11 = h_row1(h, w5[0].y, w5[1].y, w5[2].y, w5[3].y, w5[4].y) + kR;
+    const double s11 = h_row1(h, w5[0].y, w5[1].y, w5[2].y, w5[3].y, w5[4].y) + nz.r1;
     si = inv2x2(s00, s01, s10, s11);
     double zr, zphi;
     range_bearing(sx, sy, zr, zphi);
@@ -80,7 +80,7 @@ __device__ __forceinline__ double gain_state(const Sym2& si, const double& nu0, 
 // One full warp: `v` = Sigma_0(id_a, id_l) of the lane's entry.  Rebuilds the current block with the p pending factors,
 // then lane 0 leaves H_j, S^-1 and the innovation in g.
 __device__ __forceinline__ void gain_block(int lane, const GainBlockEntry& e, double v, const double2* Wp, long long ld,
-                                           int p, const Hj& h, double sx, double sy, GainSharedP& g) {
+                                           int p, const Hj& h, double sx, double sy, const Noise& nz, GainSharedP& g) {
 #pragma unroll 4
     for (int j = 0; j < p; ++j) v = apply_factor(v, g.Kidx[j][e.a], Wp[(long long)j * ld + e.idl]);
     // column l of the block: s[a'] = Sigma(id_a', id_l) sits in lane 5 a' + l
@@ -97,7 +97,7 @@ __device__ __forceinline__ void gain_block(int lane, const GainBlockEntry& e, do
     }
     if (lane == 0) {
         g.h = h;
-        gain_scalars(h, w5, sx, sy, g.si, g.nu0, g.nu1);
+        gain_scalars(h, w5, sx, sy, nz, g.si, g.nu0, g.nu1);
     }
 }
 
@@ -142,10 +142,12 @@ __device__ __forceinline__ void named_bar_sync(int id, int count) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory");
 }
 
-__global__ void __launch_bounds__(kGainThreads)
-    k_large_gain_p(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
-                   double* __restrict__ state_out, const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
-                   int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp, double2* __restrict__ Wp, int p) {
+// The body is shared by k_large_gain_p (the reference's R) and the single filter's noise variant (capi.cu).
+__device__ __forceinline__ void large_gain_p(const double* __restrict__ sig, long long ld, int N,
+                                             const double* __restrict__ state_in, double* __restrict__ state_out,
+                                             const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
+                                             int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp,
+                                             double2* __restrict__ Wp, int p, const Noise& nz) {
     __shared__ GainSharedP g;
     pdl_prologue();
     int lm = lm_arg;
@@ -172,7 +174,7 @@ __global__ void __launch_bounds__(kGainThreads)
         if (active) {
             const GainBlockEntry e = gain_block_entry(lane, i3);
             const Hj h = make_hj(state_in[i3], state_in[i3 + 1], pose_src[0], pose_src[1], pose_src[2]);
-            gain_block(lane, e, sig[e.ida * ld + e.idl], Wp, ld, p, h, sx, sy, g);
+            gain_block(lane, e, sig[e.ida * ld + e.idl], Wp, ld, p, h, sx, sy, nz, g);
         }
         __syncwarp();
         named_bar_sync(2, kGainThreads);
@@ -202,6 +204,12 @@ __global__ void __launch_bounds__(kGainThreads)
     state_out[k] = gain_column(g, s0, s1, s2, s3, s4, st_k, k, wk, kk);
     Wout[k] = wk;
     Kout[k] = kk;
+}
+__global__ void __launch_bounds__(kGainThreads)
+    k_large_gain_p(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
+                   double* __restrict__ state_out, const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
+                   int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp, double2* __restrict__ Wp, int p) {
+    large_gain_p(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p, ref_noise());
 }
 
 // prediction() with factors pending: Sigma' = A (Sigma_0 - sum_j K_j W_j) A^T + Q = [A Sigma_0 A^T + Q] - sum_j (A K_j)(W_j A^T)

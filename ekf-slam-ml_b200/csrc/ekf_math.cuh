@@ -33,6 +33,18 @@ constexpr double kGateNew = 10.0;    // ekf_slam.cpp:293
 constexpr double kGateUpdate = 1.0;  // ekf_slam.cpp:330
 constexpr double kSmallTurn = 0.000001;  // ekf_slam.cpp:79
 
+// Process and measurement noise of one filter: Q = diag(q0, q1, q2) on (theta, x, y), R = diag(r0, r1) on (range,
+// bearing).  ref_noise() holds the reference's constants; the default kernels pass it, so they compile as before, and
+// the NOISE variants read a per-filter row {q_theta, q_x, q_y, r_range, r_bearing} (ekf_set_noise,
+// ekf_batch_set_noise).
+struct Noise {
+    double q0, q1, q2, r0, r1;
+};
+__host__ __device__ constexpr Noise ref_noise() { return Noise{kQ, kQ, kQ, kR, kR}; }
+__device__ __forceinline__ Noise load_noise(const double* __restrict__ row) {
+    return Noise{row[0], row[1], row[2], row[3], row[4]};
+}
+
 // fmod(x, 2*pi), exact like the C library's: the quotient is small on this path, so one FMA recovers the
 // remainder exactly (x and q*2pi are both multiples of ulp(2pi) once |x| >= 2pi, and the remainder is
 // below 8 so it fits 53 bits).  Falls back to fmod() for large or non-finite arguments.
@@ -263,7 +275,7 @@ __device__ __forceinline__ void nis_add(double* acc, double v) {
 // row stride ld.  They are the same matrix on one GPU and two different buffers in the row-sharded engine.
 __device__ __forceinline__ double maha_distance_rows(const double* __restrict__ robot, const double* __restrict__ lm,
                                                      int64_t ld, int i, double mx, double my, double zr, double zphi,
-                                                     double theta, double x, double y) {
+                                                     double theta, double x, double y, const Noise& nz) {
     const Hj h = make_hj(mx, my, theta, x, y);
     const int64_t id[5] = {0, 1, 2, 3 + 2 * (int64_t)i, 4 + 2 * (int64_t)i};
     double wl0[5], wl1[5];
@@ -278,10 +290,10 @@ __device__ __forceinline__ double maha_distance_rows(const double* __restrict__ 
         wl1[l] = h_row1(h, s0, s1, s2, s3, s4);
     }
     // psi = (H Sigma) H^T + R
-    const double p00 = h_row0(h, wl0[1], wl0[2], wl0[3], wl0[4]) + kR;
+    const double p00 = h_row0(h, wl0[1], wl0[2], wl0[3], wl0[4]) + nz.r0;
     const double p01 = h_row1(h, wl0[0], wl0[1], wl0[2], wl0[3], wl0[4]);
     const double p10 = h_row0(h, wl1[1], wl1[2], wl1[3], wl1[4]);
-    const double p11 = h_row1(h, wl1[0], wl1[1], wl1[2], wl1[3], wl1[4]) + kR;
+    const double p11 = h_row1(h, wl1[0], wl1[1], wl1[2], wl1[3], wl1[4]) + nz.r1;
     const Sym2 pi = inv2x2(p00, p01, p10, p11);
     const double v0 = __dsub_rn(zr, h.zr), v1 = __dsub_rn(zphi, h.zphi);
     const double t0 = __dadd_rn(__dmul_rn(v0, pi.i00), __dmul_rn(v1, pi.i10));
@@ -292,8 +304,15 @@ __device__ __forceinline__ double maha_distance_rows(const double* __restrict__ 
 // Whole Sigma in one buffer (shared memory in the fused engine, global memory in the streamed one).
 __device__ __forceinline__ double maha_distance(const double* __restrict__ sig, int64_t ld, int i, double mx,
                                                 double my, double zr, double zphi, double theta, double x,
-                                                double y) {
-    return maha_distance_rows(sig, sig + (3 + 2 * (int64_t)i) * ld, ld, i, mx, my, zr, zphi, theta, x, y);
+                                                double y, const Noise& nz) {
+    return maha_distance_rows(sig, sig + (3 + 2 * (int64_t)i) * ld, ld, i, mx, my, zr, zphi, theta, x, y, nz);
+}
+
+// + Q on the robot block's diagonal after the motion Jacobian (ekf_slam.cpp:41-43, :102); s = rows 0..2, columns 0..2
+__device__ __forceinline__ void add_process_noise(double (&s)[3][3], const Noise& nz) {
+    s[0][0] += nz.q0;
+    s[1][1] += nz.q1;
+    s[2][2] += nz.q2;
 }
 
 // Motion model increments and Jacobian entries (ekf_slam.cpp:67-96): state[0..2] += u, A(1,0)=a1, A(2,0)=a2.

@@ -117,7 +117,7 @@ __global__ void __launch_bounds__(256)
         if (active_s) {
             const int i3 = ctx->i3;
             const double2 w5[5] = {Wp_slot[0], Wp_slot[1], Wp_slot[2], Wp_slot[i3], Wp_slot[i3 + 1]};
-            gain_scalars(ctx->h, w5, ctx->sx, ctx->sy, si_s, nu_s[0], nu_s[1]);
+            gain_scalars(ctx->h, w5, ctx->sx, ctx->sy, ref_noise(), si_s, nu_s[0], nu_s[1]);
         }
     }
     __syncthreads();
@@ -337,7 +337,7 @@ __global__ void __launch_bounds__(256)
                 w5[k] = make_double2(w5[k].x + b.x, w5[k].y + b.y);
             }
         }
-        gain_scalars(h, w5, z_s[0], z_s[1], si_s, nu_s[0], nu_s[1]);
+        gain_scalars(h, w5, z_s[0], z_s[1], ref_noise(), si_s, nu_s[0], nu_s[1]);
         const long long b0 = (long long)blockIdx.x << 8, b1 = b0 + 256;
         if (b0 < 3 || (i3 + 1 >= b0 && i3 < b1)) {  // this CTA's state update overwrites what thread 0 of the others reads
             while (ld_acquire_sys_u64(read_count) < read_target) {
@@ -376,7 +376,7 @@ __global__ void __launch_bounds__(256)
     double best, second;
     int best_i;
     if (assoc_scan(robot, sig_local, ld, r0, L0, L1 < known_count ? L1 : known_count, state, zr, zphi, state[0],
-                   state[1], state[2], block_partials, done_counter, best, second, best_i))
+                   state[1], state[2], block_partials, done_counter, best, second, best_i, ref_noise()))
         *out = AssocPartial{best, second, best_i, 0};
 }
 

@@ -90,6 +90,21 @@ def _as_xy(measures):
     return np.ascontiguousarray(measures, dtype=np.float64).reshape(-1)
 
 
+DEFAULT_Q = 1e-4  # EKF_DEFAULT_Q: the reference's process noise on (theta, x, y)
+DEFAULT_R = 0.01  # EKF_DEFAULT_R: the reference's measurement noise on (range, bearing)
+
+
+def noise_rows(q, r, B):
+    """[K][5] float64 rows {q_theta, q_x, q_y, r_range, r_bearing} from q (3,) / (B, 3) and r (2,) / (B, 2); None takes
+    the reference values.  K = 1 when both parts are shared by all filters, else B."""
+    q = np.full(3, DEFAULT_Q) if q is None else np.asarray(q, dtype=np.float64)
+    r = np.full(2, DEFAULT_R) if r is None else np.asarray(r, dtype=np.float64)
+    if q.shape not in ((3,), (B, 3)) or r.shape not in ((2,), (B, 2)):
+        raise ValueError(f"noise: q must be (3,) or ({B}, 3) and r (2,) or ({B}, 2), got {q.shape} and {r.shape}")
+    k = 1 if q.ndim == 1 and r.ndim == 1 else B
+    return np.ascontiguousarray(np.hstack([np.broadcast_to(q, (k, 3)), np.broadcast_to(r, (k, 2))]))
+
+
 class EKF_SLAM:
     """Drop-in for rigid2d::EKF_SLAM.  `engine` picks the fused on-chip kernel or the HBM-streamed path."""
 
@@ -270,6 +285,23 @@ class EKF_SLAM:
         """Streamed engine: let correction factors stay pending across prediction() / measurement() calls (default on;
         off = Sigma is swept at the end of every measurement(), bit-identical to one sweep per correction)."""
         check(self._L.ekf_set_carry_pending(self._h, 1 if on else 0))
+
+    def set_noise(self, q=None, r=None):
+        """Noise covariances Q = diag(q) on (theta, x, y) and R = diag(r) on (range, bearing) (ekf_set_noise).  A part
+        left as None takes the reference values (DEFAULT_Q, DEFAULT_R); set_noise() restores both.  Every entry must be
+        finite, q >= 0 and r > 0.  Takes effect from the next verb; clone() copies it."""
+        if q is None and r is None:
+            check(self._L.ekf_set_noise(self._h, None))
+            return
+        row = noise_rows(q, r, 1)
+        check(self._L.ekf_set_noise(self._h, row.ctypes.data))
+
+    @property
+    def noise(self):
+        """The filter's {q_theta, q_x, q_y, r_range, r_bearing} (5,)."""
+        out = np.empty(5)
+        check(self._L.ekf_get_noise(self._h, out.ctypes.data))
+        return out
 
     def timer_start(self):
         check(self._L.ekf_timer_start(self._h))
@@ -547,6 +579,23 @@ class EKFBatch:
         batch's stream without a synchronisation; the results are valid after sync()."""
         check(self._L.ekf_batch_nis_dev(self._h, int(d_per_filter) if d_per_filter else None,
                                         int(d_out4) if d_out4 else None, 1 if reset else 0))
+
+    def set_noise(self, q=None, r=None):
+        """Per-filter noise covariances (ekf_batch_set_noise): q is (3,) for every filter or (B, 3), r (2,) or (B, 2);
+        a part left as None takes the reference values (DEFAULT_Q, DEFAULT_R), and set_noise() returns to the default
+        kernels.  Invalid rows (not finite, q < 0, r <= 0) raise and leave the batch unchanged.  The following steps
+        run the NOISE variants of the step kernels; checkpoints do not carry the noise."""
+        if q is None and r is None:
+            check(self._L.ekf_batch_set_noise(self._h, None, 0))
+            return
+        rows = noise_rows(q, r, self.B)
+        check(self._L.ekf_batch_set_noise(self._h, rows.ctypes.data, 5 if rows.shape[0] > 1 else 0))
+
+    def noise(self):
+        """(B, 5) rows {q_theta, q_x, q_y, r_range, r_bearing} in use."""
+        out = np.empty((self.B, 5))
+        check(self._L.ekf_batch_get_noise(self._h, out.ctypes.data))
+        return out
 
     def sync(self):
         check(self._L.ekf_batch_sync(self._h))

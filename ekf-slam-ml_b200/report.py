@@ -32,10 +32,11 @@ def _anees(cs, stats, key, dof):
             "bounds_95": list(cs.chi2_bounds(dof, runs))}
 
 
-def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0):
+def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0, noise=None):
     """Returns a dict with the batch statistics after `steps` SLAM steps (11 simulator ticks each; one lap of the
     follow_circle trajectory is about 114 steps).  With nees_every = K > 0 the SLAM batch's pose ANEES is also recorded
-    after every K-th step, on the device from the simulator's truth (no host round trip per step)."""
+    after every K-th step, on the device from the simulator's truth (no host round trip per step).  noise =
+    (q_theta, q_x, q_y, r_range, r_bearing) replaces the reference's Q and R in both batches."""
     import torch
     tg = pkg.tracegen
     world = world or tg.dense_world(20)
@@ -44,6 +45,9 @@ def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0)
     slam = pkg.EKFBatch(robots, n, device=device)
     blind = pkg.EKFBatch(robots, n, device=device)
     slam.set_nis(True)  # innovation consistency of every correction, on the device
+    if noise is not None:
+        for b in (slam, blind):
+            b.set_noise(noise[:3], noise[3:])
     sim.use_stream(slam.stream)
     p = sim.device_pointers()
     no_vis = torch.zeros(robots * n, dtype=torch.uint8, device=f"cuda:{device}")
@@ -74,6 +78,7 @@ def run(pkg, robots=4096, steps=140, seed=0, device=0, world=None, nees_every=0)
                            "wheel_odometry": float(np.abs(odom[:, :2] - truth[:, :2]).max())},
         "landmark_rmse": float(np.sqrt(np.mean(lm_err ** 2))),
         "landmarks": int(nt),
+        **({"noise": [float(v) for v in noise]} if noise is not None else {}),
     }
     # consistency: NEES against the simulator's truth; slots without a tube are not scored
     lm_truth = np.full((n, 2), np.nan)
@@ -133,13 +138,17 @@ def main(argv=None):
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--nees-every", type=int, default=0, metavar="K",
                     help="also record the SLAM batch's pose ANEES after every K-th step (on the device)")
+    ap.add_argument("--noise", type=lambda s: [float(v) for v in s.split(",")], default=None, metavar="QT,QX,QY,RR,RB",
+                    help="process and measurement noise variances instead of the reference's (1e-4 and 0.01 each)")
     ap.add_argument("--json", action="store_true")
     a = ap.parse_args(argv)
+    if a.noise is not None and len(a.noise) != 5:
+        ap.error("--noise takes five comma-separated values")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     if root not in sys.path:
         sys.path.insert(0, root)
     import ekf_slam_ml_b200 as pkg
-    r = run(pkg, a.robots, a.steps, a.seed, a.device, nees_every=a.nees_every)
+    r = run(pkg, a.robots, a.steps, a.seed, a.device, nees_every=a.nees_every, noise=a.noise)
     print(json.dumps(r) if a.json else markdown(r))
 
 

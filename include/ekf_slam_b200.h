@@ -31,6 +31,11 @@ extern "C" {
 #define EKF_ERR_UNSUPPORTED (-2)
 #define EKF_ERR_STATE (-3)
 
+/* the reference's noise covariances (ekf_slam.cpp:41-43, :172-175): Q = EKF_DEFAULT_Q I_3 on (theta, x, y),
+ * R = EKF_DEFAULT_R I_2 on (range, bearing); what every filter uses until ekf_set_noise / ekf_batch_set_noise */
+#define EKF_DEFAULT_Q 0.0001
+#define EKF_DEFAULT_R 0.01
+
 /* engine selection for ekf_create_ex */
 #define EKF_ENGINE_AUTO 0  /* fused on-chip engine when Sigma fits shared memory, streamed otherwise */
 #define EKF_ENGINE_FUSED 1 /* one kernel per call, Sigma resident in shared memory (n <= 64) */
@@ -112,6 +117,13 @@ int ekf_set_max_pending(ekf_filter* h, int max_pending);
  * 0: Sigma is swept at the end of every measurement().  Every verb that reads Sigma or the update counter settles the
  * pending factors first, so the difference is only visible in rounding (1e-15 relative) and in speed. */
 int ekf_set_carry_pending(ekf_filter* h, int carry);
+/* Noise covariances of the filter: noise5 = {q_theta, q_x, q_y, r_range, r_bearing}, Q = diag(q) added to the robot
+ * block in prediction, R = diag(r) added to S in measurement(), data_association() and ekf_maha.  Every entry finite,
+ * q >= 0, r > 0, or EKF_ERR_INVALID and nothing changes; NULL restores EKF_DEFAULT_Q / EKF_DEFAULT_R.  Takes effect
+ * from the next verb (a prediction the fused engine still defers is applied first, with the old Q); noise5 may be
+ * reused on return.  ekf_clone copies it; it is configuration, not state (ekf_set_state / ekf_set_sigma keep it). */
+int ekf_set_noise(ekf_filter* h, const double* noise5);
+int ekf_get_noise(ekf_filter* h, double* out5);
 /* passes over Sigma the streamed engine has made so far (for the roofline accounting of bench.py) */
 int ekf_sweep_count(ekf_filter* h, uint64_t* out);
 /* raw device pointers for callers that live on the GPU already (bench, fused pipelines) */
@@ -226,6 +238,14 @@ int ekf_batch_set_nis(ekf_batch* b, int on);
 int ekf_batch_nis(ekf_batch* b, double* per_filter, double* out4, int reset);
 /* the same with DEVICE pointers, enqueued on ekf_batch_stream(), no synchronisation (a per-step series with reset = 1) */
 int ekf_batch_nis_dev(ekf_batch* b, double* d_per_filter, double* d_out4, int reset);
+/* Per-filter noise covariances, rows {q_theta, q_x, q_y, r_range, r_bearing} as in ekf_set_noise: stride 0 gives every
+ * filter the row at `noise`, stride 5 reads [B][5].  The following steps run the NOISE variants of the step kernels
+ * (still one launch per step); NULL returns to EKF_DEFAULT_Q / EKF_DEFAULT_R and the default kernels.  Rows are
+ * checked on the host (any invalid row: EKF_ERR_INVALID, nothing changes) and copied in stream order behind the work
+ * already enqueued; `noise` may be reused on return.  Not part of checkpoints: set it again after ekf_batch_import. */
+int ekf_batch_set_noise(ekf_batch* b, const double* noise, int64_t stride);
+/* out [B][5]: the rows in use (the defaults when none are set); synchronises */
+int ekf_batch_get_noise(ekf_batch* b, double* out);
 int ekf_batch_sync(ekf_batch* b);
 /* Raw device arrays of the batch.  state: [B][state_stride] doubles (theta, x, y, m1x, m1y, ...).  sigma:
  * [B][sigma_stride] doubles in the engine's layout:

@@ -134,6 +134,18 @@ class EKF_SLAM {
         status_ = ekf_association_log_open(h_, path);
         report("ekf_association_log_open");
     }
+    // not in the reference: process noise q = {theta, x, y} and measurement noise r = {range, bearing} variances
+    // (ekf_set_noise); both nullptr restore the reference's values, one nullptr keeps that part at them
+    void set_noise(const double q[3], const double r[2]) {
+        if (!q && !r) {
+            status_ = ekf_set_noise(h_, nullptr);
+        } else {
+            const double row[5] = {q ? q[0] : EKF_DEFAULT_Q, q ? q[1] : EKF_DEFAULT_Q, q ? q[2] : EKF_DEFAULT_Q,
+                                   r ? r[0] : EKF_DEFAULT_R, r ? r[1] : EKF_DEFAULT_R};
+            status_ = ekf_set_noise(h_, row);
+        }
+        report("ekf_set_noise");
+    }
     ekf_filter* handle() {
         pose_ok_ = false;  // the caller may change the filter behind this object
         return h_;

@@ -1,0 +1,384 @@
+"""Per-filter process and measurement noise (Q, R): EKFBatch.set_noise / noise in the tile (n = 20), staircase
+(n <= 64) and wide (64 < n <= 1,024) layouts, and EKF_SLAM.set_noise on the fused and streamed single filters.
+
+The NOISE variants of the step kernels must give the default kernels' results when the reference values are set
+explicitly, and follow tests/_noise_ref.py (the CPU oracle's arithmetic with Q and R as arguments) otherwise."""
+import numpy as np
+import pytest
+
+from _noise_ref import DEFAULT_NOISE, NoiseOracle
+from _oracle import sigma_err, state_err
+
+pytestmark = pytest.mark.gpu
+
+M_MAX = 40
+TOL = 1e-9
+NIS_RTOL = 1e-8
+# Noise classes of the parity tests.  A smaller R makes each correction remove more of Sigma, and the relative rounding
+# error of what is left grows with it; these rows keep r >= 0.002, where the 1e-9 tolerance of the default holds.
+GRID = np.array([[1e-4, 1e-4, 1e-4, 0.01, 0.01], [4e-4, 2e-4, 3e-4, 0.003, 0.002], [2e-5, 1e-3, 5e-4, 0.03, 0.004],
+                 [0.0, 0.0, 0.0, 0.004, 0.002], [1e-3, 1e-5, 2e-4, 0.008, 0.05]])
+
+
+def _sms():
+    import torch
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def _dev(a):
+    import torch
+    return torch.as_tensor(np.ascontiguousarray(a)).cuda()
+
+
+def _c(a):
+    return np.ascontiguousarray(a)
+
+
+def _world(pkg, n):
+    nx = max(d for d in range(1, int(np.sqrt(n)) + 1) if n % d == 0)
+    return pkg.tracegen.grid_world(n // nx, nx, pitch=0.35)
+
+
+def _known(pkg, n, B, T, seed, p_vis=0.5):
+    tr = pkg.tracegen.simulate_known(_world(pkg, n), B, T, seed=seed)
+    rng = np.random.default_rng(seed)
+    vis = (tr["vis"] != 0) & (rng.random(tr["vis"].shape) < p_vis)
+    vis[0] = True
+    vis = vis.astype(np.uint8)
+    return {"twists": tr["twists"], "xy": np.ascontiguousarray(tr["xy"] * vis.repeat(2, axis=2)), "vis": vis}
+
+
+def _unknown(pkg, n, B, T, seed):
+    return pkg.tracegen.simulate_unknown(pkg.tracegen.dense_world(n), B, T, seed=seed, m_max=M_MAX)
+
+
+def _step_known(pkg, bt, tr, t, form):
+    tw, xy, vis = _c(tr["twists"][t]), _c(tr["xy"][t]), _c(tr["vis"][t])
+    if form == "dense":
+        bt.step_known(tw, xy, vis)
+    elif form == "markers":
+        bt.step_known_sparse(tw, *pkg.marker_list(xy, vis))
+    else:
+        d = (_dev(tw), _dev(xy), _dev(vis))
+        bt.step_known_dev(*(x.data_ptr() for x in d))
+        bt.sync()
+
+
+def _run_known(pkg, bt, tr, form="dense"):
+    for t in range(tr["twists"].shape[0]):
+        _step_known(pkg, bt, tr, t, form)
+    bt.sync()
+
+
+def _run_unknown(bt, tr):
+    out = [bt.step_unknown(_c(tr["twists"][t]), _c(tr["meas"][t]), _c(tr["count"][t]), M_MAX, want_assoc=True)
+           for t in range(tr["twists"].shape[0])]
+    bt.sync()
+    return np.stack(out)
+
+
+def _same_checkpoint(a, b):
+    for key in ("sigma_packed", "state", "init_flag", "known"):
+        x, y = a[key], b[key]
+        if x.dtype == np.float64:
+            x, y = x.view(np.uint64), y.view(np.uint64)
+        assert np.array_equal(x, y), key
+    assert a["updates"] == b["updates"]
+
+
+def _rows(B):
+    return GRID[np.arange(B) % len(GRID)]
+
+
+def _check_filters(bt, refs, what):
+    worst_s = worst_p = 0.0
+    states = bt.states()
+    for b, o in enumerate(refs):
+        worst_s = max(worst_s, state_err(states[b], o.state))
+        worst_p = max(worst_p, sigma_err(bt.sigma(b), o.sigma))
+    print(f"{what}: state {worst_s:.2e}, sigma {worst_p:.2e}")
+    assert worst_s < TOL and worst_p < TOL, (what, worst_s, worst_p)
+
+
+# ---------------------------------------------------------------- 1. reference values set explicitly
+CASES = [("tile-dense", 20, "dense"), ("tile-markers", 20, "markers"), ("tile-device", 20, "device"),
+         ("tile-unknown", 20, "unknown"), ("stair-known", 33, "dense"), ("stair-unknown", 33, "unknown"),
+         ("stair-device", 33, "device"), ("wide-dense", 100, "dense"), ("wide-markers", 100, "markers"),
+         ("wide-device", 100, "device")]
+
+
+@pytest.mark.parametrize("name,n,form", CASES, ids=[c[0] for c in CASES])
+def test_reference_values_bit_identical(gpu_pkg, name, n, form):
+    B, T = (48, 8) if n <= 64 else (6, 5)
+    tr = _unknown(gpu_pkg, n, B, T, seed=n + 9) if form == "unknown" else _known(gpu_pkg, n, B, T, seed=n + 9)
+    plain, explicit = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
+    explicit.set_noise([1e-4] * 3, [0.01] * 2)
+    assert np.array_equal(explicit.noise(), np.tile(DEFAULT_NOISE, (B, 1)))
+    if form == "unknown":
+        assert np.array_equal(_run_unknown(plain, tr), _run_unknown(explicit, tr))
+    else:
+        _run_known(gpu_pkg, plain, tr, form)
+        _run_known(gpu_pkg, explicit, tr, form)
+    _same_checkpoint(plain.checkpoint(), explicit.checkpoint())
+    assert plain.launch_count == explicit.launch_count
+
+
+def _single_trace(pkg, n, T, seed):
+    tk = _known(pkg, n, 1, T, seed)
+    tu = _unknown(pkg, n, 1, T, seed + 1)
+    return tk, tu
+
+
+def _drive_single(f, tk, tu, t, known):
+    f.prediction(tuple(tk["twists"][t, 0]))
+    f.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
+    f.prediction(tuple(tu["twists"][t, 0]))
+    m = int(tu["count"][t, 0])
+    return f.data_association(tu["meas"][t, 0, :m], known)["assoc"]
+
+
+@pytest.mark.parametrize("engine", ["fused", "stream"])
+def test_single_reference_values_bit_identical(gpu_pkg, engine):
+    n, T = 20, 6
+    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
+    tk, tu = _single_trace(gpu_pkg, n, T, seed=31)
+    a, b = gpu_pkg.EKF_SLAM(n, engine=eng), gpu_pkg.EKF_SLAM(n, engine=eng)
+    b.set_noise([1e-4] * 3, [0.01] * 2)
+    ka, kb = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
+    for t in range(T):
+        assert np.array_equal(_drive_single(a, tk, tu, t, ka), _drive_single(b, tk, tu, t, kb))
+    assert np.array_equal(a.state.view(np.uint64), b.state.view(np.uint64))
+    assert np.array_equal(a.sigma.view(np.uint64), b.sigma.view(np.uint64))
+    assert a.calculate_maha_dis((0.3, 0.4), 2) == b.calculate_maha_dis((0.3, 0.4), 2)
+    assert a.launch_count == b.launch_count
+
+
+# ---------------------------------------------------------------- 2. per-filter noise against the reference
+@pytest.mark.parametrize("n", [20, 33, 100, 256])
+def test_known_matches_reference(gpu_pkg, n):
+    B, T = (10, 8) if n <= 64 else (5, 5)
+    tr = _known(gpu_pkg, n, B, T, seed=300 + n)
+    rows = _rows(B)
+    bt = gpu_pkg.EKFBatch(B, n)
+    bt.set_noise(rows[:, :3], rows[:, 3:])
+    assert np.array_equal(bt.noise(), rows)
+    bt.set_nis(True)
+    _run_known(gpu_pkg, bt, tr)
+    refs = [NoiseOracle(n, rows[b]) for b in range(B)]
+    for t in range(T):
+        for b, o in enumerate(refs):
+            o.prediction(*tr["twists"][t, b])
+            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+    _check_filters(bt, refs, f"known n={n}")
+    _check_nis(bt, refs, f"known n={n}")
+
+
+def _check_nis(bt, refs, what):
+    r = bt.nis(per_filter=True)
+    assert np.array_equal(r["nis_count"][:len(refs)], [o.acc[2] for o in refs]), what
+    for col, k in (("nis_sum", 0), ("nis_sq_sum", 1)):
+        want = np.array([o.acc[k] for o in refs])
+        err = np.abs(r[col][:len(refs)] - want) / np.maximum(np.abs(want), 1e-300)
+        print(f"{what}: {col} worst relative deviation {err.max():.2e}")
+        assert err.max() < NIS_RTOL, (what, col)
+
+
+@pytest.mark.parametrize("n", [20, 33])
+def test_unknown_matches_reference(gpu_pkg, n):
+    B, T = 10, 10
+    tr = _unknown(gpu_pkg, n, B, T, seed=400 + n)
+    rows = _rows(B)
+    bt = gpu_pkg.EKFBatch(B, n)
+    bt.set_noise(rows[:, :3], rows[:, 3:])
+    bt.set_nis(True)
+    assoc = _run_unknown(bt, tr)
+    refs = [NoiseOracle(n, rows[b]) for b in range(B)]
+    known = [np.zeros(n, np.uint8) for _ in range(B)]
+    for t in range(T):
+        for b, o in enumerate(refs):
+            o.prediction(*tr["twists"][t, b])
+            m = int(np.clip(tr["count"][t, b], 0, M_MAX))
+            a, _ = o.data_association(tr["meas"][t, b, :m], known[b])
+            assert np.array_equal(a, assoc[t, b, :m]), (t, b)
+    assert np.array_equal(bt.known, np.stack(known))
+    _check_filters(bt, refs, f"unknown n={n}")
+    _check_nis(bt, refs, f"unknown n={n}")
+
+
+@pytest.mark.parametrize("engine", ["fused", "stream"])
+def test_single_matches_reference(gpu_pkg, engine):
+    n, T = 20, 6
+    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
+    tk, tu = _single_trace(gpu_pkg, n, T, seed=41)
+    row = GRID[1]
+    f = gpu_pkg.EKF_SLAM(n, engine=eng)
+    f.set_noise(row[:3], row[3:])
+    assert np.array_equal(f.noise, row)
+    o = NoiseOracle(n, row)
+    kf, ko = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
+    for t in range(T):
+        a = _drive_single(f, tk, tu, t, kf)
+        o.prediction(*tk["twists"][t, 0])
+        o.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
+        o.prediction(*tu["twists"][t, 0])
+        m = int(tu["count"][t, 0])
+        assert np.array_equal(a, o.data_association(tu["meas"][t, 0, :m], ko)[0]), t
+    assert state_err(f.state, o.state) < TOL and sigma_err(f.sigma, o.sigma) < TOL
+    for i in (0, 5, 13):
+        d, want = f.calculate_maha_dis((0.3, -0.2), i), o.maha(0.3, -0.2, i)
+        assert abs(d - want) <= TOL * max(1.0, abs(want)), (i, d, want)
+
+
+@pytest.mark.parametrize("n", [100, 256])
+def test_wide_bit_identical_to_streamed(gpu_pkg, n):
+    B, T = 3, 4
+    tr = _known(gpu_pkg, n, B, T, seed=500 + n)
+    rows = _rows(B)
+    bt = gpu_pkg.EKFBatch(B, n)
+    bt.set_noise(rows[:, :3], rows[:, 3:])
+    _run_known(gpu_pkg, bt, tr)
+    for b in range(B):
+        f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
+        f.set_carry_pending(False)
+        f.set_noise(rows[b, :3], rows[b, 3:])
+        for t in range(T):
+            f.prediction(tuple(tr["twists"][t, b]))
+            f.measurement(tr["xy"][t, b], tr["vis"][t, b])
+        assert np.array_equal(f.state.view(np.uint64), bt.states()[b].view(np.uint64)), b
+        assert np.array_equal(f.sigma.view(np.uint64), bt.sigma(b).view(np.uint64)), b
+
+
+# ---------------------------------------------------------------- 3. several filters per persistent CTA
+@pytest.mark.parametrize("n,form", [(20, "known"), (20, "unknown"), (33, "known"), (65, "known")])
+def test_noise_classes_over_replicas(gpu_pkg, n, form):
+    """One trajectory for every filter, K noise classes permuted over a batch beyond one resident wave: every replica
+    is bit-identical to its class's first filter, and the class representatives match the reference."""
+    K = len(GRID)
+    B = (2 * _sms() + 5) if n > 64 else (64 * _sms() + 37)
+    T = 4 if n > 64 else 8
+    cls = np.random.default_rng(n).permutation(np.arange(B) % K)
+    one = _unknown(gpu_pkg, n, 1, T, seed=600 + n) if form == "unknown" else _known(gpu_pkg, n, 1, T, seed=600 + n)
+    tr = {k: np.ascontiguousarray(np.repeat(v, B, axis=1)) for k, v in one.items() if k in ("twists", "xy", "vis", "meas", "count")}
+    bt = gpu_pkg.EKFBatch(B, n)
+    bt.set_noise(GRID[cls, :3], GRID[cls, 3:])
+    if form == "unknown":
+        _run_unknown(bt, tr)
+    else:
+        _run_known(gpu_pkg, bt, tr)
+    st = bt.states().view(np.uint64)
+    reps = [int(np.flatnonzero(cls == k)[0]) for k in range(K)]
+    for k in range(K):
+        members = np.flatnonzero(cls == k)
+        assert (st[members] == st[reps[k]]).all(), k
+    for k in range(K):
+        o = NoiseOracle(n, GRID[k])
+        known = np.zeros(n, np.uint8)
+        for t in range(T):
+            o.prediction(*one["twists"][t, 0])
+            if form == "unknown":
+                o.data_association(one["meas"][t, 0, :int(one["count"][t, 0])], known)
+            else:
+                o.measurement(one["xy"][t, 0], one["vis"][t, 0])
+        assert state_err(bt.states()[reps[k]], o.state) < TOL and sigma_err(bt.sigma(reps[k]), o.sigma) < TOL, k
+    assert len(set(tuple(st[r]) for r in reps)) == K  # the classes really differ
+
+
+# ---------------------------------------------------------------- 4. changing the noise mid-run
+@pytest.mark.parametrize("n", [20, 33, 100])
+def test_noise_changed_mid_run(gpu_pkg, n):
+    B, T = 4, 6
+    tr = _known(gpu_pkg, n, B, T, seed=700 + n)
+    bt = gpu_pkg.EKFBatch(B, n)
+    refs = [NoiseOracle(n) for _ in range(B)]
+    for t in range(T):
+        if t == 3:
+            bt.set_noise(_rows(B)[:, :3], _rows(B)[:, 3:])
+            for b, o in enumerate(refs):
+                o.set_noise(_rows(B)[b])
+        if t == 5:
+            bt.set_noise()
+            for o in refs:
+                o.set_noise(DEFAULT_NOISE)
+        _step_known(gpu_pkg, bt, tr, t, "dense")
+        for b, o in enumerate(refs):
+            o.prediction(*tr["twists"][t, b])
+            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+    bt.sync()
+    _check_filters(bt, refs, f"mid-run n={n}")
+
+
+@pytest.mark.parametrize("engine", ["fused", "stream"])
+def test_single_noise_changed_with_prediction_pending(gpu_pkg, engine):
+    """prediction(), then set_noise(), then measurement(): the prediction uses the old Q (the fused engine still holds
+    it back when set_noise() is called), the corrections the new R."""
+    n, T = 20, 5
+    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
+    tk = _known(gpu_pkg, n, 1, T, seed=801)
+    f, o = gpu_pkg.EKF_SLAM(n, engine=eng), NoiseOracle(n)
+    for t in range(T):
+        f.prediction(tuple(tk["twists"][t, 0]))
+        o.prediction(*tk["twists"][t, 0])
+        row = GRID[1 + t % 4]
+        f.set_noise(row[:3], row[3:])
+        o.set_noise(row)
+        f.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
+        o.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
+    assert state_err(f.state, o.state) < TOL and sigma_err(f.sigma, o.sigma) < TOL
+
+
+# ---------------------------------------------------------------- 5. configuration handling
+def test_broadcast_clone_and_checkpoints(gpu_pkg):
+    n, B, T = 20, 16, 5
+    tr = _known(gpu_pkg, n, B, T, seed=901)
+    row = GRID[2]
+    shared, per = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
+    shared.set_noise(row[:3], row[3:])
+    per.set_noise(np.tile(row[:3], (B, 1)), np.tile(row[3:], (B, 1)))
+    _run_known(gpu_pkg, shared, tr)
+    _run_known(gpu_pkg, per, tr)
+    _same_checkpoint(shared.checkpoint(), per.checkpoint())
+    # checkpoints carry no noise: a restored batch keeps its own setting, a fresh one the reference values
+    ck = shared.checkpoint()
+    fresh = gpu_pkg.EKFBatch(B, n)
+    fresh.restore(ck)
+    assert np.array_equal(fresh.noise(), np.tile(DEFAULT_NOISE, (B, 1)))
+    per.set_noise(GRID[1, :3], GRID[1, 3:])
+    per.restore(ck)
+    assert np.array_equal(per.noise(), np.tile(GRID[1], (B, 1)))
+    for eng in (gpu_pkg.ENGINE_FUSED, gpu_pkg.ENGINE_STREAM):
+        f = gpu_pkg.EKF_SLAM(n, engine=eng)
+        f.set_noise(row[:3], row[3:])
+        f.prediction((0.01, 0.02))
+        g = f.clone()
+        assert np.array_equal(g.noise, row)
+        for h in (f, g):
+            h.prediction(tuple(tr["twists"][1, 0]))
+            h.measurement(tr["xy"][0, 0], tr["vis"][0, 0])
+        assert np.array_equal(f.sigma.view(np.uint64), g.sigma.view(np.uint64))
+        f.set_noise()
+        assert np.array_equal(f.noise, DEFAULT_NOISE)
+
+
+@pytest.mark.parametrize("bad", [(np.nan, 1e-4, 1e-4, 0.01, 0.01), (1e-4, -1e-6, 1e-4, 0.01, 0.01),
+                                 (1e-4, 1e-4, 1e-4, 0.0, 0.01), (1e-4, 1e-4, 1e-4, 0.01, np.inf)],
+                         ids=["nan", "negative-q", "zero-r", "inf-r"])
+def test_invalid_rows_rejected(gpu_pkg, bad):
+    n, B = 20, 8
+    bad = np.array(bad)
+    bt = gpu_pkg.EKFBatch(B, n)
+    rows = _rows(B)
+    bt.set_noise(rows[:, :3], rows[:, 3:])
+    before = bt.checkpoint()
+    mixed = rows.copy()
+    mixed[5] = bad
+    for q, r in ((mixed[:, :3], mixed[:, 3:]), (bad[:3], bad[3:])):
+        with pytest.raises(gpu_pkg.EkfError):
+            bt.set_noise(q, r)
+        assert np.array_equal(bt.noise(), rows)
+    _same_checkpoint(before, bt.checkpoint())
+    for eng in (gpu_pkg.ENGINE_FUSED, gpu_pkg.ENGINE_STREAM):
+        f = gpu_pkg.EKF_SLAM(n, engine=eng)
+        f.set_noise(GRID[1, :3], GRID[1, 3:])
+        with pytest.raises(gpu_pkg.EkfError):
+            f.set_noise(bad[:3], bad[3:])
+        assert np.array_equal(f.noise, GRID[1])
