@@ -28,6 +28,7 @@ class NoiseOracle:
         self.sigma[np.arange(3, self.N), np.arange(3, self.N)] = 100.0
         self.init_flag = False
         self.acc = np.zeros(4)
+        self.values = []  # every scored value, in order
         self.set_noise(noise)
 
     def set_noise(self, noise):
@@ -100,6 +101,7 @@ class NoiseOracle:
             v = nu0 * t0 + nu1 * t1
             if math.isfinite(v):
                 self.acc += (v, v * v, 1.0, 0.0)
+                self.values.append(v)
             else:
                 self.acc[3] += 1.0
 

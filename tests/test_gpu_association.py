@@ -12,20 +12,13 @@ import functools
 import numpy as np
 import pytest
 
+from _batch import assert_clear, robot_frame
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-9
 FAR = np.array([40.0, 35.0])  # a reading far from every landmark: a new one, or dropped when the map is full
-
-
-def _robot_frame(state, k, offset=(0.0, 0.0)):
-    """Reading of landmark k's current estimate as the robot sees it from the estimated pose, plus an offset."""
-    th, x, y = state[:3]
-    dx, dy = state[3 + 2 * k] - x, state[4 + 2 * k] - y
-    c, s = np.cos(th), np.sin(th)
-    return np.array([c * dx + s * dy + offset[0], -s * dx + c * dy + offset[1]])
 
 
 @functools.lru_cache(maxsize=None)
@@ -99,8 +92,8 @@ def _graze(o, k, known_count):
         lo, hi = 0.0, 4.0
         for _ in range(40):
             mid = 0.5 * (lo + hi)
-            lo, hi = (mid, hi) if nearest(_robot_frame(o.state, k, mid * u))[0] < 1.6 else (lo, mid)
-        xy = _robot_frame(o.state, k, hi * u)
+            lo, hi = (mid, hi) if nearest(robot_frame(o.state, k, mid * u))[0] < 1.6 else (lo, mid)
+        xy = robot_frame(o.state, k, hi * u)
         d, i = nearest(xy)
         if d < 1.0:  # every point within reach in this direction is close to some landmark
             continue
@@ -109,15 +102,6 @@ def _graze(o, k, known_count):
         first = xy if first is None else first
     assert first is not None
     return first
-
-
-def _assert_clear(dmin, second):
-    """No decision sits within 1e-6 (relative) of a gate or of the runner-up, where the device and the oracle could
-    round to different sides."""
-    has = dmin < 10.0
-    margin = np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(second - dmin)]),
-                      np.abs(second - 10.0))
-    assert np.all(margin > 1e-6 * np.maximum(1.0, np.abs(dmin))), "threshold tie in the fixture"
 
 
 def _associate(f, o, xy, known_count, tie=False, nan_entry=None):
@@ -131,7 +115,7 @@ def _associate(f, o, xy, known_count, tie=False, nan_entry=None):
     if tie:
         assert np.all(sec == dmin) and np.all(r["second"] == r["dmin"])
     else:
-        _assert_clear(dmin, sec)
+        assert_clear(dmin, sec)
     assert np.array_equal(r["assoc"], a), (r["assoc"], a)
     assert np.array_equal(r["created"], cr) and np.array_equal(kf, ko)
     np.testing.assert_allclose(r["dmin"], dmin, rtol=1e-7, atol=1e-9)
@@ -150,7 +134,7 @@ def _hit(f, o, k, partner, base):
     off = np.array([0.01, -0.005])
     c, s = np.cos(base[0][0]), np.sin(base[0][0])
     _set(f, o, *_duplicate(*base, k, partner, shift=-3.0 * np.array([c * off[0] - s * off[1], s * off[0] + c * off[1]])))
-    xy = _robot_frame(o.state, k, off)
+    xy = robot_frame(o.state, k, off)
     d_partner = o.maha(*xy, partner)
     a, dmin, sec, cr = _associate(f, o, xy, o.n)
     assert a[0] == k and cr[0] == 0 and sec[0] == d_partner
@@ -159,7 +143,7 @@ def _hit(f, o, k, partner, base):
 def _tie(f, o, i, j, base):
     """Landmark i copied into slot j: a reading of it is exactly as far from both, and the lower index wins."""
     _set(f, o, *_duplicate(*base, i, j))
-    a, _, _, _ = _associate(f, o, _robot_frame(o.state, i, (0.01, -0.005)), o.n, tie=True)
+    a, _, _, _ = _associate(f, o, robot_frame(o.state, i, (0.01, -0.005)), o.n, tie=True)
     assert a[0] == min(i, j)
 
 
@@ -210,7 +194,7 @@ def test_streamed_engine(gpu_pkg, max_pending):
     st = base[0].copy()
     st[3 + 2 * q] = np.nan
     _set(f, o, st, base[1])
-    xy = np.stack([_robot_frame(base[0], q), _robot_frame(st, q + 1, (0.01, -0.005)), _robot_frame(st, 7)])
+    xy = np.stack([robot_frame(base[0], q), robot_frame(st, q + 1, (0.01, -0.005)), robot_frame(st, 7)])
     a, _, _, _ = _associate(f, o, xy, n, nan_entry=3 + 2 * q)
     assert q not in a and a[1] == q + 1 and a[2] == 7
 
@@ -231,7 +215,7 @@ def test_sharded_local_emulation(gpu_pkg, world):
         targets += [first, last] + [k for k in (first + 255, first + 256) if k < last]
     assert len(set(targets)) == len(targets) == {2: 8, 3: 6}[world]  # 200 landmarks per rank at world = 3: one CTA
     for k in targets:
-        a, _, _, cr = _associate(f, o, _robot_frame(o.state, k, (0.01, -0.005)), n)
+        a, _, _, cr = _associate(f, o, robot_frame(o.state, k, (0.01, -0.005)), n)
         assert a[0] == k and cr[0] == 0
         a, _, _, cr = _associate(f, o, _graze(o, k, n), n)
         assert a[0] == -1 and cr[0] == 0

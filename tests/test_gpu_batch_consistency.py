@@ -7,35 +7,25 @@ leave the batch untouched."""
 import numpy as np
 import pytest
 
+from _batch import grid_world, run_known, run_unknown, sms, unknown_trace
+
 pytestmark = pytest.mark.gpu
 
 RTOL = 1e-10
 
 
-def _world(pkg, n):
-    nx = max(d for d in range(1, int(np.sqrt(n)) + 1) if n % d == 0)  # n landmarks on an nx x (n / nx) grid
-    return pkg.tracegen.grid_world(n // nx, nx, pitch=0.35)
-
-
 def _known_batch(pkg, n, B, T, seed):
-    w = _world(pkg, n)
+    w = grid_world(pkg, n)
     tr = pkg.tracegen.simulate_known(w, B, T, seed=seed)
     bt = pkg.EKFBatch(B, n)
-    for t in range(T):
-        bt.step_known(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["xy"][t]),
-                      np.ascontiguousarray(tr["vis"][t]))
-    bt.sync()
+    run_known(pkg, bt, tr)
     return bt, tr, w
 
 
 def _unknown_batch(pkg, n, B, T, seed, m_max):
-    w = pkg.tracegen.dense_world(n)
-    tr = pkg.tracegen.simulate_unknown(w, B, T, seed=seed, m_max=m_max)
+    tr = unknown_trace(pkg, n, B, T, seed, m_max)
     bt = pkg.EKFBatch(B, n)
-    for t in range(T):
-        bt.step_unknown(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["meas"][t]),
-                        np.ascontiguousarray(tr["count"][t]), m_max)
-    bt.sync()
+    run_unknown(bt, tr, m_max)
     return bt, tr
 
 
@@ -194,17 +184,12 @@ def test_unknown_association_scores_known_slots_only(gpu_pkg):
         np.testing.assert_allclose(res["landmark_nees_sum"][b], sum(vals), rtol=RTOL)
 
 
-def _sms():
-    import torch
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
 @pytest.mark.parametrize("n", [20, 33])
 def test_batch_partials_are_the_per_filter_sums_and_repeat_bit_for_bit(gpu_pkg, n):
     """B above 64 warps per SM (more filters than any grid of the kernel has warps) and not a multiple of 8 warps."""
-    B = 64 * _sms() + 37
+    B = 64 * sms() + 37
     T = 4
-    w = _world(gpu_pkg, n)
+    w = grid_world(gpu_pkg, n)
     tr = gpu_pkg.tracegen.simulate_known(w, 61, T, seed=5)  # filter b runs trajectory b mod 61
 
     def rep(a):

@@ -9,6 +9,7 @@ of the per-filter measurement count (both batch kernels)."""
 import numpy as np
 import pytest
 
+from _batch import assert_clear, dev, robot_frame, run_known, run_unknown, step_known
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
@@ -34,14 +35,6 @@ def pack_staircase(dense, N):
 
 def _strides(N):
     return (_stair_row_base(N, N) + 1) & ~1, (N + 1) & ~1  # per-filter Sigma and state strides in doubles
-
-
-def _robot_frame(state, k, offset=(0.0, 0.0)):
-    """Reading of landmark k's current estimate as the robot sees it from the estimated pose, plus an offset."""
-    th, x, y = state[:3]
-    dx, dy = state[3 + 2 * k] - x, state[4 + 2 * k] - y
-    c, s = np.cos(th), np.sin(th)
-    return np.array([c * dx + s * dy + offset[0], -s * dx + c * dy + offset[1]])
 
 
 def _grid_world(pkg, n, pitch=0.3):
@@ -83,10 +76,7 @@ def test_known_association_dense_matches_oracle(gpu_pkg, n):
     assert tr["vis"][1:].any(axis=(0, 1)).all()  # every slot is corrected at least once
     bt = gpu_pkg.EKFBatch(B, n)
     assert bt.engine == gpu_pkg.ENGINE_FUSED
-    for t in range(T):
-        bt.step_known(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["xy"][t]),
-                      np.ascontiguousarray(tr["vis"][t]))
-    bt.sync()
+    run_known(gpu_pkg, bt, tr)
     assert bt.update_count == int(tr["vis"].sum())
     states = bt.states()
     for b in _picks(B, n):
@@ -146,15 +136,6 @@ def _unknown_world(pkg):
     return pkg.tracegen.grid_world(7, 7, pitch=0.45, max_visible=3.0)
 
 
-def _assert_clear(dmin, second):
-    """No decision of the fixture sits within 1e-6 (relative) of a gate or of a tie with the runner-up, where the
-    device and the oracle could round to different sides."""
-    has = dmin < 10.0
-    margin = np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(second - dmin)]),
-                      np.abs(second - 10.0))
-    assert np.all(margin > 1e-6 * np.maximum(1.0, np.abs(dmin))), "threshold tie in the fixture: pick another seed"
-
-
 @pytest.mark.parametrize("n,m_max", [(6, 1), (6, 7), (6, 40), (33, 1), (33, 7), (33, 40), (64, 1), (64, 7), (64, 40),
                                      (20, 40)])
 def test_unknown_association_matches_oracle(gpu_pkg, n, m_max):
@@ -164,8 +145,7 @@ def test_unknown_association_matches_oracle(gpu_pkg, n, m_max):
     w.n_slots = n
     tu = gpu_pkg.tracegen.simulate_unknown(w, B, T, seed=500 + n + m_max, m_max=m_max)
     bt = gpu_pkg.EKFBatch(B, n)
-    assoc = [bt.step_unknown(np.ascontiguousarray(tu["twists"][t]), np.ascontiguousarray(tu["meas"][t]),
-                             np.ascontiguousarray(tu["count"][t]), m_max, want_assoc=True) for t in range(T)]
+    assoc = run_unknown(bt, tu, m_max)
     states, known = bt.states(), bt.known
     assert int(tu["count"].max()) == min(m_max, 49)
     created = full = 0
@@ -176,7 +156,7 @@ def test_unknown_association_matches_oracle(gpu_pkg, n, m_max):
             o.prediction(*tu["twists"][t, b])
             m = int(tu["count"][t, b])
             a, dmin, sec, cr = o.data_association(tu["meas"][t, b, :m], k)
-            _assert_clear(dmin, sec)
+            assert_clear(dmin, sec)
             assert np.array_equal(assoc[t][b, :m], a), (b, t)
             assert np.all(assoc[t][b, m:] == -1)
             created += int(cr.sum())
@@ -200,8 +180,7 @@ def test_checkpoint_resume_is_bit_identical(gpu_pkg, tmp_path, mode):
 
     def step(bt, t):
         if mode == "known":
-            bt.step_known(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["xy"][t]),
-                          np.ascontiguousarray(tr["vis"][t]))
+            step_known(gpu_pkg, bt, tr, t)
         else:
             bt.step_unknown(np.ascontiguousarray(tu["twists"][t]), np.ascontiguousarray(tu["meas"][t]),
                             np.ascontiguousarray(tu["count"][t]), M)
@@ -230,10 +209,7 @@ def test_association_ties_lowest_index_wins(gpu_pkg):
     N = 3 + 2 * n
     tr = _known_trace(gpu_pkg, n, B, 4, seed=31)
     bt = gpu_pkg.EKFBatch(B, n)
-    for t in range(4):
-        bt.step_known(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["xy"][t]),
-                      np.ascontiguousarray(tr["vis"][t]))
-    bt.sync()
+    run_known(gpu_pkg, bt, tr)
     ck = bt.checkpoint()
     ss, sts = _strides(N)
     size = _stair_row_base(N, N)
@@ -259,7 +235,7 @@ def test_association_ties_lowest_index_wins(gpu_pkg):
     meas = np.zeros((B, 1, 2))
     for b, (i, j) in enumerate(pairs):
         oracles[b].prediction(*tw[b])
-        meas[b, 0] = _robot_frame(oracles[b].state, i, (0.01, -0.005))
+        meas[b, 0] = robot_frame(oracles[b].state, i, (0.01, -0.005))
     assoc = bt.step_unknown(tw, meas, np.ones(B, np.int32), 1, want_assoc=True)
     states = bt.states()
     for b, (i, j) in enumerate(pairs):
@@ -280,10 +256,6 @@ def _count_fixture(pkg, n, B, M):
     tu = pkg.tracegen.simulate_unknown(w, B, 2, seed=40 + n, m_max=M, shuffle=False)
     assert np.all(tu["count"] == M)
     return tu
-
-
-def _dev(a, torch):
-    return torch.as_tensor(np.ascontiguousarray(a)).cuda()
 
 
 @pytest.mark.parametrize("n", [20, 33])
@@ -320,7 +292,7 @@ def test_measurement_count_is_clamped(gpu_pkg, n):
             assert np.all(assoc[b] == -1) and np.array_equal(known[b], known0[b])
         else:
             want, dmin, sec, _ = o.data_association(tu["meas"][1, b], k)
-            _assert_clear(dmin, sec)
+            assert_clear(dmin, sec)
             assert np.array_equal(assoc[b], want), (b, assoc[b], want)
             assert np.array_equal(known[b], k)
             if b == 2:
@@ -333,7 +305,7 @@ def test_measurement_count_is_clamped(gpu_pkg, n):
     bad_d = bad.copy()
     bad_d[0] = -3
     out = torch.full((B + 1, M), 77, dtype=torch.int32, device="cuda")
-    t_tw, t_me, t_ct = _dev(tw1, torch), _dev(me1, torch), _dev(bad_d, torch)
+    t_tw, t_me, t_ct = dev(tw1), dev(me1), dev(bad_d)
     torch.cuda.synchronize()
     d.step_unknown_dev(t_tw.data_ptr(), t_me.data_ptr(), t_ct.data_ptr(), M, out[1].data_ptr())
     d.sync()

@@ -15,6 +15,7 @@ import ctypes
 import numpy as np
 import pytest
 
+from _batch import assert_clear, assert_replicas, assert_same_checkpoint, dev, grid_world, replicate, sms
 from _oracle import OracleEKF, sigma_err, state_err
 from test_gpu_batch_wide import _streamed
 
@@ -29,49 +30,15 @@ KNOWN_CLASSES = (0, 1, 2, 3, 7, 20)  # corrections per step of trajectory k's cl
 WIDE_CLASSES = (0, 1, 13, 14, 15, 29)
 
 
-def _sms():
-    import torch
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-def _replicate(a, B):
-    """[T, K, ...] -> [T, B, ...]: filter b runs trajectory b mod K."""
-    return np.ascontiguousarray(a[:, np.arange(B) % K])
-
-
-def _dev(a):
-    import torch
-    return torch.as_tensor(np.ascontiguousarray(a)).cuda()
-
-
-def _assert_replicas(a, B, what):
-    """Rows b and b mod K of a [B, ...] array are bit-identical (floats compared as their bit patterns)."""
-    a = np.ascontiguousarray(a).reshape(B, -1)
-    if a.dtype == np.float64:
-        a = a.view(np.uint64)
-    for k in range(K):
-        bad = np.flatnonzero((a[k::K] != a[k]).any(axis=1))
-        assert bad.size == 0, f"{what}: filter {k + K * int(bad[0])} differs from filter {k}"
-
-
 def _assert_checkpoint_replicas(bt):
     ck = bt.checkpoint()
     for key in ("sigma_packed", "state", "init_flag", "known"):
-        _assert_replicas(ck[key], bt.B, key)
-    _assert_replicas(bt.states(), bt.B, "states()")
+        assert_replicas(ck[key], bt.B, K, key)
+    assert_replicas(bt.states(), bt.B, K, "states()")
     for k in range(K):
         last = k + K * ((bt.B - 1 - k) // K)
         assert np.array_equal(bt.sigma(last).view(np.uint64), bt.sigma(k).view(np.uint64)), (k, last)
     return ck
-
-
-def _assert_same_checkpoint(a, b):
-    for key in ("sigma_packed", "state", "init_flag", "known"):
-        x, y = a[key], b[key]
-        if x.dtype == np.float64:
-            x, y = x.view(np.uint64), y.view(np.uint64)
-        assert np.array_equal(x, y), key
-    assert a["updates"] == b["updates"]
 
 
 def _assert_tile_schedule(busy, sms):
@@ -117,7 +84,7 @@ def known_inputs(gpu_pkg):
 def _sparse_dev(bt, tw, off, ids, pts):
     """ekf_batch_step_known_sparse_dev (no Python wrapper): the marker list in device memory."""
     import torch
-    d_tw, d_off, d_ids, d_pts = _dev(tw), _dev(off), _dev(ids if ids.size else np.zeros(1, np.uint8)), _dev(pts)
+    d_tw, d_off, d_ids, d_pts = dev(tw), dev(off), dev(ids if ids.size else np.zeros(1, np.uint8)), dev(pts)
     torch.cuda.synchronize()
     rc = bt._L.ekf_batch_step_known_sparse_dev(bt._h, d_tw.data_ptr(), d_off.data_ptr(), d_ids.data_ptr(),
                                                d_pts.data_ptr(), ctypes.c_int64(int(off[-1])))
@@ -130,17 +97,16 @@ def test_tile_known_replicas_in_every_input_form(gpu_pkg, known_inputs):
     B = 64 x SMs + 37: bit-identical replicas, the four forms bit-identical to each other, the K references against
     the oracle."""
     import torch
-    sms = _sms()
-    B = 64 * sms + 37
-    tw, xy, vis = (_replicate(known_inputs[k], B) for k in ("twists", "xy", "vis"))
-    _assert_tile_schedule(vis.any(axis=2), sms)
-    host, dev, sp_host, sp_dev = (gpu_pkg.EKFBatch(B, NT) for _ in range(4))
+    B = 64 * sms() + 37
+    tw, xy, vis = (replicate(known_inputs[k], B, K) for k in ("twists", "xy", "vis"))
+    _assert_tile_schedule(vis.any(axis=2), sms())
+    host, device, sp_host, sp_dev = (gpu_pkg.EKFBatch(B, NT) for _ in range(4))
     for t in range(T_KNOWN):
         host.step_known(tw[t], xy[t], vis[t])
-        d_tw, d_xy, d_vis = _dev(tw[t]), _dev(xy[t]), _dev(vis[t])
+        d_tw, d_xy, d_vis = dev(tw[t]), dev(xy[t]), dev(vis[t])
         torch.cuda.synchronize()
-        dev.step_known_dev(d_tw.data_ptr(), d_xy.data_ptr(), d_vis.data_ptr())
-        dev.sync()
+        device.step_known_dev(d_tw.data_ptr(), d_xy.data_ptr(), d_vis.data_ptr())
+        device.sync()
         off, ids, pts = gpu_pkg.marker_list(xy[t], vis[t])
         assert (np.diff(off) == 0).any()  # some filters list no marker at all
         sp_host.step_known_sparse(tw[t], off, ids, pts)
@@ -148,8 +114,8 @@ def test_tile_known_replicas_in_every_input_form(gpu_pkg, known_inputs):
     host.sync(), sp_host.sync()
     assert host.update_count == int(vis.sum())
     ck = _assert_checkpoint_replicas(host)
-    for other in (dev, sp_host, sp_dev):
-        _assert_same_checkpoint(other.checkpoint(), ck)
+    for other in (device, sp_host, sp_dev):
+        assert_same_checkpoint(other.checkpoint(), ck)
     states = host.states()
     for k in range(K):
         o = OracleEKF(NT)
@@ -183,38 +149,28 @@ def unknown_inputs(gpu_pkg):
     return {"twists": tu["twists"], "meas": tu["meas"], "count": count}
 
 
-def _assert_clear(dmin, second):
-    """No decision within 1e-6 (relative) of a gate or of a tie with the runner-up, where the device and the oracle
-    could round to different sides."""
-    has = dmin < 10.0
-    margin = np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(second - dmin)]),
-                      np.abs(second - 10.0))
-    assert np.all(margin > 1e-6 * np.maximum(1.0, np.abs(dmin))), "threshold tie in the fixture: pick another seed"
-
-
 def test_tile_unknown_replicas_host_and_device(gpu_pkg, unknown_inputs):
     """ekf_fused_tile_kernel<true> at m_max = 40 and B = 64 x SMs + 37, through step_unknown(want_assoc=True) and
     step_unknown_dev with a device count array: bit-identical replicas in association outputs, known lists, state and
     Sigma; the K references against the oracle."""
     import torch
-    sms = _sms()
-    B = 64 * sms + 37
-    tw, meas, cnt = (_replicate(unknown_inputs[k], B) for k in ("twists", "meas", "count"))
-    _assert_tile_schedule(cnt > 0, sms)
-    host, dev = gpu_pkg.EKFBatch(B, NT), gpu_pkg.EKFBatch(B, NT)
+    B = 64 * sms() + 37
+    tw, meas, cnt = (replicate(unknown_inputs[k], B, K) for k in ("twists", "meas", "count"))
+    _assert_tile_schedule(cnt > 0, sms())
+    host, device = gpu_pkg.EKFBatch(B, NT), gpu_pkg.EKFBatch(B, NT)
     assoc = []
     out = torch.empty((B, M_MAX), dtype=torch.int32, device="cuda")
     for t in range(T_UNKNOWN):
         assoc.append(host.step_unknown(tw[t], meas[t], cnt[t], M_MAX, want_assoc=True))
-        d_tw, d_me, d_ct = _dev(tw[t]), _dev(meas[t]), _dev(cnt[t])
+        d_tw, d_me, d_ct = dev(tw[t]), dev(meas[t]), dev(cnt[t])
         out.fill_(77)
         torch.cuda.synchronize()
-        dev.step_unknown_dev(d_tw.data_ptr(), d_me.data_ptr(), d_ct.data_ptr(), M_MAX, out.data_ptr())
-        dev.sync()
+        device.step_unknown_dev(d_tw.data_ptr(), d_me.data_ptr(), d_ct.data_ptr(), M_MAX, out.data_ptr())
+        device.sync()
         assert np.array_equal(out.cpu().numpy(), assoc[t]), t
-        _assert_replicas(assoc[t], B, f"association outputs of step {t}")
+        assert_replicas(assoc[t], B, K, f"association outputs of step {t}")
     ck = _assert_checkpoint_replicas(host)
-    _assert_same_checkpoint(dev.checkpoint(), ck)
+    assert_same_checkpoint(device.checkpoint(), ck)
     states, known = host.states(), host.known
     full = 0
     for k in range(K):
@@ -224,7 +180,7 @@ def test_tile_unknown_replicas_host_and_device(gpu_pkg, unknown_inputs):
             o.prediction(*unknown_inputs["twists"][t, k])
             m = min(max(int(unknown_inputs["count"][t, k]), 0), M_MAX)
             a, dmin, sec, cr = o.data_association(unknown_inputs["meas"][t, k, :m], kn)
-            _assert_clear(dmin, sec)
+            assert_clear(dmin, sec)
             assert np.array_equal(assoc[t][k, :m], a), (k, t)
             assert np.all(assoc[t][k, m:] == -1), (k, t)
             full += int(np.sum((dmin >= 10.0) & (cr == 0)))
@@ -241,8 +197,7 @@ T_WIDE = 6
 def _wide_inputs(pkg, n):
     """K trajectories on an n-landmark grid; a class with corrections lists every slot in the first call (all n
     corrections in one step), then WIDE_CLASSES[k % 6] random slots per step."""
-    nx = max(d for d in range(1, int(np.sqrt(n)) + 1) if n % d == 0)
-    tr = pkg.tracegen.simulate_known(pkg.tracegen.grid_world(n // nx, nx, pitch=0.35), K, T_WIDE, seed=n)
+    tr = pkg.tracegen.simulate_known(grid_world(pkg, n), K, T_WIDE, seed=n)
     rng = np.random.default_rng(n)
     vis = np.zeros((T_WIDE, K, n), np.uint8)
     for k in range(K):
@@ -268,12 +223,11 @@ def _assert_wide_schedule(counts, sms):
 
 @pytest.mark.parametrize("n", [65, 256])
 def test_wide_replicas_dense_and_marker_list(gpu_pkg, n):
-    sms = _sms()
-    B = 2 * sms + 5
+    B = 2 * sms() + 5
     ref = _wide_inputs(gpu_pkg, n)
-    tw, xy, vis = (_replicate(ref[k], B) for k in ("twists", "xy", "vis"))
+    tw, xy, vis = (replicate(ref[k], B, K) for k in ("twists", "xy", "vis"))
     counts = vis.sum(axis=2)
-    _assert_wide_schedule(counts, sms)
+    _assert_wide_schedule(counts, sms())
     dense, sparse = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
     assert dense.engine == gpu_pkg.ENGINE_STREAM
     for t in range(T_WIDE):
@@ -283,7 +237,7 @@ def test_wide_replicas_dense_and_marker_list(gpu_pkg, n):
     assert dense.update_count == int(counts.sum())
     assert dense.sweep_count == int(np.ceil(counts / P).sum())
     ck = _assert_checkpoint_replicas(dense)
-    _assert_same_checkpoint(sparse.checkpoint(), ck)
+    assert_same_checkpoint(sparse.checkpoint(), ck)
     assert sparse.sweep_count == dense.sweep_count
     states = dense.states()
     for k in range(K):
@@ -330,7 +284,7 @@ def _assert_back_to_back(bt, steps, pose_bufs, want_ck, want_poses):
         step()
         bt.poses_async(buf)
     bt.sync()
-    _assert_same_checkpoint(bt.checkpoint(), want_ck)
+    assert_same_checkpoint(bt.checkpoint(), want_ck)
     for t, (got, want) in enumerate(zip(pose_bufs, want_poses)):
         assert np.array_equal(got.array.view(np.uint64), want.view(np.uint64)), t
 
@@ -339,11 +293,11 @@ def test_tile_known_back_to_back_host_steps(gpu_pkg, known_inputs):
     """Host-fed steps with one synchronisation at the end: every input in its own pinned buffer so that the copies are
     truly asynchronous, dense and marker-list steps alternating through the same two input slots, and the poses read
     back asynchronously after every step.  Reference: a batch fed from device memory, synchronised after each step."""
-    B = 64 * _sms() + 37
-    tw, xy, vis = (_replicate(known_inputs[k], B) for k in ("twists", "xy", "vis"))
+    B = 64 * sms() + 37
+    tw, xy, vis = (replicate(known_inputs[k], B, K) for k in ("twists", "xy", "vis"))
     want_ck, want_poses = _device_fed_reference(
         gpu_pkg, B, lambda bt, *d: bt.step_known_dev(*d),
-        [(_dev(tw[t]), _dev(xy[t]), _dev(vis[t])) for t in range(T_KNOWN)])
+        [(dev(tw[t]), dev(xy[t]), dev(vis[t])) for t in range(T_KNOWN)])
     inputs = [[_pinned(gpu_pkg, a) for a in ((tw[t], xy[t], vis[t]) if t % 2 == 0 else
                                              (tw[t], *gpu_pkg.marker_list(xy[t], vis[t])))] for t in range(T_KNOWN)]
     pose_bufs = [gpu_pkg.PinnedBuffer((B, 3), np.float64) for _ in range(T_KNOWN)]
@@ -356,11 +310,11 @@ def test_tile_known_back_to_back_host_steps(gpu_pkg, known_inputs):
 def test_tile_unknown_back_to_back_host_steps(gpu_pkg, unknown_inputs):
     """As above for step_unknown without association outputs (which would synchronise).  The first step enlarges the
     reading slots to m_max and synchronises while nothing else is in flight."""
-    B = 64 * _sms() + 37
-    tw, meas, cnt = (_replicate(unknown_inputs[k], B) for k in ("twists", "meas", "count"))
+    B = 64 * sms() + 37
+    tw, meas, cnt = (replicate(unknown_inputs[k], B, K) for k in ("twists", "meas", "count"))
     want_ck, want_poses = _device_fed_reference(
         gpu_pkg, B, lambda bt, *d: bt.step_unknown_dev(*d, M_MAX),
-        [(_dev(tw[t]), _dev(meas[t]), _dev(cnt[t])) for t in range(T_UNKNOWN)])
+        [(dev(tw[t]), dev(meas[t]), dev(cnt[t])) for t in range(T_UNKNOWN)])
     inputs = [[_pinned(gpu_pkg, a) for a in (tw[t], meas[t], cnt[t])] for t in range(T_UNKNOWN)]
     pose_bufs = [gpu_pkg.PinnedBuffer((B, 3), np.float64) for _ in range(T_UNKNOWN)]
     bt = gpu_pkg.EKFBatch(B, NT)

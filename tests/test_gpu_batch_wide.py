@@ -8,6 +8,7 @@ import ctypes
 import numpy as np
 import pytest
 
+from _batch import grid_world, run_known, step_known
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
@@ -16,20 +17,10 @@ TOL = 1e-9
 P = 14  # factor pairs per pass over a filter's covariance
 
 
-def _world(pkg, n):
-    nx = max(d for d in range(1, int(np.sqrt(n)) + 1) if n % d == 0)  # n landmarks on an nx x (n / nx) grid
-    return pkg.tracegen.grid_world(n // nx, nx, pitch=0.35)
-
-
 def _trace(pkg, n, B, T, seed):
-    tr = pkg.tracegen.simulate_known(_world(pkg, n), B, T, seed=seed)
+    tr = pkg.tracegen.simulate_known(grid_world(pkg, n), B, T, seed=seed)
     tr["twists"][T // 2, :, 0] = 1e-8  # the straight-line branch of the motion model
     return tr
-
-
-def _step(bt, tr, t):
-    bt.step_known(np.ascontiguousarray(tr["twists"][t]), np.ascontiguousarray(tr["xy"][t]),
-                  np.ascontiguousarray(tr["vis"][t]))
 
 
 def _streamed(pkg, n, tr, b, steps):
@@ -47,9 +38,7 @@ def test_wide_batch_is_bit_identical_to_streamed_filters(gpu_pkg, n):
     tr = _trace(gpu_pkg, n, B, T, seed=100 + n)
     bt = gpu_pkg.EKFBatch(B, n)
     assert bt.engine == gpu_pkg.ENGINE_STREAM
-    for t in range(T):
-        _step(bt, tr, t)
-    bt.sync()
+    run_known(gpu_pkg, bt, tr)
     states = bt.states()
     assert bt.update_count == int(tr["vis"].sum())
     rng = np.random.default_rng(n)
@@ -74,9 +63,7 @@ def test_wide_batch_more_corrections_than_one_group(gpu_pkg):
     tr["vis"][0] = 1
     tr["vis"][3, : B // 2] = 1
     bt = gpu_pkg.EKFBatch(B, n)
-    for t in range(T):
-        _step(bt, tr, t)
-    bt.sync()
+    run_known(gpu_pkg, bt, tr)
     c = tr["vis"].sum(axis=2)
     assert bt.update_count == int(c.sum())
     assert bt.sweep_count == int(np.ceil(c / P).sum())
@@ -123,14 +110,14 @@ def test_wide_batch_checkpoint_resume_is_bit_identical(gpu_pkg, tmp_path):
     tr = _trace(gpu_pkg, n, B, T, seed=5)
     a, b = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
     for t in range(T // 2):
-        _step(a, tr, t)
+        step_known(gpu_pkg, a, tr, t)
     path = str(tmp_path / "wide.npz")
     a.save_checkpoint(path)
     b.load_checkpoint(path)
     assert b.update_count == a.update_count
     for t in range(T // 2, T):
-        _step(a, tr, t)
-        _step(b, tr, t)
+        step_known(gpu_pkg, a, tr, t)
+        step_known(gpu_pkg, b, tr, t)
     a.sync(), b.sync()
     assert np.array_equal(a.states(), b.states()) and a.update_count == b.update_count
     for f in (0, B - 1):
@@ -153,7 +140,7 @@ def test_wide_batch_engine_boundaries(gpu_pkg):
     n, B = 100, 8
     tr = _trace(gpu_pkg, n, B, 2, seed=9)
     bt = gpu_pkg.EKFBatch(B, n)
-    _step(bt, tr, 0)
+    step_known(gpu_pkg, bt, tr, 0)
     before = bt.states()
     with pytest.raises(gpu_pkg.EkfError) as e:
         bt.step_unknown(np.ones((B, 2)), np.ones((B, 4, 2)), np.full(B, 4, np.int32), 4)
@@ -175,7 +162,7 @@ def test_wide_batch_getters(gpu_pkg):
     tr = _trace(gpu_pkg, n, B, T, seed=13)
     bt = gpu_pkg.EKFBatch(B, n)
     for t in range(T):
-        _step(bt, tr, t)
+        step_known(gpu_pkg, bt, tr, t)
     states = bt.states()
     assert np.array_equal(bt.poses(), states[:, :3])
     err = bt.pose_error(tr["truth"][-1])

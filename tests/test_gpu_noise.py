@@ -6,6 +6,7 @@ explicitly, and follow tests/_noise_ref.py (the CPU oracle's arithmetic with Q a
 import numpy as np
 import pytest
 
+from _batch import assert_same_checkpoint, known_trace, run_known, run_unknown, sms, step_known, unknown_trace
 from _noise_ref import DEFAULT_NOISE, NoiseOracle
 from _oracle import sigma_err, state_err
 
@@ -18,72 +19,6 @@ NIS_RTOL = 1e-8
 # error of what is left grows with it; these rows keep r >= 0.002, where the 1e-9 tolerance of the default holds.
 GRID = np.array([[1e-4, 1e-4, 1e-4, 0.01, 0.01], [4e-4, 2e-4, 3e-4, 0.003, 0.002], [2e-5, 1e-3, 5e-4, 0.03, 0.004],
                  [0.0, 0.0, 0.0, 0.004, 0.002], [1e-3, 1e-5, 2e-4, 0.008, 0.05]])
-
-
-def _sms():
-    import torch
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-def _dev(a):
-    import torch
-    return torch.as_tensor(np.ascontiguousarray(a)).cuda()
-
-
-def _c(a):
-    return np.ascontiguousarray(a)
-
-
-def _world(pkg, n):
-    nx = max(d for d in range(1, int(np.sqrt(n)) + 1) if n % d == 0)
-    return pkg.tracegen.grid_world(n // nx, nx, pitch=0.35)
-
-
-def _known(pkg, n, B, T, seed, p_vis=0.5):
-    tr = pkg.tracegen.simulate_known(_world(pkg, n), B, T, seed=seed)
-    rng = np.random.default_rng(seed)
-    vis = (tr["vis"] != 0) & (rng.random(tr["vis"].shape) < p_vis)
-    vis[0] = True
-    vis = vis.astype(np.uint8)
-    return {"twists": tr["twists"], "xy": np.ascontiguousarray(tr["xy"] * vis.repeat(2, axis=2)), "vis": vis}
-
-
-def _unknown(pkg, n, B, T, seed):
-    return pkg.tracegen.simulate_unknown(pkg.tracegen.dense_world(n), B, T, seed=seed, m_max=M_MAX)
-
-
-def _step_known(pkg, bt, tr, t, form):
-    tw, xy, vis = _c(tr["twists"][t]), _c(tr["xy"][t]), _c(tr["vis"][t])
-    if form == "dense":
-        bt.step_known(tw, xy, vis)
-    elif form == "markers":
-        bt.step_known_sparse(tw, *pkg.marker_list(xy, vis))
-    else:
-        d = (_dev(tw), _dev(xy), _dev(vis))
-        bt.step_known_dev(*(x.data_ptr() for x in d))
-        bt.sync()
-
-
-def _run_known(pkg, bt, tr, form="dense"):
-    for t in range(tr["twists"].shape[0]):
-        _step_known(pkg, bt, tr, t, form)
-    bt.sync()
-
-
-def _run_unknown(bt, tr):
-    out = [bt.step_unknown(_c(tr["twists"][t]), _c(tr["meas"][t]), _c(tr["count"][t]), M_MAX, want_assoc=True)
-           for t in range(tr["twists"].shape[0])]
-    bt.sync()
-    return np.stack(out)
-
-
-def _same_checkpoint(a, b):
-    for key in ("sigma_packed", "state", "init_flag", "known"):
-        x, y = a[key], b[key]
-        if x.dtype == np.float64:
-            x, y = x.view(np.uint64), y.view(np.uint64)
-        assert np.array_equal(x, y), key
-    assert a["updates"] == b["updates"]
 
 
 def _rows(B):
@@ -110,22 +45,25 @@ CASES = [("tile-dense", 20, "dense"), ("tile-markers", 20, "markers"), ("tile-de
 @pytest.mark.parametrize("name,n,form", CASES, ids=[c[0] for c in CASES])
 def test_reference_values_bit_identical(gpu_pkg, name, n, form):
     B, T = (48, 8) if n <= 64 else (6, 5)
-    tr = _unknown(gpu_pkg, n, B, T, seed=n + 9) if form == "unknown" else _known(gpu_pkg, n, B, T, seed=n + 9)
+    if form == "unknown":
+        tr = unknown_trace(gpu_pkg, n, B, T, seed=n + 9, m_max=M_MAX)
+    else:
+        tr = known_trace(gpu_pkg, n, B, T, seed=n + 9)
     plain, explicit = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
     explicit.set_noise([1e-4] * 3, [0.01] * 2)
     assert np.array_equal(explicit.noise(), np.tile(DEFAULT_NOISE, (B, 1)))
     if form == "unknown":
-        assert np.array_equal(_run_unknown(plain, tr), _run_unknown(explicit, tr))
+        assert np.array_equal(run_unknown(plain, tr, M_MAX), run_unknown(explicit, tr, M_MAX))
     else:
-        _run_known(gpu_pkg, plain, tr, form)
-        _run_known(gpu_pkg, explicit, tr, form)
-    _same_checkpoint(plain.checkpoint(), explicit.checkpoint())
+        run_known(gpu_pkg, plain, tr, form)
+        run_known(gpu_pkg, explicit, tr, form)
+    assert_same_checkpoint(plain.checkpoint(), explicit.checkpoint())
     assert plain.launch_count == explicit.launch_count
 
 
 def _single_trace(pkg, n, T, seed):
-    tk = _known(pkg, n, 1, T, seed)
-    tu = _unknown(pkg, n, 1, T, seed + 1)
+    tk = known_trace(pkg, n, 1, T, seed)
+    tu = unknown_trace(pkg, n, 1, T, seed=seed + 1, m_max=M_MAX)
     return tk, tu
 
 
@@ -157,13 +95,13 @@ def test_single_reference_values_bit_identical(gpu_pkg, engine):
 @pytest.mark.parametrize("n", [20, 33, 100, 256])
 def test_known_matches_reference(gpu_pkg, n):
     B, T = (10, 8) if n <= 64 else (5, 5)
-    tr = _known(gpu_pkg, n, B, T, seed=300 + n)
+    tr = known_trace(gpu_pkg, n, B, T, seed=300 + n)
     rows = _rows(B)
     bt = gpu_pkg.EKFBatch(B, n)
     bt.set_noise(rows[:, :3], rows[:, 3:])
     assert np.array_equal(bt.noise(), rows)
     bt.set_nis(True)
-    _run_known(gpu_pkg, bt, tr)
+    run_known(gpu_pkg, bt, tr)
     refs = [NoiseOracle(n, rows[b]) for b in range(B)]
     for t in range(T):
         for b, o in enumerate(refs):
@@ -186,12 +124,12 @@ def _check_nis(bt, refs, what):
 @pytest.mark.parametrize("n", [20, 33])
 def test_unknown_matches_reference(gpu_pkg, n):
     B, T = 10, 10
-    tr = _unknown(gpu_pkg, n, B, T, seed=400 + n)
+    tr = unknown_trace(gpu_pkg, n, B, T, seed=400 + n, m_max=M_MAX)
     rows = _rows(B)
     bt = gpu_pkg.EKFBatch(B, n)
     bt.set_noise(rows[:, :3], rows[:, 3:])
     bt.set_nis(True)
-    assoc = _run_unknown(bt, tr)
+    assoc = run_unknown(bt, tr, M_MAX)
     refs = [NoiseOracle(n, rows[b]) for b in range(B)]
     known = [np.zeros(n, np.uint8) for _ in range(B)]
     for t in range(T):
@@ -232,11 +170,11 @@ def test_single_matches_reference(gpu_pkg, engine):
 @pytest.mark.parametrize("n", [100, 256])
 def test_wide_bit_identical_to_streamed(gpu_pkg, n):
     B, T = 3, 4
-    tr = _known(gpu_pkg, n, B, T, seed=500 + n)
+    tr = known_trace(gpu_pkg, n, B, T, seed=500 + n)
     rows = _rows(B)
     bt = gpu_pkg.EKFBatch(B, n)
     bt.set_noise(rows[:, :3], rows[:, 3:])
-    _run_known(gpu_pkg, bt, tr)
+    run_known(gpu_pkg, bt, tr)
     for b in range(B):
         f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
         f.set_carry_pending(False)
@@ -254,17 +192,20 @@ def test_noise_classes_over_replicas(gpu_pkg, n, form):
     """One trajectory for every filter, K noise classes permuted over a batch beyond one resident wave: every replica
     is bit-identical to its class's first filter, and the class representatives match the reference."""
     K = len(GRID)
-    B = (2 * _sms() + 5) if n > 64 else (64 * _sms() + 37)
+    B = (2 * sms() + 5) if n > 64 else (64 * sms() + 37)
     T = 4 if n > 64 else 8
     cls = np.random.default_rng(n).permutation(np.arange(B) % K)
-    one = _unknown(gpu_pkg, n, 1, T, seed=600 + n) if form == "unknown" else _known(gpu_pkg, n, 1, T, seed=600 + n)
+    if form == "unknown":
+        one = unknown_trace(gpu_pkg, n, 1, T, seed=600 + n, m_max=M_MAX)
+    else:
+        one = known_trace(gpu_pkg, n, 1, T, seed=600 + n)
     tr = {k: np.ascontiguousarray(np.repeat(v, B, axis=1)) for k, v in one.items() if k in ("twists", "xy", "vis", "meas", "count")}
     bt = gpu_pkg.EKFBatch(B, n)
     bt.set_noise(GRID[cls, :3], GRID[cls, 3:])
     if form == "unknown":
-        _run_unknown(bt, tr)
+        run_unknown(bt, tr, M_MAX)
     else:
-        _run_known(gpu_pkg, bt, tr)
+        run_known(gpu_pkg, bt, tr)
     st = bt.states().view(np.uint64)
     reps = [int(np.flatnonzero(cls == k)[0]) for k in range(K)]
     for k in range(K):
@@ -287,7 +228,7 @@ def test_noise_classes_over_replicas(gpu_pkg, n, form):
 @pytest.mark.parametrize("n", [20, 33, 100])
 def test_noise_changed_mid_run(gpu_pkg, n):
     B, T = 4, 6
-    tr = _known(gpu_pkg, n, B, T, seed=700 + n)
+    tr = known_trace(gpu_pkg, n, B, T, seed=700 + n)
     bt = gpu_pkg.EKFBatch(B, n)
     refs = [NoiseOracle(n) for _ in range(B)]
     for t in range(T):
@@ -299,7 +240,7 @@ def test_noise_changed_mid_run(gpu_pkg, n):
             bt.set_noise()
             for o in refs:
                 o.set_noise(DEFAULT_NOISE)
-        _step_known(gpu_pkg, bt, tr, t, "dense")
+        step_known(gpu_pkg, bt, tr, t, "dense")
         for b, o in enumerate(refs):
             o.prediction(*tr["twists"][t, b])
             o.measurement(tr["xy"][t, b], tr["vis"][t, b])
@@ -313,7 +254,7 @@ def test_single_noise_changed_with_prediction_pending(gpu_pkg, engine):
     it back when set_noise() is called), the corrections the new R."""
     n, T = 20, 5
     eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
-    tk = _known(gpu_pkg, n, 1, T, seed=801)
+    tk = known_trace(gpu_pkg, n, 1, T, seed=801)
     f, o = gpu_pkg.EKF_SLAM(n, engine=eng), NoiseOracle(n)
     for t in range(T):
         f.prediction(tuple(tk["twists"][t, 0]))
@@ -329,14 +270,14 @@ def test_single_noise_changed_with_prediction_pending(gpu_pkg, engine):
 # ---------------------------------------------------------------- 5. configuration handling
 def test_broadcast_clone_and_checkpoints(gpu_pkg):
     n, B, T = 20, 16, 5
-    tr = _known(gpu_pkg, n, B, T, seed=901)
+    tr = known_trace(gpu_pkg, n, B, T, seed=901)
     row = GRID[2]
     shared, per = gpu_pkg.EKFBatch(B, n), gpu_pkg.EKFBatch(B, n)
     shared.set_noise(row[:3], row[3:])
     per.set_noise(np.tile(row[:3], (B, 1)), np.tile(row[3:], (B, 1)))
-    _run_known(gpu_pkg, shared, tr)
-    _run_known(gpu_pkg, per, tr)
-    _same_checkpoint(shared.checkpoint(), per.checkpoint())
+    run_known(gpu_pkg, shared, tr)
+    run_known(gpu_pkg, per, tr)
+    assert_same_checkpoint(shared.checkpoint(), per.checkpoint())
     # checkpoints carry no noise: a restored batch keeps its own setting, a fresh one the reference values
     ck = shared.checkpoint()
     fresh = gpu_pkg.EKFBatch(B, n)
@@ -375,7 +316,7 @@ def test_invalid_rows_rejected(gpu_pkg, bad):
         with pytest.raises(gpu_pkg.EkfError):
             bt.set_noise(q, r)
         assert np.array_equal(bt.noise(), rows)
-    _same_checkpoint(before, bt.checkpoint())
+    assert_same_checkpoint(before, bt.checkpoint())
     for eng in (gpu_pkg.ENGINE_FUSED, gpu_pkg.ENGINE_STREAM):
         f = gpu_pkg.EKF_SLAM(n, engine=eng)
         f.set_noise(GRID[1, :3], GRID[1, 3:])

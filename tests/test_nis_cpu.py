@@ -1,12 +1,12 @@
-"""Host side of the batch NIS read-out: consistency.anis_from_stats, the report's innovations row, and the NIS
-reference of tests/_nis_ref.py (a numpy replay of the CPU oracle) against nu^T S^-1 nu formed directly from the
-oracle's sigma and state."""
+"""Host side of the batch NIS read-out: consistency.anis_from_stats, the report's innovations row, and the NIS of
+tests/_noise_ref.py (the numpy restatement of the CPU oracle) against nu^T S^-1 nu formed directly from its sigma and
+state."""
 import math
 
 import numpy as np
 import pytest
 
-from _nis_ref import NisOracle, wrap
+from _noise_ref import NoiseOracle, normalize_angle
 
 
 def test_anis_from_stats_and_bounds(pkg):
@@ -33,7 +33,8 @@ def _direct_nis(state, sigma, i, sx, sy):
     H[0, [1, 2, 3 + 2 * i, 4 + 2 * i]] = [-dx / q, -dy / q, dx / q, dy / q]
     H[1, [0, 1, 2, 3 + 2 * i, 4 + 2 * i]] = [-1.0, dy / d, -dx / d, -dy / d, dx / d]
     S = H @ sigma @ H.T + 0.01 * np.eye(2)
-    nu = np.array([math.hypot(sx, sy) - q, wrap(math.atan2(sy, sx) - wrap(math.atan2(dy, dx) - th))])
+    zphi = normalize_angle(math.atan2(dy, dx) - th)
+    nu = np.array([math.hypot(sx, sy) - q, normalize_angle(math.atan2(sy, sx) - zphi)])
     return float(nu @ np.linalg.solve(S, nu))
 
 
@@ -51,10 +52,10 @@ def one_landmark_trace(pkg):
 
 def test_reference_nis_matches_direct_formula(one_landmark_trace):
     tw, xy, vis = one_landmark_trace
-    o = NisOracle(20)
+    o = NoiseOracle(20)
     for t in range(len(tw)):
         o.prediction(*tw[t])
-        st, sig = o.o.state, o.o.sigma
+        st, sig = o.state.copy(), o.sigma.copy()
         before = len(o.values)
         o.measurement(xy[t], vis[t])
         if t == 0:
@@ -70,13 +71,13 @@ def test_reference_nis_matches_direct_formula(one_landmark_trace):
 
 
 def test_reference_scoring_rule_on_the_association_path():
-    o = NisOracle(20)
+    o = NoiseOracle(20)
     known = np.zeros(20, np.uint8)
     o.prediction(0.01, 0.05)
-    a, _, _, c = o.data_association(np.array([[1.0, 0.2]]), known)
+    a, c = o.data_association(np.array([[1.0, 0.2]]), known)
     assert a[0] == 0 and c[0] == 1 and o.acc[2] == 0  # created by this reading: corrected, not scored
     o.prediction(0.01, 0.05)
-    a, _, _, c = o.data_association(np.array([[0.95, 0.2]]), known)
+    a, c = o.data_association(np.array([[0.95, 0.2]]), known)
     assert a[0] == 0 and c[0] == 0 and o.acc[2] == 1  # the same landmark again: scored
 
 
