@@ -61,6 +61,9 @@ SIGNATURES = {
     "ekf_set_carry_pending": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "ekf_set_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_get_noise": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
+    "ekf_set_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "ekf_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]),
+    "ekf_last_nis": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "ekf_set_max_pending": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "ekf_batch_create": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_void_pp]),
     "ekf_batch_destroy": (ctypes.c_int, [ctypes.c_void_p]),

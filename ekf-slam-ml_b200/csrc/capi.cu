@@ -49,15 +49,19 @@ int launch_smem_kernel(int smem, const FusedParams& p, cudaStream_t stream, int 
 }
 
 // Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.  With p.noise, the NOISE
-// variant.
-template <bool NoiseOn>
+// variant; with p.nis, the NIS variant.
+template <bool NoiseOn, bool Nis>
 int launch_fused_nz(const FusedParams& p, cudaStream_t stream, int device) {
-    const int smem = FusedSmem(p.n, p.m_max, NoiseOn).total;
-    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20, NoiseOn>>(smem, p, stream, device)
-                     : launch_smem_kernel<ekf_fused_kernel<0, NoiseOn>>(smem, p, stream, device);
+    const int smem = FusedSmem(p.n, p.m_max, NoiseOn, Nis).total;
+    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20, NoiseOn, Nis>>(smem, p, stream, device)
+                     : launch_smem_kernel<ekf_fused_kernel<0, NoiseOn, Nis>>(smem, p, stream, device);
+}
+template <bool Nis>
+int launch_fused_nis(const FusedParams& p, cudaStream_t stream, int device) {
+    return p.noise ? launch_fused_nz<true, Nis>(p, stream, device) : launch_fused_nz<false, Nis>(p, stream, device);
 }
 int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
-    return p.noise ? launch_fused_nz<true>(p, stream, device) : launch_fused_nz<false>(p, stream, device);
+    return p.nis ? launch_fused_nis<true>(p, stream, device) : launch_fused_nis<false>(p, stream, device);
 }
 
 // Batch with n <= 64, n != 20: symmetric staircase Sigma (ekf_fused_sym.cuh).
@@ -133,6 +137,17 @@ __global__ void __launch_bounds__(kGainThreads)
                          const UpdateCmd* __restrict__ cmd, int lm_arg, double sx_arg, double sy_arg,
                          double2* __restrict__ Kp, double2* __restrict__ Wp, int p, const Noise nz) {
     large_gain_p(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p, nz);
+}
+// NIS variants of both (ekf_set_nis): nis_acc = the handle's 8 accumulators, nis_out = the call's slot of this correction
+template <bool NoiseOn>
+__global__ void __launch_bounds__(kGainThreads)
+    k_large_gain_p_nis(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
+                       double* __restrict__ state_out, const double* __restrict__ pose_src,
+                       const UpdateCmd* __restrict__ cmd, int lm_arg, double sx_arg, double sy_arg,
+                       double2* __restrict__ Kp, double2* __restrict__ Wp, int p, const Noise nz, double* nis_acc,
+                       double* nis_out, int nis_flags) {
+    large_gain_p<true>(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p,
+                       NoiseOn ? nz : ref_noise(), nis_acc, nis_out, nis_flags);
 }
 __global__ void __launch_bounds__(256)
     k_large_assoc_noise(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
@@ -262,6 +277,16 @@ struct ekf_filter {
     bool noise_on = false;
     Noise noise = ref_noise();
     double* d_noise = nullptr;
+    // ekf_set_nis: with nis_on the NIS variants run.  d_nis = {sum, sum^2, #scored, #non-finite} accumulators, then the
+    // streamed engine's sums of the open call (folded by the next call's first gain kernel, or by ekf_nis on the host);
+    // d_nis_vals = the last NIS call's values (m_cap entries).  Both allocated on first use.
+    bool nis_on = false;
+    double* d_nis = nullptr;
+    double* d_nis_vals = nullptr;
+    int nis_flags = 0;             // streamed engine: kNisScore / kNisFold of the next gain kernel of this call
+    int nis_count = 0;             // entries of the last NIS call (n after measurement(), m after data_association())
+    bool nis_masked = false;       // streamed engine: d_nis_vals holds scored entries only, nis_mask says which
+    std::vector<uint8_t> nis_mask;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
 };
 
@@ -294,6 +319,8 @@ int free_filter(ekf_filter* h) {
     cudaFree(h->d_done);
     cudaFree(h->d_known_count);
     cudaFree(h->d_noise);
+    cudaFree(h->d_nis);
+    cudaFree(h->d_nis_vals);
     for (int i = 0; i < kRing; ++i) {
         if (h->h_ring[i]) cudaFreeHost(h->h_ring[i]);
         if (h->ring_ev[i]) cudaEventDestroy(h->ring_ev[i]);
@@ -327,6 +354,13 @@ int ensure_m_cap(ekf_filter* h, int m) {
     CU(cudaMalloc(&h->d_dmin, sizeof(double) * cap));
     CU(cudaMalloc(&h->d_second, sizeof(double) * cap));
     CU(cudaMalloc(&h->d_created, cap));
+    if (h->d_nis_vals) {  // the last NIS call's values survive the resize
+        double* vals = nullptr;
+        CU(cudaMalloc(&vals, sizeof(double) * cap));
+        CU(cudaMemcpy(vals, h->d_nis_vals, sizeof(double) * h->m_cap, cudaMemcpyDeviceToDevice));
+        cudaFree(h->d_nis_vals);
+        h->d_nis_vals = vals;
+    }
     const size_t need = sizeof(double) * 2 * cap + h->n + 64;
     if (need > h->ring_bytes) {
         for (int i = 0; i < kRing; ++i) {
@@ -374,6 +408,8 @@ FusedParams fused_params(ekf_filter* h, int mode, int m_max) {
     p.sig_stride = (int)h->sig_elems;
     p.st_stride = h->st_stride;
     p.noise = h->noise_on ? h->d_noise : nullptr;
+    p.nis = h->nis_on ? h->d_nis : nullptr;
+    p.nis_out = h->nis_on ? h->d_nis_vals : nullptr;
     return p;
 }
 
@@ -389,10 +425,22 @@ int stream_flush(ekf_filter* h, int n_counted, const UpdateCmd* cmd) {
 }
 
 // One landmark correction on the stream engine: the gain kernel appends a factor pair; Sigma itself is only
-// touched when kMaxPending factors have piled up or the verb ends.
-int stream_correct(ekf_filter* h, const double* pose_src, const UpdateCmd* cmd, int lm, double sx, double sy) {
+// touched when kMaxPending factors have piled up or the verb ends.  With NIS on, the gain kernel's NIS variant scores
+// the correction into slot `nis_slot` of the call's values.
+int stream_correct(ekf_filter* h, const double* pose_src, const UpdateCmd* cmd, int lm, double sx, double sy,
+                   int nis_slot) {
     const int gb = (int)((h->ld + 255) / 256);
-    if (h->noise_on)
+    if (h->nis_on) {
+        if (h->noise_on)
+            CU(launch_pdl(k_large_gain_p_nis<true>, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
+                          h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise,
+                          h->d_nis, h->d_nis_vals + nis_slot, h->nis_flags));
+        else
+            CU(launch_pdl(k_large_gain_p_nis<false>, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
+                          h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise,
+                          h->d_nis, h->d_nis_vals + nis_slot, h->nis_flags));
+        h->nis_flags &= ~kNisFold;
+    } else if (h->noise_on)
         CU(launch_pdl(k_large_gain_p_noise, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
                       h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise));
     else
@@ -419,6 +467,7 @@ int fused_flush_predict(ekf_filter* h) {
     tw[0] = h->pred_tw[0];
     tw[1] = h->pred_tw[1];
     FusedParams p = fused_params(h, kDoPredict, 1);
+    p.nis = p.nis_out = nullptr;  // a prediction alone has nothing to score
     p.twists = tw;  // read through the device mapping of the pinned slot
     rc = launch_fused(p, h->stream, h->device);
     CU(cudaEventRecord(ev, h->stream));
@@ -435,6 +484,24 @@ int stream_settle(ekf_filter* h) {
     if (h->engine == EKF_ENGINE_FUSED) return fused_flush_predict(h);
     if (h->pending == 0) return EKF_OK;
     return stream_flush(h, h->pending, nullptr);
+}
+
+// A measurement() / data_association() call with NIS on: its `count` values replace the last call's.  The fused kernel
+// writes every entry (-1 where unscored); the streamed engine's gain kernels write the scored ones, which nis_mask marks.
+void nis_begin_call(ekf_filter* h, int count, bool masked) {
+    h->nis_count = count;
+    h->nis_masked = masked;
+    if (masked) h->nis_mask.assign((size_t)count, 0);
+}
+
+// NIS accumulators and value buffer, allocated and zeroed on first use
+int nis_alloc(ekf_filter* h) {
+    if (h->d_nis) return EKF_OK;
+    CU(cudaMalloc(&h->d_nis, 8 * sizeof(double)));
+    CU(cudaMemsetAsync(h->d_nis, 0, 8 * sizeof(double), h->stream));
+    CU(cudaMalloc(&h->d_nis_vals, sizeof(double) * h->m_cap));
+    h->nis_count = 0;
+    return EKF_OK;
 }
 
 // Buffers and initial state (Sigma0, zero state) of a new filter; on failure the caller frees the half-made handle.
@@ -581,11 +648,23 @@ int ekf_clone(ekf_filter* src, ekf_filter** out) {
         const Noise nz = src->noise;
         const double row[5] = {nz.q0, nz.q1, nz.q2, nz.r0, nz.r1};
         rc = ekf_set_noise(h, row);
-        if (rc) {
-            free_filter(h);
-            *out = nullptr;
-            return rc;
+    }
+    if (!rc && src->d_nis) {  // the NIS switch and the accumulators, open call included
+        rc = nis_alloc(h);
+        if (!rc) {
+            e = cudaMemcpyAsync(h->d_nis, src->d_nis, 8 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+            if (e != cudaSuccess) {
+                cudaGetLastError();
+                rc = fail((int)e, "ekf_clone: %s", cudaGetErrorString(e));
+            }
         }
+        h->nis_on = src->nis_on;
+    }
+    if (rc) {
+        free_filter(h);
+        *out = nullptr;
+        return rc;
     }
     return EKF_OK;
 }
@@ -647,10 +726,12 @@ int ekf_measurement(ekf_filter* h, const double* xy, const uint8_t* visible) {
         CU(cudaEventRecord(ev, h->stream));
         h->launches += 1;
         h->pose_host_ok = rc == EKF_OK;
+        if (h->nis_on) nis_begin_call(h, n, false);
         return rc;
     }
     // stream engine: the host sequences one (gain, sweep) pair per visible landmark; readings travel as kernel
     // arguments, the entry-time pose is snapshotted on the device (ekf_slam.cpp:109-111).
+    bool score = true;
     if (!h->init_flag_host) {
         unsigned char* slot;
         cudaEvent_t ev;
@@ -662,11 +743,17 @@ int ekf_measurement(ekf_filter* h, const double* xy, const uint8_t* visible) {
         k_large_init_landmarks<<<(n + 255) / 256, 256, 0, h->stream>>>(h->d_state, h->d_in, n, h->d_init_flag);
         h->launches += 1;
         h->init_flag_host = 1;
+        score = false;  // the first call's readings initialised every landmark: nu ~ 0
+    }
+    if (h->nis_on) {  // the scored slots: the visible ones, unless this call initialised the map
+        nis_begin_call(h, n, true);
+        h->nis_flags = kNisFold | (score ? kNisScore : 0);
+        for (int i = 0; i < n; ++i) h->nis_mask[i] = score && visible[i];
     }
     CU(cudaMemcpyAsync(h->d_pose0, h->d_state, 3 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
     for (int i = 0; i < n; ++i) {
         if (!visible[i]) continue;
-        int rc = stream_correct(h, h->d_pose0, nullptr, i, xy[2 * i], xy[2 * i + 1]);
+        int rc = stream_correct(h, h->d_pose0, nullptr, i, xy[2 * i], xy[2 * i + 1], i);
         if (rc) return rc;
     }
     // with carry_pending the factors wait for more corrections (up to max_pending) before Sigma is swept
@@ -682,7 +769,10 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
         if (rc_) return rc_;
     }
     const int n = h->n;
-    if (m == 0) return EKF_OK;
+    if (m == 0) {
+        if (h->nis_on) nis_begin_call(h, 0, false);
+        return EKF_OK;
+    }
     int rc = ensure_m_cap(h, m);
     if (rc) return rc;
     unsigned char* slot;
@@ -724,9 +814,14 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
         h->launches += 1;
         h->pose_host_ok = rc == EKF_OK;
         if (rc) return rc;
+        if (h->nis_on) nis_begin_call(h, m, false);
         CU(cudaStreamSynchronize(h->stream));
         memcpy(o_known, slot + sizeof(double) * 2 * m, n);
     } else {
+        if (h->nis_on) {
+            nis_begin_call(h, m, true);
+            h->nis_flags = kNisFold;
+        }
         CU(cudaMemcpyAsync(h->d_in, slot, sizeof(double) * 2 * m, cudaMemcpyHostToDevice, h->stream));
         CU(cudaMemcpyAsync(h->d_flags, slot + sizeof(double) * 2 * m, n, cudaMemcpyHostToDevice, h->stream));
         CU(cudaMemcpyAsync(h->d_known_count, slot_i + 1, sizeof(int), cudaMemcpyHostToDevice, h->stream));
@@ -743,7 +838,7 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
                                                                        h->d_created);
             h->launches += 1;
             // the next measurement's distances need the corrected Sigma: one factor, applied at once
-            rc = stream_correct(h, h->d_state, h->d_cmd, 0, 0.0, 0.0);
+            rc = stream_correct(h, h->d_state, h->d_cmd, 0, 0.0, 0.0, j);
             if (rc) return rc;
             rc = stream_flush(h, 1, h->d_cmd);
             if (rc) return rc;
@@ -754,6 +849,8 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
         CU(cudaMemcpyAsync(o_created, h->d_created, m, cudaMemcpyDeviceToHost, h->stream));
         CU(cudaMemcpyAsync(o_kc, h->d_known_count, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
         CU(cudaStreamSynchronize(h->stream));
+        if (h->nis_on)  // scored: every applied correction but that of a landmark the same reading created
+            for (int j = 0; j < m; ++j) h->nis_mask[j] = o_assoc[j] >= 0 && !o_created[j];
     }
     if (assoc_out) memcpy(assoc_out, o_assoc, sizeof(int32_t) * m);
     if (dmin_out) memcpy(dmin_out, o_dmin, sizeof(double) * m);
@@ -825,6 +922,43 @@ int ekf_set_noise(ekf_filter* h, const double* noise5) {
         CU(cudaMemcpyAsync(h->d_noise, &h->noise, sizeof(Noise), cudaMemcpyHostToDevice, h->stream));
     }
     h->noise_on = true;
+    return EKF_OK;
+}
+
+int ekf_set_nis(ekf_filter* h, int on) {
+    if (!h) return fail(EKF_ERR_INVALID, "null handle");
+    if (on) {
+        DeviceGuard g(h->device);
+        int rc = nis_alloc(h);
+        if (rc) return rc;
+    }
+    h->nis_on = on != 0;
+    return EKF_OK;
+}
+
+int ekf_nis(ekf_filter* h, double* out4, int reset) {
+    if (!h || !out4) return fail(EKF_ERR_INVALID, "null argument");
+    if (!h->d_nis) return fail(EKF_ERR_STATE, "NIS was never enabled on this filter (ekf_set_nis)");
+    DeviceGuard g(h->device);
+    double acc[8];
+    CU(cudaMemcpyAsync(acc, h->d_nis, sizeof(acc), cudaMemcpyDeviceToHost, h->stream));
+    if (reset) CU(cudaMemsetAsync(h->d_nis, 0, sizeof(acc), h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    for (int k = 0; k < 4; ++k) out4[k] = acc[k] + acc[4 + k];  // the open call's sums, as its fold would add them
+    return EKF_OK;
+}
+
+int ekf_last_nis(ekf_filter* h, double* out, int* count_out) {
+    if (!h || !count_out) return fail(EKF_ERR_INVALID, "null argument");
+    if (!h->d_nis) return fail(EKF_ERR_STATE, "NIS was never enabled on this filter (ekf_set_nis)");
+    *count_out = h->nis_count;
+    if (!out || h->nis_count == 0) return EKF_OK;
+    DeviceGuard g(h->device);
+    CU(cudaMemcpyAsync(out, h->d_nis_vals, sizeof(double) * h->nis_count, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    if (h->nis_masked)
+        for (int j = 0; j < h->nis_count; ++j)
+            if (!h->nis_mask[j]) out[j] = -1.0;
     return EKF_OK;
 }
 

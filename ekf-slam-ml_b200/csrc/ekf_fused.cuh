@@ -39,14 +39,16 @@ struct FusedParams {
     long long sparse_total;  // marker-list mode: number of listed markers (offsets are checked against it)
     double* nis;             // [B][4] NIS accumulators of the batch kernels' NIS variants (nis() / nis_add())
     const double* noise;     // [B][5] per-filter {q_theta, q_x, q_y, r_range, r_bearing} of the NOISE variants
+    double* nis_out;         // single filter's NIS variant: the call's NIS per slot (measurement) or per reading
+                             // (association), -1 where no correction was scored
 };
 
 __host__ __device__ inline int fused_round16(int v) { return (v + 15) & ~15; }
 
 // shared memory carve-up (bytes), identical on host and device
 struct FusedSmem {
-    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_noise, total;
-    __host__ __device__ FusedSmem(int n, int m_max, bool noise = false) {
+    int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_noise, off_nis, total;
+    __host__ __device__ FusedSmem(int n, int m_max, bool noise = false, bool nis = false) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;
@@ -69,6 +71,8 @@ struct FusedSmem {
         o += 16;
         off_noise = o;  // NOISE only: the filter's row, read where it is used instead of held in registers
         o += noise ? (int)sizeof(Noise) : 0;
+        off_nis = o;  // NIS only: the call's sums {sum, sum^2, #scored, #non-finite}, kept by lane 0
+        o += nis ? 4 * 8 : 0;
         total = o;
     }
 };
@@ -82,9 +86,10 @@ __device__ __forceinline__ double apply_pair(double v, double2 k, double2 w) {
 // If PEND, Sigma in shared memory is still missing the factor pair (Kpend, Wpend) of the previous correction; the
 // five rows and five columns that this correction needs are rebuilt on the fly with exactly the FMAs the rank-2
 // update would have applied (so the result is bit-identical to updating Sigma after every correction).
-// All lanes enter with identical (i, h, zr, zphi); h = H_j / z_hat of landmark i from the current state.
+// All lanes enter with identical (i, h, zr, zphi); h = H_j / z_hat of landmark i from the current state.  Returns the
+// correction's NIS from the S^-1 and nu formed here (warp-uniform; only the NIS variants use it).
 template <bool PEND>
-__device__ __forceinline__ void warp_gain(const double* __restrict__ sig, double* __restrict__ st,
+__device__ __forceinline__ double warp_gain(const double* __restrict__ sig, double* __restrict__ st,
                                           const double2* __restrict__ Kpend, const double2* __restrict__ Wpend,
                                           double2* __restrict__ Kout, double2* __restrict__ Wout, const int N,
                                           const int lane, const int i, const Hj h, const double zr, const double zphi,
@@ -138,6 +143,7 @@ __device__ __forceinline__ void warp_gain(const double* __restrict__ sig, double
         st[r] = ns;
     }
     __syncwarp();
+    return nis(si, nu0, nu1);
 }
 
 // Sigma <- Sigma - Ka Wa [- Kb Wb]   ((I - K Hj) Sigma, ekf_slam.cpp:191-192, for one or two corrections in ONE pass
@@ -269,8 +275,8 @@ __device__ __forceinline__ int fused_assoc_inputs(const FusedParams& p, const lo
 // data_association(): Mahalanobis nearest neighbour + landmark initialisation (ekf_slam.cpp:278-402) for the m
 // readings in zbuf.  The Sigma layout enters through two calls only:
 //   dist(i, zr, zphi, theta, x, y)  distance of known landmark i (each lane scans its own landmarks);
-//   correct(i, h, zr, zphi, created) gain, state update and rank-2 update of landmark i (whole warp; h from the live
-//                                    pose); `created` is set when this very reading initialised the landmark.
+//   correct(i, h, zr, zphi, created, j) gain, state update and rank-2 update of landmark i for reading j (whole warp;
+//                                    h from the live pose); `created` is set when this very reading initialised it.
 template <class Dist, class Correct>
 __device__ __forceinline__ void fused_association(const FusedParams& p, const long long b, const int n, const int m,
                                                   const int lane, double* st, const double* zbuf,
@@ -350,7 +356,7 @@ __device__ __forceinline__ void fused_association(const FusedParams& p, const lo
         if (min_d < kGateUpdate) {  // :330
             const double th_l = st[0], x_l = st[1], y_l = st[2];  // live pose (:331-333)
             const Hj h = make_hj(st[3 + 2 * min_idx], st[4 + 2 * min_idx], th_l, x_l, y_l);
-            correct(min_idx, h, zr, zphi, created);  // the next distances need the new Sigma
+            correct(min_idx, h, zr, zphi, created, j);  // the next distances need the new Sigma
             ++n_corr;
             assoc = min_idx;
         }
@@ -372,12 +378,15 @@ __device__ __forceinline__ void fused_association(const FusedParams& p, const lo
 }
 
 // NOISE: Q and R from p.noise (one row: this kernel runs the single fused filter), kept in shared memory by lane 0.
-template <int NL, bool NOISE>
+// NIS: the call's scored corrections (none in a filter's first measurement(), none for a landmark its own reading
+// created) write their NIS to p.nis_out and are summed in correction order by lane 0, in shared memory; the sums are
+// added to p.nis at write-back.
+template <int NL, bool NOISE, bool NIS>
 __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int n = NL ? NL : p.n;
     const int N = 3 + 2 * n;
-    const FusedSmem L(n, p.m_max, NOISE);
+    const FusedSmem L(n, p.m_max, NOISE, NIS);
     double* sig = reinterpret_cast<double*>(smem_raw + L.off_sig);
     double* st = reinterpret_cast<double*>(smem_raw + L.off_st);
     double2* K2 = reinterpret_cast<double2*>(smem_raw + L.off_k2);
@@ -387,6 +396,7 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     double* zbuf = reinterpret_cast<double*>(smem_raw + L.off_z);
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + L.off_bar);
     Noise* nzs = reinterpret_cast<Noise*>(smem_raw + L.off_noise);
+    double* nacc = reinterpret_cast<double*>(smem_raw + L.off_nis);
     const auto nz = [&]() { return NOISE ? *nzs : ref_noise(); };
 
     const int lane = threadIdx.x;
@@ -412,6 +422,11 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     }
     int init_flag = p.init_flag[b];
     if (NOISE && lane == 0) *nzs = load_noise(p.noise + 5 * b);
+    if (NIS) {  // every entry of the call starts unscored
+        if (lane == 0) nacc[0] = nacc[1] = nacc[2] = nacc[3] = 0.0;
+        const int count = (p.mode & kDoMeasurement) ? n : (p.mode & kDoAssociation) ? p.m_max : 0;
+        for (int j = lane; j < count; j += 32) p.nis_out[b * count + j] = -1.0;
+    }
     int m = 0;
     if (p.mode & kDoMeasurement) {
         // z = (range, bearing) of every slot's reading, lane-parallel (ekf_slam.cpp:140-146)
@@ -436,6 +451,7 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     // ---- measurement(): known association (ekf_slam.cpp:108-197)
     if (p.mode & kDoMeasurement) {
         const double theta = st[0], x = st[1], y = st[2];  // read once; stale for later i (:109-111)
+        const bool score = init_flag != 0;  // the first call's readings initialised every landmark: nu ~ 0
         if (!init_flag) {
             for (int i = lane; i < n; i += 32) {
                 double mx, my;
@@ -464,13 +480,23 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
             while (rem) {
                 const int ia = base + __ffs(rem) - 1;
                 rem &= rem - 1;
-                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, ia, h, zbuf[2 * ia], zbuf[2 * ia + 1], nz());
+                const double va =
+                    warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, ia, h, zbuf[2 * ia], zbuf[2 * ia + 1], nz());
+                if (NIS && score && lane == 0) {
+                    nis_add(nacc, va);
+                    p.nis_out[b * n + ia] = va;
+                }
                 ++n_corr;
                 if (rem) {
                     const int ib = base + __ffs(rem) - 1;
                     rem &= rem - 1;
                     h = make_hj(st[3 + 2 * ib], st[4 + 2 * ib], theta, x, y);
-                    warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, ib, h, zbuf[2 * ib], zbuf[2 * ib + 1], nz());
+                    const double vb =
+                        warp_gain<true>(sig, st, K2, W2, K2b, W2b, N, lane, ib, h, zbuf[2 * ib], zbuf[2 * ib + 1], nz());
+                    if (NIS && score && lane == 0) {
+                        nis_add(nacc, vb);
+                        p.nis_out[b * n + ib] = vb;
+                    }
                     ++n_corr;
                     if (rem) {
                         const int in = base + __ffs(rem) - 1;
@@ -491,8 +517,12 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
             [&](int i, double zr, double zphi, double theta, double x, double y) {
                 return maha_distance(sig, N, i, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y, nz());
             },
-            [&](int i, const Hj& h, double zr, double zphi, int) {
-                warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, i, h, zr, zphi, nz());
+            [&](int i, const Hj& h, double zr, double zphi, int created, int j) {
+                const double v = warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, i, h, zr, zphi, nz());
+                if (NIS && !created && lane == 0) {  // a new landmark starts at its reading
+                    nis_add(nacc, v);
+                    p.nis_out[b * p.m_max + j] = v;
+                }
                 warp_rank2<NL, 1>(sig, K2, W2, nullptr, nullptr, N, lane);
             });
     }
@@ -508,6 +538,10 @@ __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
         bulk_commit();
         p.init_flag[b] = init_flag;
         if (p.n_updates && n_corr) atomicAdd(p.n_updates, n_corr);
+        if (NIS) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) p.nis[4 * b + k] += nacc[k];
+        }
         bulk_wait_all();
     }
 }

@@ -401,7 +401,7 @@ __global__ void __launch_bounds__(32) ekf_fused_sym_kernel(const FusedParams p) 
                 return sym_maha_distance(sig, N, i, rob, st[3 + 2 * i], st[4 + 2 * i], zr, zphi, theta, x, y,
                                          NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);
             },
-            [&](int i, const Hj& h, double zr, double zphi, int created) {
+            [&](int i, const Hj& h, double zr, double zphi, int created, int) {
                 const double nu0 = __dsub_rn(zr, h.zr), nu1 = normalize_angle(__dsub_rn(zphi, h.zphi));  // :182-183
                 const Sym2 si = sym_warp_gain<false>(sig, st, nullptr, nullptr, K2, W2, N, lane, cmv, i, h, nu0, nu1,
                                                      NOISE ? nzs->r0 : kR, NOISE ? nzs->r1 : kR);

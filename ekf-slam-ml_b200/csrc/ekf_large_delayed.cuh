@@ -142,12 +142,41 @@ __device__ __forceinline__ void named_bar_sync(int id, int count) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory");
 }
 
-// The body is shared by k_large_gain_p (the reference's R) and the single filter's noise variant (capi.cu).
+// NIS variants (the single filter's ekf_set_nis): nis_flags bits of the gain kernel.
+enum : int {
+    kNisScore = 1,  // measurement(): the correction is scored (the filter's landmarks were initialised before the call)
+    kNisFold = 2,   // first gain of a call: fold the previous call's sums into the accumulators before scoring
+};
+// acc = {sum, sum^2, #scored, #non-finite} accumulators, then the sums of the open call: the first gain of a call adds
+// the previous call's sums to the accumulators and zeroes them, each scored correction adds its NIS to them, so every
+// call is summed on its own, in correction order, and added as a whole (the rule of the batch kernels).
+__device__ __forceinline__ void gain_nis(const GainSharedP& g, const UpdateCmd* __restrict__ cmd, bool active,
+                                         double* __restrict__ acc, double* __restrict__ nis_out, int nis_flags) {
+    if (nis_flags & kNisFold) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            acc[k] += acc[4 + k];
+            acc[4 + k] = 0.0;
+        }
+    }
+    // data_association(): every applied correction except that of a landmark the same reading created
+    const bool score = cmd ? (cmd->do_update && !cmd->created) : (nis_flags & kNisScore) != 0;
+    if (active && score) {
+        const double v = nis(g.si, g.nu0, g.nu1);
+        *nis_out = v;
+        nis_add(acc + 4, v);
+    }
+}
+
+// The body is shared by k_large_gain_p (the reference's R) and the single filter's noise and NIS variants (capi.cu).
+// NIS: lane 0 of the scalar warp in CTA 0 scores the correction (gain_nis) and writes its value to *nis_out.
+template <bool NIS = false>
 __device__ __forceinline__ void large_gain_p(const double* __restrict__ sig, long long ld, int N,
                                              const double* __restrict__ state_in, double* __restrict__ state_out,
                                              const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
                                              int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp,
-                                             double2* __restrict__ Wp, int p, const Noise& nz) {
+                                             double2* __restrict__ Wp, int p, const Noise& nz, double* nis_acc = nullptr,
+                                             double* nis_out = nullptr, int nis_flags = 0) {
     __shared__ GainSharedP g;
     pdl_prologue();
     int lm = lm_arg;
@@ -176,6 +205,7 @@ __device__ __forceinline__ void large_gain_p(const double* __restrict__ sig, lon
             const Hj h = make_hj(state_in[i3], state_in[i3 + 1], pose_src[0], pose_src[1], pose_src[2]);
             gain_block(lane, e, sig[e.ida * ld + e.idl], Wp, ld, p, h, sx, sy, nz, g);
         }
+        if (NIS && lane == 0 && blockIdx.x == 0) gain_nis(g, cmd, active, nis_acc, nis_out, nis_flags);
         __syncwarp();
         named_bar_sync(2, kGainThreads);
         return;

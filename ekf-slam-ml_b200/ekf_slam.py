@@ -303,6 +303,35 @@ class EKF_SLAM:
         check(self._L.ekf_get_noise(self._h, out.ctypes.data))
         return out
 
+    def set_nis(self, on=True):
+        """ekf_set_nis: with on, the following measurement() / data_association() calls also score the normalised
+        innovation squared of their corrections (NIS = nu^T S^-1 nu; the accumulators are allocated and zeroed on first
+        use), with the scoring rule of EKFBatch.set_nis; with off, the plain kernels run again and the accumulators are
+        kept.  clone() copies both."""
+        check(self._L.ekf_set_nis(self._h, 1 if on else 0))
+
+    def nis(self, reset=False):
+        """NIS read-out, the consistency test that needs no truth: consistency.anis_from_stats() of
+        {sum NIS, sum NIS^2, #scored, #non-finite} (also returned as "stats").  reset zeroes the accumulators after the
+        read.  Raises before set_nis() was ever called."""
+        from .consistency import anis_from_stats
+        out = np.zeros(4)
+        check(self._L.ekf_nis(self._h, out.ctypes.data, 1 if reset else 0))
+        res = anis_from_stats(out)
+        res["stats"] = out
+        return res
+
+    def last_nis(self):
+        """NIS of each correction of the last measurement() / data_association() call that ran with NIS on: n values in
+        slot order after measurement(), m values in measurement order after data_association(); -1 where no
+        correction was scored.  Raises before set_nis() was ever called."""
+        count = ctypes.c_int()
+        check(self._L.ekf_last_nis(self._h, None, ctypes.byref(count)))
+        out = np.empty(count.value)
+        if count.value:
+            check(self._L.ekf_last_nis(self._h, out.ctypes.data, ctypes.byref(count)))
+        return out
+
     def timer_start(self):
         check(self._L.ekf_timer_start(self._h))
 

@@ -124,6 +124,26 @@ int ekf_set_carry_pending(ekf_filter* h, int carry);
  * reused on return.  ekf_clone copies it; it is configuration, not state (ekf_set_state / ekf_set_sigma keep it). */
 int ekf_set_noise(ekf_filter* h, const double* noise5);
 int ekf_get_noise(ekf_filter* h, double* out5);
+/* Normalised innovation squared of the single filter, with the scoring rule of ekf_batch_set_nis: every correction a
+ * measurement() / data_association() call applies is scored from exactly the S^-1 and nu of its gain, except those of
+ * the filter's first measurement() (landmark_init_flag == 0 on entry) and a data_association() correction of a landmark
+ * created by the same reading.  A call's values are summed in correction order and the sum is then added to
+ * {sum NIS, sum NIS^2, #scored, #non-finite}, so a streamed filter with ekf_set_carry_pending(h, 0) gets accumulators
+ * bit-identical to the same filter in a wide batch.  No kernel launch is added: ekf_launch_count is the same either way.
+ *
+ * 1: the following measurement() / data_association() calls run the NIS variants of the filter's kernels and
+ * accumulate (buffers allocated and zeroed on first use); 0: the plain kernels again, accumulators kept.  ekf_clone
+ * copies the switch and the accumulators; ekf_set_state, ekf_set_sigma and ekf_set_noise leave them alone. */
+int ekf_set_nis(ekf_filter* h, int on);
+/* out4 = {sum NIS, sum NIS^2, #scored, #non-finite}; reset != 0 zeroes them after the read.  EKF_ERR_STATE before NIS
+ * was ever enabled.  Synchronises. */
+int ekf_nis(ekf_filter* h, double* out4, int reset);
+/* The NIS of the last measurement() / data_association() call that ran with NIS on, aligned with that call's inputs:
+ * n values (slot order) after measurement(), m values (measurement order) after data_association(); *count_out says
+ * which (0 before the first such call).  -1.0 where no correction was scored; a scored value that is not finite is
+ * written as it is.  out may be NULL to ask for the count only.  EKF_ERR_STATE before NIS was ever enabled.
+ * Synchronises. */
+int ekf_last_nis(ekf_filter* h, double* out, int* count_out);
 /* passes over Sigma the streamed engine has made so far (for the roofline accounting of bench.py) */
 int ekf_sweep_count(ekf_filter* h, uint64_t* out);
 /* raw device pointers for callers that live on the GPU already (bench, fused pipelines) */

@@ -9,6 +9,7 @@
 #ifndef EKF_SLAM_INCLUDE_GUARD_HPP
 #define EKF_SLAM_INCLUDE_GUARD_HPP
 
+#include <array>
 #include <cstdint>
 #include <cstdio>
 #include <utility>
@@ -145,6 +146,31 @@ class EKF_SLAM {
             status_ = ekf_set_noise(h_, row);
         }
         report("ekf_set_noise");
+    }
+    // not in the reference: normalised innovation squared of the following measurement() / data_association() calls
+    // (ekf_set_nis); copies of this object carry the switch and the accumulators
+    void set_nis(bool on) {
+        status_ = ekf_set_nis(h_, on ? 1 : 0);
+        report("ekf_set_nis");
+    }
+    // {sum NIS, sum NIS^2, #scored, #non-finite} (ekf_nis); reset zeroes them after the read.  Zeros on failure.
+    std::array<double, 4> nis(bool reset = false) {
+        std::array<double, 4> out = {0.0, 0.0, 0.0, 0.0};
+        status_ = ekf_nis(h_, out.data(), reset ? 1 : 0);
+        report("ekf_nis");
+        if (status_ != 0) out = {0.0, 0.0, 0.0, 0.0};
+        return out;
+    }
+    // NIS per slot (after measurement()) or per measurement (after data_association()) of the last call that ran with
+    // NIS on, -1 where nothing was scored (ekf_last_nis).  Empty on failure.
+    std::vector<double> last_nis() {
+        int count = 0;
+        status_ = ekf_last_nis(h_, nullptr, &count);
+        std::vector<double> out(status_ == 0 ? (size_t)count : 0);
+        if (status_ == 0 && count > 0) status_ = ekf_last_nis(h_, out.data(), &count);
+        report("ekf_last_nis");
+        if (status_ != 0) out.clear();
+        return out;
     }
     ekf_filter* handle() {
         pose_ok_ = false;  // the caller may change the filter behind this object
