@@ -48,56 +48,52 @@ int launch_smem_kernel(int smem, const FusedParams& p, cudaStream_t stream, int 
     return EKF_OK;
 }
 
-// Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.  With p.noise, the NOISE
-// variant; with p.nis, the NIS variant.
-template <bool NoiseOn, bool Nis>
-int launch_fused_nz(const FusedParams& p, cudaStream_t stream, int device) {
-    const int smem = FusedSmem(p.n, p.m_max, NoiseOn, Nis).total;
-    return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20, NoiseOn, Nis>>(smem, p, stream, device)
-                     : launch_smem_kernel<ekf_fused_kernel<0, NoiseOn, Nis>>(smem, p, stream, device);
-}
-template <bool Nis>
-int launch_fused_nis(const FusedParams& p, cudaStream_t stream, int device) {
-    return p.noise ? launch_fused_nz<true, Nis>(p, stream, device) : launch_fused_nz<false, Nis>(p, stream, device);
-}
+// Single filter: dense Sigma (ekf_fused.cuh); n = 20 gets the fully unrolled rank-2 pass.  With p.nis, the NIS
+// variant; with p.noise, the NOISE variant.
 int launch_fused(const FusedParams& p, cudaStream_t stream, int device) {
-    return p.nis ? launch_fused_nis<true>(p, stream, device) : launch_fused_nis<false>(p, stream, device);
+    return with_flags(
+        [&](auto nis, auto noise) {
+            const int smem = FusedSmem(p.n, p.m_max, nis, noise).total;
+            return p.n == 20 ? launch_smem_kernel<ekf_fused_kernel<20, nis, noise>>(smem, p, stream, device)
+                             : launch_smem_kernel<ekf_fused_kernel<0, nis, noise>>(smem, p, stream, device);
+        },
+        p.nis != nullptr, p.noise != nullptr);
 }
 
 // Batch with n <= 64, n != 20: symmetric staircase Sigma (ekf_fused_sym.cuh).
-template <bool Nis>
-int launch_fused_staircase_nis(const FusedParams& p, cudaStream_t stream, int device) {
-    return p.noise ? launch_smem_kernel<ekf_fused_sym_kernel<Nis, true>>(SymSmem(p.n, p.m_max, Nis, true).total, p, stream,
-                                                                        device)
-                   : launch_smem_kernel<ekf_fused_sym_kernel<Nis, false>>(SymSmem(p.n, p.m_max, Nis).total, p, stream,
-                                                                         device);
-}
 int launch_fused_staircase(const FusedParams& p, cudaStream_t stream, int device) {
-    return p.nis ? launch_fused_staircase_nis<true>(p, stream, device) : launch_fused_staircase_nis<false>(p, stream, device);
+    return with_flags(
+        [&](auto nis, auto noise) {
+            return launch_smem_kernel<ekf_fused_sym_kernel<nis, noise>>(SymSmem(p.n, p.m_max, nis, noise).total, p,
+                                                                        stream, device);
+        },
+        p.nis != nullptr, p.noise != nullptr);
 }
 
-// Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh).
-template <bool Assoc, bool Nis, bool NoiseOn>
-int launch_fused_tile(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
-    const tile::TileSmem L(p.m_max, Assoc, Nis, NoiseOn);
-    if (L.total > max_smem_optin(device))
-        return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for m_max=%d", L.total, p.m_max);
-    if (p.sig_stride != tile::kStride || p.st_stride != tile::kStride || p.n != tile::kNL ||
-        p.state != p.sigma + tile::kStOff)
-        return fail(EKF_ERR_STATE, "tile engine: unexpected batch layout");
-    if (p.B <= 0) return EKF_OK;
-    // persistent warps: as many single-warp CTAs as fit the device at once, each walking filters b, b + grid, ...
-    int per_sm = 0;
-    CU((kernel_setup<tile::ekf_fused_tile_kernel<Assoc, Nis, NoiseOn>>(device, 32, L.total, true, &per_sm)));
-    const long long resident = (long long)sm_count * std::max(per_sm, 1);
-    tile::ekf_fused_tile_kernel<Assoc, Nis, NoiseOn><<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
-    CU(cudaGetLastError());
-    return EKF_OK;
-}
-template <bool Assoc, bool Nis>
-int launch_fused_tile_nis(const FusedParams& p, cudaStream_t stream, int device, int sm_count) {
-    return p.noise ? launch_fused_tile<Assoc, Nis, true>(p, stream, device, sm_count)
-                   : launch_fused_tile<Assoc, Nis, false>(p, stream, device, sm_count);
+// Batched engine at the reference's map size (n = 20): Sigma resident in registers (ekf_fused_tile.cuh); with
+// `association` (kDoAssociation), the ASSOC variant.
+int launch_fused_tile(const FusedParams& p, bool association, cudaStream_t stream, int device, int sm_count) {
+    return with_flags(
+        [&](auto assoc, auto nis, auto noise) {
+            const tile::TileSmem L(p.m_max, assoc, nis, noise);
+            if (L.total > max_smem_optin(device))
+                return fail(EKF_ERR_UNSUPPORTED, "fused engine: %d B of shared memory needed for m_max=%d", L.total,
+                            p.m_max);
+            if (p.sig_stride != tile::kStride || p.st_stride != tile::kStride || p.n != tile::kNL ||
+                p.state != p.sigma + tile::kStOff)
+                return fail(EKF_ERR_STATE, "tile engine: unexpected batch layout");
+            if (p.B <= 0) return EKF_OK;
+            // persistent warps: as many single-warp CTAs as fit the device at once, each walking filters
+            // b, b + grid, ...
+            int per_sm = 0;
+            CU((kernel_setup<tile::ekf_fused_tile_kernel<assoc, nis, noise>>(device, 32, L.total, true, &per_sm)));
+            const long long resident = (long long)sm_count * std::max(per_sm, 1);
+            tile::ekf_fused_tile_kernel<assoc, nis, noise>
+                <<<(unsigned)std::min<long long>(p.B, resident), 32, L.total, stream>>>(p);
+            CU(cudaGetLastError());
+            return EKF_OK;
+        },
+        association, p.nis != nullptr, p.noise != nullptr);
 }
 
 // Sigma0 = blockdiag(0_3, 100 I) (ekf_slam.cpp:29-36) for B filters of an already-zeroed buffer: dense rows of stride
@@ -109,54 +105,14 @@ __global__ void k_init_sigma(double* __restrict__ sigma, long long B, int N, lon
     sigma[b * stride + k * ld + k] = kSigma0;
 }
 
-__device__ __forceinline__ void maha_one(const double* sig, long long ld, const double* state, int i, double sx,
-                                         double sy, double* out, const Noise& nz) {
+// NOISE: Q and R from `nz` (the handle's row, ekf_set_noise); otherwise the reference's.
+template <bool NOISE>
+__global__ void k_maha_one(const double* sig, long long ld, const double* state, int i, double sx, double sy,
+                           double* out, const Noise nz) {
     double zr, zphi;
     range_bearing(sx, sy, zr, zphi);
-    *out = maha_distance(sig, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, state[0], state[1], state[2], nz);
-}
-__global__ void k_maha_one(const double* sig, long long ld, const double* state, int i, double sx, double sy,
-                           double* out) {
-    maha_one(sig, ld, state, i, sx, sy, out, ref_noise());
-}
-
-// NOISE variants of the single filter's kernels that use Q or R (ekf_set_noise): the handle's row travels as a kernel
-// argument.  The fused engine reads it from the device copy instead (FusedParams::noise).
-__global__ void k_maha_one_noise(const double* sig, long long ld, const double* state, int i, double sx, double sy,
-                                 double* out, const Noise nz) {
-    maha_one(sig, ld, state, i, sx, sy, out, nz);
-}
-__global__ void k_large_motion_noise(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
-                                     double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
-                                     double2* __restrict__ Wp, int pending, const Noise nz) {
-    large_motion(state, sig, ld, dtheta, dx, motion_out, Kp, Wp, pending, nz);
-}
-__global__ void __launch_bounds__(kGainThreads)
-    k_large_gain_p_noise(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
-                         double* __restrict__ state_out, const double* __restrict__ pose_src,
-                         const UpdateCmd* __restrict__ cmd, int lm_arg, double sx_arg, double sy_arg,
-                         double2* __restrict__ Kp, double2* __restrict__ Wp, int p, const Noise nz) {
-    large_gain_p(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p, nz);
-}
-// NIS variants of both (ekf_set_nis): nis_acc = the handle's 8 accumulators, nis_out = the call's slot of this correction
-template <bool NoiseOn>
-__global__ void __launch_bounds__(kGainThreads)
-    k_large_gain_p_nis(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
-                       double* __restrict__ state_out, const double* __restrict__ pose_src,
-                       const UpdateCmd* __restrict__ cmd, int lm_arg, double sx_arg, double sy_arg,
-                       double2* __restrict__ Kp, double2* __restrict__ Wp, int p, const Noise nz, double* nis_acc,
-                       double* nis_out, int nis_flags) {
-    large_gain_p<true>(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p,
-                       NoiseOn ? nz : ref_noise(), nis_acc, nis_out, nis_flags);
-}
-__global__ void __launch_bounds__(256)
-    k_large_assoc_noise(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
-                        const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
-                        AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
-                        UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
-                        double* __restrict__ second_out, uint8_t* __restrict__ created_out, const Noise nz) {
-    large_assoc(sig, ld, state, n, meas, j, known_count_p, partials, done_counter, cmd, assoc_out, dmin_out, second_out,
-                created_out, nz);
+    *out = maha_distance(sig, ld, i, state[3 + 2 * i], state[4 + 2 * i], zr, zphi, state[0], state[1], state[2],
+                         NOISE ? nz : ref_noise());
 }
 
 // Rows {q_theta, q_x, q_y, r_range, r_bearing}: every entry finite, q >= 0, r > 0.
@@ -430,22 +386,14 @@ int stream_flush(ekf_filter* h, int n_counted, const UpdateCmd* cmd) {
 int stream_correct(ekf_filter* h, const double* pose_src, const UpdateCmd* cmd, int lm, double sx, double sy,
                    int nis_slot) {
     const int gb = (int)((h->ld + 255) / 256);
-    if (h->nis_on) {
-        if (h->noise_on)
-            CU(launch_pdl(k_large_gain_p_nis<true>, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
-                          h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise,
-                          h->d_nis, h->d_nis_vals + nis_slot, h->nis_flags));
-        else
-            CU(launch_pdl(k_large_gain_p_nis<false>, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
-                          h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise,
-                          h->d_nis, h->d_nis_vals + nis_slot, h->nis_flags));
-        h->nis_flags &= ~kNisFold;
-    } else if (h->noise_on)
-        CU(launch_pdl(k_large_gain_p_noise, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N,
-                      h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending, h->noise));
-    else
-        CU(launch_pdl(k_large_gain_p, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld, h->N, h->d_state,
-                      h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending));
+    CU(with_flags(
+        [&](auto nis, auto noise) {
+            return launch_pdl(k_large_gain_p<nis, noise>, dim3(gb), dim3(kGainThreads), 0, h->stream, h->d_sigma, h->ld,
+                              h->N, h->d_state, h->d_state_alt, pose_src, cmd, lm, sx, sy, h->d_K2, h->d_W2, h->pending,
+                              h->noise, h->d_nis, nis ? h->d_nis_vals + nis_slot : nullptr, h->nis_flags);
+        },
+        h->nis_on, h->noise_on));
+    if (h->nis_on) h->nis_flags &= ~kNisFold;
     h->launches += 1;
     std::swap(h->d_state, h->d_state_alt);
     h->pending += 1;
@@ -691,12 +639,12 @@ int ekf_predict(ekf_filter* h, double dtheta, double dx) {
     }
     // motion model + robot block + the pending factors carried across the prediction (ekf_large_delayed.cuh), then
     // the robot-landmark strips
-    if (h->noise_on)
-        CU(launch_pdl(k_large_motion_noise, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld, dtheta, dx,
-                      h->d_motion, h->d_K2, h->d_W2, h->pending, h->noise));
-    else
-        CU(launch_pdl(k_large_motion, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld, dtheta, dx,
-                      h->d_motion, h->d_K2, h->d_W2, h->pending));
+    CU(with_flags(
+        [&](auto noise) {
+            return launch_pdl(k_large_motion<noise>, dim3(1), dim3(32), 0, h->stream, h->d_state, h->d_sigma, h->ld,
+                              dtheta, dx, h->d_motion, h->d_K2, h->d_W2, h->pending, h->noise);
+        },
+        h->noise_on));
     CU(launch_pdl(k_large_predict_strips, dim3((h->N - 3 + 255) / 256), dim3(256), 0, h->stream, h->d_sigma, h->ld, h->N,
                   (const double*)h->d_motion));
     h->launches += 2;
@@ -827,15 +775,13 @@ int ekf_data_association(ekf_filter* h, const double* xy, int m, uint8_t* known,
         CU(cudaMemcpyAsync(h->d_known_count, slot_i + 1, sizeof(int), cudaMemcpyHostToDevice, h->stream));
         CU(cudaEventRecord(ev, h->stream));
         for (int j = 0; j < m; ++j) {
-            if (h->noise_on)
-                k_large_assoc_noise<<<h->assoc_blocks, 256, 0, h->stream>>>(
-                    h->d_sigma, h->ld, h->d_state, n, h->d_in, j, h->d_known_count, h->d_partials, h->d_done, h->d_cmd,
-                    h->d_assoc, h->d_dmin, h->d_second, h->d_created, h->noise);
-            else
-                k_large_assoc<<<h->assoc_blocks, 256, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, n, h->d_in, j,
-                                                                       h->d_known_count, h->d_partials, h->d_done,
-                                                                       h->d_cmd, h->d_assoc, h->d_dmin, h->d_second,
-                                                                       h->d_created);
+            with_flags(
+                [&](auto noise) {
+                    k_large_assoc<noise><<<h->assoc_blocks, 256, 0, h->stream>>>(
+                        h->d_sigma, h->ld, h->d_state, n, h->d_in, j, h->d_known_count, h->d_partials, h->d_done,
+                        h->d_cmd, h->d_assoc, h->d_dmin, h->d_second, h->d_created, h->noise);
+                },
+                h->noise_on);
             h->launches += 1;
             // the next measurement's distances need the corrected Sigma: one factor, applied at once
             rc = stream_correct(h, h->d_state, h->d_cmd, 0, 0.0, 0.0, j);
@@ -892,10 +838,12 @@ int ekf_maha(ekf_filter* h, double mx, double my, int landmark, double* d_out) {
         int rc_ = stream_settle(h);
         if (rc_) return rc_;
     }
-    if (h->noise_on)
-        k_maha_one_noise<<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar, h->noise);
-    else
-        k_maha_one<<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar);
+    with_flags(
+        [&](auto noise) {
+            k_maha_one<noise><<<1, 1, 0, h->stream>>>(h->d_sigma, h->ld, h->d_state, landmark, mx, my, h->d_scalar,
+                                                      h->noise);
+        },
+        h->noise_on);
     h->launches += 1;
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(d_out, h->d_scalar, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -1443,12 +1391,8 @@ int launch_wide(ekf_batch* b, const double* twists, const double* xy, const uint
     p.st_stride = b->st_stride;
     p.nis = b->nis_on ? b->d_nis : nullptr;
     p.noise = b->noise_on ? b->d_noise : nullptr;
-    if (p.nis)
-        CU((p.noise ? launch_wide_step<true, true>(p, b->grid, b->stream, b->device)
-                    : launch_wide_step<true, false>(p, b->grid, b->stream, b->device)));
-    else
-        CU((p.noise ? launch_wide_step<false, true>(p, b->grid, b->stream, b->device)
-                    : launch_wide_step<false, false>(p, b->grid, b->stream, b->device)));
+    CU(with_flags([&](auto nis, auto noise) { return launch_wide_step<nis, noise>(p, b->grid, b->stream, b->device); },
+                  p.nis != nullptr, p.noise != nullptr));
     return EKF_OK;
 }
 
@@ -1487,14 +1431,8 @@ int batch_launch(ekf_batch* b, int mode, int m_max, const double* tw, const doub
         p.sparse_total = total;
         p.nis = b->nis_on ? b->d_nis : nullptr;
         p.noise = b->noise_on ? b->d_noise : nullptr;
-        if (b->layout == Layout::Stair)
-            rc = launch_fused_staircase(p, b->stream, b->device);
-        else if (association)
-            rc = p.nis ? launch_fused_tile_nis<true, true>(p, b->stream, b->device, b->sm_count)
-                       : launch_fused_tile_nis<true, false>(p, b->stream, b->device, b->sm_count);
-        else
-            rc = p.nis ? launch_fused_tile_nis<false, true>(p, b->stream, b->device, b->sm_count)
-                       : launch_fused_tile_nis<false, false>(p, b->stream, b->device, b->sm_count);
+        rc = b->layout == Layout::Stair ? launch_fused_staircase(p, b->stream, b->device)
+                                        : launch_fused_tile(p, association, b->stream, b->device, b->sm_count);
     }
     b->launches += 1;
     return rc;

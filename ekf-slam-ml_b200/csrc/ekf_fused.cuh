@@ -48,7 +48,7 @@ __host__ __device__ inline int fused_round16(int v) { return (v + 15) & ~15; }
 // shared memory carve-up (bytes), identical on host and device
 struct FusedSmem {
     int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_noise, off_nis, total;
-    __host__ __device__ FusedSmem(int n, int m_max, bool noise = false, bool nis = false) {
+    __host__ __device__ FusedSmem(int n, int m_max, bool nis, bool noise) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;
@@ -381,12 +381,12 @@ __device__ __forceinline__ void fused_association(const FusedParams& p, const lo
 // NIS: the call's scored corrections (none in a filter's first measurement(), none for a landmark its own reading
 // created) write their NIS to p.nis_out and are summed in correction order by lane 0, in shared memory; the sums are
 // added to p.nis at write-back.
-template <int NL, bool NOISE, bool NIS>
+template <int NL, bool NIS, bool NOISE>
 __global__ void __launch_bounds__(32) ekf_fused_kernel(const FusedParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int n = NL ? NL : p.n;
     const int N = 3 + 2 * n;
-    const FusedSmem L(n, p.m_max, NOISE, NIS);
+    const FusedSmem L(n, p.m_max, NIS, NOISE);
     double* sig = reinterpret_cast<double*>(smem_raw + L.off_sig);
     double* st = reinterpret_cast<double*>(smem_raw + L.off_st);
     double2* K2 = reinterpret_cast<double2*>(smem_raw + L.off_k2);

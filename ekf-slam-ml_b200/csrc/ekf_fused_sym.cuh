@@ -38,7 +38,7 @@ __host__ __device__ constexpr int sym_st_stride(int N) { return (N + 1) & ~1; }
 
 struct SymSmem {
     int off_sig, off_st, off_k2, off_w2, off_k2b, off_w2b, off_z, off_bar, off_nis, off_noise, total;
-    __host__ __device__ SymSmem(int n, int m_max, bool nis = false, bool noise = false) {
+    __host__ __device__ SymSmem(int n, int m_max, bool nis, bool noise) {
         const int N = 3 + 2 * n;
         int o = 0;
         off_sig = o;

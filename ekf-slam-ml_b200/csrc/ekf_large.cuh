@@ -40,7 +40,8 @@ __device__ __forceinline__ void pdl_prologue() {
 // One warp: lane 0 does the motion model, state[0..2], the 3x3 robot block of At*Sigma*At^T + Q, and (a1, a2) for the
 // strips; lane j < pending carries pending factor j across the prediction (ekf_large_delayed.cuh).  The row-sharded
 // engine runs it on every rank: `sig` is then the rank's 3 x ld copy of rows 0..2, or its own rows on rank 0.
-// The body is shared by k_large_motion (the reference's Q) and the single filter's noise variant (capi.cu).
+// k_large_motion<NOISE> runs it with Q from `nz` (the single filter's row, ekf_set_noise), otherwise with the
+// reference's.
 __device__ __forceinline__ void large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld,
                                              double dtheta, double dx, double* __restrict__ motion_out,
                                              double2* __restrict__ Kp, double2* __restrict__ Wp, int pending,
@@ -83,10 +84,11 @@ __device__ __forceinline__ void large_motion(double* __restrict__ state, double*
     motion_out[0] = m.a1;
     motion_out[1] = m.a2;
 }
+template <bool NOISE>
 __global__ void k_large_motion(double* __restrict__ state, double* __restrict__ sig, long long ld, double dtheta,
                                double dx, double* __restrict__ motion_out, double2* __restrict__ Kp,
-                               double2* __restrict__ Wp, int pending) {
-    large_motion(state, sig, ld, dtheta, dx, motion_out, Kp, Wp, pending, ref_noise());
+                               double2* __restrict__ Wp, int pending, const Noise nz) {
+    large_motion(state, sig, ld, dtheta, dx, motion_out, Kp, Wp, pending, NOISE ? nz : ref_noise());
 }
 
 // Robot-landmark strips: rows 1,2 += a*row0 and cols 1,2 += a*col0 for indices k >= 3.  6N doubles touched.
@@ -230,7 +232,8 @@ __device__ __forceinline__ void assoc_decide(double best, double second, int bes
     if (created_out) created_out[j] = (uint8_t)created;
 }
 
-// The body is shared by k_large_assoc (the reference's R) and the single filter's noise variant (capi.cu).
+// k_large_assoc<NOISE> runs it with R from `nz` (the single filter's row, ekf_set_noise), otherwise with the
+// reference's.
 __device__ __forceinline__ void large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state,
                                             int n, const double* __restrict__ meas, int j,
                                             int* __restrict__ known_count_p, AssocPartial* __restrict__ partials,
@@ -251,14 +254,15 @@ __device__ __forceinline__ void large_assoc(const double* __restrict__ sig, long
     assoc_decide(best, second, best_i, known_count, n, j, sx, sy, theta, x, y, state, known_count_p, cmd, assoc_out,
                  dmin_out, second_out, created_out);
 }
+template <bool NOISE>
 __global__ void __launch_bounds__(256)
     k_large_assoc(const double* __restrict__ sig, long long ld, double* __restrict__ state, int n,
                   const double* __restrict__ meas, int j, int* __restrict__ known_count_p,
                   AssocPartial* __restrict__ partials, unsigned int* __restrict__ done_counter,
                   UpdateCmd* __restrict__ cmd, int32_t* __restrict__ assoc_out, double* __restrict__ dmin_out,
-                  double* __restrict__ second_out, uint8_t* __restrict__ created_out) {
+                  double* __restrict__ second_out, uint8_t* __restrict__ created_out, const Noise nz) {
     large_assoc(sig, ld, state, n, meas, j, known_count_p, partials, done_counter, cmd, assoc_out, dmin_out, second_out,
-                created_out, ref_noise());
+                created_out, NOISE ? nz : ref_noise());
 }
 
 // ---------------------------------------------------------------- 256-bit global accesses (LDG/STG.E.256 on sm_100a)

@@ -168,15 +168,16 @@ __device__ __forceinline__ void gain_nis(const GainSharedP& g, const UpdateCmd* 
     }
 }
 
-// The body is shared by k_large_gain_p (the reference's R) and the single filter's noise and NIS variants (capi.cu).
-// NIS: lane 0 of the scalar warp in CTA 0 scores the correction (gain_nis) and writes its value to *nis_out.
-template <bool NIS = false>
+// k_large_gain_p<NIS, NOISE> runs it with R from `nz` (the single filter's row, ekf_set_noise) under NOISE, otherwise
+// with the reference's.  NIS (ekf_set_nis): lane 0 of the scalar warp in CTA 0 scores the correction (gain_nis) into
+// nis_acc (the handle's 8 accumulators) and writes its value to *nis_out (the call's slot of this correction).
+template <bool NIS>
 __device__ __forceinline__ void large_gain_p(const double* __restrict__ sig, long long ld, int N,
                                              const double* __restrict__ state_in, double* __restrict__ state_out,
                                              const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
                                              int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp,
-                                             double2* __restrict__ Wp, int p, const Noise& nz, double* nis_acc = nullptr,
-                                             double* nis_out = nullptr, int nis_flags = 0) {
+                                             double2* __restrict__ Wp, int p, const Noise& nz, double* nis_acc,
+                                             double* nis_out, int nis_flags) {
     __shared__ GainSharedP g;
     pdl_prologue();
     int lm = lm_arg;
@@ -235,11 +236,14 @@ __device__ __forceinline__ void large_gain_p(const double* __restrict__ sig, lon
     Wout[k] = wk;
     Kout[k] = kk;
 }
+template <bool NIS, bool NOISE>
 __global__ void __launch_bounds__(kGainThreads)
     k_large_gain_p(const double* __restrict__ sig, long long ld, int N, const double* __restrict__ state_in,
                    double* __restrict__ state_out, const double* __restrict__ pose_src, const UpdateCmd* __restrict__ cmd,
-                   int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp, double2* __restrict__ Wp, int p) {
-    large_gain_p(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p, ref_noise());
+                   int lm_arg, double sx_arg, double sy_arg, double2* __restrict__ Kp, double2* __restrict__ Wp, int p,
+                   const Noise nz, double* nis_acc, double* nis_out, int nis_flags) {
+    large_gain_p<NIS>(sig, ld, N, state_in, state_out, pose_src, cmd, lm_arg, sx_arg, sy_arg, Kp, Wp, p,
+                      NOISE ? nz : ref_noise(), nis_acc, nis_out, nis_flags);
 }
 
 // prediction() with factors pending: Sigma' = A (Sigma_0 - sum_j K_j W_j) A^T + Q = [A Sigma_0 A^T + Q] - sum_j (A K_j)(W_j A^T)

@@ -6,6 +6,7 @@
 
 #include <cstdarg>
 #include <cstdio>
+#include <type_traits>
 
 namespace {
 
@@ -66,6 +67,18 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+// Runtime flags to compile-time ones: with_flags(f, b0, b1, ...) calls f(std::bool_constant<b0>{},
+// std::bool_constant<b1>{}, ...), so that a generic lambda can instantiate the kernel variant the flags select.
+template <class F>
+decltype(auto) with_flags(F&& f) {
+    return f();
+}
+template <class F, class... Flags>
+decltype(auto) with_flags(F&& f, bool b, Flags... rest) {
+    if (b) return with_flags([&](auto... c) { return f(std::true_type{}, c...); }, rest...);
+    return with_flags([&](auto... c) { return f(std::false_type{}, c...); }, rest...);
 }
 
 // Set-up of one kernel on `device` (the current device), cached per kernel and device: raises the kernel's dynamic

@@ -864,7 +864,8 @@ int ekf_sharded_predict(ekf_sharded* h, double dtheta, double dx) {
     }
     for (auto& s : h->sh) {
         // on ranks > 0 this updates the copy of rows 0..2, which exchange_robot_rows overwrites before it is read
-        k_large_motion<<<1, 32, 0, h->stream>>>(s.state, s.robot, h->ld, dtheta, dx, s.motion, s.K2, s.W2, h->pending);
+        k_large_motion<false><<<1, 32, 0, h->stream>>>(s.state, s.robot, h->ld, dtheta, dx, s.motion, s.K2, s.W2,
+                                                       h->pending, ref_noise());
         h->launches++;
         int lr_begin = 0;
         if (s.rank == 0) {
