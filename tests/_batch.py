@@ -1,6 +1,7 @@
 """Helpers shared by the GPU batch tests: device shorthands, the grid world and traces the batch tests run, the step
-loops over EKFBatch's input forms, and the bit-identity checks of checkpoints and replicas.  What differs between test
-files (number of trajectories, m_max, tolerances) is passed in."""
+loops over EKFBatch's input forms, the bit-identity checks of checkpoints and replicas, the association tie margin and
+the staircase layout's strides.  What differs between test files (number of trajectories, m_max, tolerances) is
+passed in."""
 import numpy as np
 
 
@@ -89,13 +90,30 @@ def assert_replicas(a, B, K, what):
         assert bad.size == 0, f"{what}: filter {k + K * int(bad[0])} differs from filter {k}"
 
 
+def tie_margin(dmin, second):
+    """How far each association decision is from flipping: dmin's distance to the gates (1 and 10) and to the
+    runner-up, or, when no candidate is below the gate (dmin == 10 exactly), the runner-up's distance to the gate."""
+    has = dmin < 10.0
+    return np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(second - dmin)]),
+                    np.abs(second - 10.0))
+
+
 def assert_clear(dmin, second):
     """No decision sits within 1e-6 (relative) of a gate or of a tie with the runner-up, where the device and the
     oracle could round to different sides."""
-    has = dmin < 10.0
-    margin = np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(second - dmin)]),
-                      np.abs(second - 10.0))
+    margin = tie_margin(dmin, second)
     assert np.all(margin > 1e-6 * np.maximum(1.0, np.abs(dmin))), "threshold tie in the fixture: pick another seed"
+
+
+def stair_row_base(r, N):
+    """Offset of row r in the packed staircase layout of csrc/ekf_fused_sym.cuh (the batch layout of n <= 64, n != 20):
+    row r keeps the columns [16 floor(r / 16), N)."""
+    rb = r >> 4
+    return 16 * rb * N - 128 * rb * (rb - 1) + (r - 16 * rb) * (N - 16 * rb)
+
+
+def stair_strides(N):
+    return (stair_row_base(N, N) + 1) & ~1, (N + 1) & ~1  # per-filter Sigma and state strides in doubles
 
 
 def robot_frame(state, k, offset=(0.0, 0.0)):

@@ -12,6 +12,7 @@ import functools
 import numpy as np
 import pytest
 
+import _single as single
 from _batch import assert_clear, robot_frame
 from _oracle import OracleEKF, sigma_err, state_err
 
@@ -44,17 +45,13 @@ def _map(n):
     return steps, o.state, o.sigma
 
 
-def _sigma(f):
-    return f.sigma_full_local() if hasattr(f, "sigma_full_local") else f.sigma
-
-
 def _built(f, n):
     """Runs the map inputs through the device filter f; returns an oracle holding the same map."""
     steps, st, sg = _map(n)
     for tw, xy, vis in steps:
         f.prediction(tw)
         f.measurement(xy, vis)
-    assert state_err(f.state, st) < TOL and sigma_err(_sigma(f), sg) < TOL
+    assert state_err(f.state, st) < TOL and sigma_err(single.sigma(f), sg) < TOL
     o = OracleEKF(n)
     o.state, o.sigma, o.init_flag = st, sg, True
     return o
@@ -125,7 +122,7 @@ def _associate(f, o, xy, known_count, tie=False, nan_entry=None):
         assert np.isnan(fs[nan_entry]) and np.isnan(os_[nan_entry])
         fs[nan_entry] = os_[nan_entry] = 0.0
     assert state_err(fs, os_) < TOL
-    assert sigma_err(_sigma(f), o.sigma) < TOL
+    assert sigma_err(single.sigma(f), o.sigma) < TOL
     return a, dmin, sec, cr
 
 

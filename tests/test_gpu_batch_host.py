@@ -6,7 +6,7 @@ sym_sig_stride(N) and sym_st_stride(N); wide layout (64 < n <= 1,024) N * ld and
 import numpy as np
 import pytest
 
-from test_gpu_batch_staircase import _strides
+from _batch import stair_strides
 
 pytestmark = pytest.mark.gpu
 
@@ -17,7 +17,7 @@ def _expected(n):
     if n == 20:
         return 1136, 44, 1136
     if n <= 64:
-        sig, st = _strides(N)
+        sig, st = stair_strides(N)
         return sig, st, st
     ld = (N + 15) & ~15
     return N * ld, ld, ld

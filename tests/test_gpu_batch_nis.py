@@ -8,6 +8,7 @@ rule, bit-identical replicas when persistent CTAs carry several filters, and the
 import numpy as np
 import pytest
 
+import _single as single
 from _batch import (assert_replicas, assert_same_checkpoint, known_trace, replicate, run_known, run_unknown, sms,
                     step_known, unknown_trace)
 from _noise_ref import NoiseOracle
@@ -69,11 +70,7 @@ def test_nis_known_matches_reference(gpu_pkg, n):
     bt = gpu_pkg.EKFBatch(B, n)
     bt.set_nis(True)
     run_known(gpu_pkg, bt, tr, "dense")
-    refs = [NoiseOracle(n) for _ in range(B)]
-    for t in range(T):
-        for b, o in enumerate(refs):
-            o.prediction(*tr["twists"][t, b])
-            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+    refs = [single.run_known(NoiseOracle(n), tr, b) for b in range(B)]
     _compare(bt.nis(per_filter=True), refs, f"known n={n}")
 
 
@@ -85,14 +82,10 @@ def test_nis_unknown_matches_reference(gpu_pkg, n):
     bt.set_nis(True)
     assoc = run_unknown(bt, tr, M_MAX)
     refs = [NoiseOracle(n) for _ in range(B)]
-    known = [np.zeros(n, np.uint8) for _ in range(B)]
     created = dropped = 0
-    for t in range(T):
-        for b, o in enumerate(refs):
-            o.prediction(*tr["twists"][t, b])
-            m = int(np.clip(tr["count"][t, b], 0, M_MAX))
-            a, c = o.data_association(tr["meas"][t, b, :m], known[b])
-            assert np.array_equal(a, assoc[t, b, :m]), (t, b)
+    for b, o in enumerate(refs):
+        for t, (a, c) in enumerate(single.run_unknown(o, tr, np.zeros(n, np.uint8), b)):
+            assert np.array_equal(a, assoc[t, b, :len(a)]), (t, b)
             created += int(c.sum())
             dropped += int((a < 0).sum())
     assert created > 0 and dropped > 0  # the rule's exceptions are exercised: new landmarks and readings between gates
@@ -191,7 +184,7 @@ def test_back_to_back_host_steps(gpu_pkg):
     for row in bufs:
         bt.step_known(*row)
     bt.sync()
-    assert np.array_equal(_per_filter(bt).view(np.uint64), _per_filter(ref).view(np.uint64))
+    assert np.array_equal(single.bits(_per_filter(bt)), single.bits(_per_filter(ref)))
 
 
 # ---------------------------------------------------------------- 5. read-out
@@ -205,8 +198,8 @@ def test_readout(gpu_pkg):
     bt.set_nis(True)
     run_known(gpu_pkg, bt, tr, "dense")
     r1, r2 = bt.nis(per_filter=True), bt.nis(per_filter=True)
-    assert np.array_equal(r1["stats"].view(np.uint64), r2["stats"].view(np.uint64))
-    assert np.array_equal(r1["nis_sum"].view(np.uint64), r2["nis_sum"].view(np.uint64))
+    assert np.array_equal(single.bits(r1["stats"]), single.bits(r2["stats"]))
+    assert np.array_equal(single.bits(r1["nis_sum"]), single.bits(r2["nis_sum"]))
     assert r1["stats"][2] == r1["nis_count"].sum() and r1["stats"][3] == 0
     np.testing.assert_allclose(r1["stats"][0], r1["nis_sum"].sum(), rtol=1e-12)
     np.testing.assert_allclose(r1["stats"][1], r1["nis_sq_sum"].sum(), rtol=1e-12)
@@ -215,8 +208,8 @@ def test_readout(gpu_pkg):
     d_out, d_pf = torch.zeros(4, dtype=torch.float64, device="cuda"), torch.zeros(B, 4, dtype=torch.float64, device="cuda")
     bt.nis_dev(d_out.data_ptr(), d_pf.data_ptr(), reset=True)
     bt.sync()
-    assert np.array_equal(d_out.cpu().numpy().view(np.uint64), r1["stats"].view(np.uint64))
-    assert np.array_equal(d_pf.cpu().numpy()[:, 0].view(np.uint64), r1["nis_sum"].view(np.uint64))
+    assert np.array_equal(single.bits(d_out.cpu().numpy()), single.bits(r1["stats"]))
+    assert np.array_equal(single.bits(d_pf.cpu().numpy()[:, 0]), single.bits(r1["nis_sum"]))
     assert np.all(bt.nis()["stats"] == 0)
     # a null out4 is refused
     assert bt._L.ekf_batch_nis(bt._h, None, None, 0) != 0
@@ -245,5 +238,5 @@ def test_nan_covariance_counts_nonfinite(gpu_pkg, n):
         bt.sync()
     pa, pb = _per_filter(a), _per_filter(b)
     others = np.arange(B) != bad
-    assert np.array_equal(pa[others].view(np.uint64), pb[others].view(np.uint64))
+    assert np.array_equal(single.bits(pa[others]), single.bits(pb[others]))
     assert pb[bad, 3] == tr["vis"][1:, bad].sum() and pb[bad, 2] == 0 and pb[bad, 0] == 0

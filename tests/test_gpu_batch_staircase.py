@@ -9,7 +9,8 @@ of the per-filter measurement count (both batch kernels)."""
 import numpy as np
 import pytest
 
-from _batch import assert_clear, dev, robot_frame, run_known, run_unknown, step_known
+import _single as single
+from _batch import assert_clear, dev, robot_frame, run_known, run_unknown, stair_row_base, stair_strides, step_known
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
@@ -18,23 +19,14 @@ TOL = 1e-9
 
 
 # ---------------------------------------------------------------- staircase layout (formulas of ekf_fused_sym.cuh)
-def _stair_row_base(r, N):
-    rb = r >> 4
-    return 16 * rb * N - 128 * rb * (rb - 1) + (r - 16 * rb) * (N - 16 * rb)
-
-
 def pack_staircase(dense, N):
     """Dense N x N -> the stored part of the staircase: row r keeps the columns [16 floor(r / 16), N)."""
-    out = np.zeros(_stair_row_base(N, N))
+    out = np.zeros(stair_row_base(N, N))
     for r in range(N):
         c0 = r & ~15
-        base = _stair_row_base(r, N)
+        base = stair_row_base(r, N)
         out[base:base + N - c0] = dense[r, c0:]
     return out
-
-
-def _strides(N):
-    return (_stair_row_base(N, N) + 1) & ~1, (N + 1) & ~1  # per-filter Sigma and state strides in doubles
 
 
 def _grid_world(pkg, n, pitch=0.3):
@@ -54,16 +46,6 @@ def _known_trace(pkg, n, B, T, seed):
     return tr
 
 
-def _oracle_known(tr, b, n, xy=None, vis=None):
-    xy = tr["xy"] if xy is None else xy
-    vis = tr["vis"] if vis is None else vis
-    o = OracleEKF(n)
-    for t in range(tr["twists"].shape[0]):
-        o.prediction(*tr["twists"][t, b])
-        o.measurement(xy[t, b], vis[t, b])
-    return o
-
-
 def _picks(B, seed):
     return [0, B - 1] + [int(v) for v in np.random.default_rng(seed).choice(np.arange(1, B - 1), 2, replace=False)]
 
@@ -80,7 +62,7 @@ def test_known_association_dense_matches_oracle(gpu_pkg, n):
     assert bt.update_count == int(tr["vis"].sum())
     states = bt.states()
     for b in _picks(B, n):
-        o = _oracle_known(tr, b, n)
+        o = single.run_known(OracleEKF(n), tr, b)
         assert state_err(states[b], o.state) < TOL, b
         assert sigma_err(bt.sigma(b), o.sigma) < TOL, b
 
@@ -124,8 +106,9 @@ def test_marker_list_matches_oracle(gpu_pkg, n):
     bt.sync()
     assert bt.update_count == int(vis.sum())
     states = bt.states()
+    listed = dict(tr, xy=xy, vis=vis)
     for b in range(B):
-        o = _oracle_known(tr, b, n, xy=xy, vis=vis)
+        o = single.run_known(OracleEKF(n), listed, b)
         assert state_err(states[b], o.state) < TOL, b
         assert sigma_err(bt.sigma(b), o.sigma) < TOL, b
 
@@ -152,10 +135,8 @@ def test_unknown_association_matches_oracle(gpu_pkg, n, m_max):
     for b in range(B):
         o = OracleEKF(n)
         k = np.zeros(n, np.uint8)
-        for t in range(T):
-            o.prediction(*tu["twists"][t, b])
-            m = int(tu["count"][t, b])
-            a, dmin, sec, cr = o.data_association(tu["meas"][t, b, :m], k)
+        for t, (a, dmin, sec, cr) in enumerate(single.run_unknown(o, tu, k, b)):
+            m = len(a)
             assert_clear(dmin, sec)
             assert np.array_equal(assoc[t][b, :m], a), (b, t)
             assert np.all(assoc[t][b, m:] == -1)
@@ -211,8 +192,8 @@ def test_association_ties_lowest_index_wins(gpu_pkg):
     bt = gpu_pkg.EKFBatch(B, n)
     run_known(gpu_pkg, bt, tr)
     ck = bt.checkpoint()
-    ss, sts = _strides(N)
-    size = _stair_row_base(N, N)
+    ss, sts = stair_strides(N)
+    size = stair_row_base(N, N)
     pairs = [(3, 9), (5, 37)]
     oracles = []
     for b, (i, j) in enumerate(pairs):
@@ -282,7 +263,7 @@ def test_measurement_count_is_clamped(gpu_pkg, n):
     known0 = a.known
     assoc = a.step_unknown(tw1, me1, bad, M, want_assoc=True)
     states, known = a.states(), a.known
-    for b in range(B):
+    for b in range(B):  # by hand: filter 3's second step is a prediction only
         o = OracleEKF(n)
         k = np.zeros(n, np.uint8)
         o.prediction(*tu["twists"][0, b])

@@ -15,9 +15,9 @@ import ctypes
 import numpy as np
 import pytest
 
+import _single as single
 from _batch import assert_clear, assert_replicas, assert_same_checkpoint, dev, grid_world, replicate, sms
 from _oracle import OracleEKF, sigma_err, state_err
-from test_gpu_batch_wide import _streamed
 
 pytestmark = pytest.mark.gpu
 
@@ -37,7 +37,7 @@ def _assert_checkpoint_replicas(bt):
     assert_replicas(bt.states(), bt.B, K, "states()")
     for k in range(K):
         last = k + K * ((bt.B - 1 - k) // K)
-        assert np.array_equal(bt.sigma(last).view(np.uint64), bt.sigma(k).view(np.uint64)), (k, last)
+        assert np.array_equal(single.bits(bt.sigma(last)), single.bits(bt.sigma(k))), (k, last)
     return ck
 
 
@@ -118,10 +118,7 @@ def test_tile_known_replicas_in_every_input_form(gpu_pkg, known_inputs):
         assert_same_checkpoint(other.checkpoint(), ck)
     states = host.states()
     for k in range(K):
-        o = OracleEKF(NT)
-        for t in range(T_KNOWN):
-            o.prediction(*known_inputs["twists"][t, k])
-            o.measurement(known_inputs["xy"][t, k], known_inputs["vis"][t, k])
+        o = single.run_known(OracleEKF(NT), known_inputs, k)
         assert state_err(states[k], o.state) < TOL, k
         assert sigma_err(host.sigma(k), o.sigma) < TOL, k
 
@@ -176,10 +173,8 @@ def test_tile_unknown_replicas_host_and_device(gpu_pkg, unknown_inputs):
     for k in range(K):
         o = OracleEKF(NT)
         kn = np.zeros(NT, np.uint8)
-        for t in range(T_UNKNOWN):
-            o.prediction(*unknown_inputs["twists"][t, k])
-            m = min(max(int(unknown_inputs["count"][t, k]), 0), M_MAX)
-            a, dmin, sec, cr = o.data_association(unknown_inputs["meas"][t, k, :m], kn)
+        for t, (a, dmin, sec, cr) in enumerate(single.run_unknown(o, unknown_inputs, kn, k)):
+            m = len(a)
             assert_clear(dmin, sec)
             assert np.array_equal(assoc[t][k, :m], a), (k, t)
             assert np.all(assoc[t][k, m:] == -1), (k, t)
@@ -241,15 +236,12 @@ def test_wide_replicas_dense_and_marker_list(gpu_pkg, n):
     assert sparse.sweep_count == dense.sweep_count
     states = dense.states()
     for k in range(K):
-        f = _streamed(gpu_pkg, n, ref, k, range(T_WIDE))
-        assert np.array_equal(states[k].view(np.uint64), f.state.view(np.uint64)), k
-        assert np.array_equal(dense.sigma(k).view(np.uint64), f.sigma.view(np.uint64)), k
+        f = single.streamed(gpu_pkg, n, ref, k, range(T_WIDE))
+        assert np.array_equal(single.bits(states[k]), single.bits(f.state)), k
+        assert np.array_equal(single.bits(dense.sigma(k)), single.bits(f.sigma)), k
         f.close()
     k = WIDE_CLASSES.index(29)
-    o = OracleEKF(n)
-    for t in range(T_WIDE):
-        o.prediction(*ref["twists"][t, k])
-        o.measurement(ref["xy"][t, k], ref["vis"][t, k])
+    o = single.run_known(OracleEKF(n), ref, k)
     assert state_err(states[k], o.state) < TOL
     assert sigma_err(dense.sigma(k), o.sigma) < TOL
 
@@ -286,7 +278,7 @@ def _assert_back_to_back(bt, steps, pose_bufs, want_ck, want_poses):
     bt.sync()
     assert_same_checkpoint(bt.checkpoint(), want_ck)
     for t, (got, want) in enumerate(zip(pose_bufs, want_poses)):
-        assert np.array_equal(got.array.view(np.uint64), want.view(np.uint64)), t
+        assert np.array_equal(single.bits(got.array), single.bits(want)), t
 
 
 def test_tile_known_back_to_back_host_steps(gpu_pkg, known_inputs):

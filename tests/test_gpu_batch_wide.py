@@ -8,6 +8,7 @@ import ctypes
 import numpy as np
 import pytest
 
+import _single as single
 from _batch import grid_world, run_known, step_known
 from _oracle import OracleEKF, sigma_err, state_err
 
@@ -23,15 +24,6 @@ def _trace(pkg, n, B, T, seed):
     return tr
 
 
-def _streamed(pkg, n, tr, b, steps):
-    f = pkg.EKF_SLAM(n, engine=pkg.ENGINE_STREAM)
-    f.set_carry_pending(False)
-    for t in steps:
-        f.prediction(tuple(tr["twists"][t, b]))
-        f.measurement(tr["xy"][t, b], tr["vis"][t, b])
-    return f
-
-
 @pytest.mark.parametrize("n", [65, 100, 256])
 def test_wide_batch_is_bit_identical_to_streamed_filters(gpu_pkg, n):
     B, T = 48, 20
@@ -43,15 +35,12 @@ def test_wide_batch_is_bit_identical_to_streamed_filters(gpu_pkg, n):
     assert bt.update_count == int(tr["vis"].sum())
     rng = np.random.default_rng(n)
     for b in [0, B - 1] + list(rng.choice(np.arange(1, B - 1), 4, replace=False)):
-        f = _streamed(gpu_pkg, n, tr, b, range(T))
+        f = single.streamed(gpu_pkg, n, tr, b, range(T))
         assert np.array_equal(states[b], f.state), b
         assert np.array_equal(bt.sigma(b), f.sigma), b
     # oracle parity on a few filters
     for b in (0, B // 2):
-        o = OracleEKF(n)
-        for t in range(T):
-            o.prediction(*tr["twists"][t, b])
-            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+        o = single.run_known(OracleEKF(n), tr, b)
         assert state_err(states[b], o.state) < TOL
         assert sigma_err(bt.sigma(b), o.sigma) < TOL
 
@@ -69,7 +58,7 @@ def test_wide_batch_more_corrections_than_one_group(gpu_pkg):
     assert bt.sweep_count == int(np.ceil(c / P).sum())
     states = bt.states()
     for b in (0, B // 2 - 1, B // 2, B - 1):
-        f = _streamed(gpu_pkg, n, tr, b, range(T))
+        f = single.streamed(gpu_pkg, n, tr, b, range(T))
         assert np.array_equal(states[b], f.state), b
         assert np.array_equal(bt.sigma(b), f.sigma), b
 

@@ -5,6 +5,8 @@ state and covariance within 1e-9 in the scaled metric of tests/_oracle.py (sigma
 import numpy as np
 import pytest
 
+import _single as single
+from _batch import tie_margin
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
@@ -18,29 +20,13 @@ def _trace(pkg, n_slots, steps, seed, world=None):
     return tg.simulate_known(w, 1, steps, seed=seed)
 
 
-def _run_known(filt, oracle, tr, check_every=1):
-    worst_s = worst_x = 0.0
-    T = tr["twists"].shape[0]
-    for t in range(T):
-        dth, dx = tr["twists"][t, 0]
-        filt.prediction((dth, dx))
-        oracle.prediction(dth, dx)
-        filt.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
-        oracle.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
-        if t % check_every == 0 or t == T - 1:
-            worst_x = max(worst_x, state_err(filt.state, oracle.state))
-            worst_s = max(worst_s, sigma_err(filt.sigma, oracle.sigma))
-    return worst_x, worst_s
-
-
 @pytest.mark.parametrize("engine", ["fused", "stream"])
 def test_known_association_default_world(gpu_pkg, engine):
     """cfg1: nuslam known association on the default 10-tube world, n = 20 slots."""
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
     tr = _trace(gpu_pkg, 20, 150, seed=11)
-    f = gpu_pkg.EKF_SLAM(20, engine=eng)
+    f = gpu_pkg.EKF_SLAM(20, engine=single.engine(gpu_pkg, engine))
     o = OracleEKF(20)
-    ex, es = _run_known(f, o, tr, check_every=10)
+    ex, es = single.parity_known(f, o, tr, check_every=10)
     assert f.init_flag and o.init_flag
     assert f.update_count == int(tr["vis"].sum())
     assert ex < TOL and es < TOL, (ex, es)
@@ -50,13 +36,12 @@ def test_known_association_default_world(gpu_pkg, engine):
                                       (100, "stream")])
 def test_known_association_other_sizes(gpu_pkg, n, engine):
     """Generic-n code paths (the n=20 kernel is a specialised instantiation)."""
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
     rng = np.random.default_rng(n)
     lm = rng.uniform(-1.5, 1.5, (n, 2))
-    f = gpu_pkg.EKF_SLAM(n, engine=eng)
+    f = gpu_pkg.EKF_SLAM(n, engine=single.engine(gpu_pkg, engine))
     o = OracleEKF(n)
     worst = 0.0
-    for t in range(25):
+    for t in range(25):  # by hand: each step's readings are taken from the oracle's current pose
         dth, dx = 0.05 + rng.normal(0, 0.01), 0.01 + rng.normal(0, 0.002)
         if t % 7 == 3:
             dth = 1e-8  # straight-line branch of the motion model (ekf_slam.cpp:79)
@@ -87,21 +72,11 @@ def _unknown_run(gpu_pkg, n, eng, steps, seed, n_tubes=None):
     worst = 0.0
     n_meas = n_tie = 0
     for t in range(steps):
-        dth, dx = tr["twists"][t, 0]
-        f.prediction((dth, dx))
-        o.prediction(dth, dx)
-        m = int(tr["count"][t, 0])
-        meas = tr["meas"][t, 0, :m]
-        res = f.data_association(meas, kf)
-        a_o, dmin_o, sec_o, cr_o = o.data_association(meas, ko)
+        res = single.step_unknown(f, tr, t, kf)
+        a_o, dmin_o, sec_o, cr_o = single.step_unknown(o, tr, t, ko)
         # a decision is "away from a tie" when neither gate nor the runner-up is within 1e-6 (relative) of dmin
-        # (dmin == 10.0 exactly means "no candidate below the gate": then only the runner-up's distance to the
-        # gate matters)
-        has = dmin_o < 10.0
-        margin = np.where(has, np.minimum.reduce([np.abs(dmin_o - 10.0), np.abs(dmin_o - 1.0), np.abs(sec_o - dmin_o)]),
-                          np.abs(sec_o - 10.0))
-        clear = margin > 1e-6 * np.maximum(1.0, np.abs(dmin_o))
-        n_meas += m
+        clear = tie_margin(dmin_o, sec_o) > 1e-6 * np.maximum(1.0, np.abs(dmin_o))
+        n_meas += len(a_o)
         n_tie += int((~clear).sum())
         assert np.array_equal(res["assoc"][clear], a_o[clear]), (t, res["assoc"], a_o)
         assert np.array_equal(res["created"][clear], cr_o[clear])
@@ -114,8 +89,7 @@ def _unknown_run(gpu_pkg, n, eng, steps, seed, n_tubes=None):
 @pytest.mark.parametrize("engine", ["fused", "stream"])
 def test_unknown_association(gpu_pkg, engine):
     """cfg2 filter side: Mahalanobis gating + landmark initialisation, n = 20 slots, 10 tubes."""
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
-    worst, n_meas, n_tie, known = _unknown_run(gpu_pkg, 20, eng, 120, seed=5)
+    worst, n_meas, n_tie, known = _unknown_run(gpu_pkg, 20, single.engine(gpu_pkg, engine), 120, seed=5)
     assert n_meas > 300 and known >= 5
     assert n_tie == 0
     assert worst < TOL, worst
@@ -132,7 +106,7 @@ def test_maha_seam_and_getters(gpu_pkg):
     tr = _trace(gpu_pkg, 20, 30, seed=2)
     f = gpu_pkg.EKF_SLAM(20)
     o = OracleEKF(20)
-    _run_known(f, o, tr, check_every=100)
+    single.parity_known(f, o, tr, check_every=100)
     for i in (0, 3, 9):
         d_f = f.calculate_maha_dis((0.3, -0.2), i)
         d_o = o.maha(0.3, -0.2, i)
@@ -151,7 +125,7 @@ def test_pose_read_path_follows_every_way_the_state_can_change(gpu_pkg):
     tr = _trace(gpu_pkg, 20, 6, seed=8)
     f = gpu_pkg.EKF_SLAM(20)
     o = OracleEKF(20)
-    for t in range(3):
+    for t in range(3):  # by hand: the getters are read between prediction() and measurement()
         f.prediction(tuple(tr["twists"][t, 0]))
         o.prediction(*tr["twists"][t, 0])
         assert abs(f.getStateTheta() - o.state[0]) < 1e-12 and abs(f.getStateX() - o.state[1]) < 1e-12
@@ -233,7 +207,7 @@ def test_normalize_angle_device_twin_is_bit_exact(gpu_pkg):
                            np.nextafter(np.pi * np.arange(-8, 9), np.inf), np.nextafter(np.pi * np.arange(-8, 9), -np.inf)])
     got = gpu_pkg.normalize_angle(vals)
     want = np.array([L.oracle_normalize_angle(float(v)) for v in vals])
-    assert np.array_equal(got.view(np.uint64), want.view(np.uint64))
+    assert np.array_equal(single.bits(got), single.bits(want))
     # golden values of rigid2d/tests/tests.cpp:322-331
     g = gpu_pkg.normalize_angle(np.deg2rad([30.0, 230.0, -330.0]))
     np.testing.assert_allclose(g, [0.523599, -2.26893, 0.523599], rtol=1.2e-5)
@@ -283,10 +257,7 @@ def test_batch_matches_per_filter_oracle(gpu_pkg):
     assert bt.update_count == int(tr["vis"].sum())
     worst = 0.0
     for b in range(0, B, 5):
-        o = OracleEKF(20)
-        for t in range(T):
-            o.prediction(*tr["twists"][t, b])
-            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+        o = single.run_known(OracleEKF(20), tr, b)
         worst = max(worst, state_err(states[b], o.state), sigma_err(bt.sigma(b), o.sigma))
     assert worst < TOL, worst
     poses = bt.poses()
@@ -383,12 +354,9 @@ def test_batch_unknown_matches_oracle(gpu_pkg):
     for b in range(0, B, 3):
         o = OracleEKF(20)
         k = np.zeros(20, np.uint8)
-        for t in range(T):
-            o.prediction(*tr["twists"][t, b])
-            m = int(tr["count"][t, b])
-            a, _, _, _ = o.data_association(tr["meas"][t, b, :m], k)
-            assert np.array_equal(assoc[t][b, :m], a)
-            assert np.all(assoc[t][b, m:] == -1)
+        for t, (a, _, _, _) in enumerate(single.run_unknown(o, tr, k, b)):
+            assert np.array_equal(assoc[t][b, :len(a)], a)
+            assert np.all(assoc[t][b, len(a):] == -1)
         assert np.array_equal(known[b], k)
         worst = max(worst, state_err(states[b], o.state), sigma_err(bt.sigma(b), o.sigma))
     assert worst < TOL, worst
@@ -403,14 +371,14 @@ def test_large_map_stream_engine(gpu_pkg):
     f = gpu_pkg.EKF_SLAM(n)
     assert f.engine == gpu_pkg.ENGINE_STREAM
     o = OracleEKF(n)
-    ex, es = _run_known(f, o, tr, check_every=4)
+    ex, es = single.parity_known(f, o, tr, check_every=4)
     assert int(tr["vis"].sum()) > 40
     assert ex < TOL and es < TOL, (ex, es)
     # then unknown association on top of the converged map: all landmarks known
     known_f = np.ones(n, np.uint8)
     known_o = np.ones(n, np.uint8)
     tu = tg.simulate_unknown(w, 1, 3, seed=1)
-    for t in range(3):
+    for t in range(3):  # by hand: association only, no prediction in between
         m = int(tu["count"][t, 0])
         meas = tu["meas"][t, 0, :m]
         # measurements come from a different trajectory prefix, so most will be gated out: both sides must agree
@@ -432,10 +400,8 @@ def test_large_map_cfg4_size(gpu_pkg):
     o = OracleEKF(n)
     done = t = 0
     while done < 10:
-        f.prediction(tuple(tr["twists"][t, 0]))
-        f.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
-        o.prediction(*tr["twists"][t, 0])
-        o.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
+        single.step_known(f, tr, t)
+        single.step_known(o, tr, t)
         done += int(tr["vis"][t, 0].sum()) if t else 0
         t += 1
     assert f.sweep_count <= 1  # the corrections went through (at most) one sweep so far, the rest is pending
@@ -464,11 +430,7 @@ def test_update_count_with_one_sweep_per_correction(gpu_pkg):
     f.set_max_pending(1)
     o = OracleEKF(n)
     for obj in (f, o):
-        if obj is f:
-            obj.prediction(tuple(tr["twists"][0, 0]))
-        else:
-            obj.prediction(*tr["twists"][0, 0])
-        obj.measurement(tr["xy"][0, 0], tr["vis"][0, 0])
+        single.step_known(obj, tr, 0)
     ids = np.flatnonzero(tr["vis"][1, 0])[:4]
     xy = tr["xy"][1, 0].reshape(-1, 2)[ids]
     meas = np.concatenate([xy, [[55.0, 55.0]]])  # the last one is far from everything: gated out, no correction
@@ -493,7 +455,7 @@ def test_streamed_filter_on_a_second_device(gpu_pkg):
     for dev in (0, 1):
         f = gpu_pkg.EKF_SLAM(n, device=dev, engine=gpu_pkg.ENGINE_STREAM)
         o = OracleEKF(n)
-        ex, es = _run_known(f, o, tr, check_every=2)
+        ex, es = single.parity_known(f, o, tr, check_every=2)
         assert ex < TOL and es < TOL, (dev, ex, es)
 
 
@@ -507,7 +469,7 @@ def test_association_log(gpu_pkg, tmp_path):
     f.association_log(log)
     kf, ko = np.zeros(20, np.uint8), np.zeros(20, np.uint8)
     expect = []
-    for t in range(12):
+    for t in range(12):  # by hand: no data_association() call for a step without readings
         m = int(tu["count"][t, 0])
         f.prediction(tuple(tu["twists"][t, 0]))
         o.prediction(*tu["twists"][t, 0])
@@ -561,10 +523,10 @@ _GOLD = _os.path.join(_os.path.dirname(_os.path.abspath(__file__)), "golden")
 def test_golden_known_association(gpu_pkg, engine):
     """tests/golden/ekf_known_n20.npz: state / Sigma checkpoints and Mahalanobis probes produced by the reference."""
     g = np.load(_os.path.join(_GOLD, "ekf_known_n20.npz"))
-    f = gpu_pkg.EKF_SLAM(20, engine=gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM)
+    f = gpu_pkg.EKF_SLAM(20, engine=single.engine(gpu_pkg, engine))
     ck = list(g["checkpoints"])
     worst = 0.0
-    for t in range(g["twists"].shape[0]):
+    for t in range(g["twists"].shape[0]):  # by hand: the golden arrays have no trajectory axis
         f.prediction(tuple(g["twists"][t]))
         f.measurement(g["xy"][t], g["vis"][t])
         if t in ck:
@@ -586,11 +548,11 @@ def test_golden_unknown_association(gpu_pkg, engine):
     oracle/ekf_oracle.c on the same run; the reference-owned checkpoints of state and Sigma are what close the loop on
     those indices (a different association would move them far beyond the tolerance)."""
     g = np.load(_os.path.join(_GOLD, "ekf_unknown_n20.npz"))
-    f = gpu_pkg.EKF_SLAM(20, engine=gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM)
+    f = gpu_pkg.EKF_SLAM(20, engine=single.engine(gpu_pkg, engine))
     known = np.zeros(20, np.uint8)
     ck = list(g["checkpoints"])
     worst = 0.0
-    for t in range(g["twists"].shape[0]):
+    for t in range(g["twists"].shape[0]):  # by hand: the golden arrays have no trajectory axis
         f.prediction(tuple(g["twists"][t]))
         m = int(g["count"][t])
         r = f.data_association(g["meas"][t, :m], known)
@@ -605,7 +567,7 @@ def test_golden_unknown_association(gpu_pkg, engine):
 def test_golden_n100(gpu_pkg):
     g = np.load(_os.path.join(_GOLD, "ekf_known_n100.npz"))
     f = gpu_pkg.EKF_SLAM(100)
-    for t in range(g["twists"].shape[0]):
+    for t in range(g["twists"].shape[0]):  # by hand: the golden arrays have no trajectory axis
         f.prediction(tuple(g["twists"][t]))
         f.measurement(g["xy"][t], g["vis"][t])
     assert state_err(f.state, g["state"]) < TOL and sigma_err(f.sigma, g["sigma"]) < TOL
@@ -625,7 +587,7 @@ def test_scan_to_map_pipeline(gpu_pkg):
     o = OracleEKF(20)
     kf, ko = np.zeros(20, np.uint8), np.zeros(20, np.uint8)
     n_meas = 0
-    for t in range(T):
+    for t in range(T):  # by hand: the readings are the circle fit's, not the trace's
         centers, counts = cf.run_batch(s["ranges"][t])
         k = int(counts[0])
         c_o, _ = co.approx_circle_positions(s["ranges"][t, 0].astype(np.float64))
@@ -636,10 +598,7 @@ def test_scan_to_map_pipeline(gpu_pkg):
         if k:
             r = f.data_association(centers[0, :k], kf)
             a, dmin, sec, cr = o.data_association(c_o, ko)
-            has = dmin < 10.0
-            margin = np.where(has, np.minimum.reduce([np.abs(dmin - 10.0), np.abs(dmin - 1.0), np.abs(sec - dmin)]),
-                              np.abs(sec - 10.0))
-            assert np.all(margin > 1e-6), "threshold tie in the fixture: pick another seed"
+            assert np.all(tie_margin(dmin, sec) > 1e-6), "threshold tie in the fixture: pick another seed"
             assert np.array_equal(r["assoc"], a) and np.array_equal(kf, ko)
             n_meas += k
     assert n_meas > 100 and ko.sum() >= 5
@@ -659,14 +618,12 @@ def test_delayed_application_is_bit_identical(gpu_pkg):
         f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
         f.set_max_pending(k)
         f.set_carry_pending(False)  # groups end with the measurement() call
-        for t in range(8):
-            f.prediction(tuple(tr["twists"][t, 0]))
-            f.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
+        single.run_known(f, tr)
         outs.append((f.state, f.sigma, f.launch_count))
     assert int(tr["vis"][1:].sum(axis=2).max()) > 15  # some steps need more than one group at k = 8 and fill a group of 15+
     for st, sg, _ in outs[1:]:
-        assert np.array_equal(st.view(np.uint64), outs[0][0].view(np.uint64))
-        assert np.array_equal(sg.view(np.uint64), outs[0][1].view(np.uint64))
+        assert np.array_equal(single.bits(st), single.bits(outs[0][0]))
+        assert np.array_equal(single.bits(sg), single.bits(outs[0][1]))
     assert outs[ks.index(20)][2] < outs[ks.index(8)][2] < outs[0][2]  # fewer launches: fewer sweeps
 
 
@@ -683,10 +640,9 @@ def test_pending_factors_carried_across_prediction(gpu_pkg):
     b = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
     b.set_carry_pending(False)
     o = OracleEKF(n)
-    for t in range(T):
+    for t in range(T):  # by hand: a getter is read in the middle of the run
         for f in (a, b, o):
-            f.prediction(tuple(tr["twists"][t, 0])) if f is not o else f.prediction(*tr["twists"][t, 0])
-            f.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
+            single.step_known(f, tr, t)
         if t == T // 2:  # a getter in the middle settles the factors without changing the outcome
             assert sigma_err(a.sigma, o.sigma) < TOL
     assert a.sweep_count < b.sweep_count             # fewer passes over Sigma

@@ -6,6 +6,7 @@ explicitly, and follow tests/_noise_ref.py (the CPU oracle's arithmetic with Q a
 import numpy as np
 import pytest
 
+import _single as single
 from _batch import assert_same_checkpoint, known_trace, run_known, run_unknown, sms, step_known, unknown_trace
 from _noise_ref import DEFAULT_NOISE, NoiseOracle
 from _oracle import sigma_err, state_err
@@ -61,32 +62,22 @@ def test_reference_values_bit_identical(gpu_pkg, name, n, form):
     assert plain.launch_count == explicit.launch_count
 
 
-def _single_trace(pkg, n, T, seed):
-    tk = known_trace(pkg, n, 1, T, seed)
-    tu = unknown_trace(pkg, n, 1, T, seed=seed + 1, m_max=M_MAX)
-    return tk, tu
-
-
-def _drive_single(f, tk, tu, t, known):
-    f.prediction(tuple(tk["twists"][t, 0]))
-    f.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
-    f.prediction(tuple(tu["twists"][t, 0]))
-    m = int(tu["count"][t, 0])
-    return f.data_association(tu["meas"][t, 0, :m], known)["assoc"]
-
-
 @pytest.mark.parametrize("engine", ["fused", "stream"])
 def test_single_reference_values_bit_identical(gpu_pkg, engine):
     n, T = 20, 6
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
-    tk, tu = _single_trace(gpu_pkg, n, T, seed=31)
+    eng = single.engine(gpu_pkg, engine)
+    tk, tu = single.traces(gpu_pkg, n, T, seed=31, m_max=M_MAX)
     a, b = gpu_pkg.EKF_SLAM(n, engine=eng), gpu_pkg.EKF_SLAM(n, engine=eng)
     b.set_noise([1e-4] * 3, [0.01] * 2)
     ka, kb = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
     for t in range(T):
-        assert np.array_equal(_drive_single(a, tk, tu, t, ka), _drive_single(b, tk, tu, t, kb))
-    assert np.array_equal(a.state.view(np.uint64), b.state.view(np.uint64))
-    assert np.array_equal(a.sigma.view(np.uint64), b.sigma.view(np.uint64))
+        assoc = []
+        for f, k in ((a, ka), (b, kb)):
+            single.step_known(f, tk, t)
+            assoc.append(single.step_unknown(f, tu, t, k)["assoc"])
+        assert np.array_equal(*assoc)
+    assert np.array_equal(single.bits(a.state), single.bits(b.state))
+    assert np.array_equal(single.bits(a.sigma), single.bits(b.sigma))
     assert a.calculate_maha_dis((0.3, 0.4), 2) == b.calculate_maha_dis((0.3, 0.4), 2)
     assert a.launch_count == b.launch_count
 
@@ -102,11 +93,7 @@ def test_known_matches_reference(gpu_pkg, n):
     assert np.array_equal(bt.noise(), rows)
     bt.set_nis(True)
     run_known(gpu_pkg, bt, tr)
-    refs = [NoiseOracle(n, rows[b]) for b in range(B)]
-    for t in range(T):
-        for b, o in enumerate(refs):
-            o.prediction(*tr["twists"][t, b])
-            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+    refs = [single.run_known(NoiseOracle(n, rows[b]), tr, b) for b in range(B)]
     _check_filters(bt, refs, f"known n={n}")
     _check_nis(bt, refs, f"known n={n}")
 
@@ -132,12 +119,9 @@ def test_unknown_matches_reference(gpu_pkg, n):
     assoc = run_unknown(bt, tr, M_MAX)
     refs = [NoiseOracle(n, rows[b]) for b in range(B)]
     known = [np.zeros(n, np.uint8) for _ in range(B)]
-    for t in range(T):
-        for b, o in enumerate(refs):
-            o.prediction(*tr["twists"][t, b])
-            m = int(np.clip(tr["count"][t, b], 0, M_MAX))
-            a, _ = o.data_association(tr["meas"][t, b, :m], known[b])
-            assert np.array_equal(a, assoc[t, b, :m]), (t, b)
+    for b, o in enumerate(refs):
+        for t, (a, _) in enumerate(single.run_unknown(o, tr, known[b], b)):
+            assert np.array_equal(a, assoc[t, b, :len(a)]), (t, b)
     assert np.array_equal(bt.known, np.stack(known))
     _check_filters(bt, refs, f"unknown n={n}")
     _check_nis(bt, refs, f"unknown n={n}")
@@ -146,21 +130,18 @@ def test_unknown_matches_reference(gpu_pkg, n):
 @pytest.mark.parametrize("engine", ["fused", "stream"])
 def test_single_matches_reference(gpu_pkg, engine):
     n, T = 20, 6
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
-    tk, tu = _single_trace(gpu_pkg, n, T, seed=41)
+    tk, tu = single.traces(gpu_pkg, n, T, seed=41, m_max=M_MAX)
     row = GRID[1]
-    f = gpu_pkg.EKF_SLAM(n, engine=eng)
+    f = gpu_pkg.EKF_SLAM(n, engine=single.engine(gpu_pkg, engine))
     f.set_noise(row[:3], row[3:])
     assert np.array_equal(f.noise, row)
     o = NoiseOracle(n, row)
     kf, ko = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
     for t in range(T):
-        a = _drive_single(f, tk, tu, t, kf)
-        o.prediction(*tk["twists"][t, 0])
-        o.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
-        o.prediction(*tu["twists"][t, 0])
-        m = int(tu["count"][t, 0])
-        assert np.array_equal(a, o.data_association(tu["meas"][t, 0, :m], ko)[0]), t
+        single.step_known(f, tk, t)
+        a = single.step_unknown(f, tu, t, kf)["assoc"]
+        single.step_known(o, tk, t)
+        assert np.array_equal(a, single.step_unknown(o, tu, t, ko)[0]), t
     assert state_err(f.state, o.state) < TOL and sigma_err(f.sigma, o.sigma) < TOL
     for i in (0, 5, 13):
         d, want = f.calculate_maha_dis((0.3, -0.2), i), o.maha(0.3, -0.2, i)
@@ -179,11 +160,9 @@ def test_wide_bit_identical_to_streamed(gpu_pkg, n):
         f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
         f.set_carry_pending(False)
         f.set_noise(rows[b, :3], rows[b, 3:])
-        for t in range(T):
-            f.prediction(tuple(tr["twists"][t, b]))
-            f.measurement(tr["xy"][t, b], tr["vis"][t, b])
-        assert np.array_equal(f.state.view(np.uint64), bt.states()[b].view(np.uint64)), b
-        assert np.array_equal(f.sigma.view(np.uint64), bt.sigma(b).view(np.uint64)), b
+        single.run_known(f, tr, b)
+        assert np.array_equal(single.bits(f.state), single.bits(bt.states()[b])), b
+        assert np.array_equal(single.bits(f.sigma), single.bits(bt.sigma(b))), b
 
 
 # ---------------------------------------------------------------- 3. several filters per persistent CTA
@@ -206,20 +185,17 @@ def test_noise_classes_over_replicas(gpu_pkg, n, form):
         run_unknown(bt, tr, M_MAX)
     else:
         run_known(gpu_pkg, bt, tr)
-    st = bt.states().view(np.uint64)
+    st = single.bits(bt.states())
     reps = [int(np.flatnonzero(cls == k)[0]) for k in range(K)]
     for k in range(K):
         members = np.flatnonzero(cls == k)
         assert (st[members] == st[reps[k]]).all(), k
     for k in range(K):
         o = NoiseOracle(n, GRID[k])
-        known = np.zeros(n, np.uint8)
-        for t in range(T):
-            o.prediction(*one["twists"][t, 0])
-            if form == "unknown":
-                o.data_association(one["meas"][t, 0, :int(one["count"][t, 0])], known)
-            else:
-                o.measurement(one["xy"][t, 0], one["vis"][t, 0])
+        if form == "unknown":
+            single.run_unknown(o, one, np.zeros(n, np.uint8))
+        else:
+            single.run_known(o, one)
         assert state_err(bt.states()[reps[k]], o.state) < TOL and sigma_err(bt.sigma(reps[k]), o.sigma) < TOL, k
     assert len(set(tuple(st[r]) for r in reps)) == K  # the classes really differ
 
@@ -242,8 +218,7 @@ def test_noise_changed_mid_run(gpu_pkg, n):
                 o.set_noise(DEFAULT_NOISE)
         step_known(gpu_pkg, bt, tr, t, "dense")
         for b, o in enumerate(refs):
-            o.prediction(*tr["twists"][t, b])
-            o.measurement(tr["xy"][t, b], tr["vis"][t, b])
+            single.step_known(o, tr, t, b)
     bt.sync()
     _check_filters(bt, refs, f"mid-run n={n}")
 
@@ -253,10 +228,9 @@ def test_single_noise_changed_with_prediction_pending(gpu_pkg, engine):
     """prediction(), then set_noise(), then measurement(): the prediction uses the old Q (the fused engine still holds
     it back when set_noise() is called), the corrections the new R."""
     n, T = 20, 5
-    eng = gpu_pkg.ENGINE_FUSED if engine == "fused" else gpu_pkg.ENGINE_STREAM
     tk = known_trace(gpu_pkg, n, 1, T, seed=801)
-    f, o = gpu_pkg.EKF_SLAM(n, engine=eng), NoiseOracle(n)
-    for t in range(T):
+    f, o = gpu_pkg.EKF_SLAM(n, engine=single.engine(gpu_pkg, engine)), NoiseOracle(n)
+    for t in range(T):  # by hand: set_noise() falls between prediction() and measurement()
         f.prediction(tuple(tk["twists"][t, 0]))
         o.prediction(*tk["twists"][t, 0])
         row = GRID[1 + t % 4]
@@ -295,7 +269,7 @@ def test_broadcast_clone_and_checkpoints(gpu_pkg):
         for h in (f, g):
             h.prediction(tuple(tr["twists"][1, 0]))
             h.measurement(tr["xy"][0, 0], tr["vis"][0, 0])
-        assert np.array_equal(f.sigma.view(np.uint64), g.sigma.view(np.uint64))
+        assert np.array_equal(single.bits(f.sigma), single.bits(g.sigma))
         f.set_noise()
         assert np.array_equal(f.noise, DEFAULT_NOISE)
 

@@ -8,6 +8,7 @@ import sys
 import numpy as np
 import pytest
 
+import _single as single
 from _oracle import OracleEKF, sigma_err, state_err
 
 pytestmark = pytest.mark.gpu
@@ -37,16 +38,9 @@ def test_local_emulation_known_association(gpu_pkg, n, world):
     assert all(bounds[g][1] == bounds[g + 1][0] for g in range(world - 1))
     assert all(b[0] % 2 == 1 for b in bounds[1:])
     assert [b[0] for b in bounds] + [f.N] == gpu_pkg.sharding.landmark_row_blocks(n, world)
-    worst = 0.0
-    for t in range(10):
-        f.prediction(tuple(tr["twists"][t, 0]))
-        o.prediction(*tr["twists"][t, 0])
-        f.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
-        o.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
-        if t % 3 == 0 or t == 9:
-            worst = max(worst, state_err(f.state, o.state), sigma_err(f.sigma_full_local(), o.sigma))
+    ex, es = single.parity_known(f, o, tr, check_every=3)
     assert f.update_count == int(tr["vis"].sum()) > 10
-    assert worst < TOL, worst
+    assert ex < TOL and es < TOL, (ex, es)
 
 
 @pytest.mark.parametrize("n,world", [(20, 2), (20, 4), (150, 3)])
@@ -58,7 +52,7 @@ def test_local_emulation_unknown_association(gpu_pkg, n, world):
     f = ShardedEKF.local_emulation(n, world)
     o = OracleEKF(n)
     kf, ko = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
-    for t in range(25):
+    for t in range(25):  # by hand: no data_association() call for a step without readings
         f.prediction(tuple(tr["twists"][t, 0]))
         o.prediction(*tr["twists"][t, 0])
         m = int(tr["count"][t, 0])
@@ -79,6 +73,7 @@ sys.path.insert(0, sys.argv[1]); sys.path.insert(0, os.path.join(sys.argv[1], "t
 import torch, torch.distributed as dist
 import ekf_slam_ml_b200 as pkg
 from ekf_slam_ml_b200.sharded import ShardedEKF
+import _single as single
 from _oracle import OracleEKF, sigma_err, state_err
 local = int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
@@ -91,12 +86,10 @@ w = tg.grid_world(nx, 15, pitch=0.45, n_slots=n, max_visible=1.0)
 tr = tg.simulate_known(w, 1, 8, seed=5)
 tu = tg.simulate_unknown(w, 1, 3, seed=6, m_max=8)
 f = ShardedEKF.from_process_group(n, dist, local)
-o = OracleEKF(n)
-for t in range(8):
-    f.prediction(tuple(tr["twists"][t, 0])); o.prediction(*tr["twists"][t, 0])
-    f.measurement(tr["xy"][t, 0], tr["vis"][t, 0]); o.measurement(tr["xy"][t, 0], tr["vis"][t, 0])
+single.run_known(f, tr)
+o = single.run_known(OracleEKF(n), tr)
 kf, ko = np.ones(n, np.uint8), np.ones(n, np.uint8)
-for t in range(3):
+for t in range(3):  # by hand: association only, no prediction in between
     m = int(tu["count"][t, 0])
     r = f.data_association(tu["meas"][t, 0, :m], kf)
     a, dmin, sec, cr = o.data_association(tu["meas"][t, 0, :m], ko)

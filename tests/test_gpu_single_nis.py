@@ -8,7 +8,8 @@ the accumulators of the same filter in a wide batch, bit for bit."""
 import numpy as np
 import pytest
 
-from _batch import grid_world, known_trace, robot_frame, run_known, unknown_trace
+import _single as single
+from _batch import known_trace, robot_frame, run_known
 from _noise_ref import DEFAULT_NOISE, NoiseOracle
 
 pytestmark = pytest.mark.gpu
@@ -22,50 +23,10 @@ FILTERS = [("fused", 20), ("fused", 33), ("stream", 20), ("stream", 100)]
 
 
 def _make(pkg, engine, n, noise=None):
-    f = pkg.EKF_SLAM(n, engine=pkg.ENGINE_FUSED if engine == "fused" else pkg.ENGINE_STREAM)
+    f = pkg.EKF_SLAM(n, engine=single.engine(pkg, engine))
     if noise is not None:
         f.set_noise(noise[:3], noise[3:])
     return f
-
-
-def _traces(pkg, n, T, seed):
-    if n <= 33:
-        tu = unknown_trace(pkg, n, 1, T, seed=seed + 1, m_max=M_MAX)
-    else:  # the dense world holds about 33 tubes; larger maps take the grid of the known traces
-        tu = pkg.tracegen.simulate_unknown(grid_world(pkg, n), 1, T, seed=seed + 1, m_max=M_MAX)
-    return known_trace(pkg, n, 1, T, seed), tu
-
-
-def _known_step(f, tk, t):
-    f.prediction(tuple(tk["twists"][t, 0]))
-    f.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
-
-
-def _unknown_step(f, tu, t, known):
-    f.prediction(tuple(tu["twists"][t, 0]))
-    m = int(tu["count"][t, 0])
-    return f.data_association(tu["meas"][t, 0, :m], known)
-
-
-def _oracle_known(o, tk, t):
-    """The oracle's step t and its expected last_nis(): n values, -1 where nothing was scored."""
-    o.prediction(*tk["twists"][t, 0])
-    k0, score = len(o.values), o.init_flag
-    o.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
-    want = np.full(o.n, -1.0)
-    if score:
-        want[np.flatnonzero(tk["vis"][t, 0])] = o.values[k0:]
-    return want
-
-
-def _oracle_unknown(o, tu, t, known):
-    o.prediction(*tu["twists"][t, 0])
-    m = int(tu["count"][t, 0])
-    k0 = len(o.values)
-    a, cr = o.data_association(tu["meas"][t, 0, :m], known)
-    want = np.full(m, -1.0)
-    want[(a >= 0) & (cr == 0)] = o.values[k0:]
-    return a, cr, want
 
 
 def _nis_dev(got, want, what):
@@ -78,31 +39,27 @@ def _nis_dev(got, want, what):
     return float((np.abs(got[m] - want[m]) / np.maximum(np.abs(want[m]), 1e-300)).max())
 
 
-def _bits(a):
-    return np.ascontiguousarray(a, dtype=np.float64).view(np.uint64)
-
-
 # ---------------------------------------------------------------- 1. the NIS variants do not change the filter
 @pytest.mark.parametrize("noise", ["reference", "grid"])
 @pytest.mark.parametrize("engine,n", FILTERS, ids=[f"{e}-{n}" for e, n in FILTERS])
 def test_nis_leaves_filter_unchanged(gpu_pkg, engine, n, noise):
     T = 6
     row = NOISE_ROW if noise == "grid" else None
-    tk, tu = _traces(gpu_pkg, n, T, seed=10 + n)
+    tk, tu = single.traces(gpu_pkg, n, T, seed=10 + n, m_max=M_MAX)
     plain, scored = _make(gpu_pkg, engine, n, row), _make(gpu_pkg, engine, n, row)
     scored.set_nis(True)
     kp, ks = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
     for t in range(T):
         for f in (plain, scored):
-            _known_step(f, tk, t)
-        a, b = _unknown_step(plain, tu, t, kp), _unknown_step(scored, tu, t, ks)
+            single.step_known(f, tk, t)
+        a, b = single.step_unknown(plain, tu, t, kp), single.step_unknown(scored, tu, t, ks)
         for key in ("assoc", "created"):
             assert np.array_equal(a[key], b[key]), (t, key)
         for key in ("dmin", "second"):
-            assert np.array_equal(_bits(a[key]), _bits(b[key])), (t, key)
+            assert np.array_equal(single.bits(a[key]), single.bits(b[key])), (t, key)
         assert np.array_equal(kp, ks), t
-    assert np.array_equal(_bits(plain.state), _bits(scored.state))
-    assert np.array_equal(_bits(plain.sigma), _bits(scored.sigma))
+    assert np.array_equal(single.bits(plain.state), single.bits(scored.state))
+    assert np.array_equal(single.bits(plain.sigma), single.bits(scored.sigma))
     assert plain.update_count == scored.update_count
     assert plain.launch_count == scored.launch_count
     r = scored.nis()
@@ -116,18 +73,18 @@ def test_nis_leaves_filter_unchanged(gpu_pkg, engine, n, noise):
 def test_nis_matches_reference(gpu_pkg, engine, n, mode, noise):
     T = 8
     row = NOISE_ROW if noise == "grid" else np.array(DEFAULT_NOISE)
-    tk, tu = _traces(gpu_pkg, n, T, seed=100 + n)
+    tk, tu = single.traces(gpu_pkg, n, T, seed=100 + n, m_max=M_MAX)
     f, o = _make(gpu_pkg, engine, n, row), NoiseOracle(n, row)
     f.set_nis(True)
     worst = 0.0
     kf, ko = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
     for t in range(T):
         if mode == "known":
-            _known_step(f, tk, t)
-            want = _oracle_known(o, tk, t)
+            single.step_known(f, tk, t)
+            want = single.nis_step_known(o, tk, t)
         else:
-            got = _unknown_step(f, tu, t, kf)
-            a, _, want = _oracle_unknown(o, tu, t, ko)
+            got = single.step_unknown(f, tu, t, kf)
+            a, _, want = single.nis_step_unknown(o, tu, t, ko)
             assert np.array_equal(got["assoc"], a), t
         worst = max(worst, _nis_dev(f.last_nis(), want, f"{engine} n={n} {mode} call {t}"))
     r = f.nis()
@@ -150,9 +107,7 @@ def test_streamed_equals_wide(gpu_pkg, carry):
     f = gpu_pkg.EKF_SLAM(n, engine=gpu_pkg.ENGINE_STREAM)
     f.set_carry_pending(carry)
     f.set_nis(True)
-    for t in range(T):
-        f.prediction(tuple(tr["twists"][t, b]))
-        f.measurement(tr["xy"][t, b], tr["vis"][t, b])
+    single.run_known(f, tr, b)
     want = bt.nis(per_filter=True)
     want = np.array([want["nis_sum"][b], want["nis_sq_sum"][b], want["nis_count"][b], want["nis_nonfinite"][b]])
     got = f.nis()["stats"]
@@ -161,7 +116,7 @@ def test_streamed_equals_wide(gpu_pkg, carry):
         assert got[2] == want[2] and got[3] == want[3]
         np.testing.assert_allclose(got[:2], want[:2], rtol=1e-8)
     else:
-        assert np.array_equal(_bits(got), _bits(want)), (got, want)
+        assert np.array_equal(single.bits(got), single.bits(want)), (got, want)
 
 
 # ---------------------------------------------------------------- 4. the scoring rule on hand-built inputs
@@ -223,7 +178,7 @@ def test_scoring_rule(gpu_pkg, engine, n):
 @pytest.mark.parametrize("engine,n", FILTERS, ids=[f"{e}-{n}" for e, n in FILTERS])
 def test_readout(gpu_pkg, engine, n):
     T = 6
-    tk, tu = _traces(gpu_pkg, n, T, seed=900 + n)
+    tk, tu = single.traces(gpu_pkg, n, T, seed=900 + n, m_max=M_MAX)
     f = _make(gpu_pkg, engine, n)
     out, cnt = np.zeros(4), np.zeros(1, np.int32)
     assert f._L.ekf_nis(f._h, out.ctypes.data, 0) == -3  # EKF_ERR_STATE: NIS never enabled
@@ -234,28 +189,29 @@ def test_readout(gpu_pkg, engine, n):
     f.set_nis(True)
     known = np.zeros(n, np.uint8)
     for t in range(3):
-        _known_step(f, tk, t)
-        _unknown_step(f, tu, t, known)
+        single.step_known(f, tk, t)
+        single.step_unknown(f, tu, t, known)
     s1 = f.nis()["stats"]
-    assert s1[2] > 0 and np.array_equal(_bits(f.nis()["stats"]), _bits(s1))  # a read changes nothing
+    assert s1[2] > 0 and np.array_equal(single.bits(f.nis()["stats"]), single.bits(s1))  # a read changes nothing
     # steps with NIS off leave the accumulators and the last call's values alone
     last = f.last_nis()
     f.set_nis(False)
-    _known_step(f, tk, 3)
-    _unknown_step(f, tu, 3, known)
-    assert np.array_equal(_bits(f.nis()["stats"]), _bits(s1))
-    assert np.array_equal(_bits(f.last_nis()), _bits(last))
+    single.step_known(f, tk, 3)
+    single.step_unknown(f, tu, 3, known)
+    assert np.array_equal(single.bits(f.nis()["stats"]), single.bits(s1))
+    assert np.array_equal(single.bits(f.last_nis()), single.bits(last))
     # a clone continues bit-identically, accumulators included
     f.set_nis(True)
     g, kg = f.clone(), known.copy()
-    assert np.array_equal(_bits(g.nis()["stats"]), _bits(s1))
+    assert np.array_equal(single.bits(g.nis()["stats"]), single.bits(s1))
     for t in range(4, T):
         for h, k in ((f, known), (g, kg)):
-            _known_step(h, tk, t)
-            _unknown_step(h, tu, t, k)
-    assert np.array_equal(_bits(f.nis()["stats"]), _bits(g.nis()["stats"]))
-    assert np.array_equal(_bits(f.last_nis()), _bits(g.last_nis()))
-    assert np.array_equal(_bits(f.state), _bits(g.state)) and np.array_equal(_bits(f.sigma), _bits(g.sigma))
+            single.step_known(h, tk, t)
+            single.step_unknown(h, tu, t, k)
+    assert np.array_equal(single.bits(f.nis()["stats"]), single.bits(g.nis()["stats"]))
+    assert np.array_equal(single.bits(f.last_nis()), single.bits(g.last_nis()))
+    assert np.array_equal(single.bits(f.state), single.bits(g.state))
+    assert np.array_equal(single.bits(f.sigma), single.bits(g.sigma))
     # reset zeroes after the read
     s2 = f.nis(reset=True)["stats"]
     assert s2[2] > s1[2]
@@ -263,7 +219,7 @@ def test_readout(gpu_pkg, engine, n):
     # clone of a filter that has NIS switched off carries the switch: its steps leave the accumulators alone
     f.set_nis(False)
     h = f.clone()
-    _known_step(h, tk, 0)
+    single.step_known(h, tk, 0)
     assert np.all(h.nis()["stats"] == 0)
 
 
@@ -272,9 +228,9 @@ def test_toggle_with_prediction_deferred(gpu_pkg, n):
     """The fused engine defers prediction() into the next kernel; switching NIS on or off in between changes nothing
     else: same state, covariance, launches and accumulators as switching before the prediction."""
     T = 5
-    tk, _ = _traces(gpu_pkg, n, T, seed=950 + n)
+    tk, _ = single.traces(gpu_pkg, n, T, seed=950 + n, m_max=M_MAX)
     a, b = _make(gpu_pkg, "fused", n), _make(gpu_pkg, "fused", n)
-    for t in range(T):
+    for t in range(T):  # by hand: set_nis() falls between prediction() and measurement()
         on = t % 2 == 0
         a.set_nis(on)
         a.prediction(tuple(tk["twists"][t, 0]))
@@ -282,8 +238,9 @@ def test_toggle_with_prediction_deferred(gpu_pkg, n):
         b.set_nis(on)  # the prediction is still deferred here
         for f in (a, b):
             f.measurement(tk["xy"][t, 0], tk["vis"][t, 0])
-    assert np.array_equal(_bits(a.state), _bits(b.state)) and np.array_equal(_bits(a.sigma), _bits(b.sigma))
+    assert np.array_equal(single.bits(a.state), single.bits(b.state))
+    assert np.array_equal(single.bits(a.sigma), single.bits(b.sigma))
     assert a.launch_count == b.launch_count
-    assert np.array_equal(_bits(a.nis()["stats"]), _bits(b.nis()["stats"]))
-    assert np.array_equal(_bits(a.last_nis()), _bits(b.last_nis()))
+    assert np.array_equal(single.bits(a.nis()["stats"]), single.bits(b.nis()["stats"]))
+    assert np.array_equal(single.bits(a.last_nis()), single.bits(b.last_nis()))
     assert a.nis()["count"] > 0
