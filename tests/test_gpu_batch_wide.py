@@ -24,7 +24,7 @@ def _trace(pkg, n, B, T, seed):
     return tr
 
 
-@pytest.mark.parametrize("n", [65, 100, 256])
+@pytest.mark.parametrize("n", [65, 100, 256, 512, 1024])
 def test_wide_batch_is_bit_identical_to_streamed_filters(gpu_pkg, n):
     B, T = 48, 20
     tr = _trace(gpu_pkg, n, B, T, seed=100 + n)
@@ -135,15 +135,20 @@ def test_wide_batch_engine_boundaries(gpu_pkg):
         bt.step_unknown(np.ones((B, 2)), np.ones((B, 4, 2)), np.full(B, 4, np.int32), 4)
     assert e.value.code == -2
     assert np.array_equal(bt.states(), before)
-    # a 1,024-landmark step runs (every slot visible on the first call: 74 groups of factors)
-    tw = np.full((2, 2), 0.01)
+    # a 1,024-landmark step (every slot visible on the first call: 74 groups of factors) gives the bits of two streamed
+    # filters
+    tw = np.full((1, 2, 2), 0.01)
     rng = np.random.default_rng(4)
     r, phi = rng.uniform(0.5, 2.0, (2, 1024)), rng.uniform(-np.pi, np.pi, (2, 1024))
-    xy = np.ascontiguousarray(np.stack([r * np.cos(phi), r * np.sin(phi)], axis=2).reshape(2, 2048))
-    big.step_known(tw, xy, np.ones((2, 1024), np.uint8))
-    big.sync()
+    xy = np.stack([r * np.cos(phi), r * np.sin(phi)], axis=2).reshape(1, 2, 2048)
+    one = {"twists": tw, "xy": xy, "vis": np.ones((1, 2, 1024), np.uint8)}
+    run_known(gpu_pkg, big, one)
     assert big.update_count == 2 * 1024 and big.sweep_count == 2 * int(np.ceil(1024 / P))
-    assert np.all(np.isfinite(big.states()))
+    states = big.states()
+    for b in range(2):
+        f = single.streamed(gpu_pkg, 1024, one, b, range(1))
+        assert np.array_equal(single.bits(states[b]), single.bits(f.state)), b
+        assert np.array_equal(single.bits(big.sigma(b)), single.bits(f.sigma)), b
 
 
 def test_wide_batch_getters(gpu_pkg):

@@ -43,7 +43,7 @@ def test_local_emulation_known_association(gpu_pkg, n, world):
     assert ex < TOL and es < TOL, (ex, es)
 
 
-@pytest.mark.parametrize("n,world", [(20, 2), (20, 4), (150, 3)])
+@pytest.mark.parametrize("n,world", [(20, 2), (20, 4), (20, 8), (150, 3)])  # (20, 8): rank 7 owns no row
 def test_local_emulation_unknown_association(gpu_pkg, n, world):
     from ekf_slam_ml_b200.sharded import ShardedEKF
     tg = gpu_pkg.tracegen
